@@ -1111,6 +1111,29 @@ uint64_t mm_b200_batch_digest(const mm_b200_batch_t *b, int64_t *n_hits)
 	return h;
 }
 
+/* the hits of a mapped batch as rows of MM_B200_HIT_COLS integers, in read order, and their CIGARs concatenated in the same order */
+int64_t mm_b200_batch_hits(const mm_b200_batch_t *b, int64_t *rows, uint32_t *cigar, int64_t *n_cigar)
+{
+	const step_t *s = (const step_t*)b;
+	int64_t n = 0, nc = 0;
+	int i, j;
+	for (i = 0; i < s->n_seq; ++i)
+		for (j = 0; j < s->n_reg[i]; ++j, ++n) {
+			const mm_reg1_t *r = &s->reg[i][j];
+			const uint32_t k = r->p ? r->p->n_cigar : 0;
+			if (rows) {
+				int64_t *o = rows + n * MM_B200_HIT_COLS;
+				o[0] = i, o[1] = r->rid, o[2] = r->rs, o[3] = r->re, o[4] = r->qs, o[5] = r->qe, o[6] = r->rev, o[7] = r->mapq;
+				o[8] = r->score, o[9] = r->parent == r->id, o[10] = r->sam_pri, o[11] = r->proper_frag, o[12] = r->mlen, o[13] = r->blen;
+				o[14] = r->p ? r->p->dp_score : 0, o[15] = r->p ? r->p->dp_max : 0, o[16] = k;
+			}
+			if (cigar && k) memcpy(cigar + nc, r->p->cigar, k * sizeof(uint32_t));
+			nc += k;
+		}
+	if (n_cigar) *n_cigar = nc;
+	return n;
+}
+
 void mm_b200_write_batch(const mm_idx_t *mi, const mm_mapopt_t *opt, mm_b200_batch_t *b)
 {
 	pipeline_t pl;

@@ -16,6 +16,8 @@ reference.  One step = one mini-batch of pairs through the whole hot path (sketc
              records are compared byte for byte with the reference fork's (oracle/_ref/minimap2_B); at N>1 every rank
              maps the same prefix with its replica of the index and the digests must agree
   roofline : the dominant kernel by CUDA-event time inside the timed region
+  --dump-outputs DIR : the hits of the last mini-batch of the resident timed pass, one float64 array per field (dump_outputs), so
+             that two builds can be compared hit for hit on the same seeded inputs
   --impl reference / cpu_baseline : the reference fork's own mapping step (worker_pipeline step 1 = kt_for(worker_for) ->
              mm_map_frag, unmodified objects in oracle/_ref/libmm2ref.so driven by oracle/ref_mapstep.c) on all host
              cores, same files, same mini-batch size; parsing and SAM formatting run but are not in the step time
@@ -46,6 +48,13 @@ K4_INT_ROOFLINE_GCUPS = 148 * 128 * 1.965 / 30.0
 
 METRIC = "remapped reads/sec at 1/2/4/8 B200; ksw2 GCUPS; seed-lookup HBM GB/s"
 PARITY_PAIRS = 100_000
+# --dump-outputs: the columns of mm_b200_batch_hits (include/minimap_b200.h), and the size cap of all files together (npy headers aside)
+HIT_FIELDS = ("read", "rid", "rs", "re", "qs", "qe", "rev", "mapq", "score", "primary", "sam_pri", "proper_frag", "mlen", "blen",
+              "dp_score", "dp_max", "n_cigar")
+DUMP_BYTES = (64 << 20) - (1 << 16)
+# (workload, genome bp, contigs, parity units) -> (records, sha256) of oracle/_ref/minimap2_B's SAM records of the parity prefix,
+# from runs where the reference fork was built (profiles/bench_r02_n1.json, "reference_sha256"): without it the gate compares with these
+REF_PARITY = {("sr", 3_100_000_000, 24, PARITY_PAIRS): (200_000, "18d83c22c05360e9b758914f3a2637e4e1b1ede46a93dbd87c2d5ca13616f2a2")}
 
 
 class IdxOpt(C.Structure):
@@ -101,6 +110,8 @@ def load_lib():
     L.mm_b200_write_batch.argtypes = [C.c_void_p, C.POINTER(MapOptFull), C.c_void_p]
     L.mm_b200_batch_digest.restype = C.c_uint64
     L.mm_b200_batch_digest.argtypes = [C.c_void_p, C.POINTER(C.c_int64)]
+    L.mm_b200_batch_hits.restype = C.c_int64
+    L.mm_b200_batch_hits.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int64)]
     L.mm_b200_stats.argtypes = [C.POINTER(Stats), C.c_int]
     L.mm_b200_profile.argtypes = [C.c_void_p, C.c_int]
     L.mm_b200_set_serial.argtypes = [C.c_int]
@@ -337,6 +348,36 @@ def first_difference(p1, p2):
     return None
 
 
+def batch_hits(L, b):
+    """the hits of a mapped batch as its caller receives them: (rows of HIT_FIELDS in read order, their CIGAR words concatenated)"""
+    import numpy as np
+    n_cig = C.c_int64(0)
+    n = L.mm_b200_batch_hits(b, None, None, C.byref(n_cig))
+    rows = np.zeros((n, len(HIT_FIELDS)), dtype=np.int64)
+    cig = np.zeros(n_cig.value, dtype=np.uint32)
+    L.mm_b200_batch_hits(b, rows.ctypes.data, cig.ctypes.data, C.byref(n_cig))
+    return rows, cig
+
+
+def dump_outputs(out_dir, rows, cig, n_reads):
+    """Writes out_dir/<field>.npy (one float64 per hit, fields of HIT_FIELDS) and out_dir/cigar.npy (the CIGAR words of those hits in
+    hit order; n_cigar.npy splits them).  Over DUMP_BYTES, whole reads are kept in a fixed seeded order until the budget is spent,
+    so that equal hits give equal files.  Returns (hits written, reads kept)."""
+    import numpy as np
+    n_cigar = rows[:, HIT_FIELDS.index("n_cigar")]
+    hit_bytes = 8 * (len(HIT_FIELDS) + n_cigar)
+    read_bytes = np.bincount(rows[:, 0], weights=hit_bytes, minlength=n_reads)
+    order = np.random.default_rng(0).permutation(n_reads)
+    keep_read = np.zeros(n_reads, dtype=bool)
+    keep_read[order[np.cumsum(read_bytes[order]) <= DUMP_BYTES]] = True
+    keep = keep_read[rows[:, 0]]
+    os.makedirs(out_dir, exist_ok=True)
+    for j, name in enumerate(HIT_FIELDS):
+        np.save(os.path.join(out_dir, f"{name}.npy"), rows[keep, j].astype(np.float64))
+    np.save(os.path.join(out_dir, "cigar.npy"), cig[np.repeat(keep, n_cigar)].astype(np.float64))
+    return int(keep.sum()), int(keep_read.sum())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -354,7 +395,12 @@ def main():
     ap.add_argument("--no-cli", action="store_true", help="skip the whole-CLI (parse + map + SAM) timing at N=1")
     ap.add_argument("--lanes", type=int, default=4, help="streams per GPU: two mini-batches in flight, each cut into lanes/2 shards")
     ap.add_argument("--in-flight", type=int, default=2, help="mini-batches in flight (each on lanes/in_flight streams)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the hits of the last timed mini-batch to DIR/<field>.npy (float64); --impl b200 only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 path computes; --impl reference has no such outputs")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -512,6 +558,13 @@ def main():
                     parity["first_difference"] = first_difference(ours, theirs)
                     sys.stderr.write(f"[bench] PARITY MISMATCH: {parity}\n")
                 os.unlink(theirs)
+            elif (wl.kind, wl.G, wl.n_ctg, par_units) in REF_PARITY:
+                n_ref, h_ref = REF_PARITY[(wl.kind, wl.G, wl.n_ctg, par_units)]
+                ok = (n_ref == n_ours and h_ref == h_ours and ranks_equal is not False)
+                parity.update({"checked": True, "ok": ok, "reference_records": n_ref, "reference_sha256": h_ref,
+                               "why": "every SAM record of the prefix identical to minimap2_B's, by its stored digest (REF_PARITY)" if ok else "MISMATCH"})
+                if not ok:
+                    sys.stderr.write(f"[bench] PARITY MISMATCH: {parity}\n")
             os.unlink(ours)
         else:
             L.mm_b200_free_batch(pb)
@@ -552,9 +605,10 @@ def main():
     for b in wb:
         L.mm_b200_free_batch(b)
 
-    def timed(mode_resident, in_flight=1, profile=False):
+    def timed(mode_resident, in_flight=1, profile=False, capture=False):
         """K steps; returns (seconds max over ranks, reads of all ranks, stats, kernel profile, launches, clocks, digest).
-        in_flight: mini-batches resident at a time in the resident pass (1 when the shards take turns on the device)."""
+        in_flight: mini-batches resident at a time in the resident pass (1 when the shards take turns on the device).
+        capture: keep the hits of the last step in timed.last_hits (rows, cigar, reads of that step)."""
         L.mm_b200_stats(None, 1)
         L.mmg_growth_counts((C.c_uint64 * 2)(), 1)
         L.mm_b200_path_counts(mi, (C.c_uint64 * 8)(), 1)
@@ -608,6 +662,10 @@ def main():
         L.mm_b200_path_counts(mi, pc, 0)
         timed.paths = {"rechained": pc[0], "heap_rank_replay": pc[1], "heap_literal_replay": pc[2], "warp_tree": pc[3], "zdrop_rounds": pc[4],
                        "zdrop_cuts": pc[5], "replayed_hits": pc[6]}
+        if capture:   # before the reset below drops the hits
+            ns = C.c_int(0)
+            L.mm_b200_batch_info(batches[-1], C.byref(ns), None, None)
+            timed.last_hits = batch_hits(L, batches[-1]) + (ns.value,)
         digest = 0
         for b in batches:  # the three passes must produce the same hits
             digest ^= L.mm_b200_batch_digest(b, None)
@@ -644,7 +702,7 @@ def main():
             sys.stderr.write(f"[bench] {nm}: total {st.t_total:.3f} upload {st.t_upload:.3f} seed/chain {st.t_seedchain:.3f} (kernels {st.t_seedchain_kernels:.3f}) dp {st.t_ksw_total:.3f} (kernel {st.t_ksw_kernel:.3f}) finish {st.t_finish:.3f}\n")
         sys.stderr.write(f"[bench] e2e pass 1 {secs_e2e * 1e3 / args.steps:.1f} ms/step (buffer re-allocations {growths_e2e}), pass 2 {s2 * 1e3 / args.steps:.1f} ms/step ({timed.growths})\n")
     in_flight = L.mm_b200_batches_in_flight(mi, C.byref(opt))   # 1 for the presets whose post-chaining stages run on the host
-    secs_res, reads_res, st_res, prof_val, launches_res, clocks_res, dig_res = timed(True, in_flight=in_flight)
+    secs_res, reads_res, st_res, prof_val, launches_res, clocks_res, dig_res = timed(True, in_flight=in_flight, capture=bool(args.dump_outputs))
     per_rank_ms = timed.per_rank_ms
     # Kernel profile: a third pass in which the shards of a GPU take turns on the device.  In the timed passes the two shards'
     # kernels overlap on purpose, which stretches every per-kernel CUDA-event interval; the roofline figures need clean ones.
@@ -769,6 +827,10 @@ def main():
                                         "tests/test_gpu_e2e.py, tests/test_gpu_paths.py and the golden CLI cases"}
         except Exception as e:  # noqa
             out["long_read"] = {"value": None, "why": f"failed: {e}"}
+    if rank == 0 and args.dump_outputs:
+        rows, cig, n_last = timed.last_hits
+        n_kept, reads_kept = dump_outputs(args.dump_outputs, rows, cig, n_last)
+        out["dump_outputs"] = {"dir": args.dump_outputs, "reads": n_last, "hits": len(rows), "reads_written": reads_kept, "hits_written": n_kept}
     if rank == 0:
         print(json.dumps(out))
 

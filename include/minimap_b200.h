@@ -211,6 +211,12 @@ void mm_b200_batch_info(const mm_b200_batch_t *b, int *n_seq, int *n_frag, int64
 int  mm_b200_map_batch(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_threads, mm_b200_batch_t *b, int mode);
 void mm_b200_reset_batch(mm_b200_batch_t *b);
 uint64_t mm_b200_batch_digest(const mm_b200_batch_t *b, int64_t *n_hits);
+/* columns of a row of mm_b200_batch_hits: read (index in the batch), rid, rs, re, qs, qe, rev, mapq, score, primary (parent == id),
+ * sam_pri, proper_frag, mlen, blen, dp_score, dp_max, n_cigar */
+#define MM_B200_HIT_COLS 17
+/* the hits of a mapped batch: one row per hit into rows (n_hits x MM_B200_HIT_COLS) and the CIGARs of all hits, concatenated,
+ * into cigar; either may be 0 to only count.  Returns the number of hits; *n_cigar receives the number of CIGAR words. */
+int64_t mm_b200_batch_hits(const mm_b200_batch_t *b, int64_t *rows, uint32_t *cigar, int64_t *n_cigar);
 void mm_b200_write_batch(const mm_idx_t *mi, const mm_mapopt_t *opt, mm_b200_batch_t *b); /* prints and frees */
 void mm_b200_free_batch(mm_b200_batch_t *b);
 /* n mini-batches through mm_b200_map_batch with two of them in flight (needs an even number of lanes >= 2): batch i uses lane

@@ -2,8 +2,11 @@
 when present), the plain-C oracle port (oracle/_ref/libmm2oracle.so) and helpers.
 Test infrastructure only."""
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
+import tempfile
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -74,6 +77,49 @@ def oracle():
 
 def have_ref():
     return os.path.exists(REF_SO)
+
+
+def have_ref_bin():
+    return os.path.exists(REF_BIN_B)
+
+
+DIGESTS = os.path.join(ROOT, "tests", "golden", "digests.json")
+
+
+def _bytes(out):
+    if isinstance(out, (list, tuple)):
+        return b"\n".join(l if isinstance(l, bytes) else l.encode() for l in out)
+    return out
+
+
+def check_digest(key, out):
+    """Where the reference fork (oracle/_ref) is not built, an output that the tests compare with the reference's is compared
+    with the size and sha256 kept for key in tests/golden/digests.json; each entry's "source" says whose output it is.
+    out: bytes, or a list of lines (str or bytes).  On a mismatch the output is saved to a temporary file for a line-by-line
+    diff against a run of the reference elsewhere."""
+    with open(DIGESTS) as f:
+        want = json.load(f).get(key)
+    assert want is not None, f"no recorded digest for {key!r} in {DIGESTS}"
+    b = _bytes(out)
+    got = {"bytes": len(b), "sha256": hashlib.sha256(b).hexdigest()}
+    if got != {k: want[k] for k in got}:
+        fd, path = tempfile.mkstemp(prefix="airlift_digest_", suffix=".out")
+        with os.fdopen(fd, "wb") as f:
+            f.write(b)
+        raise AssertionError(f"{key}: output {got} differs from the recorded one {want}; output saved to {path}")
+
+
+def record_reference_digest(key, want):
+    """With AIRLIFT_RECORD_REFERENCE_DIGESTS=1, stores the digest of want -- the REFERENCE's output, already compared with this
+    project's by the caller -- as the entry of key in tests/golden/digests.json.  Only the reference branches of the tests call it."""
+    if os.environ.get("AIRLIFT_RECORD_REFERENCE_DIGESTS") != "1":
+        return
+    b = _bytes(want)
+    with open(DIGESTS) as f:
+        d = json.load(f)
+    d[key] = {"bytes": len(b), "sha256": hashlib.sha256(b).hexdigest(), "source": "reference fork (oracle/_ref)"}
+    with open(DIGESTS, "w") as f:
+        json.dump(d, f, indent=1, sort_keys=True)
 
 
 class mm128_v(C.Structure):

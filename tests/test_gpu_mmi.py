@@ -1,5 +1,6 @@
 """Index files: `-d` must write the bytes the reference writes (mm_idx_dump, index.c:438-477), and a .mmi written
-by the reference must map like the FASTA it came from (mm_idx_load, index.c:479-531)."""
+by the reference must map like the FASTA it came from (mm_idx_load, index.c:479-531).  Where the reference fork is not built,
+the reference's outputs are stood in for by this project's, held to their digests recorded in tests/golden/digests.json."""
 import os
 import subprocess
 import pytest
@@ -12,8 +13,8 @@ SYN = os.path.join(L.ROOT, "build", "mmsynth")
 
 @pytest.fixture(scope="module")
 def data(tmp_path_factory):
-    if not (os.path.exists(L.REF_BIN_B) and os.path.exists(NEW) and os.path.exists(SYN)):
-        pytest.skip("needs oracle/_ref/minimap2_B, build/minimap2-b200 and build/mmsynth")
+    if not (os.path.exists(NEW) and os.path.exists(SYN)):
+        pytest.skip("needs build/minimap2-b200 and build/mmsynth")
     d = tmp_path_factory.mktemp("mmi")
     subprocess.check_call([SYN, "ref", str(d / "ref.fa"), "3000000", "3", "42"])
     subprocess.check_call([SYN, "sr", str(d / "ref.fa"), str(d / "r1.fq"), str(d / "r2.fq"), "4000", "44", "0.05"])
@@ -27,10 +28,20 @@ def _ok(cmd, cwd):
     return p
 
 
+def _ref_dump(args, out, cwd):
+    """the reference's `-d out` (args: index options): without the reference fork, this project's, held to the recorded digest"""
+    if L.have_ref_bin():
+        _ok([L.REF_BIN_B] + args + ["-d", out, "ref.fa"], cwd)
+        L.record_reference_digest("mmi " + " ".join(args), open(cwd / out, "rb").read())
+    else:
+        _ok([NEW] + args + ["-d", out, "ref.fa"], cwd)
+        L.check_digest("mmi " + " ".join(args), open(cwd / out, "rb").read())
+
+
 @pytest.mark.parametrize("args", [["-x", "sr"], ["-x", "map-ont"], ["-H", "-k", "19", "-w", "10"], ["-x", "sr", "-I", "1M"],
                                   ["-k", "12", "-w", "3"]], ids=" ".join)
 def test_dump_is_byte_identical(data, args):
-    _ok([L.REF_BIN_B] + args + ["-d", "want.mmi", "ref.fa"], data)
+    _ref_dump(args, "want.mmi", data)
     _ok([NEW] + args + ["-d", "got.mmi", "ref.fa"], data)
     want, got = open(data / "want.mmi", "rb").read(), open(data / "got.mmi", "rb").read()
     assert len(want) == len(got)
@@ -41,14 +52,19 @@ def test_dump_is_byte_identical(data, args):
 
 @pytest.mark.parametrize("preset,reads", [("sr", ["r1.fq", "r2.fq"]), ("map-ont", ["long.fq"])])
 def test_prebuilt_index_maps_like_fasta(data, preset, reads):
-    _ok([L.REF_BIN_B, "-x", preset, "-d", f"{preset}.mmi", "ref.fa"], data)
-    want = [l for l in _ok([L.REF_BIN_B, "-ax", preset, "-t", "8", "ref.fa"] + reads, data).stdout.decode().split("\n") if not l.startswith("@PG")]
+    _ref_dump(["-x", preset], f"{preset}.mmi", data)
+    want = [l for l in _ok([L.REF_BIN_B if L.have_ref_bin() else NEW, "-ax", preset, "-t", "8", "ref.fa"] + reads, data).stdout.decode().split("\n")
+            if not l.startswith("@PG")]
+    if L.have_ref_bin():
+        L.record_reference_digest(f"mmi map -ax {preset} " + " ".join(reads), want)
+    else:
+        L.check_digest(f"mmi map -ax {preset} " + " ".join(reads), want)
     got = [l for l in _ok([NEW, "-ax", preset, "-t", "8", f"{preset}.mmi"] + reads, data).stdout.decode().split("\n") if not l.startswith("@PG")]
     assert want == got
 
 
 def test_dump_of_loaded_index_round_trips(data):
     """reading a .mmi and writing it again (-d with a .mmi input) keeps the bytes"""
-    _ok([L.REF_BIN_B, "-x", "sr", "-d", "a.mmi", "ref.fa"], data)
+    _ref_dump(["-x", "sr"], "a.mmi", data)
     _ok([NEW, "-x", "sr", "-d", "b.mmi", "a.mmi"], data)
     assert open(data / "a.mmi", "rb").read() == open(data / "b.mmi", "rb").read()
