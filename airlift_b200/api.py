@@ -105,6 +105,8 @@ def lib():
                                     C.c_int8, C.c_int8, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(Extz), C.c_void_p]
         L.mmg_seed_chain_batch.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(MapOpt), C.POINTER(Batch), C.POINTER(Chains)]
         L.mmg_batch_upload.argtypes = [C.c_void_p, C.POINTER(MapOpt), C.POINTER(Batch)]
+        L.mmg_batch_upload_flips.argtypes = [C.c_void_p, C.POINTER(MapOpt), C.POINTER(Batch), C.c_void_p]
+        L.mmg_staging_flips_slot.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]
         L.mmg_seed_chain_resident.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(MapOpt), C.POINTER(Chains), C.c_int]
         L.mmg_ksw_batch.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(MapOpt), C.c_int, C.c_void_p, C.c_void_p,
                                     C.POINTER(C.POINTER(C.c_uint32)), C.POINTER(C.c_double), C.POINTER(C.c_uint64)]
@@ -210,8 +212,16 @@ class Context:
         _check(lib().mmg_seed_chain_batch(self.h, idx.h, C.byref(opt), C.byref(batch), C.byref(out)))
         return out
 
-    def batch_upload(self, opt, batch):
-        _check(lib().mmg_batch_upload(self.h, C.byref(opt), C.byref(batch)))
+    def batch_upload(self, opt, batch, flips=None):
+        """flips: None (mates flipped per opt.pe_ori within each fragment) or one 0/1 per read: 1 = reverse-complemented before
+        mapping, whatever fragment the read is in (how --no-pairing maps the mates of a pair one by one)."""
+        if flips is None:
+            _check(lib().mmg_batch_upload(self.h, C.byref(opt), C.byref(batch)))
+            return
+        flips = np.ascontiguousarray(flips, dtype=np.uint8)
+        if len(flips) != batch.n_seq:
+            raise ValueError(f"{len(flips)} flips for {batch.n_seq} reads")
+        _check(lib().mmg_batch_upload_flips(self.h, C.byref(opt), C.byref(batch), flips.ctypes.data))
 
     def seed_chain_resident(self, idx, opt, download=True):
         out = Chains()

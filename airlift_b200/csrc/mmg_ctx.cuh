@@ -137,6 +137,7 @@ struct mmg_ctx_s {
 	// after z-drop cuts, [5] hits cut at a z-drop
 	uint64_t path[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 	PinBuf h_tab, h_tab_b, h_in_b;     // input tables of the batch being uploaded (mmg_staging_tables); second staging slot
+	PinBuf h_flip, h_flip_b;           // per-read flips of the two staging slots (mmg_staging_flips_slot)
 	PinBuf h_path;                     // device counters of the pass in flight land here
 	PinBuf h_p_hash, h_p_nreg, h_p_offs, h_p_blob, h_p_rep;
 	PinBuf h_in, h_meta, h_out_meta, h_out_u, h_out_a, h_out_mini, h_k_jobs, h_k_res, h_k_cig;

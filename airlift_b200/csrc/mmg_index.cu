@@ -58,7 +58,8 @@ extern "C" void mmg_destroy(mmg_ctx_t *c)
 	for (DevBuf *b : bufs) b->release();
 	for (DevBuf &b : c->pb) b.release();
 	PinBuf *pins[] = {&c->h_in, &c->h_meta, &c->h_out_meta, &c->h_out_u, &c->h_out_a, &c->h_out_mini, &c->h_k_jobs, &c->h_k_res, &c->h_k_cig,
-	                  &c->h_p_hash, &c->h_p_nreg, &c->h_p_offs, &c->h_p_blob, &c->h_p_rep, &c->h_path, &c->h_tab, &c->h_tab_b, &c->h_in_b};
+	                  &c->h_p_hash, &c->h_p_nreg, &c->h_p_offs, &c->h_p_blob, &c->h_p_rep, &c->h_path, &c->h_tab, &c->h_tab_b, &c->h_in_b,
+	                  &c->h_flip, &c->h_flip_b};
 	for (PinBuf *b : pins) b->release();
 	if (getenv("MM2_B200_TRACE")) fprintf(stderr, "[T::buffers] released in %.3f s\n", (mmg_now_ns() - t_rel) * 1e-9);
 	for (int i = 0; i < 4; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);

@@ -1421,9 +1421,11 @@ struct UnitsOfLen { __host__ __device__ int64_t operator()(int32_t len) const { 
 // what the sketch and the later stages need per read and per fragment, from the lengths alone: the sketch work units
 // (one per MMG_READ_CHUNK positions of a read), the mates to flip (pe_ori, map.c:467-469), the fragments' unit ranges and
 // query lengths.  (The host used to build these 60 bytes per read and copy them over from pageable memory, every batch.)
+// flip_given: flip[] already holds the per-read decision (mmg_batch_upload_flips), it is not derived from the fragment here
 __global__ void k_batch_tables(int n_frag, int n_seq, const int32_t *__restrict__ n_seg, const int32_t *__restrict__ seg_off,
                                const int32_t *__restrict__ seq_len, const uint64_t *__restrict__ q_off, const int64_t *__restrict__ unit0, int pe_ori,
-                               SketchUnit *__restrict__ units, uint8_t *__restrict__ flip, int32_t *__restrict__ frag_unit0, int32_t *__restrict__ frag_qlen)
+                               int flip_given, SketchUnit *__restrict__ units, uint8_t *__restrict__ flip, int32_t *__restrict__ frag_unit0,
+                               int32_t *__restrict__ frag_qlen)
 {
 	const int f = blockIdx.x * blockDim.x + threadIdx.x;
 	if (f > n_frag) return;
@@ -1433,7 +1435,7 @@ __global__ void k_batch_tables(int n_frag, int n_seq, const int32_t *__restrict_
 	frag_unit0[f] = (int32_t)unit0[off];
 	for (int j = 0; j < ns; ++j) {
 		const int r = off + j, len = seq_len[r];
-		flip[r] = (ns == 2 && ((j == 0 && (pe_ori >> 1 & 1)) || (j == 1 && (pe_ori & 1)))) ? 1 : 0;
+		if (!flip_given) flip[r] = (ns == 2 && ((j == 0 && (pe_ori >> 1 & 1)) || (j == 1 && (pe_ori & 1)))) ? 1 : 0;
 		int64_t uu = unit0[r];
 		for (int st = 0; st < len; st += MMG_READ_CHUNK) {
 			SketchUnit u;
@@ -1446,7 +1448,28 @@ __global__ void k_batch_tables(int n_frag, int n_seq, const int32_t *__restrict_
 	frag_qlen[f] = sum;
 }
 
-extern "C" int mmg_batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t *b)
+extern "C" int mmg_staging_flips_slot(mmg_ctx_t *c, int slot, int n_seq, uint8_t **flip)
+{
+	cudaSetDevice(c->dev);
+	PinBuf &fl = slot ? c->h_flip_b : c->h_flip;
+	MMG_TRY(fl.ensure((size_t)n_seq + 16));
+	if (c->h_flip_b.p || slot) MMG_TRY((slot ? c->h_flip : c->h_flip_b).ensure((size_t)n_seq + 16)); // both slots grow together, as the tables do
+	*flip = fl.as<uint8_t>();
+	return MMG_OK;
+}
+
+static int batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t *b, const uint8_t *flip_in);
+
+extern "C" int mmg_batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t *b) { return batch_upload(c, opt, b, nullptr); }
+
+extern "C" int mmg_batch_upload_flips(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t *b, const uint8_t *flip)
+{
+	if (flip == nullptr) { mmg_set_error("mmg_batch_upload_flips: no flip table"); return MMG_EINVAL; }
+	return batch_upload(c, opt, b, flip);
+}
+
+// flip_in (n_seq bytes, or null): which reads are reverse-complemented before mapping; null derives it from pe_ori and each fragment's mates
+static int batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t *b, const uint8_t *flip_in)
 {
 	MMG_CUDA(cudaSetDevice(c->dev));
 	ResidentBatch &rb = c->rb;
@@ -1500,6 +1523,15 @@ extern "C" int mmg_batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg
 	MMG_H2D(c, c->d_seq_off.p, t_off, (size_t)(n_seq + 1) * 8);
 	MMG_H2D(c, c->d_misc.p, t_nseg, (size_t)n_frag * 4);
 	MMG_H2D(c, c->d_fseg_off.p, t_segoff, (size_t)n_frag * 4);
+	if (flip_in) { // the per-read flips, from pinned memory like the tables (in place when the caller used mmg_staging_flips_slot)
+		const uint8_t *src = flip_in;
+		if (src != c->h_flip.p && src != c->h_flip_b.p) {
+			MMG_TRY(c->h_flip.ensure((size_t)n_seq + 16));
+			memcpy(c->h_flip.p, flip_in, (size_t)n_seq);
+			src = c->h_flip.as<uint8_t>();
+		}
+		if (n_seq > 0) MMG_H2D(c, c->d_flip.p, src, (size_t)n_seq);
+	}
 	{ // packed (8-base aligned) offset of every read, first sketch unit of every read
 		cub::TransformInputIterator<uint64_t, PadLen8, const int32_t*> it_q(c->d_seq_len.as<int32_t>(), PadLen8());
 		cub::TransformInputIterator<int64_t, UnitsOfLen, const int32_t*> it_u(c->d_seq_len.as<int32_t>(), UnitsOfLen());
@@ -1512,7 +1544,7 @@ extern "C" int mmg_batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg
 		c->launches += 2;
 	}
 	MMG_LAUNCH(c, k_batch_tables, mmg_blocks((size_t)n_frag + 1, 256), 256, 0, n_frag, n_seq, c->d_misc.as<int32_t>(), c->d_fseg_off.as<int32_t>(),
-	           c->d_seq_len.as<int32_t>(), c->d_q_off.as<uint64_t>(), c->d_unit0.as<int64_t>(), opt->pe_ori, c->d_units.as<SketchUnit>(),
+	           c->d_seq_len.as<int32_t>(), c->d_q_off.as<uint64_t>(), c->d_unit0.as<int64_t>(), opt->pe_ori, flip_in ? 1 : 0, c->d_units.as<SketchUnit>(),
 	           c->d_flip.as<uint8_t>(), c->d_frag_unit0.as<int32_t>(), c->d_frag_qlen.as<int32_t>());
 	if (rb.q_words)
 		MMG_LAUNCH(c, k_encode_reads, mmg_blocks(rb.q_words, 256), 256, 0, c->d_ascii.as<uint8_t>(), c->d_seq_off.as<uint64_t>(),

@@ -98,11 +98,18 @@ typedef struct {          /* one GPU's share of a mini-batch */
 	int rc;
 	int slot, stage_mode; /* staging slot of the ctx; 0: stage and upload, 1: stage only (host), 2: upload what an earlier stage-only call left in the slot */
 	const void *batch;    /* the mini-batch the shard belongs to (identifies what a slot holds) */
+	const uint8_t *flip;  /* --no-pairing: [read] 1 if the read is mapped reverse-complemented, decided by the pair it was read in; 0: by pe_ori and the fragment */
 } shard_t;
 
 static inline int mate_is_flipped(const mm_mapopt_t *opt, int n_segs, int j)
 { /* map.c:468 */
 	return n_segs == 2 && ((j == 0 && (opt->pe_ori >> 1 & 1)) || (j == 1 && (opt->pe_ori & 1)));
+}
+
+/* segment j of a fragment of ns reads whose first read is `off` */
+static inline int read_is_flipped(const shard_t *sh, int ns, int j, int off)
+{
+	return sh->flip ? sh->flip[off + j] : mate_is_flipped(sh->opt, ns, j);
 }
 
 static int chain_gap_ref(const mm_mapopt_t *opt, int qlen_sum)
@@ -138,7 +145,7 @@ static void stage_hits(void *data, long i, int tid)
 	if (fr->qlen_sum == 0 || ns <= 0 || ns > MM_MAX_SEG) return;
 	if (opt->max_qlen > 0 && fr->qlen_sum > opt->max_qlen) return;
 	for (j = 0; j < ns; ++j) /* host copy in mapping orientation, undone in stage_finish (map.c:467-469,489) */
-		if (mate_is_flipped(opt, ns, j)) mm_revcomp_bseq(&sh->seq[off + j]);
+		if (read_is_flipped(sh, ns, j, off)) mm_revcomp_bseq(&sh->seq[off + j]);
 	fr->hash = mm_frag_hash(sh->seq[off].name, fr->qlen_sum, opt->seed);
 	fr->frag_gap = chain_gap_ref(opt, fr->qlen_sum);
 	fr->rep_len = ch->rep_len[i];
@@ -256,7 +263,7 @@ static void stage_finish(void *data, long i, int tid)
 		if (ns == 2 && opt->pe_ori >= 0 && (opt->flag & MM_F_CIGAR))
 			mm_pair(fr->frag_gap, opt->pe_bonus, opt->a * 2 + opt->b, opt->a, fr->qlens, &sh->n_reg[off], &sh->reg[off]);
 		for (j = 0; j < ns; ++j)
-			if (mate_is_flipped(opt, ns, j)) {
+			if (read_is_flipped(sh, ns, j, off)) {
 				mm_revcomp_bseq(&sh->seq[off + j]);
 				for (k = 0; k < sh->n_reg[off + j]; ++k) {
 					mm_reg1_t *r = &sh->reg[off + j][k];
@@ -295,6 +302,7 @@ static void *shard_upload(void *data)
 	char *bases;
 	int32_t *n_seg, *seg_off, *seq_len;
 	uint64_t *seq_off;
+	uint8_t *flip = 0;
 	mmg_batch_t b;
 	double t0;
 	sh->rc = 0;
@@ -307,12 +315,21 @@ static void *shard_upload(void *data)
 		n_seq = B->staged[ci][sh->slot].n_seq, n_bases = B->staged[ci][sh->slot].n_bases;
 		bases = (char*)mmg_staging_slot(sh->ctx, sh->slot, n_bases + 1);
 		mmg_staging_tables_slot(sh->ctx, sh->slot, n_seq, nf, &seq_len, &seq_off, &n_seg, &seg_off);
+		if (sh->flip && mmg_staging_flips_slot(sh->ctx, sh->slot, n_seq, &flip) != MMG_OK) {
+			shard_fail(sh, "cannot allocate the staging buffers"); if (sh->up_token) pthread_mutex_unlock(sh->up_token); return 0;
+		}
 	} else {
 		for (i = sh->f0; i < sh->f1; ++i) n_seq += sh->n_seg[i];
 		for (i = 0; i < n_seq; ++i) n_bases += sh->seq[sh->s0 + i].l_seq;
 		bases = (char*)mmg_staging_slot(sh->ctx, sh->slot, n_bases + 1);
 		if (bases == 0 || mmg_staging_tables_slot(sh->ctx, sh->slot, n_seq, nf, &seq_len, &seq_off, &n_seg, &seg_off) != MMG_OK) {
 			shard_fail(sh, "cannot allocate the staging buffers"); if (mode != 1 && sh->up_token) pthread_mutex_unlock(sh->up_token); return 0;
+		}
+		if (sh->flip) { /* the reads are uploaded as read; the device flips them from this table */
+			if (mmg_staging_flips_slot(sh->ctx, sh->slot, n_seq, &flip) != MMG_OK) {
+				shard_fail(sh, "cannot allocate the staging buffers"); if (mode != 1 && sh->up_token) pthread_mutex_unlock(sh->up_token); return 0;
+			}
+			memcpy(flip, sh->flip + sh->s0, (size_t)n_seq);
 		}
 		for (i = 0, o = 0; i < n_seq; ++i) {
 			seq_len[i] = sh->seq[sh->s0 + i].l_seq, seq_off[i] = o;
@@ -330,7 +347,7 @@ static void *shard_upload(void *data)
 		}
 	}
 	b.n_frag = nf, b.n_seq = n_seq, b.n_seg = n_seg, b.seg_off = seg_off, b.seq_len = seq_len, b.seq_off = seq_off, b.bases = bases, b.n_bases = n_bases;
-	if (mmg_batch_upload(sh->ctx, &sh->dopt, &b) != MMG_OK) shard_fail(sh, "read upload failed");
+	if ((flip ? mmg_batch_upload_flips(sh->ctx, &sh->dopt, &b, flip) : mmg_batch_upload(sh->ctx, &sh->dopt, &b)) != MMG_OK) shard_fail(sh, "read upload failed");
 	if (getenv("MM2_B200_TRACE")) fprintf(stderr, "[T::upload] +device upload %.4f s\n", realtime() - t0);
 	sh->st.n_frag += nf, sh->st.n_reads += n_seq, sh->st.n_bases += n_bases;
 	sh->st.t_upload += realtime() - t0;
@@ -386,7 +403,7 @@ static void stage_dev_finish(void *data, long i, int tid)
 		if (ns == 2 && opt->pe_ori >= 0 && (opt->flag & MM_F_CIGAR))
 			mm_pair(frag_gap, opt->pe_bonus, opt->a * 2 + opt->b, opt->a, qlens, &sh->n_reg[off], &sh->reg[off]);
 		for (j = 0; j < ns; ++j)
-			if (mate_is_flipped(opt, ns, j)) /* the host copy of the read was never flipped on this path: only the coordinates are */
+			if (read_is_flipped(sh, ns, j, off)) /* the host copy of the read was never flipped on this path: only the coordinates are */
 				for (k = 0; k < sh->n_reg[off + j]; ++k) {
 					mm_reg1_t *r = &sh->reg[off + j][k];
 					const int t = r->qs;
@@ -573,10 +590,23 @@ static int map_step_group(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_thre
 	int d, f = 0, rc = 0, pass;
 	int64_t tot = 0, acc = 0;
 	const double t_start = realtime();
+	/* the mapping units: the fragments as read, or with --no-pairing every read on its own (worker_for, map.c:475-485); the
+	 * writer keeps the step's own fragment tables, so that records still print as pairs */
+	int n_unit = s->n_frag, *u_seg = s->n_seg, *u_off = s->seg_off, *u_tab = 0;
+	uint8_t *u_flip = 0;
 	mm_b200_tune_malloc();
 	if (mm_b200_check_opt(opt) < 0) { free(sh); free(tid); return -1; }
+	if (opt->flag & MM_F_INDEPEND_SEG) {
+		int k, j;
+		u_tab = (int*)malloc(2 * (size_t)s->n_seq * sizeof(int) + 1);
+		u_flip = (uint8_t*)malloc((size_t)s->n_seq + 1);
+		n_unit = s->n_seq, u_seg = u_tab, u_off = u_tab + s->n_seq;
+		for (d = 0; d < s->n_seq; ++d) u_seg[d] = 1, u_off[d] = d;
+		for (k = 0; k < s->n_frag; ++k) /* the mates are still flipped as the pair they were read in (map.c:467-469) */
+			for (j = 0; j < s->n_seg[k]; ++j) u_flip[s->seg_off[k] + j] = mate_is_flipped(opt, s->n_seg[k], j);
+	}
 	for (d = 0; d < s->n_seq; ++d) tot += s->seq[d].l_seq;
-	for (d = 0; d < n_dev; ++d) { /* contiguous fragment ranges balanced by bases; a fragment is never cut */
+	for (d = 0; d < n_dev; ++d) { /* contiguous unit ranges balanced by bases; a unit is never cut (with --no-pairing a pair may be) */
 		shard_t *h = &sh[d];
 		/* device path with two shards per GPU: the first shard is the smaller one, so that its upload (the only one no kernel
 		 * can hide) is short and the second, larger upload runs under its kernels */
@@ -592,15 +622,16 @@ static int map_step_group(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_thre
 		h->gpu_token = B->lanes > 1 && (!use_device_path(mi, opt) || g_serial_shards) ? &B->gpu_token[gpu] : 0;
 		h->up_token = B->lanes > 1 && use_device_path(mi, opt) ? &B->up_token[gpu] : 0;
 		h->slot = slot, h->stage_mode = stage_mode, h->batch = s;
-		h->seq = s->seq, h->n_seg = s->n_seg, h->seg_off = s->seg_off, h->n_reg = s->n_reg, h->rep_len = s->rep_len, h->frag_gap = s->frag_gap, h->reg = s->reg;
+		h->seq = s->seq, h->n_seg = u_seg, h->seg_off = u_off, h->n_reg = s->n_reg, h->rep_len = s->rep_len, h->frag_gap = s->frag_gap, h->reg = s->reg;
+		h->flip = u_flip;
 		h->f0 = f;
-		while (f < s->n_frag && (acc < goal || d == n_dev - 1)) {
+		while (f < n_unit && (acc < goal || d == n_dev - 1)) {
 			int j;
-			for (j = 0; j < s->n_seg[f]; ++j) acc += s->seq[s->seg_off[f] + j].l_seq;
+			for (j = 0; j < u_seg[f]; ++j) acc += s->seq[u_off[f] + j].l_seq;
 			++f;
 		}
 		h->f1 = f;
-		if (h->f1 > h->f0) h->s0 = s->seg_off[h->f0];
+		if (h->f1 > h->f0) h->s0 = u_off[h->f0];
 	}
 	if (stage_mode == 1) mode = 1; /* host staging only */
 	for (pass = 0; pass < 2; ++pass) {
@@ -634,7 +665,7 @@ static int map_step_group(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_thre
 			fprintf(stderr, "[T::map_step] at %.3f: %.3f s, shard %d: %d frags, upload %.3f seed/chain %.3f (kernels %.3f) hits %.3f align %.3f dp %.3f (kernel %.3f) finish %.3f\n",
 					realtime() - mm_realtime0, realtime() - t_start, d, sh[d].f1 - sh[d].f0, t->t_upload, t->t_seedchain, t->t_seedchain_kernels, t->t_hits, t->t_align_host, t->t_ksw_total, t->t_ksw_kernel, t->t_finish);
 		}
-	free(sh); free(tid);
+	free(sh); free(tid); free(u_tab); free(u_flip);
 	return rc;
 }
 
@@ -970,7 +1001,6 @@ int mm_b200_check_opt(const mm_mapopt_t *opt)
 { /* what the device stages do not implement is refused with a message; nothing is silently dropped */
 	const char *what = 0;
 	if (opt->flag & MM_F_SPLICE) what = "spliced alignment (--splice, ksw_exts2)";
-	else if (opt->flag & MM_F_INDEPEND_SEG) what = "--no-pairing";
 	else if (opt->flag & (MM_F_NO_DIAG | MM_F_NO_DUAL)) what = "the self/dual-hit filters of the all-vs-all modes (-D, -X, --dual=no, ava-ont, ava-pb; map.c:128-137)";
 	else if (opt->sdust_thres > 0) what = "SDUST masking of query minimizers (-T, map.c:41-62)";
 	else if (opt->split_prefix) what = "--split-prefix (the index is a single part in HBM)";
@@ -1002,7 +1032,9 @@ void mm_map_frag(const mm_idx_t *mi, int n_segs, const int *qlens, const char **
 	}
 	memset(&sh, 0, sizeof(sh));
 	mm_arena_init(&sh.arena);
-	/* worker_for flips the mates of a pair around this call (map.c:467-469,486-497); callers of the library API
+	/* MM_F_INDEPEND_SEG is read by the file and batch drivers only (worker_for, map.c:475-485): the reference's mm_map_frag maps
+	 * the segments it is given jointly whatever the flag, and so does this one (shard_t::flip stays 0).
+	 * worker_for flips the mates of a pair around this call (map.c:467-469,486-497); callers of the library API
 	 * pass sequences already in mapping orientation, so neither the host nor the device flips here.
 	 * pe_ori = 0 keeps `pe_ori >= 0` (pairing on, map.c:404) while naming no mate to flip. */
 	o2 = *opt;

@@ -193,9 +193,11 @@ mm_idx_t *mm_b200_idx_alloc_named(const mm_idxopt_t *opt, int n_seq, const char 
                                   const mmg_idx_image_t *shape, mmg_idx_image_t *ptrs); /* same, without re-reading the FASTA */
 int mm_b200_idx_seq(const mm_idx_t *mi, int i, const char **name, uint32_t *len);
 int mm_b200_idx_finalize(mm_idx_t *mi);
-/* options this build does not implement (splice, --no-pairing, -D/-X/--dual=no, -T, --split-prefix) are refused, never
- * ignored: 0 if opt can be mapped with, else -1 after an [ERROR] line.  mm_map_frag()/mm_map() take turns on a lock (one
- * resident batch per GPU context), so concurrent callers are safe but serialised. */
+/* options this build does not implement (splice, -D/-X/--dual=no, -T, --split-prefix) are refused, never ignored: 0 if
+ * opt can be mapped with, else -1 after an [ERROR] line.  MM_F_INDEPEND_SEG (--no-pairing) maps the two reads of a pair
+ * one by one in mm_map_file_frag() and mm_b200_map_batch(es); mm_map_frag() maps the segments it is given jointly, as the
+ * reference does.  mm_map_frag()/mm_map() take turns on a lock (one resident batch per GPU context), so concurrent
+ * callers are safe but serialised. */
 int mm_b200_check_opt(const mm_mapopt_t *opt);
 int mm_b200_set_lanes(int lanes); /* streams (with their arenas) per GPU, 1..8; before building the index */
 

@@ -168,6 +168,12 @@ int  mmg_staging_tables(mmg_ctx_t *ctx, int n_seq, int n_frag, int32_t **seq_len
 /* the same with an explicit slot (0 or 1): a caller can fill slot 1 for its next batch while the batch staged in slot 0 is mapped */
 void *mmg_staging_slot(mmg_ctx_t *ctx, int slot, size_t bytes);
 int  mmg_staging_tables_slot(mmg_ctx_t *ctx, int slot, int n_seq, int n_frag, int32_t **seq_len, uint64_t **seq_off, int32_t **n_seg, int32_t **seg_off);
+/* mmg_batch_upload with the flip of every read given (flip[n_seq]: 1 = reverse-complement the read before mapping) instead of
+ * derived from pe_ori and each fragment's segment count.  For batches whose fragments are single reads cut from pairs
+ * (--no-pairing, map.c:458-498): the mates are still flipped as for a pair, but mapped one by one. */
+int  mmg_batch_upload_flips(mmg_ctx_t *ctx, const mmg_mapopt_t *opt, const mmg_batch_t *batch, const uint8_t *flip);
+/* pinned array of the ctx for that flip table in slot 0 or 1 (n_seq bytes): fill it and pass it to skip a host copy */
+int  mmg_staging_flips_slot(mmg_ctx_t *ctx, int slot, int n_seq, uint8_t **flip);
 /* page-locked job / result arrays owned by the ctx (kept across batches) for mmg_ksw_batch; plain malloc'd arrays work too, slower */
 
 int  mmg_seed_chain_resident(mmg_ctx_t *ctx, const mmg_idx_t *idx, const mmg_mapopt_t *opt, mmg_chains_t *out, int download);
