@@ -19,7 +19,7 @@ all: lib tools cli emu
 lib: $(LIB)
 tools: $(BUILD)/mmsynth
 cli: $(if $(wildcard $(HOST)/main.c),$(BUILD)/minimap2-b200)
-emu: $(BUILD)/libmmg_emu.so
+emu: $(BUILD)/libmmg_emu.so $(BUILD)/libmmg_emu_named.so
 
 $(BUILD):
 	mkdir -p $(BUILD)
@@ -43,6 +43,9 @@ $(BUILD)/mmsynth: tools/mmsynth.c | $(BUILD)
 
 # CPU emulation of the per-thread device code (test harness only; never linked into the product)
 $(BUILD)/libmmg_emu.so: tests/emu/emu.cpp $(CUHDR) | $(BUILD)
+	g++ -O2 -g -std=c++17 -fPIC -shared -ffp-contract=off -I$(CSRC) $< -o $@
+
+$(BUILD)/libmmg_emu_named.so: tests/emu/emu_named.cpp tests/emu/emu.cpp $(CUHDR) | $(BUILD)
 	g++ -O2 -g -std=c++17 -fPIC -shared -ffp-contract=off -I$(CSRC) $< -o $@
 
 oracle:

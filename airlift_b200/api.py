@@ -23,6 +23,9 @@ MM_F_2_IO_THREADS = 0x8000
 MM_F_FOR_ONLY = 0x100000
 MM_F_REV_ONLY = 0x200000
 MM_F_HEAP_SORT = 0x400000
+MM_F_NO_DIAG = 0x001
+MM_F_NO_DUAL = 0x002
+NAME_NONE = 0xffffffff  # MMG_NAME_NONE: the unit key of a fragment without a name
 
 
 class MmgError(RuntimeError):
@@ -108,6 +111,14 @@ def lib():
         L.mmg_batch_upload_flips.argtypes = [C.c_void_p, C.POINTER(MapOpt), C.POINTER(Batch), C.c_void_p]
         L.mmg_staging_flips_slot.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]
         L.mmg_seed_chain_resident.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(MapOpt), C.POINTER(Chains), C.c_int]
+        L.mmg_collect_seeds_named.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_uint32,
+                                              C.c_void_p, C.c_int64, C.POINTER(C.c_int64), C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_void_p]
+        L.mmg_idx_set_name_keys.argtypes = [C.c_void_p, C.c_void_p]
+        L.mmg_batch_set_name_keys.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
+        L.mm_b200_name_order.argtypes = [C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), C.c_void_p]
+        L.mm_b200_name_ukey.restype = C.c_uint32
+        L.mm_b200_name_ukey.argtypes = [C.c_int, C.POINTER(C.c_char_p), C.c_char_p]
+        L.mmg_path_counts.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
         L.mmg_ksw_batch.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(MapOpt), C.c_int, C.c_void_p, C.c_void_p,
                                     C.POINTER(C.POINTER(C.c_uint32)), C.POINTER(C.c_double), C.POINTER(C.c_uint64)]
         _lib = L
@@ -166,14 +177,25 @@ class Context:
         _check(lib().mmg_sketch(self.h, seq, len(seq), w, k, rid, hpc, out.ctypes.data, len(out), C.byref(n)))
         return out[:n.value].copy()
 
-    def collect_seeds(self, idx, heap_sort, flag, max_occ, mv, qlen, cap):
+    def collect_seeds(self, idx, heap_sort, flag, max_occ, mv, qlen, cap, name=False):
+        """name: the fragment's name (bytes, or None for no name) against an Index whose set_names() was called; False: no
+        self/dual filtering (mmg_collect_seeds)"""
         mv = np.ascontiguousarray(mv)
         a = np.zeros(cap + 1, dtype=mm128)
         mp = np.zeros(len(mv) + 1, dtype=np.uint64)
         n_a, rep, nm = C.c_int64(0), C.c_int(0), C.c_int(0)
-        _check(lib().mmg_collect_seeds(self.h, idx.h, int(heap_sort), flag, max_occ, len(mv), mv.ctypes.data, qlen, a.ctypes.data, cap,
-                                       C.byref(n_a), C.byref(rep), C.byref(nm), mp.ctypes.data))
+        if name is False:
+            _check(lib().mmg_collect_seeds(self.h, idx.h, int(heap_sort), flag, max_occ, len(mv), mv.ctypes.data, qlen, a.ctypes.data, cap,
+                                           C.byref(n_a), C.byref(rep), C.byref(nm), mp.ctypes.data))
+        else:
+            _check(lib().mmg_collect_seeds_named(self.h, idx.h, int(heap_sort), flag, max_occ, len(mv), mv.ctypes.data, qlen, idx.unit_key(name),
+                                                 a.ctypes.data, cap, C.byref(n_a), C.byref(rep), C.byref(nm), mp.ctypes.data))
         return a[:n_a.value].copy(), rep.value, mp[:nm.value].copy()
+
+    def path_counts(self, reset=False):
+        out = np.zeros(8, dtype=np.uint64)
+        lib().mmg_path_counts(self.h, out.ctypes.data, 1 if reset else 0)
+        return out
 
     def chain_dp(self, params, a):
         a = np.ascontiguousarray(a.copy())
@@ -212,16 +234,23 @@ class Context:
         _check(lib().mmg_seed_chain_batch(self.h, idx.h, C.byref(opt), C.byref(batch), C.byref(out)))
         return out
 
-    def batch_upload(self, opt, batch, flips=None):
+    def batch_upload(self, opt, batch, flips=None, names=None, idx=None):
         """flips: None (mates flipped per opt.pe_ori within each fragment) or one 0/1 per read: 1 = reverse-complemented before
-        mapping, whatever fragment the read is in (how --no-pairing maps the mates of a pair one by one)."""
+        mapping, whatever fragment the read is in (how --no-pairing maps the mates of a pair one by one).
+        names: one name (bytes, or None) per fragment for the self/dual filters (-D, --dual=no), ordered against the target names
+        given to idx.set_names()."""
         if flips is None:
             _check(lib().mmg_batch_upload(self.h, C.byref(opt), C.byref(batch)))
-            return
-        flips = np.ascontiguousarray(flips, dtype=np.uint8)
-        if len(flips) != batch.n_seq:
-            raise ValueError(f"{len(flips)} flips for {batch.n_seq} reads")
-        _check(lib().mmg_batch_upload_flips(self.h, C.byref(opt), C.byref(batch), flips.ctypes.data))
+        else:
+            flips = np.ascontiguousarray(flips, dtype=np.uint8)
+            if len(flips) != batch.n_seq:
+                raise ValueError(f"{len(flips)} flips for {batch.n_seq} reads")
+            _check(lib().mmg_batch_upload_flips(self.h, C.byref(opt), C.byref(batch), flips.ctypes.data))
+        if names is not None:
+            if idx is None or len(names) != batch.n_frag:
+                raise ValueError("names needs one name per fragment and the Index they are ordered against")
+            ukey = np.array([idx.unit_key(n) for n in names], dtype=np.uint32)
+            _check(lib().mmg_batch_set_name_keys(self.h, batch.n_frag, ukey.ctypes.data))
 
     def seed_chain_resident(self, idx, opt, download=True):
         out = Chains()
@@ -258,6 +287,20 @@ class Index:
         if self.h:
             lib().mmg_idx_free(self.h)
             self.h = C.c_void_p()
+
+    def set_names(self, names):
+        """the targets' names (bytes, one per sequence): computes and uploads their name keys for the self/dual filters"""
+        n = len(names)
+        self._names = (C.c_char_p * max(n, 1))(*names)  # the sorted table points into these
+        self._sorted = (C.c_char_p * max(n, 1))()
+        tkey = np.zeros(max(n, 1), dtype=np.uint32)
+        lib().mm_b200_name_order(n, self._names, self._sorted, tkey.ctypes.data)
+        self._n_names = n
+        _check(lib().mmg_idx_set_name_keys(self.h, tkey.ctypes.data))
+
+    def unit_key(self, name):
+        """the name key of a fragment named `name` (None: no name) against the names of set_names()"""
+        return lib().mm_b200_name_ukey(self._n_names, self._sorted, name)
 
     def n_minimizers(self):
         return lib().mmg_idx_n_minimizers(self.h)

@@ -23,8 +23,12 @@ struct mm128 { uint64_t x, y; };
 #define MMG_NONE 0xffffffffffffffffULL
 #define MMG_MAX_W 64               // ring buffer size of the sketch state machine (reference allows 255)
 #define MMG_SEED_TANDEM (1ULL << 42)  // mmpriv.h:18
+#define MMG_SEED_SELF (1ULL << 43)    // mmpriv.h:19
 #define MMG_SEED_SEG_SHIFT 48         // mmpriv.h:21
 #define MMG_SEED_SEG_MASK (0xffULL << MMG_SEED_SEG_SHIFT)
+#define MMG_NAME_NONE 0xffffffffu     // name key of a unit without a name (include/mmg.h)
+#define MMG_F_NO_DIAG 0x001LL         // minimap.h:8
+#define MMG_F_NO_DUAL 0x002LL
 #define MMG_F_FOR_ONLY 0x100000LL     // minimap.h:28
 #define MMG_F_REV_ONLY 0x200000LL
 #define MMG_F_HEAP_SORT 0x400000LL
@@ -170,6 +174,7 @@ struct IdxView {
 	const uint32_t *S;
 	const uint64_t *seq_off;
 	const uint32_t *seq_len;
+	const uint32_t *tkey;      // name key of every target (mmg_idx_set_name_keys); null until set
 	const IdxSlot *slots;
 	const uint64_t *pos;
 	uint64_t slot_mask;
@@ -223,13 +228,41 @@ MMG_HDN inline int64_t mmg_frag_plan(const mm128 *mv, const int32_t *m_n, int n_
 	return n_a;
 }
 
-MMG_HD bool mmg_skip_seed(int64_t flag, uint64_t r, uint32_t q_pos)  // skip_seed, map.c:139-145 (strand filters only)
+// The self/dual-hit filters of skip_seed compare the mapping unit's name with the target's.  The device sees the names only as
+// the order keys of include/mmg.h: tkey[rid] per target, ukey per unit (MMG_NAME_NONE: the filters are off for the unit).
+struct NameFilt { const uint32_t *tkey, *tlen; uint32_t ukey; };
+
+#define MMG_SKIP_KEEP 0
+#define MMG_SKIP_STRAND 1  // dropped by --for-only / --rev-only
+#define MMG_SKIP_NAME 2    // dropped by -D (diagonal of a self-hit) or --dual=no (target name sorts below the unit's)
+
+// skip_seed, map.c:125-147; qlen is the unit's summed length.  *is_self: same-strand anchor of a unit mapped onto the target of
+// its own name and length (MMG_SEED_SELF).  Nothing is read from nf unless a name filter is on.
+MMG_HD int mmg_skip_seed(int64_t flag, uint64_t r, uint32_t q_pos, const NameFilt &nf, int qlen, bool *is_self)
 {
-	if (flag & (MMG_F_FOR_ONLY | MMG_F_REV_ONLY)) {
-		if ((r & 1) == (q_pos & 1)) { if (flag & MMG_F_REV_ONLY) return true; }
-		else if (flag & MMG_F_FOR_ONLY) return true;
+	*is_self = false;
+	if ((flag & (MMG_F_NO_DIAG | MMG_F_NO_DUAL)) && nf.ukey != MMG_NAME_NONE) {
+		const uint32_t rid = (uint32_t)(r >> 32), tk = nf.tkey[rid];
+		if ((flag & MMG_F_NO_DIAG) && tk == nf.ukey && (int)nf.tlen[rid] == qlen) {
+			if ((uint32_t)r >> 1 == q_pos >> 1) return MMG_SKIP_NAME;
+			if ((r & 1) == (q_pos & 1)) *is_self = true;
+		}
+		if ((flag & MMG_F_NO_DUAL) && tk < nf.ukey) return MMG_SKIP_NAME;
 	}
-	return false;
+	if (flag & (MMG_F_FOR_ONLY | MMG_F_REV_ONLY)) {
+		if ((r & 1) == (q_pos & 1)) { if (flag & MMG_F_REV_ONLY) return MMG_SKIP_STRAND; }
+		else if (flag & MMG_F_FOR_ONLY) return MMG_SKIP_STRAND;
+	}
+	return MMG_SKIP_KEEP;
+}
+
+// Strand-only forms of the functions below, for callers without name keys (the self/dual filters off): the strand filters,
+// no self bit, no count of hits dropped by name
+MMG_HD bool mmg_skip_seed(int64_t flag, uint64_t r, uint32_t q_pos)
+{
+	const NameFilt nf = {nullptr, nullptr, MMG_NAME_NONE};
+	bool self;
+	return mmg_skip_seed(flag, r, q_pos, nf, 0, &self) != MMG_SKIP_KEEP;
 }
 
 MMG_HD bool mmg_is_tandem(const mm128 *mv, int n_mv, int i)  // map.c:113-115
@@ -238,7 +271,7 @@ MMG_HD bool mmg_is_tandem(const mm128 *mv, int n_mv, int i)  // map.c:113-115
 	return (i > 0 && h == mv[i - 1].x >> 8) || (i < n_mv - 1 && h == mv[i + 1].x >> 8);
 }
 
-MMG_HD mm128 mmg_make_anchor(uint64_t r, const mm128 &m, bool tandem, int qlen)  // map.c:176-187 / 232-241
+MMG_HD mm128 mmg_make_anchor(uint64_t r, const mm128 &m, bool tandem, bool self, int qlen)  // map.c:176-187 / 232-241
 {
 	const uint32_t q_pos = (uint32_t)m.y, q_span = (uint32_t)(m.x & 0xff), seg_id = (uint32_t)(m.y >> 32);
 	const uint32_t rpos = (uint32_t)r >> 1;
@@ -252,8 +285,10 @@ MMG_HD mm128 mmg_make_anchor(uint64_t r, const mm128 &m, bool tandem, int qlen) 
 	}
 	p.y |= (uint64_t)seg_id << MMG_SEED_SEG_SHIFT;
 	if (tandem) p.y |= MMG_SEED_TANDEM;
+	if (self) p.y |= MMG_SEED_SELF;
 	return p;
 }
+MMG_HD mm128 mmg_make_anchor(uint64_t r, const mm128 &m, bool tandem, int qlen) { return mmg_make_anchor(r, m, tandem, false, qlen); }
 
 MMG_HD uint64_t mmg_hit_pos(const uint64_t *pos, int n, uint64_t val, uint32_t j) { return n == 1 ? val : pos[val + j]; }
 
@@ -273,11 +308,16 @@ MMG_HD void mmg_heap_down(size_t i, size_t n, mm128 *l)
 // collect_seed_hits_heap (map.c:149-213): k-way merge of the per-minimizer position lists.
 // heap[] is scratch with room for n_mv entries.  a[] has room for n_a_planned anchors.
 // Equal-x anchors come out in the heap's own order (SURVEY.md H2), hence the literal replay.
+// *n_named receives the hits the self/dual filters dropped (here and in mmg_fill_flat).  kNamed = false compiles the filters out
+// (options without MMG_F_NO_DIAG / MMG_F_NO_DUAL), so that the kernels of the other presets keep their registers.
+#define MMG_NAMED_FLAG(kNamed, flag) ((kNamed) ? (flag) : (flag) & ~(MMG_F_NO_DIAG | MMG_F_NO_DUAL))
+template <bool kNamed = true>
 MMG_HDN inline int64_t mmg_fill_heap(const mm128 *mv, const int32_t *m_n, const uint64_t *m_val, int n_mv, int max_occ,
-                                     const uint64_t *pos, int64_t flag, int qlen, int64_t n_a_planned, mm128 *heap, mm128 *a)
+                                     const uint64_t *pos, int64_t flag, const NameFilt &nf, int qlen, int64_t n_a_planned, mm128 *heap,
+                                     mm128 *a, int64_t *n_named)
 {
 	size_t hs = 0;
-	int64_t n_for = 0, n_rev = 0, n_a = n_a_planned;
+	int64_t n_for = 0, n_rev = 0, n_a = n_a_planned, n_nm = 0;
 	for (int i = 0; i < n_mv; ++i)
 		if (m_n[i] > 0 && m_n[i] < max_occ) {
 			heap[hs].x = mmg_hit_pos(pos, m_n[i], m_val[i], 0);
@@ -288,11 +328,13 @@ MMG_HDN inline int64_t mmg_fill_heap(const mm128 *mv, const int32_t *m_n, const 
 	while (hs > 0) {
 		const int i = (int)(heap[0].y >> 32);
 		const uint64_t r = heap[0].x;
-		if (!mmg_skip_seed(flag, r, (uint32_t)mv[i].y)) {
-			const mm128 an = mmg_make_anchor(r, mv[i], mmg_is_tandem(mv, n_mv, i), qlen);
+		bool self;
+		const int sk = mmg_skip_seed(MMG_NAMED_FLAG(kNamed, flag), r, (uint32_t)mv[i].y, nf, qlen, &self);
+		if (sk == MMG_SKIP_KEEP) {
+			const mm128 an = mmg_make_anchor(r, mv[i], mmg_is_tandem(mv, n_mv, i), self, qlen);
 			if ((r & 1) == ((uint32_t)mv[i].y & 1)) a[n_for++] = an;
 			else a[n_a - (++n_rev)] = an;
-		}
+		} else n_nm += sk == MMG_SKIP_NAME;
 		if ((uint32_t)heap[0].y < (uint32_t)m_n[i] - 1) {
 			++heap[0].y;
 			heap[0].x = mmg_hit_pos(pos, m_n[i], m_val[i], (uint32_t)heap[0].y);
@@ -307,11 +349,19 @@ MMG_HDN inline int64_t mmg_fill_heap(const mm128 *mv, const int32_t *m_n, const 
 		a[n_a - 1 - j] = a[n_a - (n_rev - j)];
 		a[n_a - (n_rev - j)] = t;
 	}
-	if (n_a > n_for + n_rev) { // map.c:208-211 (only with strand filters)
+	if (n_a > n_for + n_rev) { // map.c:208-211 (only with strand or self/dual filters)
 		for (int64_t j = 0; j < n_rev; ++j) a[n_for + j] = a[n_a - n_rev + j];
 		n_a = n_for + n_rev;
 	}
+	*n_named = n_nm;
 	return n_a;
+}
+MMG_HDN inline int64_t mmg_fill_heap(const mm128 *mv, const int32_t *m_n, const uint64_t *m_val, int n_mv, int max_occ,
+                                     const uint64_t *pos, int64_t flag, int qlen, int64_t n_a_planned, mm128 *heap, mm128 *a)
+{
+	const NameFilt nf = {nullptr, nullptr, MMG_NAME_NONE};
+	int64_t nn;
+	return mmg_fill_heap<false>(mv, m_n, m_val, n_mv, max_occ, pos, flag, nf, qlen, n_a_planned, heap, a, &nn);
 }
 
 // The same merge replayed on RANKS.  Which of two equal positions leaves the heap first depends on the heap's shape, so the
@@ -410,21 +460,33 @@ MMG_HDN inline void mmg_rs_sort_exact(T *a, int64_t n, RsFrame *stack, KeyFn key
 struct KeyX { MMG_HD uint64_t operator()(const mm128 &v) const { return v.x; } };
 
 // collect_seed_hits (map.c:215-247): fill in query order, then radix_sort_128x
+template <bool kNamed = true>
 MMG_HDN inline int64_t mmg_fill_flat(const mm128 *mv, const int32_t *m_n, const uint64_t *m_val, int n_mv, int max_occ,
-                                     const uint64_t *pos, int64_t flag, int qlen, mm128 *a, RsFrame *stack)
+                                     const uint64_t *pos, int64_t flag, const NameFilt &nf, int qlen, mm128 *a, RsFrame *stack,
+                                     int64_t *n_named)
 {
-	int64_t o = 0;
+	int64_t o = 0, n_nm = 0;
 	for (int i = 0; i < n_mv; ++i) {
 		if (m_n[i] <= 0 || m_n[i] >= max_occ) continue;
 		const bool tandem = mmg_is_tandem(mv, n_mv, i);
 		for (uint32_t j = 0; j < (uint32_t)m_n[i]; ++j) {
 			const uint64_t r = mmg_hit_pos(pos, m_n[i], m_val[i], j);
-			if (mmg_skip_seed(flag, r, (uint32_t)mv[i].y)) continue;
-			a[o++] = mmg_make_anchor(r, mv[i], tandem, qlen);
+			bool self;
+			const int sk = mmg_skip_seed(MMG_NAMED_FLAG(kNamed, flag), r, (uint32_t)mv[i].y, nf, qlen, &self);
+			if (sk != MMG_SKIP_KEEP) { n_nm += sk == MMG_SKIP_NAME; continue; }
+			a[o++] = mmg_make_anchor(r, mv[i], tandem, self, qlen);
 		}
 	}
 	mmg_rs_sort_exact(a, o, stack, KeyX());
+	*n_named = n_nm;
 	return o;
+}
+MMG_HDN inline int64_t mmg_fill_flat(const mm128 *mv, const int32_t *m_n, const uint64_t *m_val, int n_mv, int max_occ,
+                                     const uint64_t *pos, int64_t flag, int qlen, mm128 *a, RsFrame *stack)
+{
+	const NameFilt nf = {nullptr, nullptr, MMG_NAME_NONE};
+	int64_t nn;
+	return mmg_fill_flat<false>(mv, m_n, m_val, n_mv, max_occ, pos, flag, nf, qlen, a, stack, &nn);
 }
 
 // ------------------------------------------------------------------ K3: chaining

@@ -84,11 +84,12 @@ struct mmg_idx_s {
 	IdxSlot *d_slots = nullptr;
 	uint64_t *d_pos = nullptr;
 	uint32_t *d_counts = nullptr;      // occurrences per distinct minimizer (for mm_idx_cal_max_occ)
+	uint32_t *d_tkey = nullptr;        // name key of every target (mmg_idx_set_name_keys); null until set
 	std::vector<uint64_t> h_seq_off;   // host copies: job generation needs them
 	std::vector<uint32_t> h_seq_len;
 	IdxView view() const {
 		IdxView v;
-		v.S = d_S, v.seq_off = d_seq_off, v.seq_len = d_seq_len, v.slots = d_slots, v.pos = d_pos;
+		v.S = d_S, v.seq_off = d_seq_off, v.seq_len = d_seq_len, v.tkey = d_tkey, v.slots = d_slots, v.pos = d_pos;
 		v.slot_mask = n_slots - 1, v.slot_shift = slot_shift, v.n_seq = n_seq, v.w = w, v.k = k;
 		return v;
 	}
@@ -97,6 +98,7 @@ struct mmg_idx_s {
 // state of the mini-batch currently resident on the device
 struct ResidentBatch {
 	int32_t n_frag = 0, n_seq = 0, n_units = 0, max_len = 0;
+	int32_t n_ukey = -1;             // fragments whose name keys were set for this batch (mmg_batch_set_name_keys); -1: none
 	uint64_t n_bases = 0, q_words = 0;
 	std::vector<int32_t> n_seg, seg_off, seq_len;
 };
@@ -118,13 +120,14 @@ struct mmg_ctx_s {
 	DevBuf d_ascii, d_Q, d_seq_len, d_seq_off, d_q_off, d_flip, d_units, d_unit_cnt, d_unit_off, d_mv, d_m_n, d_m_val,
 	       d_frag_unit0, d_frag_qlen, d_frag_na, d_frag_aoff, d_frag_rep, d_frag_nmini, d_mini, d_a, d_work, d_u, d_b, d_heap,
 	       d_stack, d_frag_nu, d_frag_nv, d_frag_flag, d_frag_iter, d_cub, d_out_u, d_out_a, d_out_mini, d_uoff, d_voff, d_moff,
-	       d_frag_list, d_misc, d_seg_head, d_seg_start, d_seg_avg, d_replay, d_skey, d_sval, d_sseg, d_tie, d_m_aoff, d_hrank, d_hpop, d_hlist, d_seg_li, d_seg_long, d_unit0, d_fseg_off, d_sk_stage, d_heavy;
+	       d_frag_list, d_misc, d_seg_head, d_seg_start, d_seg_avg, d_replay, d_skey, d_sval, d_sseg, d_tie, d_m_aoff, d_hrank, d_hpop, d_hlist, d_seg_li, d_seg_long, d_unit0, d_fseg_off, d_sk_stage, d_heavy, d_ukey;
 	// second-pass (re-chain with max_occ) arenas
 	DevBuf d2_frag_na, d2_frag_aoff, d2_frag_rep, d2_frag_nmini, d2_mini, d2_a, d2_work, d2_u, d2_b, d2_stack, d2_frag_nu, d2_frag_nv;
 	// ksw arenas
 	DevBuf k_jobs, k_mem, k_H, k_p, k_cig, k_res, k_cig_out, k_cig_off;
 	const void *k_last_res = nullptr; // device {ez, cigar offset} array of the last ksw_launch
 	uint64_t k_last_jobs_fast = 0, k_last_cells_fast = 0, k_last_jobs_literal = 0, k_last_cells_literal = 0;
+	std::vector<uint32_t> h_k_cig_parts; // CIGARs of an mmg_ksw_batch call that ran in parts
 	// post-chaining stages on the device (mmg_post.cu): flat arrays sized by prefix sums, kept across batches
 	enum { PB_SHARD, PB_HASH, PB_SEGOFF, PB_READ_FRAG, PB_PERM, PB_CNT, PB_PRE, PB_KEY_IN, PB_VAL_IN, PB_KEY, PB_ASCNT, PB_R0, PB_W, PB_COV, PB_BIG, PB_STACK, PB_N0,
 	       PB_CAP, PB_ROFF, PB_NREG, PB_R1, PB_TMP1, PB_PLAN, PB_XSIZE, PB_XOFF, PB_SKEY, PB_SIDX, PB_SBIG, PB_SSTACK, PB_A1, PB_A1OFF, PB_JOBS, PB_CTR, PB_XW,
@@ -134,21 +137,24 @@ struct mmg_ctx_s {
 	int64_t last_tot_u = 0, last_tot_v = 0; // chains / chained anchors left on the device by the last mmg_seed_chain_resident
 	// how many work items took each data-dependent path (mmg_path_counts): [0] fragments re-chained with max_occ, [1] fragments whose
 	// heap order was replayed on ranks, [2] ... replayed literally, [3] fragments whose hit tree was built by a warp, [4] extra DP rounds
-	// after z-drop cuts, [5] hits cut at a z-drop
+	// after z-drop cuts, [5] hits cut at a z-drop, [6] seed hits whose merge order was replayed, [7] seed hits the self/dual filters dropped
 	uint64_t path[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 	PinBuf h_tab, h_tab_b, h_in_b;     // input tables of the batch being uploaded (mmg_staging_tables); second staging slot
 	PinBuf h_flip, h_flip_b;           // per-read flips of the two staging slots (mmg_staging_flips_slot)
+	PinBuf h_ukey, h_ukey_b;           // per-fragment name keys of the two staging slots (mmg_staging_name_keys_slot)
 	PinBuf h_path;                     // device counters of the pass in flight land here
 	PinBuf h_p_hash, h_p_nreg, h_p_offs, h_p_blob, h_p_rep;
 	PinBuf h_in, h_meta, h_out_meta, h_out_u, h_out_a, h_out_mini, h_k_jobs, h_k_res, h_k_cig;
 };
 
-#define MMG_LAUNCH(ctx, kern, grid, block, smem, ...) do { \
-	ProfRec pr_ = {#kern, nullptr, nullptr}; \
+#define MMG_LAUNCH(ctx, kern, grid, block, smem, ...) MMG_LAUNCH_AS(ctx, #kern, kern, grid, block, smem, __VA_ARGS__)
+// the same under a given profile name (the instantiations of one kernel template share their template's name)
+#define MMG_LAUNCH_AS(ctx, label, kern, grid, block, smem, ...) do { \
+	ProfRec pr_ = {label, nullptr, nullptr}; \
 	if ((ctx)->prof_on) { pr_.a = (ctx)->prof_event(); pr_.b = (ctx)->prof_event(); cudaEventRecord(pr_.a, (ctx)->stream); } \
 	kern<<<(grid), (block), (smem), (ctx)->stream>>>(__VA_ARGS__); ++(ctx)->launches; \
 	if ((ctx)->prof_on) { cudaEventRecord(pr_.b, (ctx)->stream); (ctx)->prof.push_back(pr_); } \
-	cudaError_t e_ = cudaGetLastError(); if (e_ != cudaSuccess) { mmg_set_error("launch %s: %s", #kern, cudaGetErrorString(e_)); return MMG_ECUDA; } } while (0)
+	cudaError_t e_ = cudaGetLastError(); if (e_ != cudaSuccess) { mmg_set_error("launch %s: %s", label, cudaGetErrorString(e_)); return MMG_ECUDA; } } while (0)
 
 // a library call (cub) on the context's stream, timed like a launch when profiling is on
 #define MMG_TIMED(ctx, label, call) do { \

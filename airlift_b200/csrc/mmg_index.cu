@@ -48,7 +48,7 @@ extern "C" void mmg_destroy(mmg_ctx_t *c)
 		&c->d_unit_off, &c->d_mv, &c->d_m_n, &c->d_m_val, &c->d_frag_unit0, &c->d_frag_qlen, &c->d_frag_na, &c->d_frag_aoff,
 		&c->d_frag_rep, &c->d_frag_nmini, &c->d_mini, &c->d_a, &c->d_work, &c->d_u, &c->d_b, &c->d_heap, &c->d_stack, &c->d_frag_nu,
 		&c->d_frag_nv, &c->d_frag_flag, &c->d_frag_iter, &c->d_cub, &c->d_out_u, &c->d_out_a, &c->d_out_mini, &c->d_uoff, &c->d_voff,
-		&c->d_moff, &c->d_frag_list, &c->d_misc, &c->d_seg_head, &c->d_seg_start, &c->d_seg_avg, &c->d_replay, &c->d_skey, &c->d_sval, &c->d_sseg, &c->d_tie, &c->d_m_aoff, &c->d_hrank, &c->d_hpop, &c->d_hlist, &c->d_seg_li, &c->d_seg_long, &c->d_unit0, &c->d_fseg_off, &c->d_sk_stage, &c->d_heavy, &c->d2_frag_na, &c->d2_frag_aoff, &c->d2_frag_rep, &c->d2_frag_nmini, &c->d2_mini,
+		&c->d_moff, &c->d_frag_list, &c->d_misc, &c->d_seg_head, &c->d_seg_start, &c->d_seg_avg, &c->d_replay, &c->d_skey, &c->d_sval, &c->d_sseg, &c->d_tie, &c->d_m_aoff, &c->d_hrank, &c->d_hpop, &c->d_hlist, &c->d_seg_li, &c->d_seg_long, &c->d_unit0, &c->d_fseg_off, &c->d_sk_stage, &c->d_heavy, &c->d_ukey, &c->d2_frag_na, &c->d2_frag_aoff, &c->d2_frag_rep, &c->d2_frag_nmini, &c->d2_mini,
 		&c->d2_a, &c->d2_work, &c->d2_u, &c->d2_b, &c->d2_stack, &c->d2_frag_nu, &c->d2_frag_nv, &c->k_jobs, &c->k_mem, &c->k_H,
 		&c->k_p, &c->k_cig, &c->k_res, &c->k_cig_out, &c->k_cig_off};
 	if (getenv("MM2_B200_TRACE"))
@@ -59,7 +59,7 @@ extern "C" void mmg_destroy(mmg_ctx_t *c)
 	for (DevBuf &b : c->pb) b.release();
 	PinBuf *pins[] = {&c->h_in, &c->h_meta, &c->h_out_meta, &c->h_out_u, &c->h_out_a, &c->h_out_mini, &c->h_k_jobs, &c->h_k_res, &c->h_k_cig,
 	                  &c->h_p_hash, &c->h_p_nreg, &c->h_p_offs, &c->h_p_blob, &c->h_p_rep, &c->h_path, &c->h_tab, &c->h_tab_b, &c->h_in_b,
-	                  &c->h_flip, &c->h_flip_b};
+	                  &c->h_flip, &c->h_flip_b, &c->h_ukey, &c->h_ukey_b};
 	for (PinBuf *b : pins) b->release();
 	if (getenv("MM2_B200_TRACE")) fprintf(stderr, "[T::buffers] released in %.3f s\n", (mmg_now_ns() - t_rel) * 1e-9);
 	for (int i = 0; i < 4; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
@@ -268,8 +268,17 @@ extern "C" void mmg_idx_free(mmg_idx_t *mi)
 {
 	if (!mi) return;
 	cudaSetDevice(mi->dev);
-	cudaFree(mi->d_S); cudaFree(mi->d_seq_off); cudaFree(mi->d_seq_len); cudaFree(mi->d_slots); cudaFree(mi->d_pos); cudaFree(mi->d_counts);
+	cudaFree(mi->d_S); cudaFree(mi->d_seq_off); cudaFree(mi->d_seq_len); cudaFree(mi->d_slots); cudaFree(mi->d_pos); cudaFree(mi->d_counts); cudaFree(mi->d_tkey);
 	delete mi;
+}
+
+extern "C" int mmg_idx_set_name_keys(mmg_idx_t *mi, const uint32_t *tkey)
+{
+	if (tkey == nullptr) { mmg_set_error("mmg_idx_set_name_keys: no key table"); return MMG_EINVAL; }
+	MMG_CUDA(cudaSetDevice(mi->dev));
+	if (mi->d_tkey == nullptr) MMG_CUDA(cudaMalloc(&mi->d_tkey, (size_t)(mi->n_seq + 1) * 4));
+	MMG_CUDA(cudaMemcpy(mi->d_tkey, tkey, (size_t)mi->n_seq * 4, cudaMemcpyHostToDevice));
+	return MMG_OK;
 }
 
 static int idx_alloc(mmg_idx_t *mi)

@@ -948,10 +948,13 @@ template <class T> static int scan_excl(mmg_ctx_t *c, const T *d_in, int64_t *d_
 	return MMG_OK;
 }
 
-// d_jobs: n jobs already on the device.  q_off/read_len/ref_off: device tables the jobs index into.
+#define KSW_SPLIT 1 // ksw_launch: the jobs' DP state exceeds the budget given; nothing was run
+
+// d_jobs: n jobs already on the device.  q_off/read_len/ref_off: device tables the jobs index into.  budget: device bytes the
+// jobs' DP state may take (0: any); above it, and with more than one job, KSW_SPLIT is returned instead.
 static int ksw_launch(mmg_ctx_t *c, const mmg_ksw_job_t *d_jobs, int n, const uint32_t *d_Q, const uint32_t *d_S, const uint64_t *d_q_off,
                       const int32_t *d_read_len, const uint64_t *d_ref_off, const KswScore &sc, mmg_ksw_res_t *res, const uint32_t **cigars,
-                      double *kernel_ms, uint64_t *cells, bool to_host = true)
+                      double *kernel_ms, uint64_t *cells, bool to_host = true, size_t budget = 0)
 {
 	// scratch layout in k_cig_off: mem_sz | p_sz | cig_sz (u64, n+1 each) | their scans (i64, n+1 each) | ncig scan (i64, n+1) | cells, class counts |
 	// key, key2 (u32) | idx, order (i32) | ncig (i32, n+1)
@@ -980,6 +983,7 @@ static int ksw_launch(mmg_ctx_t *c, const mmg_ksw_job_t *d_jobs, int n, const ui
 	MMG_D2H(c, &tot[0], mem_off + n, 8); MMG_D2H(c, &tot[1], p_off + n, 8); MMG_D2H(c, &tot[2], cg_off + n, 8);
 	MMG_D2H(c, h_cells, d_cells, sizeof(h_cells)); MMG_D2H(c, h_cls, d_cls, sizeof(h_cls));
 	MMG_CUDA(cudaStreamSynchronize(c->stream));
+	if (budget && n > 1 && (size_t)(tot[0] + tot[1] + tot[2] * 4) > budget) return KSW_SPLIT;
 	if (cells) *cells = h_cells[0];
 	c->k_last_jobs_literal = h_cls[KSW_CLS_LITERAL] + h_cls[KSW_CLS_LITERAL_WIDE] + h_cls[KSW_CLS_BLOCK1] + h_cls[KSW_CLS_BLOCK2]; // the wavefront form counts as a fast form
 	c->k_last_cells_literal = h_cells[1 + KSW_CLS_LITERAL] + h_cells[1 + KSW_CLS_LITERAL_WIDE] + h_cells[1 + KSW_CLS_BLOCK1] + h_cells[1 + KSW_CLS_BLOCK2];
@@ -1117,6 +1121,32 @@ extern "C" void mmg_ksw_last_split(const mmg_ctx_t *c, uint64_t *jobs_fast, uint
 	if (cells_literal) *cells_literal = c->k_last_cells_literal;
 }
 
+// jobs [0, n) of an mmg_ksw_batch call whose DP state does not fit at once: halves until a part fits, each part's CIGARs appended
+// to c->h_k_cig_parts (an all-vs-all round asks for hundreds of GB of traceback for 10^5 overlaps of 10 kb reads)
+static int ksw_batch_parts(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, int n, const mmg_ksw_job_t *jobs, mmg_ksw_res_t *res,
+                           size_t budget, double *kernel_ms, uint64_t *cells, uint64_t split[4])
+{
+	MMG_H2D(c, c->k_jobs.p, jobs, (size_t)n * sizeof(mmg_ksw_job_t));
+	const uint32_t *cg = nullptr;
+	double ms = 0; uint64_t cl = 0;
+	const int rc = ksw_launch(c, c->k_jobs.as<mmg_ksw_job_t>(), n, c->d_Q.as<uint32_t>(), mi->d_S, c->d_q_off.as<uint64_t>(), c->d_seq_len.as<int32_t>(),
+	                          mi->d_seq_off, make_score(opt), res, &cg, &ms, &cl, true, budget);
+	if (rc == KSW_SPLIT) {
+		const int h = n / 2;
+		MMG_TRY(ksw_batch_parts(c, mi, opt, h, jobs, res, budget, kernel_ms, cells, split));
+		return ksw_batch_parts(c, mi, opt, n - h, jobs + h, res + h, budget, kernel_ms, cells, split);
+	}
+	MMG_TRY(rc);
+	std::vector<uint32_t> &all = c->h_k_cig_parts;
+	const uint64_t base = all.size();
+	size_t n_cig = 0;
+	for (int i = 0; i < n; ++i) { n_cig += (size_t)res[i].ez.n_cigar; res[i].cigar_off += base; }
+	all.insert(all.end(), cg, cg + n_cig);
+	*kernel_ms += ms, *cells += cl;
+	split[0] += c->k_last_jobs_fast, split[1] += c->k_last_cells_fast, split[2] += c->k_last_jobs_literal, split[3] += c->k_last_cells_literal;
+	return MMG_OK;
+}
+
 extern "C" int mmg_ksw_batch(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, int n_jobs, const mmg_ksw_job_t *jobs,
                              mmg_ksw_res_t *res, const uint32_t **cigars, double *kernel_ms, uint64_t *cells)
 {
@@ -1132,8 +1162,22 @@ extern "C" int mmg_ksw_batch(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt
 		}
 	MMG_TRY(c->k_jobs.ensure((size_t)(n_jobs + 1) * sizeof(mmg_ksw_job_t)));
 	MMG_H2D(c, c->k_jobs.p, jobs, (size_t)n_jobs * sizeof(mmg_ksw_job_t));
-	return ksw_launch(c, c->k_jobs.as<mmg_ksw_job_t>(), n_jobs, c->d_Q.as<uint32_t>(), mi->d_S, c->d_q_off.as<uint64_t>(), c->d_seq_len.as<int32_t>(),
-	                  mi->d_seq_off, make_score(opt), res, cigars, kernel_ms, cells);
+	// the DP state may take a third of what the device has free (the ctx's own DP buffers count as free: they are reused)
+	size_t fr = 0, total = 0;
+	MMG_CUDA(cudaMemGetInfo(&fr, &total));
+	const size_t budget = (fr + c->k_mem.cap + c->k_p.cap + c->k_cig.cap) / 3;
+	const int rc = ksw_launch(c, c->k_jobs.as<mmg_ksw_job_t>(), n_jobs, c->d_Q.as<uint32_t>(), mi->d_S, c->d_q_off.as<uint64_t>(), c->d_seq_len.as<int32_t>(),
+	                          mi->d_seq_off, make_score(opt), res, cigars, kernel_ms, cells, true, budget);
+	if (rc != KSW_SPLIT) return rc;
+	c->h_k_cig_parts.clear();
+	double ms = 0; uint64_t cl = 0, split[4] = {0, 0, 0, 0};
+	MMG_TRY(ksw_batch_parts(c, mi, opt, n_jobs, jobs, res, budget, &ms, &cl, split));
+	c->k_last_jobs_fast = split[0], c->k_last_cells_fast = split[1], c->k_last_jobs_literal = split[2], c->k_last_cells_literal = split[3];
+	if (kernel_ms) *kernel_ms = ms;
+	if (cells) *cells = cl;
+	c->h_k_cig_parts.push_back(0);
+	*cigars = c->h_k_cig_parts.data();
+	return MMG_OK;
 }
 
 // single pair, sequences given as 0..4 codes (parity-test entry point for ksw_extd2_sse, ksw2.h:60)

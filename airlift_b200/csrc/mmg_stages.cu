@@ -57,6 +57,17 @@ struct FragTab {  // per-fragment tables of the resident batch
 	const int32_t *qlen;       // [n_frag] summed segment lengths
 };
 
+struct NameTabs {  // the self/dual filters' name keys (include/mmg.h): per target of the index, per fragment of the resident batch
+	const uint32_t *tkey, *tlen, *ukey;  // ukey null: the filters are off
+};
+
+__device__ __forceinline__ NameFilt name_filt(const NameTabs &nt, int f)
+{
+	NameFilt n;
+	n.tkey = nt.tkey, n.tlen = nt.tlen, n.ukey = nt.ukey ? nt.ukey[f] : MMG_NAME_NONE;
+	return n;
+}
+
 __device__ __forceinline__ int frag_of_anchor(const int64_t *aoff, int n_list, int64_t g)
 { // last li with aoff[li] <= g
 	int lo = 0, hi = n_list - 1;
@@ -106,10 +117,12 @@ __global__ void k_plan(FragTab ft, const int32_t *__restrict__ list, int n_list,
 
 // K2c, sort form (fragments without repeated hashes): every planned anchor slot finds its (minimizer, hit), and emits the
 // heap's pop key (strand class, reference position incl. strand bit) with the anchor's y as payload
+template <bool kNamed>
 __global__ void k_expand(FragTab ft, const int32_t *__restrict__ list, int n_list, const mm128 *__restrict__ mv, const int32_t *__restrict__ m_n,
                          const uint64_t *__restrict__ m_val, const uint64_t *__restrict__ pos, int max_occ, int64_t flag,
                          const int64_t *__restrict__ aoff, const uint8_t *__restrict__ replay, int64_t n_total,
-                         uint64_t *__restrict__ key, uint64_t *__restrict__ val, int32_t *__restrict__ n_skipped, const int32_t *__restrict__ m_aoff)
+                         uint64_t *__restrict__ key, uint64_t *__restrict__ val, int32_t *__restrict__ n_skipped, const int32_t *__restrict__ m_aoff,
+                         NameTabs nt, unsigned long long *__restrict__ n_named)
 {
 	const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if (g >= n_total) return;
@@ -128,10 +141,16 @@ __global__ void k_expand(FragTab ft, const int32_t *__restrict__ list, int n_lis
 	const mm128 mz = mv[b + m];
 	const uint64_t r = mmg_hit_pos(pos, m_n[b + m], m_val[b + m], (uint32_t)i);
 	if (replay[li] == 1) { key[g] = r, val[g] = (uint64_t)(g - aoff[li]); return; } // heap replay: ordered by position alone, the planned slot as payload
-	if (mmg_skip_seed(flag, r, (uint32_t)mz.y)) { key[g] = MMG_NONE, val[g] = 0; atomicAdd(&n_skipped[li], 1); return; }
-	const mm128 an = mmg_make_anchor(r, mz, mmg_is_tandem(mv + b, (int)(e - b), m), ft.qlen[f]);
+	bool self;
+	const int sk = mmg_skip_seed(MMG_NAMED_FLAG(kNamed, flag), r, (uint32_t)mz.y, name_filt(nt, f), kNamed ? ft.qlen[f] : 0, &self);
+	if (sk != MMG_SKIP_KEEP) {
+		key[g] = MMG_NONE, val[g] = 0; atomicAdd(&n_skipped[li], 1);
+		if (kNamed && sk == MMG_SKIP_NAME) atomicAdd(n_named, 1ULL);
+		return;
+	}
+	const mm128 an = mmg_make_anchor(r, mz, mmg_is_tandem(mv + b, (int)(e - b), m), self, ft.qlen[f]);
 	key[g] = (an.x & (1ULL << 63)) | r; // r < 2^63
-	val[g] = an.y;
+	val[g] = an.y; // the self bit rides here
 }
 
 __global__ void k_sort_segments(int n_list, const int64_t *__restrict__ aoff, const uint8_t *__restrict__ replay, int64_t *__restrict__ seg_b, int64_t *__restrict__ seg_e)
@@ -428,10 +447,12 @@ __device__ __forceinline__ int block_excl_scan(int v, int *s_w, int *total)
 // pop order (map.c:176-211).  (One warp did this after its replay: 2 x 5 000 rounds of dependent global loads for a fragment
 // with 1.6 x 10^5 hits, as long as the replay itself.)
 #define HEAP_EMIT_THREADS 512
+template <bool kNamed>
 __global__ void __launch_bounds__(HEAP_EMIT_THREADS)
 k_heap_emit(FragTab ft, const int32_t *__restrict__ list, const int32_t *__restrict__ rlist, const mm128 *__restrict__ mv, const int32_t *__restrict__ m_n,
             const uint64_t *__restrict__ m_val, const int32_t *__restrict__ m_aoff, const uint64_t *__restrict__ pos, int max_occ, int64_t flag,
-            const int64_t *__restrict__ aoff, uint32_t *__restrict__ P, int32_t *__restrict__ na, mm128 *__restrict__ a, unsigned long long *__restrict__ n_pops)
+            const int64_t *__restrict__ aoff, uint32_t *__restrict__ P, int32_t *__restrict__ na, mm128 *__restrict__ a, unsigned long long *__restrict__ n_pops,
+            NameTabs nt, unsigned long long *__restrict__ n_named)
 {
 	__shared__ int32_t s_first[HEAP_MAX_LISTS], s_m[HEAP_MAX_LISTS], s_w[32], s_tot[3];
 	const int tid = threadIdx.x, lane = tid & 31, NT = blockDim.x;
@@ -439,6 +460,7 @@ k_heap_emit(FragTab ft, const int32_t *__restrict__ list, const int32_t *__restr
 	const int li = rlist[blockIdx.x], f = list ? list[li] : li;
 	const int64_t b = ft.unit_off[ft.unit0[f]], e = ft.unit_off[ft.unit0[f + 1]], ao = aoff[li];
 	const int n_mv = (int)(e - b), qlen = ft.qlen[f];
+	const NameFilt nfl = name_filt(nt, f);
 	if (tid < 32) { // the kept minimizers, in query order (as in k_heap_replay)
 		int n_lists = 0, n_a = 0;
 		for (int i0 = 0; i0 < n_mv; i0 += 32) {
@@ -454,7 +476,7 @@ k_heap_emit(FragTab ft, const int32_t *__restrict__ list, const int32_t *__restr
 	__syncthreads();
 	const int n_lists = s_tot[0], n_a = s_tot[2];
 	// pass 1: strand class of every pop (kept in the two top bits of its word), number of forward-strand hits
-	int my_for = 0;
+	int my_for = 0, my_named = 0;
 	for (int tt = tid; tt < n_a; tt += NT) {
 		const uint32_t slot = P[ao + tt];
 		int lo = 0, hi = n_lists - 1; // list of the slot
@@ -462,12 +484,18 @@ k_heap_emit(FragTab ft, const int32_t *__restrict__ list, const int32_t *__restr
 		const int m = s_m[lo];
 		const uint64_t r = mmg_hit_pos(pos, m_n[b + m], m_val[b + m], slot - (uint32_t)s_first[lo]);
 		const uint32_t qp = (uint32_t)mv[b + m].y;
-		const int cls = mmg_skip_seed(flag, r, qp) ? 0 : ((r & 1) == (qp & 1) ? 1 : 2);
+		bool self;
+		const int sk = mmg_skip_seed(MMG_NAMED_FLAG(kNamed, flag), r, qp, nfl, qlen, &self);
+		const int cls = sk != MMG_SKIP_KEEP ? 0 : ((r & 1) == (qp & 1) ? 1 : 2);
 		P[ao + tt] = slot | (uint32_t)cls << 30;
-		my_for += cls == 1;
+		my_for += cls == 1, my_named += sk == MMG_SKIP_NAME;
 	}
 	my_for = __reduce_add_sync(FULL, my_for);
 	if (lane == 0 && my_for) atomicAdd(&s_tot[1], my_for);
+	if (kNamed) {
+		my_named = __reduce_add_sync(FULL, my_named);
+		if (lane == 0 && my_named) atomicAdd(n_named, (unsigned long long)my_named);
+	}
 	__syncthreads();
 	const int n_for = s_tot[1];
 	// pass 2: anchors; forward hits in the low half of the packed scan value, reverse hits in the high half
@@ -483,7 +511,9 @@ k_heap_emit(FragTab ft, const int32_t *__restrict__ list, const int32_t *__restr
 			while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if ((uint32_t)s_first[mid] <= slot) lo = mid; else hi = mid - 1; }
 			const int m = s_m[lo];
 			const uint64_t r = mmg_hit_pos(pos, m_n[b + m], m_val[b + m], slot - (uint32_t)s_first[lo]);
-			const mm128 an = mmg_make_anchor(r, mv[b + m], mmg_is_tandem(mv + b, n_mv, m), qlen);
+			bool self;
+			mmg_skip_seed(MMG_NAMED_FLAG(kNamed, flag), r, (uint32_t)mv[b + m].y, nfl, qlen, &self); // kept (pass 1); asked again for the self bit
+			const mm128 an = mmg_make_anchor(r, mv[b + m], mmg_is_tandem(mv + b, n_mv, m), self, qlen);
 			if (cls == 1) a[ao + run_for + (ex & 0xffff)] = an;
 			else a[ao + n_for + run_rev + (ex >> 16)] = an;
 		}
@@ -495,11 +525,13 @@ k_heap_emit(FragTab ft, const int32_t *__restrict__ list, const int32_t *__restr
 // mmg_fill_heap (mmg_core.h) for one fragment per warp: same pops in the same order; the heap and the next position of every
 // list live in shared memory, and the position after that is fetched while the heap is sifted, so that the L2 latency of the
 // position arrays is off the critical path of the serial replay (a repeat-family fragment makes ~2 x 10^5 pops).
+template <bool kNamed>
 __device__ int64_t fill_heap_prefetch(const mm128 *mv, const int32_t *m_n, const uint64_t *m_val, int n_mv, int max_occ, const uint64_t *pos,
-                                      int64_t flag, int qlen, int64_t n_a_planned, mm128 *heap, uint64_t *nxt, mm128 *a)
+                                      int64_t flag, const NameFilt &nf, int qlen, int64_t n_a_planned, mm128 *heap, uint64_t *nxt, mm128 *a,
+                                      int64_t *n_named)
 {
 	size_t hs = 0;
-	int64_t n_for = 0, n_rev = 0, n_a = n_a_planned;
+	int64_t n_for = 0, n_rev = 0, n_a = n_a_planned, n_nm = 0;
 	for (int i = 0; i < n_mv; ++i)
 		if (m_n[i] > 0 && m_n[i] < max_occ) {
 			heap[hs].x = mmg_hit_pos(pos, m_n[i], m_val[i], 0);
@@ -520,11 +552,13 @@ __device__ int64_t fill_heap_prefetch(const mm128 *mv, const int32_t *m_n, const
 		if (more) { ++heap[0].y; heap[0].x = nxt[i]; }
 		else { heap[0] = heap[hs - 1]; --hs; }
 		if (hs > 0) mmg_heap_down(0, hs, heap);
-		if (!mmg_skip_seed(flag, r, (uint32_t)mz.y)) {
-			const mm128 an = mmg_make_anchor(r, mz, mmg_is_tandem(mv, n_mv, i), qlen);
+		bool self;
+		const int sk = mmg_skip_seed(MMG_NAMED_FLAG(kNamed, flag), r, (uint32_t)mz.y, nf, qlen, &self);
+		if (sk == MMG_SKIP_KEEP) {
+			const mm128 an = mmg_make_anchor(r, mz, mmg_is_tandem(mv, n_mv, i), self, qlen);
 			if ((r & 1) == ((uint32_t)mz.y & 1)) a[n_for++] = an;
 			else a[n_a - (++n_rev)] = an;
-		}
+		} else n_nm += sk == MMG_SKIP_NAME;
 		if (more) nxt[i] = pending;
 	}
 	for (int64_t j = 0; j < n_rev >> 1; ++j) { // map.c:203-207
@@ -532,18 +566,21 @@ __device__ int64_t fill_heap_prefetch(const mm128 *mv, const int32_t *m_n, const
 		a[n_a - 1 - j] = a[n_a - (n_rev - j)];
 		a[n_a - (n_rev - j)] = t;
 	}
-	if (n_a > n_for + n_rev) { // map.c:208-211 (only with strand filters)
+	if (n_a > n_for + n_rev) { // map.c:208-211 (only with strand or self/dual filters)
 		for (int64_t j = 0; j < n_rev; ++j) a[n_for + j] = a[n_a - n_rev + j];
 		n_a = n_for + n_rev;
 	}
+	*n_named = n_nm;
 	return n_a;
 }
 
 // K2c: anchors per fragment, in the reference's order (map.c:149-247)
+template <bool kNamed>
 __global__ void k_fill(FragTab ft, const int32_t *__restrict__ list, int n_list, const mm128 *__restrict__ mv, const int32_t *__restrict__ m_n,
                        const uint64_t *__restrict__ m_val, const uint64_t *__restrict__ pos, int max_occ, int64_t flag,
                        const int64_t *__restrict__ aoff, int32_t *__restrict__ na, mm128 *__restrict__ a, mm128 *__restrict__ heap, RsFrame *__restrict__ stack,
-                       const uint8_t *__restrict__ replay /* null: every fragment */, int want /* value of replay[] that selects a fragment */, int per_warp)
+                       const uint8_t *__restrict__ replay /* null: every fragment */, int want /* value of replay[] that selects a fragment */, int per_warp,
+                       NameTabs nt, unsigned long long *__restrict__ n_named)
 {
 	// per_warp: one fragment per warp (lane 0 works).  The re-chain pass lists a few hundred fragments of ~10^5 anchors each; as
 	// neighbouring threads of one warp their serial replays diverged and ran one after the other (36 ms for 192 fragments)
@@ -553,17 +590,19 @@ __global__ void k_fill(FragTab ft, const int32_t *__restrict__ list, int n_list,
 	const int f = list ? list[li] : li;
 	const int64_t b = ft.unit_off[ft.unit0[f]], e = ft.unit_off[ft.unit0[f + 1]];
 	const int64_t ao = aoff[li];
-	int64_t n;
+	const NameFilt nf = name_filt(nt, f);
+	int64_t n, nn;
 	if (flag & MMG_F_HEAP_SORT) {
 		__shared__ mm128 s_heap[2][128];
 		__shared__ uint64_t s_nxt[2][128];
 		if (per_warp && e - b <= 128)
-			n = fill_heap_prefetch(mv + b, m_n + b, m_val + b, (int)(e - b), max_occ, pos, flag, ft.qlen[f], na[li], s_heap[threadIdx.x >> 5], s_nxt[threadIdx.x >> 5], a + ao);
-		else n = mmg_fill_heap(mv + b, m_n + b, m_val + b, (int)(e - b), max_occ, pos, flag, ft.qlen[f], na[li], heap + b, a + ao);
+			n = fill_heap_prefetch<kNamed>(mv + b, m_n + b, m_val + b, (int)(e - b), max_occ, pos, flag, nf, ft.qlen[f], na[li], s_heap[threadIdx.x >> 5], s_nxt[threadIdx.x >> 5], a + ao, &nn);
+		else n = mmg_fill_heap<kNamed>(mv + b, m_n + b, m_val + b, (int)(e - b), max_occ, pos, flag, nf, ft.qlen[f], na[li], heap + b, a + ao, &nn);
 	}
 	else
-		n = mmg_fill_flat(mv + b, m_n + b, m_val + b, (int)(e - b), max_occ, pos, flag, ft.qlen[f], a + ao, stack + ao / 65 + 2 * (int64_t)li);
+		n = mmg_fill_flat<kNamed>(mv + b, m_n + b, m_val + b, (int)(e - b), max_occ, pos, flag, nf, ft.qlen[f], a + ao, stack + ao / 65 + 2 * (int64_t)li, &nn);
 	na[li] = (int32_t)n;
+	if (kNamed && nn) atomicAdd(n_named, (unsigned long long)nn);
 }
 
 struct ChainOptDev { int32_t bw, max_gap, max_gap_ref, max_frag_len, max_skip, max_iter, min_cnt, min_sc, is_cdna, is_sr; };
@@ -1460,6 +1499,35 @@ extern "C" int mmg_staging_flips_slot(mmg_ctx_t *c, int slot, int n_seq, uint8_t
 
 static int batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t *b, const uint8_t *flip_in);
 
+extern "C" int mmg_staging_name_keys_slot(mmg_ctx_t *c, int slot, int n_frag, uint32_t **ukey)
+{
+	cudaSetDevice(c->dev);
+	PinBuf &k = slot ? c->h_ukey_b : c->h_ukey;
+	MMG_TRY(k.ensure(((size_t)n_frag + 4) * 4));
+	if (c->h_ukey_b.p || slot) MMG_TRY((slot ? c->h_ukey : c->h_ukey_b).ensure(((size_t)n_frag + 4) * 4)); // both slots grow together, as the tables do
+	*ukey = k.as<uint32_t>();
+	return MMG_OK;
+}
+
+extern "C" int mmg_batch_set_name_keys(mmg_ctx_t *c, int n_frag, const uint32_t *ukey)
+{
+	if (ukey == nullptr || n_frag != c->rb.n_frag) {
+		mmg_set_error("mmg_batch_set_name_keys: %d keys for a resident batch of %d fragments", ukey ? n_frag : 0, c->rb.n_frag);
+		return MMG_EINVAL;
+	}
+	MMG_CUDA(cudaSetDevice(c->dev));
+	const uint32_t *src = ukey;
+	if (src != c->h_ukey.as<uint32_t>() && src != c->h_ukey_b.as<uint32_t>()) { // from pinned memory, like the tables
+		MMG_TRY(c->h_ukey.ensure(((size_t)n_frag + 4) * 4));
+		memcpy(c->h_ukey.p, ukey, (size_t)n_frag * 4);
+		src = c->h_ukey.as<uint32_t>();
+	}
+	MMG_TRY(c->d_ukey.ensure(((size_t)n_frag + 4) * 4));
+	if (n_frag > 0) MMG_H2D(c, c->d_ukey.p, src, (size_t)n_frag * 4);
+	c->rb.n_ukey = n_frag;
+	return MMG_OK;
+}
+
 extern "C" int mmg_batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t *b) { return batch_upload(c, opt, b, nullptr); }
 
 extern "C" int mmg_batch_upload_flips(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t *b, const uint8_t *flip)
@@ -1485,6 +1553,7 @@ static int batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t
 	MMG_H2D(c, c->d_ascii.p, src_bases, b->n_bases);
 	const int n_seq = b->n_seq, n_frag = b->n_frag;
 	rb.n_frag = n_frag, rb.n_seq = n_seq, rb.n_bases = b->n_bases;
+	rb.n_ukey = -1; // name keys belong to one batch
 	rb.n_seg.assign(b->n_seg, b->n_seg + n_frag);
 	rb.seg_off.assign(b->seg_off, b->seg_off + n_frag);
 	rb.seq_len.assign(b->seq_len, b->seq_len + n_seq);
@@ -1558,9 +1627,11 @@ struct PassBufs {
 };
 
 // plan -> scan -> fill -> chain for the fragments in `list` (null = all) with cut-off max_occ
-static int run_pass(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, const FragTab &ft, const int32_t *d_list, int n_list,
+static int run_pass(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, const FragTab &ft, const NameTabs &nt, const int32_t *d_list, int n_list,
                     int64_t n_mv, int max_occ, const PassBufs &pb, bool want_mini, uint8_t *d_flag, int64_t *n_anchors)
 {
+	unsigned long long *n_named = c->d_frag_iter.as<unsigned long long>() + 2;
+	const bool named = nt.ukey != nullptr;
 	*n_anchors = 0;
 	if (n_list == 0) return MMG_OK;
 	MMG_TRY(pb.na->ensure((size_t)(n_list + 1) * 4));
@@ -1614,8 +1685,9 @@ static int run_pass(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, 
 		int64_t *seg_b = c->d_sseg.as<int64_t>(), *seg_e = seg_b + n_list + 1;
 		int32_t *n_skipped = reinterpret_cast<int32_t*>(seg_e + n_list + 1);
 		MMG_CUDA(cudaMemsetAsync(n_skipped, 0, (size_t)n_list * 4, c->stream));
-		MMG_LAUNCH(c, k_expand, mmg_blocks(tot, 256), 256, 0, ft, d_list, n_list, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(), c->d_m_val.as<uint64_t>(),
-		           mi->d_pos, max_occ, opt->flag, pb.aoff->as<int64_t>(), c->d_replay.as<uint8_t>(), tot, k0, v0, n_skipped, c->d_m_aoff.as<int32_t>());
+		MMG_LAUNCH_AS(c, "k_expand", (named ? k_expand<true> : k_expand<false>), mmg_blocks(tot, 256), 256, 0, ft, d_list, n_list, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(), c->d_m_val.as<uint64_t>(),
+		           mi->d_pos, max_occ, opt->flag, pb.aoff->as<int64_t>(), c->d_replay.as<uint8_t>(), tot, k0, v0, n_skipped, c->d_m_aoff.as<int32_t>(),
+			           nt, n_named);
 		MMG_LAUNCH(c, k_sort_segments, mmg_blocks(n_list, 256), 256, 0, n_list, pb.aoff->as<int64_t>(), c->d_replay.as<uint8_t>(), seg_b, seg_e);
 		{
 			size_t tmp = 0;
@@ -1635,9 +1707,9 @@ static int run_pass(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, 
 			MMG_LAUNCH(c, k_heap_rank, mmg_blocks(tot, 256), 256, 0, n_list, pb.aoff->as<int64_t>(), c->d_replay.as<uint8_t>(), tot, k1, v1, c->d_hrank.as<uint32_t>());
 			MMG_LAUNCH(c, k_heap_replay, hp[0] < 148 * 8 ? hp[0] : 148 * 8, 32, 0, ft, d_list, rlist, counters, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(), c->d_m_val.as<uint64_t>(),
 			           c->d_m_aoff.as<int32_t>(), mi->d_pos, max_occ, opt->flag, pb.aoff->as<int64_t>(), c->d_hrank.as<uint32_t>(), c->d_hpop.as<uint32_t>());
-			MMG_LAUNCH(c, k_heap_emit, hp[0], HEAP_EMIT_THREADS, 0, ft, d_list, rlist, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(), c->d_m_val.as<uint64_t>(),
+			MMG_LAUNCH_AS(c, "k_heap_emit", (named ? k_heap_emit<true> : k_heap_emit<false>), hp[0], HEAP_EMIT_THREADS, 0, ft, d_list, rlist, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(), c->d_m_val.as<uint64_t>(),
 			           c->d_m_aoff.as<int32_t>(), mi->d_pos, max_occ, opt->flag, pb.aoff->as<int64_t>(), c->d_hpop.as<uint32_t>(), pb.na->as<int32_t>(), pb.a->as<mm128>(),
-			           c->d_frag_iter.as<unsigned long long>() + 1);
+			           c->d_frag_iter.as<unsigned long long>() + 1, nt, n_named);
 		}
 	}
 	// literal replay: the heap merge for the few fragments the rank replay does not take; fill + klib radix sort for the non-heap presets
@@ -1647,9 +1719,9 @@ static int run_pass(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, 
 			           c->d_sval.as<uint64_t>(), pb.na->as<int32_t>(), pb.a->as<mm128>(), pb.work->as<int32_t>(), pb.stack->as<RsFrame>());
 	} else {
 		const int per_warp = d_flag == nullptr || n_list <= 4096 ? 1 : 0; // the re-chain pass (and any small list): spread over warps
-		MMG_LAUNCH(c, k_fill, mmg_blocks(per_warp ? (size_t)n_list * 32 : (size_t)n_list, 64), 64, 0, ft, d_list, n_list, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(),
+		MMG_LAUNCH_AS(c, "k_fill", (named ? k_fill<true> : k_fill<false>), mmg_blocks(per_warp ? (size_t)n_list * 32 : (size_t)n_list, 64), 64, 0, ft, d_list, n_list, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(),
 		           c->d_m_val.as<uint64_t>(), mi->d_pos, max_occ, opt->flag, pb.aoff->as<int64_t>(), pb.na->as<int32_t>(), pb.a->as<mm128>(), c->d_heap.as<mm128>(),
-		           pb.stack->as<RsFrame>(), heap_path ? c->d_replay.as<uint8_t>() : d_tie, heap_path ? 2 : 1, per_warp);
+		           pb.stack->as<RsFrame>(), heap_path ? c->d_replay.as<uint8_t>() : d_tie, heap_path ? 2 : 1, per_warp, nt, n_named);
 	}
 	if (getenv("MMG_TRACE")) { // distribution of the literal-replay work of this pass (debug aid; synchronises)
 		std::vector<uint8_t> hr((size_t)n_list); std::vector<int32_t> hn((size_t)n_list);
@@ -1751,6 +1823,12 @@ extern "C" int mmg_seed_chain_resident(mmg_ctx_t *c, const mmg_idx_t *mi, const 
 	out->n_frag = nf;
 	if (nf == 0) return MMG_OK;
 	if (mi->w > MMG_MAX_W) { mmg_set_error("w=%d exceeds the device limit %d", mi->w, MMG_MAX_W); return MMG_ELIMIT; }
+	NameTabs nt = {nullptr, nullptr, nullptr};
+	if (opt->flag & (MMG_F_NO_DIAG | MMG_F_NO_DUAL)) { // never filter on keys of another index or batch
+		if (mi->d_tkey == nullptr) { mmg_set_error("the self/dual filters need the target name keys (mmg_idx_set_name_keys)"); return MMG_EINVAL; }
+		if (rb.n_ukey != nf) { mmg_set_error("the self/dual filters need the name keys of this batch (mmg_batch_set_name_keys)"); return MMG_EINVAL; }
+		nt.tkey = mi->d_tkey, nt.tlen = mi->d_seq_len, nt.ukey = c->d_ukey.as<uint32_t>();
+	}
 	MMG_CUDA(cudaEventRecord(c->ev[0], c->stream));
 	// K1
 	int64_t n_mv = 0;
@@ -1765,15 +1843,15 @@ extern "C" int mmg_seed_chain_resident(mmg_ctx_t *c, const mmg_idx_t *mi, const 
 	ft.unit0 = c->d_frag_unit0.as<int32_t>(), ft.unit_off = c->d_unit_off.as<int64_t>(), ft.qlen = c->d_frag_qlen.as<int32_t>();
 	const bool want_mini = !(opt->flag & MMG_F_SR); // only mm_est_err reads mini_pos (map.c:388)
 	MMG_TRY(c->d_frag_flag.ensure((size_t)nf + 16));
-	MMG_TRY(c->d_frag_iter.ensure(16));
+	MMG_TRY(c->d_frag_iter.ensure(32)); // chain iterations | replayed merge pops | hits the self/dual filters dropped
 	MMG_CUDA(cudaMemsetAsync(c->d_frag_flag.p, 0, (size_t)nf + 16, c->stream));
-	MMG_CUDA(cudaMemsetAsync(c->d_frag_iter.p, 0, 16, c->stream));
+	MMG_CUDA(cudaMemsetAsync(c->d_frag_iter.p, 0, 32, c->stream));
 	MMG_TRY(c->h_path.ensure(64));
 	memset(c->h_path.p, 0, 64);
 	PassBufs p1 = {&c->d_frag_na, &c->d_frag_aoff, &c->d_frag_rep, &c->d_frag_nmini, &c->d_mini, &c->d_a, &c->d_work, &c->d_u, &c->d_b,
 	               &c->d_stack, &c->d_frag_nu, &c->d_frag_nv};
 	int64_t n_anch1 = 0, n_anch2 = 0;
-	MMG_TRY(run_pass(c, mi, opt, ft, nullptr, nf, n_mv, opt->mid_occ, p1, want_mini, c->d_frag_flag.as<uint8_t>(), &n_anch1));
+	MMG_TRY(run_pass(c, mi, opt, ft, nt, nullptr, nf, n_mv, opt->mid_occ, p1, want_mini, c->d_frag_flag.as<uint8_t>(), &n_anch1));
 	// second pass: fragments whose best chain misses a segment, with the higher cut-off (map.c:353-375)
 	std::vector<int32_t> list;
 	std::vector<uint8_t> hflag(nf);
@@ -1790,7 +1868,7 @@ extern "C" int mmg_seed_chain_resident(mmg_ctx_t *c, const mmg_idx_t *mi, const 
 	const int n2 = (int)list.size();
 	if (n2) {
 		MMG_H2D(c, d_list, list.data(), (size_t)n2 * 4);
-		MMG_TRY(run_pass(c, mi, opt, ft, d_list, n2, n_mv, opt->max_occ, p2, want_mini, nullptr, &n_anch2));
+		MMG_TRY(run_pass(c, mi, opt, ft, nt, d_list, n2, n_mv, opt->max_occ, p2, want_mini, nullptr, &n_anch2));
 		MMG_LAUNCH(c, k_merge_pass2, mmg_blocks(n2, 128), 128, 0, n2, d_list, c->d2_frag_nu.as<int32_t>(), c->d2_frag_nv.as<int32_t>(),
 		           c->d2_frag_rep.as<int32_t>(), c->d2_frag_nmini.as<int32_t>(), c->d_frag_nu.as<int32_t>(), c->d_frag_nv.as<int32_t>(),
 		           c->d_frag_rep.as<int32_t>(), c->d_frag_nmini.as<int32_t>(), d_src);
@@ -1820,7 +1898,7 @@ extern "C" int mmg_seed_chain_resident(mmg_ctx_t *c, const mmg_idx_t *mi, const 
 	MMG_CUDA(cudaEventRecord(c->ev[1], c->stream));
 	unsigned long long iters = 0;
 	MMG_D2H(c, &iters, c->d_frag_iter.p, 8);
-	MMG_D2H(c, c->h_path.as<unsigned long long>() + 5, c->d_frag_iter.as<unsigned long long>() + 1, 8); // hits whose merge order was replayed
+	MMG_D2H(c, c->h_path.as<unsigned long long>() + 5, c->d_frag_iter.as<unsigned long long>() + 1, 16); // hits whose merge order was replayed, hits dropped by name
 	out->n_minimizers = (uint64_t)n_mv, out->n_anchors = (uint64_t)(n_anch1 + n_anch2);
 	if (download) {
 		// meta: n_u | n_a | rep_len | n_mini | rechained (int32 each) then u_off | a_off | mini_off (uint64 each, nf+1)
@@ -1855,7 +1933,7 @@ extern "C" int mmg_seed_chain_resident(mmg_ctx_t *c, const mmg_idx_t *mi, const 
 	{ // path counters of this batch (the stream is idle here)
 		const int32_t *hp = c->h_path.as<int32_t>();
 		c->path[0] += (uint64_t)n2, c->path[1] += (uint64_t)(hp[0] + hp[4]), c->path[2] += (uint64_t)(hp[2] + hp[6]);
-		c->path[6] += c->h_path.as<unsigned long long>()[5];
+		c->path[6] += c->h_path.as<unsigned long long>()[5], c->path[7] += c->h_path.as<unsigned long long>()[6];
 	}
 	float ms = 0;
 	cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]); out->t_kernels_ms = ms;
@@ -1904,7 +1982,7 @@ extern "C" int mmg_sketch(mmg_ctx_t *c, const char *str, int len, int w, int k, 
 	return MMG_OK;
 }
 
-__global__ void k_collect_one(IdxView ix, const mm128 *mv, int n_mv, int heap_sort, int64_t flag, int max_occ, int qlen,
+__global__ void k_collect_one(IdxView ix, const mm128 *mv, int n_mv, int heap_sort, int64_t flag, int max_occ, int qlen, uint32_t ukey,
                               int32_t *m_n, uint64_t *m_val, mm128 *heap, mm128 *a, int64_t a_cap, RsFrame *stack, int64_t *out4, uint64_t *mini)
 {
 	if (blockIdx.x || threadIdx.x) return;
@@ -1913,13 +1991,35 @@ __global__ void k_collect_one(IdxView ix, const mm128 *mv, int n_mv, int heap_so
 	int64_t n_a = mmg_frag_plan(mv, m_n, n_mv, max_occ, &rep, &nm, mini);
 	out4[0] = n_a, out4[1] = rep, out4[2] = nm;
 	if (n_a > a_cap) return;
-	if (heap_sort) n_a = mmg_fill_heap(mv, m_n, m_val, n_mv, max_occ, ix.pos, flag, qlen, n_a, heap, a);
-	else n_a = mmg_fill_flat(mv, m_n, m_val, n_mv, max_occ, ix.pos, flag, qlen, a, stack);
+	NameFilt nf; nf.tkey = ix.tkey, nf.tlen = ix.seq_len, nf.ukey = ukey;
+	int64_t nn;
+	if (heap_sort) n_a = mmg_fill_heap(mv, m_n, m_val, n_mv, max_occ, ix.pos, flag, nf, qlen, n_a, heap, a, &nn);
+	else n_a = mmg_fill_flat(mv, m_n, m_val, n_mv, max_occ, ix.pos, flag, nf, qlen, a, stack, &nn);
 	out4[0] = n_a;
 }
 
+static int collect_seeds(mmg_ctx_t *c, const mmg_idx_t *mi, int heap_sort, int64_t flag, int max_occ, int n_mv, const mmg128_t *mv,
+                         int qlen, uint32_t ukey, mmg128_t *a_out, int64_t a_cap, int64_t *n_a, int *rep_len, int *n_mini_pos, uint64_t *mini_pos);
+
 extern "C" int mmg_collect_seeds(mmg_ctx_t *c, const mmg_idx_t *mi, int heap_sort, int64_t flag, int max_occ, int n_mv, const mmg128_t *mv,
                                  int qlen, mmg128_t *a_out, int64_t a_cap, int64_t *n_a, int *rep_len, int *n_mini_pos, uint64_t *mini_pos)
+{
+	return collect_seeds(c, mi, heap_sort, flag, max_occ, n_mv, mv, qlen, MMG_NAME_NONE, a_out, a_cap, n_a, rep_len, n_mini_pos, mini_pos);
+}
+
+extern "C" int mmg_collect_seeds_named(mmg_ctx_t *c, const mmg_idx_t *mi, int heap_sort, int64_t flag, int max_occ, int n_mv, const mmg128_t *mv,
+                                       int qlen, uint32_t ukey, mmg128_t *a_out, int64_t a_cap, int64_t *n_a, int *rep_len, int *n_mini_pos,
+                                       uint64_t *mini_pos)
+{
+	if ((flag & (MMG_F_NO_DIAG | MMG_F_NO_DUAL)) && ukey != MMG_NAME_NONE && mi->d_tkey == nullptr) {
+		mmg_set_error("mmg_collect_seeds_named: the index has no name keys (mmg_idx_set_name_keys)");
+		return MMG_EINVAL;
+	}
+	return collect_seeds(c, mi, heap_sort, flag, max_occ, n_mv, mv, qlen, ukey, a_out, a_cap, n_a, rep_len, n_mini_pos, mini_pos);
+}
+
+static int collect_seeds(mmg_ctx_t *c, const mmg_idx_t *mi, int heap_sort, int64_t flag, int max_occ, int n_mv, const mmg128_t *mv,
+                         int qlen, uint32_t ukey, mmg128_t *a_out, int64_t a_cap, int64_t *n_a, int *rep_len, int *n_mini_pos, uint64_t *mini_pos)
 {
 	MMG_CUDA(cudaSetDevice(c->dev));
 	DevBuf dmv, dn, dval, dheap, da, dstack, dout, dmini;
@@ -1930,7 +2030,7 @@ extern "C" int mmg_collect_seeds(mmg_ctx_t *c, const mmg_idx_t *mi, int heap_sor
 	CS_TRY(dheap.ensure((size_t)(n_mv + 1) * 16)); CS_TRY(da.ensure((size_t)(a_cap + 1) * 16)); CS_TRY(dstack.ensure((size_t)(a_cap / 65 + 4) * sizeof(RsFrame)));
 	CS_TRY(dout.ensure(64)); CS_TRY(dmini.ensure((size_t)(n_mv + 1) * 8));
 	if (n_mv) cudaMemcpyAsync(dmv.p, mv, (size_t)n_mv * 16, cudaMemcpyHostToDevice, c->stream);
-	k_collect_one<<<1, 32, 0, c->stream>>>(mi->view(), dmv.as<mm128>(), n_mv, heap_sort, flag, max_occ, qlen, dn.as<int32_t>(), dval.as<uint64_t>(),
+	k_collect_one<<<1, 32, 0, c->stream>>>(mi->view(), dmv.as<mm128>(), n_mv, heap_sort, flag, max_occ, qlen, ukey, dn.as<int32_t>(), dval.as<uint64_t>(),
 	                                      dheap.as<mm128>(), da.as<mm128>(), a_cap, dstack.as<RsFrame>(), dout.as<int64_t>(), dmini.as<uint64_t>());
 	++c->launches;
 	int64_t o4[4] = {0, 0, 0, 0};

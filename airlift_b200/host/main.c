@@ -273,7 +273,7 @@ int main(int argc, char *argv[])
 		fprintf(stderr, "[ERROR] incorrect input: in the sr mode, please specify no more than two query files.\n");
 		return 1;
 	}
-	if (mm_b200_check_opt(&opt) < 0) return 1; /* splice, -D/-X/--dual=no, -T, --split-prefix: refused, not ignored */
+	if (mm_b200_check_opt(&opt) < 0) return 1; /* splice, -D/-X/--dual=no with the sr presets, -T, --split-prefix: refused, not ignored */
 	/* two shards per GPU: the host stages (or, for the short-read presets whose bookkeeping runs on the GPU, the upload and
 	 * the latency-bound kernel tails) of one overlap the kernels of the other */
 	mm_b200_set_lanes(4); /* two lane groups of two streams: two mini-batches in flight on the device path (mm_map_file_frag) */

@@ -17,7 +17,18 @@
 /* ------------------------------------------------------------------ work / time counters (for bench.py and -v4) */
 
 static mm_b200_stats_t g_stats;
+static double g_t_name_keys; /* kept apart: mm_b200_stats_t is mirrored by callers */
 static pthread_mutex_t g_stats_mu = PTHREAD_MUTEX_INITIALIZER;
+
+double mm_b200_name_key_time(int reset)
+{
+	double t;
+	pthread_mutex_lock(&g_stats_mu);
+	t = g_t_name_keys;
+	if (reset) g_t_name_keys = 0;
+	pthread_mutex_unlock(&g_stats_mu);
+	return t;
+}
 
 void mm_b200_stats(mm_b200_stats_t *out, int reset)
 {
@@ -99,6 +110,8 @@ typedef struct {          /* one GPU's share of a mini-batch */
 	int slot, stage_mode; /* staging slot of the ctx; 0: stage and upload, 1: stage only (host), 2: upload what an earlier stage-only call left in the slot */
 	const void *batch;    /* the mini-batch the shard belongs to (identifies what a slot holds) */
 	const uint8_t *flip;  /* --no-pairing: [read] 1 if the read is mapped reverse-complemented, decided by the pair it was read in; 0: by pe_ori and the fragment */
+	uint32_t *ukey;       /* self/dual filters: name key of every unit of the shard, in a pinned staging slot of the ctx */
+	double t_name_keys;
 } shard_t;
 
 static inline int mate_is_flipped(const mm_mapopt_t *opt, int n_segs, int j)
@@ -289,6 +302,14 @@ static void stage_copy_read(void *data, long i, int tid)
 	memcpy(sh->stage_dst + sh->stage_off[i], t->seq, t->l_seq);
 }
 
+static inline int use_name_filters(const mm_mapopt_t *opt) { return (opt->flag & (MM_F_NO_DIAG | MM_F_NO_DUAL)) != 0; }
+
+static void stage_unit_key(void *data, long i, int tid)
+{ /* the unit's name is its first read's (worker_for passes it to mm_map_frag, map.c:475-485) */
+	shard_t *sh = (shard_t*)data;
+	sh->ukey[i] = mm_b200_unit_key(sh->mi, sh->seq[sh->seg_off[sh->f0 + i]].name);
+}
+
 /* stage the reads of fragments [f0,f1) on the shard's GPU: the host part fills one of the ctx's two pinned staging slots
  * (concatenated reads and the four tables), the device part is mmg_batch_upload (H2D + 4-bit encode).  mm_b200_map_batches
  * runs the host part of a lane group's next mini-batch while the current one is mapped. */
@@ -315,7 +336,8 @@ static void *shard_upload(void *data)
 		n_seq = B->staged[ci][sh->slot].n_seq, n_bases = B->staged[ci][sh->slot].n_bases;
 		bases = (char*)mmg_staging_slot(sh->ctx, sh->slot, n_bases + 1);
 		mmg_staging_tables_slot(sh->ctx, sh->slot, n_seq, nf, &seq_len, &seq_off, &n_seg, &seg_off);
-		if (sh->flip && mmg_staging_flips_slot(sh->ctx, sh->slot, n_seq, &flip) != MMG_OK) {
+		if ((sh->flip && mmg_staging_flips_slot(sh->ctx, sh->slot, n_seq, &flip) != MMG_OK) ||
+		    (use_name_filters(sh->opt) && mmg_staging_name_keys_slot(sh->ctx, sh->slot, nf, &sh->ukey) != MMG_OK)) {
 			shard_fail(sh, "cannot allocate the staging buffers"); if (sh->up_token) pthread_mutex_unlock(sh->up_token); return 0;
 		}
 	} else {
@@ -330,6 +352,14 @@ static void *shard_upload(void *data)
 				shard_fail(sh, "cannot allocate the staging buffers"); if (mode != 1 && sh->up_token) pthread_mutex_unlock(sh->up_token); return 0;
 			}
 			memcpy(flip, sh->flip + sh->s0, (size_t)n_seq);
+		}
+		if (use_name_filters(sh->opt)) {
+			const double tk = realtime();
+			if (mmg_staging_name_keys_slot(sh->ctx, sh->slot, nf, &sh->ukey) != MMG_OK) {
+				shard_fail(sh, "cannot allocate the staging buffers"); if (mode != 1 && sh->up_token) pthread_mutex_unlock(sh->up_token); return 0;
+			}
+			parallel_for(sh->n_threads, stage_unit_key, sh, nf);
+			sh->t_name_keys += realtime() - tk;
 		}
 		for (i = 0, o = 0; i < n_seq; ++i) {
 			seq_len[i] = sh->seq[sh->s0 + i].l_seq, seq_off[i] = o;
@@ -348,6 +378,7 @@ static void *shard_upload(void *data)
 	}
 	b.n_frag = nf, b.n_seq = n_seq, b.n_seg = n_seg, b.seg_off = seg_off, b.seq_len = seq_len, b.seq_off = seq_off, b.bases = bases, b.n_bases = n_bases;
 	if ((flip ? mmg_batch_upload_flips(sh->ctx, &sh->dopt, &b, flip) : mmg_batch_upload(sh->ctx, &sh->dopt, &b)) != MMG_OK) shard_fail(sh, "read upload failed");
+	else if (use_name_filters(sh->opt) && mmg_batch_set_name_keys(sh->ctx, nf, sh->ukey) != MMG_OK) shard_fail(sh, "name key upload failed");
 	if (getenv("MM2_B200_TRACE")) fprintf(stderr, "[T::upload] +device upload %.4f s\n", realtime() - t0);
 	sh->st.n_frag += nf, sh->st.n_reads += n_seq, sh->st.n_bases += n_bases;
 	sh->st.t_upload += realtime() - t0;
@@ -595,7 +626,7 @@ static int map_step_group(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_thre
 	int n_unit = s->n_frag, *u_seg = s->n_seg, *u_off = s->seg_off, *u_tab = 0;
 	uint8_t *u_flip = 0;
 	mm_b200_tune_malloc();
-	if (mm_b200_check_opt(opt) < 0) { free(sh); free(tid); return -1; }
+	if (mm_b200_check_opt(opt) < 0 || (use_name_filters(opt) && mm_b200_name_keys_ready(mi) < 0)) { free(sh); free(tid); return -1; }
 	if (opt->flag & MM_F_INDEPEND_SEG) {
 		int k, j;
 		u_tab = (int*)malloc(2 * (size_t)s->n_seq * sizeof(int) + 1);
@@ -656,6 +687,7 @@ static int map_step_group(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_thre
 		g_stats.n_anchors += t->n_anchors, g_stats.n_chain_iter += t->n_chain_iter, g_stats.n_dp_jobs += t->n_dp_jobs;
 		g_stats.n_dp_cells += t->n_dp_cells, g_stats.n_dp_rounds += t->n_dp_rounds, g_stats.h2d_bytes += h2d, g_stats.d2h_bytes += d2h;
 		g_stats.n_dp_jobs_fast += t->n_dp_jobs_fast, g_stats.n_dp_cells_fast += t->n_dp_cells_fast;
+		g_t_name_keys += sh[d].t_name_keys;
 	}
 	g_stats.t_total += realtime() - t_start;
 	pthread_mutex_unlock(&g_stats_mu);
@@ -1001,7 +1033,8 @@ int mm_b200_check_opt(const mm_mapopt_t *opt)
 { /* what the device stages do not implement is refused with a message; nothing is silently dropped */
 	const char *what = 0;
 	if (opt->flag & MM_F_SPLICE) what = "spliced alignment (--splice, ksw_exts2)";
-	else if (opt->flag & (MM_F_NO_DIAG | MM_F_NO_DUAL)) what = "the self/dual-hit filters of the all-vs-all modes (-D, -X, --dual=no, ava-ont, ava-pb; map.c:128-137)";
+	/* the short-read presets' device post stages (aln_plan_sr, mmg_aln.h) do not bound the extension of a self-chain (MM_SEED_SELF) */
+	else if ((opt->flag & (MM_F_NO_DIAG | MM_F_NO_DUAL)) && (opt->flag & MM_F_SR)) what = "the self/dual-hit filters of the all-vs-all modes (-D, -X, --dual=no, ava-ont, ava-pb; map.c:128-137)";
 	else if (opt->sdust_thres > 0) what = "SDUST masking of query minimizers (-T, map.c:41-62)";
 	else if (opt->split_prefix) what = "--split-prefix (the index is a single part in HBM)";
 	if (what == 0) return 0;
@@ -1022,7 +1055,7 @@ void mm_map_frag(const mm_idx_t *mi, int n_segs, const int *qlens, const char **
 	for (j = 0; j < n_segs; ++j) n_regs[j] = 0, regs[j] = 0;
 	if (n_segs <= 0 || n_segs > MM_MAX_SEG) return;
 	if (mi == 0 || mi->B == 0 || mi->B->n_dev < 1) { fprintf(stderr, "[ERROR] the index is not resident on a GPU\n"); exit(1); }
-	if (mm_b200_check_opt(opt) < 0) exit(1);
+	if (mm_b200_check_opt(opt) < 0 || (use_name_filters(opt) && mm_b200_name_keys_ready(mi) < 0)) exit(1);
 	/* the resident batch, staging buffers and pools belong to ctx[0], not to the caller's mm_tbuf_t: one call at a time */
 	pthread_mutex_lock(&mi->B->api_mu);
 	seq = (mm_bseq1_t*)calloc(n_segs, sizeof(mm_bseq1_t));

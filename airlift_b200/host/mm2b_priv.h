@@ -62,6 +62,8 @@ struct mm_idx_bucket_s {
 	pthread_mutex_t gpu_token[16]; /* with lanes > 1: one shard per GPU runs device stages at a time, the others do their host stages */
 	int32_t max_occ_cache_set; float max_occ_cache_f; int32_t max_occ_cache;
 	pthread_mutex_t api_mu; /* mm_map_frag()/mm_map() share ctx[0]: concurrent callers take turns */
+	pthread_mutex_t key_mu; /* guards the lazy set-up of the name keys */
+	const char **sorted_names; /* the target names in strcmp order, once the name keys were made (namekey.c) */
 };
 
 extern unsigned char seq_nt4_table[256];
@@ -220,6 +222,10 @@ MM_FN void mm_aln_end(mm_alnseg_t *s);
 void mm_write_paf3(mm_str_t *s, const mm_idx_t *mi, const mm_bseq1_t *t, const mm_reg1_t *r, int opt_flag, int rep_len);
 void mm_write_sam3(mm_str_t *s, const mm_idx_t *mi, const mm_bseq1_t *t, int seg_idx, int reg_idx, int n_seg, const int *n_regss,
                    const mm_reg1_t *const* regss, int opt_flag, int rep_len);
+
+/* namekey.c: name keys of the self/dual-hit filters (include/mmg.h) */
+int mm_b200_name_keys_ready(const mm_idx_t *mi);  /* target keys on every device replica (first call computes them); 0 or -1 */
+uint32_t mm_b200_unit_key(const mm_idx_t *mi, const char *qname); /* after mm_b200_name_keys_ready */
 
 /* mapper.c */
 mmg_ctx_t *mm_b200_ctx(const mm_idx_t *mi, int dev_slot);

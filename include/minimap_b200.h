@@ -199,6 +199,13 @@ int mm_b200_idx_finalize(mm_idx_t *mi);
  * reference does.  mm_map_frag()/mm_map() take turns on a lock (one resident batch per GPU context), so concurrent
  * callers are safe but serialised. */
 int mm_b200_check_opt(const mm_mapopt_t *opt);
+/* name keys of the self/dual-hit filters (see "name keys" in mmg.h): sorted[] receives the n names in strcmp order (a NULL name
+ * counts as ""), tkey[] the target key of each; mm_b200_name_ukey gives the unit key of qname against those sorted names
+ * (MMG_NAME_NONE for a NULL qname) */
+void mm_b200_name_order(int n, const char *const *names, const char **sorted, uint32_t *tkey);
+uint32_t mm_b200_name_ukey(int n, const char *const *sorted, const char *qname);
+/* host seconds spent on unit keys by the mappers since the last reset (summed over shards) */
+double mm_b200_name_key_time(int reset);
 int mm_b200_set_lanes(int lanes); /* streams (with their arenas) per GPU, 1..8; before building the index */
 
 /* Batch interface = the drop-in cut point of SURVEY.md §8b (worker_pipeline step 1, map.c:590-593): a mini-batch of
