@@ -47,7 +47,7 @@ class MapOpt(C.Structure):  # mmg_mapopt_t
 
 class Batch(C.Structure):  # mmg_batch_t
     _fields_ = [("n_frag", C.c_int32), ("n_seq", C.c_int32), ("n_seg", C.c_void_p), ("seg_off", C.c_void_p), ("seq_len", C.c_void_p),
-                ("seq_off", C.c_void_p), ("bases", C.c_void_p), ("n_bases", C.c_uint64)]
+                ("seq_off", C.c_void_p), ("bases", C.c_void_p), ("n_bases", C.c_uint64), ("flip", C.c_void_p), ("ukey", C.c_void_p)]
 
 
 class Chains(C.Structure):  # mmg_chains_t
@@ -108,13 +108,10 @@ def lib():
                                     C.c_int8, C.c_int8, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(Extz), C.c_void_p]
         L.mmg_seed_chain_batch.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(MapOpt), C.POINTER(Batch), C.POINTER(Chains)]
         L.mmg_batch_upload.argtypes = [C.c_void_p, C.POINTER(MapOpt), C.POINTER(Batch)]
-        L.mmg_batch_upload_flips.argtypes = [C.c_void_p, C.POINTER(MapOpt), C.POINTER(Batch), C.c_void_p]
-        L.mmg_staging_flips_slot.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]
         L.mmg_seed_chain_resident.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(MapOpt), C.POINTER(Chains), C.c_int]
         L.mmg_collect_seeds_named.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_uint32,
                                               C.c_void_p, C.c_int64, C.POINTER(C.c_int64), C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_void_p]
         L.mmg_idx_set_name_keys.argtypes = [C.c_void_p, C.c_void_p]
-        L.mmg_batch_set_name_keys.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         L.mm_b200_name_order.argtypes = [C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), C.c_void_p]
         L.mm_b200_name_ukey.restype = C.c_uint32
         L.mm_b200_name_ukey.argtypes = [C.c_int, C.POINTER(C.c_char_p), C.c_char_p]
@@ -239,18 +236,18 @@ class Context:
         mapping, whatever fragment the read is in (how --no-pairing maps the mates of a pair one by one).
         names: one name (bytes, or None) per fragment for the self/dual filters (-D, --dual=no), ordered against the target names
         given to idx.set_names()."""
-        if flips is None:
-            _check(lib().mmg_batch_upload(self.h, C.byref(opt), C.byref(batch)))
-        else:
+        b = Batch.from_buffer_copy(batch)  # the caller's batch keeps no pointer into the arrays made here
+        if flips is not None:
             flips = np.ascontiguousarray(flips, dtype=np.uint8)
             if len(flips) != batch.n_seq:
                 raise ValueError(f"{len(flips)} flips for {batch.n_seq} reads")
-            _check(lib().mmg_batch_upload_flips(self.h, C.byref(opt), C.byref(batch), flips.ctypes.data))
+            b.flip = flips.ctypes.data
         if names is not None:
             if idx is None or len(names) != batch.n_frag:
                 raise ValueError("names needs one name per fragment and the Index they are ordered against")
             ukey = np.array([idx.unit_key(n) for n in names], dtype=np.uint32)
-            _check(lib().mmg_batch_set_name_keys(self.h, batch.n_frag, ukey.ctypes.data))
+            b.ukey = ukey.ctypes.data
+        _check(lib().mmg_batch_upload(self.h, C.byref(opt), C.byref(b)))
 
     def seed_chain_resident(self, idx, opt, download=True):
         out = Chains()

@@ -95,10 +95,19 @@ struct mmg_idx_s {
 	}
 };
 
+// one pinned staging slot (mmg_stage): the batch it holds and the event after the last copy out of it
+struct StageSlot {
+	PinBuf bases, tab, flip, ukey;
+	cudaEvent_t drained = nullptr;   // recorded by mmg_upload_stage behind its last copy out of the slot
+	int32_t n_frag = 0, n_seq = 0;
+	uint64_t n_bases = 0;
+	bool has_flip = false, has_ukey = false;
+};
+
 // state of the mini-batch currently resident on the device
 struct ResidentBatch {
 	int32_t n_frag = 0, n_seq = 0, n_units = 0, max_len = 0;
-	int32_t n_ukey = -1;             // fragments whose name keys were set for this batch (mmg_batch_set_name_keys); -1: none
+	bool has_ukey = false;           // uploaded with unit keys
 	uint64_t n_bases = 0, q_words = 0;
 	std::vector<int32_t> n_seg, seg_off, seq_len;
 };
@@ -139,13 +148,15 @@ struct mmg_ctx_s {
 	// heap order was replayed on ranks, [2] ... replayed literally, [3] fragments whose hit tree was built by a warp, [4] extra DP rounds
 	// after z-drop cuts, [5] hits cut at a z-drop, [6] seed hits whose merge order was replayed, [7] seed hits the self/dual filters dropped
 	uint64_t path[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-	PinBuf h_tab, h_tab_b, h_in_b;     // input tables of the batch being uploaded (mmg_staging_tables); second staging slot
-	PinBuf h_flip, h_flip_b;           // per-read flips of the two staging slots (mmg_staging_flips_slot)
-	PinBuf h_ukey, h_ukey_b;           // per-fragment name keys of the two staging slots (mmg_staging_name_keys_slot)
+	StageSlot stage[MMG_STAGE_SLOTS];
 	PinBuf h_path;                     // device counters of the pass in flight land here
 	PinBuf h_p_hash, h_p_nreg, h_p_offs, h_p_blob, h_p_rep;
-	PinBuf h_in, h_meta, h_out_meta, h_out_u, h_out_a, h_out_mini, h_k_jobs, h_k_res, h_k_cig;
+	PinBuf h_meta, h_out_meta, h_out_u, h_out_a, h_out_mini, h_k_jobs, h_k_res, h_k_cig;
 };
+
+// wait until the device has read what slot's last upload copied, then make its buffer `buf` hold `bytes`.  Once slot 1 is in
+// use, both slots grow together: page-locking is slow and synchronises the device, so it should happen once, not per slot.
+int mmg_stage_grow(mmg_ctx_t *c, int slot, PinBuf StageSlot::*buf, size_t bytes);
 
 #define MMG_LAUNCH(ctx, kern, grid, block, smem, ...) MMG_LAUNCH_AS(ctx, #kern, kern, grid, block, smem, __VA_ARGS__)
 // the same under a given profile name (the instantiations of one kernel template share their template's name)

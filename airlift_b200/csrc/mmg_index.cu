@@ -35,6 +35,7 @@ extern "C" int mmg_init(int device, mmg_ctx_t **out)
 	c->dev = device;
 	MMG_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
 	for (int i = 0; i < 4; ++i) MMG_CUDA(cudaEventCreate(&c->ev[i]));
+	for (StageSlot &s : c->stage) MMG_CUDA(cudaEventCreateWithFlags(&s.drained, cudaEventDisableTiming));
 	*out = c;
 	return MMG_OK;
 }
@@ -57,10 +58,13 @@ extern "C" void mmg_destroy(mmg_ctx_t *c)
 	const unsigned long long t_rel = mmg_now_ns();
 	for (DevBuf *b : bufs) b->release();
 	for (DevBuf &b : c->pb) b.release();
-	PinBuf *pins[] = {&c->h_in, &c->h_meta, &c->h_out_meta, &c->h_out_u, &c->h_out_a, &c->h_out_mini, &c->h_k_jobs, &c->h_k_res, &c->h_k_cig,
-	                  &c->h_p_hash, &c->h_p_nreg, &c->h_p_offs, &c->h_p_blob, &c->h_p_rep, &c->h_path, &c->h_tab, &c->h_tab_b, &c->h_in_b,
-	                  &c->h_flip, &c->h_flip_b, &c->h_ukey, &c->h_ukey_b};
+	PinBuf *pins[] = {&c->h_meta, &c->h_out_meta, &c->h_out_u, &c->h_out_a, &c->h_out_mini, &c->h_k_jobs, &c->h_k_res, &c->h_k_cig,
+	                  &c->h_p_hash, &c->h_p_nreg, &c->h_p_offs, &c->h_p_blob, &c->h_p_rep, &c->h_path};
 	for (PinBuf *b : pins) b->release();
+	for (StageSlot &s : c->stage) {
+		s.bases.release(), s.tab.release(), s.flip.release(), s.ukey.release();
+		if (s.drained) cudaEventDestroy(s.drained);
+	}
 	if (getenv("MM2_B200_TRACE")) fprintf(stderr, "[T::buffers] released in %.3f s\n", (mmg_now_ns() - t_rel) * 1e-9);
 	for (int i = 0; i < 4; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
 	for (const ProfRec &r : c->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
@@ -319,13 +323,13 @@ extern "C" int mmg_idx_build(mmg_ctx_t *c, int w, int k, int is_hpc, int n_seq, 
 #define IDX_CUDA(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { mmg_set_error("%s:%d: %s: %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); cleanup(); mmg_idx_free(mi); return MMG_ECUDA; } } while (0)
 #define IDX_TRY(call) do { rc = (call); if (rc != MMG_OK) { cleanup(); mmg_idx_free(mi); return rc; } } while (0)
 
-	// 1. upload ASCII (staged through pinned memory), pack to 4 bits
+	// 1. upload ASCII (through the pinned bases buffer of staging slot 0), pack to 4 bits
 	IDX_CUDA(cudaMalloc(&d_ascii, tot + 16));
 	IDX_CUDA(cudaMalloc(&mi->d_S, ((tot + 7) / 8 + 4) * 4));
 	{
 		const size_t stage = 64u << 20;
-		IDX_TRY(c->h_in.ensure(stage));
-		uint8_t *h = c->h_in.as<uint8_t>();
+		IDX_TRY(mmg_stage_grow(c, 0, &StageSlot::bases, stage));
+		uint8_t *h = c->stage[0].bases.as<uint8_t>();
 		size_t fill = 0; uint64_t done = 0;
 		for (int i = 0; i < n_seq; ++i) {
 			uint64_t o = 0;

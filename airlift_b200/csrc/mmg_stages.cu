@@ -1409,16 +1409,6 @@ static int scan_i32_to_i64(mmg_ctx_t *c, const int32_t *d_in, int64_t *d_out, in
 	return MMG_OK;
 }
 
-extern "C" void *mmg_staging_slot(mmg_ctx_t *c, int slot, size_t bytes)
-{ // pinned host buffer owned by the ctx (one of two, so that the next batch can be staged while the current one is mapped)
-	cudaSetDevice(c->dev);
-	PinBuf &in = slot ? c->h_in_b : c->h_in;
-	if (in.ensure(bytes + 64) != MMG_OK) return nullptr;
-	if ((c->h_in_b.p || slot) && (slot ? c->h_in : c->h_in_b).ensure(bytes + 64) != MMG_OK) return nullptr; // both slots grow together
-	return in.p;
-}
-extern "C" void *mmg_staging(mmg_ctx_t *c, size_t bytes) { return mmg_staging_slot(c, 0, bytes); }
-
 extern "C" int mmg_job_buffers(mmg_ctx_t *c, size_t n_jobs, mmg_ksw_job_t **jobs, mmg_ksw_res_t **res)
 { // page-locked, owned by the ctx, grown on demand and kept across batches (allocating pinned memory is slow)
 	cudaSetDevice(c->dev);
@@ -1428,8 +1418,7 @@ extern "C" int mmg_job_buffers(mmg_ctx_t *c, size_t n_jobs, mmg_ksw_job_t **jobs
 	return MMG_OK;
 }
 
-// pinned table block of the ctx: seq_len[n_seq+1] | seq_off[n_seq+1] | n_seg[n_frag] | seg_off[n_frag]; callers that fill it in place
-// (and pass these pointers in mmg_batch_t) save mmg_batch_upload a copy
+// pinned table block of a staging slot: seq_off[n_seq+2] | seq_len[n_seq+2] | n_seg[n_frag+2] | seg_off[n_frag+2]
 static void tab_layout(void *base, int n_seq, int n_frag, int32_t **seq_len, uint64_t **seq_off, int32_t **n_seg, int32_t **seg_off)
 {
 	uint8_t *p = static_cast<uint8_t*>(base);
@@ -1440,18 +1429,38 @@ static void tab_layout(void *base, int n_seq, int n_frag, int32_t **seq_len, uin
 }
 static size_t tab_bytes(int n_seq, int n_frag) { return ((size_t)n_seq + 2) * 12 + ((size_t)n_frag + 2) * 8 + 64; }
 
-extern "C" int mmg_staging_tables_slot(mmg_ctx_t *c, int slot, int n_seq, int n_frag, int32_t **seq_len, uint64_t **seq_off, int32_t **n_seg, int32_t **seg_off)
+int mmg_stage_grow(mmg_ctx_t *c, int slot, PinBuf StageSlot::*buf, size_t bytes)
 {
-	cudaSetDevice(c->dev);
-	PinBuf &tab = slot ? c->h_tab_b : c->h_tab;
-	MMG_TRY(tab.ensure(tab_bytes(n_seq, n_frag)));
-	if (c->h_tab_b.p || slot) MMG_TRY((slot ? c->h_tab : c->h_tab_b).ensure(tab_bytes(n_seq, n_frag))); // both slots grow together: page-locking is slow and synchronises the device
-	tab_layout(tab.p, n_seq, n_frag, seq_len, seq_off, n_seg, seg_off);
+	const bool together = slot != 0 || (c->stage[1].*buf).p != nullptr;
+	for (int k = 0; k < MMG_STAGE_SLOTS; ++k) {
+		const int s = (slot + k) % MMG_STAGE_SLOTS;
+		PinBuf &b = c->stage[s].*buf;
+		if (s == slot) MMG_CUDA(cudaEventSynchronize(c->stage[s].drained));
+		if ((s != slot && !together) || bytes <= b.cap) continue;
+		if (s != slot) MMG_CUDA(cudaEventSynchronize(c->stage[s].drained));
+		MMG_TRY(b.ensure(bytes));
+	}
 	return MMG_OK;
 }
-extern "C" int mmg_staging_tables(mmg_ctx_t *c, int n_seq, int n_frag, int32_t **seq_len, uint64_t **seq_off, int32_t **n_seg, int32_t **seg_off)
+
+extern "C" int mmg_stage(mmg_ctx_t *c, int slot, int n_frag, int n_seq, uint64_t n_bases, int with_flip, int with_ukey, mmg_stage_t *out)
 {
-	return mmg_staging_tables_slot(c, 0, n_seq, n_frag, seq_len, seq_off, n_seg, seg_off);
+	if (slot < 0 || slot >= MMG_STAGE_SLOTS || n_frag < 0 || n_seq < 0) {
+		mmg_set_error("mmg_stage: slot %d, %d fragments, %d reads", slot, n_frag, n_seq);
+		return MMG_EINVAL;
+	}
+	MMG_CUDA(cudaSetDevice(c->dev));
+	StageSlot &s = c->stage[slot];
+	MMG_TRY(mmg_stage_grow(c, slot, &StageSlot::bases, n_bases + 65));
+	MMG_TRY(mmg_stage_grow(c, slot, &StageSlot::tab, tab_bytes(n_seq, n_frag)));
+	if (with_flip) MMG_TRY(mmg_stage_grow(c, slot, &StageSlot::flip, (size_t)n_seq + 16));
+	if (with_ukey) MMG_TRY(mmg_stage_grow(c, slot, &StageSlot::ukey, ((size_t)n_frag + 4) * 4));
+	s.n_frag = n_frag, s.n_seq = n_seq, s.n_bases = n_bases, s.has_flip = with_flip != 0, s.has_ukey = with_ukey != 0;
+	out->bases = s.bases.as<char>();
+	tab_layout(s.tab.p, n_seq, n_frag, &out->seq_len, &out->seq_off, &out->n_seg, &out->seg_off);
+	out->flip = s.has_flip ? s.flip.as<uint8_t>() : nullptr;
+	out->ukey = s.has_ukey ? s.ukey.as<uint32_t>() : nullptr;
+	return MMG_OK;
 }
 
 struct PadLen8 { __host__ __device__ uint64_t operator()(int32_t len) const { return ((uint64_t)len + 7) / 8 * 8; } };
@@ -1460,7 +1469,7 @@ struct UnitsOfLen { __host__ __device__ int64_t operator()(int32_t len) const { 
 // what the sketch and the later stages need per read and per fragment, from the lengths alone: the sketch work units
 // (one per MMG_READ_CHUNK positions of a read), the mates to flip (pe_ori, map.c:467-469), the fragments' unit ranges and
 // query lengths.  (The host used to build these 60 bytes per read and copy them over from pageable memory, every batch.)
-// flip_given: flip[] already holds the per-read decision (mmg_batch_upload_flips), it is not derived from the fragment here
+// flip_given: flip[] already holds the per-read decision (mmg_batch_t.flip), it is not derived from the fragment here
 __global__ void k_batch_tables(int n_frag, int n_seq, const int32_t *__restrict__ n_seg, const int32_t *__restrict__ seg_off,
                                const int32_t *__restrict__ seq_len, const uint64_t *__restrict__ q_off, const int64_t *__restrict__ unit0, int pe_ori,
                                int flip_given, SketchUnit *__restrict__ units, uint8_t *__restrict__ flip, int32_t *__restrict__ frag_unit0,
@@ -1487,89 +1496,27 @@ __global__ void k_batch_tables(int n_frag, int n_seq, const int32_t *__restrict_
 	frag_qlen[f] = sum;
 }
 
-extern "C" int mmg_staging_flips_slot(mmg_ctx_t *c, int slot, int n_seq, uint8_t **flip)
+extern "C" int mmg_upload_stage(mmg_ctx_t *c, const mmg_mapopt_t *opt, int slot)
 {
-	cudaSetDevice(c->dev);
-	PinBuf &fl = slot ? c->h_flip_b : c->h_flip;
-	MMG_TRY(fl.ensure((size_t)n_seq + 16));
-	if (c->h_flip_b.p || slot) MMG_TRY((slot ? c->h_flip : c->h_flip_b).ensure((size_t)n_seq + 16)); // both slots grow together, as the tables do
-	*flip = fl.as<uint8_t>();
-	return MMG_OK;
-}
-
-static int batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t *b, const uint8_t *flip_in);
-
-extern "C" int mmg_staging_name_keys_slot(mmg_ctx_t *c, int slot, int n_frag, uint32_t **ukey)
-{
-	cudaSetDevice(c->dev);
-	PinBuf &k = slot ? c->h_ukey_b : c->h_ukey;
-	MMG_TRY(k.ensure(((size_t)n_frag + 4) * 4));
-	if (c->h_ukey_b.p || slot) MMG_TRY((slot ? c->h_ukey : c->h_ukey_b).ensure(((size_t)n_frag + 4) * 4)); // both slots grow together, as the tables do
-	*ukey = k.as<uint32_t>();
-	return MMG_OK;
-}
-
-extern "C" int mmg_batch_set_name_keys(mmg_ctx_t *c, int n_frag, const uint32_t *ukey)
-{
-	if (ukey == nullptr || n_frag != c->rb.n_frag) {
-		mmg_set_error("mmg_batch_set_name_keys: %d keys for a resident batch of %d fragments", ukey ? n_frag : 0, c->rb.n_frag);
+	if (slot < 0 || slot >= MMG_STAGE_SLOTS || c->stage[slot].tab.p == nullptr) {
+		mmg_set_error("mmg_upload_stage: slot %d holds no batch (mmg_stage)", slot);
 		return MMG_EINVAL;
 	}
 	MMG_CUDA(cudaSetDevice(c->dev));
-	const uint32_t *src = ukey;
-	if (src != c->h_ukey.as<uint32_t>() && src != c->h_ukey_b.as<uint32_t>()) { // from pinned memory, like the tables
-		MMG_TRY(c->h_ukey.ensure(((size_t)n_frag + 4) * 4));
-		memcpy(c->h_ukey.p, ukey, (size_t)n_frag * 4);
-		src = c->h_ukey.as<uint32_t>();
-	}
-	MMG_TRY(c->d_ukey.ensure(((size_t)n_frag + 4) * 4));
-	if (n_frag > 0) MMG_H2D(c, c->d_ukey.p, src, (size_t)n_frag * 4);
-	c->rb.n_ukey = n_frag;
-	return MMG_OK;
-}
-
-extern "C" int mmg_batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t *b) { return batch_upload(c, opt, b, nullptr); }
-
-extern "C" int mmg_batch_upload_flips(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t *b, const uint8_t *flip)
-{
-	if (flip == nullptr) { mmg_set_error("mmg_batch_upload_flips: no flip table"); return MMG_EINVAL; }
-	return batch_upload(c, opt, b, flip);
-}
-
-// flip_in (n_seq bytes, or null): which reads are reverse-complemented before mapping; null derives it from pe_ori and each fragment's mates
-static int batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t *b, const uint8_t *flip_in)
-{
-	MMG_CUDA(cudaSetDevice(c->dev));
+	const StageSlot &s = c->stage[slot];
 	ResidentBatch &rb = c->rb;
 	// the reads go first: their copy runs while the host looks at the lengths below
-	const size_t sz_bases = (b->n_bases + 15) & ~(size_t)15;
-	const void *src_bases = b->bases;
-	if (src_bases != c->h_in.p && src_bases != c->h_in_b.p) { // callers that filled mmg_staging() skip this copy
-		MMG_TRY(c->h_in.ensure(sz_bases + 64));
-		memcpy(c->h_in.p, b->bases, b->n_bases);
-		src_bases = c->h_in.p;
-	}
+	const size_t sz_bases = (s.n_bases + 15) & ~(size_t)15;
 	MMG_TRY(c->d_ascii.ensure(sz_bases + 64));
-	MMG_H2D(c, c->d_ascii.p, src_bases, b->n_bases);
-	const int n_seq = b->n_seq, n_frag = b->n_frag;
-	rb.n_frag = n_frag, rb.n_seq = n_seq, rb.n_bases = b->n_bases;
-	rb.n_ukey = -1; // name keys belong to one batch
-	rb.n_seg.assign(b->n_seg, b->n_seg + n_frag);
-	rb.seg_off.assign(b->seg_off, b->seg_off + n_frag);
-	rb.seq_len.assign(b->seq_len, b->seq_len + n_seq);
-	// the four input tables in pinned memory (in place already when the caller used mmg_staging_tables)
+	MMG_H2D(c, c->d_ascii.p, s.bases.p, s.n_bases);
+	const int n_seq = s.n_seq, n_frag = s.n_frag;
 	int32_t *t_len, *t_nseg, *t_segoff; uint64_t *t_off;
-	if (c->h_tab_b.p && c->h_tab_b.cap >= tab_bytes(n_seq, n_frag) && (const void*)b->seq_off == c->h_tab_b.p) // filled in place in the second slot
-		tab_layout(c->h_tab_b.p, n_seq, n_frag, &t_len, &t_off, &t_nseg, &t_segoff);
-	else {
-		MMG_TRY(c->h_tab.ensure(tab_bytes(n_seq, n_frag)));
-		tab_layout(c->h_tab.p, n_seq, n_frag, &t_len, &t_off, &t_nseg, &t_segoff);
-	}
-	if (b->seq_len != t_len) memcpy(t_len, b->seq_len, (size_t)n_seq * 4);
-	if (b->seq_off != t_off) memcpy(t_off, b->seq_off, (size_t)n_seq * 8);
-	if (b->n_seg != t_nseg) memcpy(t_nseg, b->n_seg, (size_t)n_frag * 4);
-	if (b->seg_off != t_segoff) memcpy(t_segoff, b->seg_off, (size_t)n_frag * 4);
-	t_len[n_seq] = 0, t_off[n_seq] = b->n_bases; // the scans below run over n_seq + 1 items
+	tab_layout(s.tab.p, n_seq, n_frag, &t_len, &t_off, &t_nseg, &t_segoff);
+	rb.n_frag = n_frag, rb.n_seq = n_seq, rb.n_bases = s.n_bases, rb.has_ukey = s.has_ukey;
+	rb.n_seg.assign(t_nseg, t_nseg + n_frag);
+	rb.seg_off.assign(t_segoff, t_segoff + n_frag);
+	rb.seq_len.assign(t_len, t_len + n_seq);
+	t_len[n_seq] = 0, t_off[n_seq] = s.n_bases; // the scans below run over n_seq + 1 items
 	uint64_t qo = 0; int64_t nu = 0;
 	int max_len = 0;
 	for (int r = 0; r < n_seq; ++r) { qo += PadLen8()(t_len[r]); nu += UnitsOfLen()(t_len[r]); max_len = max_len > t_len[r] ? max_len : t_len[r]; }
@@ -1592,15 +1539,12 @@ static int batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t
 	MMG_H2D(c, c->d_seq_off.p, t_off, (size_t)(n_seq + 1) * 8);
 	MMG_H2D(c, c->d_misc.p, t_nseg, (size_t)n_frag * 4);
 	MMG_H2D(c, c->d_fseg_off.p, t_segoff, (size_t)n_frag * 4);
-	if (flip_in) { // the per-read flips, from pinned memory like the tables (in place when the caller used mmg_staging_flips_slot)
-		const uint8_t *src = flip_in;
-		if (src != c->h_flip.p && src != c->h_flip_b.p) {
-			MMG_TRY(c->h_flip.ensure((size_t)n_seq + 16));
-			memcpy(c->h_flip.p, flip_in, (size_t)n_seq);
-			src = c->h_flip.as<uint8_t>();
-		}
-		if (n_seq > 0) MMG_H2D(c, c->d_flip.p, src, (size_t)n_seq);
+	if (s.has_flip && n_seq > 0) MMG_H2D(c, c->d_flip.p, s.flip.p, (size_t)n_seq);
+	if (s.has_ukey) {
+		MMG_TRY(c->d_ukey.ensure(((size_t)n_frag + 4) * 4));
+		if (n_frag > 0) MMG_H2D(c, c->d_ukey.p, s.ukey.p, (size_t)n_frag * 4);
 	}
+	MMG_CUDA(cudaEventRecord(s.drained, c->stream)); // the next mmg_stage of this slot waits for it
 	{ // packed (8-base aligned) offset of every read, first sketch unit of every read
 		cub::TransformInputIterator<uint64_t, PadLen8, const int32_t*> it_q(c->d_seq_len.as<int32_t>(), PadLen8());
 		cub::TransformInputIterator<int64_t, UnitsOfLen, const int32_t*> it_u(c->d_seq_len.as<int32_t>(), UnitsOfLen());
@@ -1613,13 +1557,26 @@ static int batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t
 		c->launches += 2;
 	}
 	MMG_LAUNCH(c, k_batch_tables, mmg_blocks((size_t)n_frag + 1, 256), 256, 0, n_frag, n_seq, c->d_misc.as<int32_t>(), c->d_fseg_off.as<int32_t>(),
-	           c->d_seq_len.as<int32_t>(), c->d_q_off.as<uint64_t>(), c->d_unit0.as<int64_t>(), opt->pe_ori, flip_in ? 1 : 0, c->d_units.as<SketchUnit>(),
+	           c->d_seq_len.as<int32_t>(), c->d_q_off.as<uint64_t>(), c->d_unit0.as<int64_t>(), opt->pe_ori, s.has_flip ? 1 : 0, c->d_units.as<SketchUnit>(),
 	           c->d_flip.as<uint8_t>(), c->d_frag_unit0.as<int32_t>(), c->d_frag_qlen.as<int32_t>());
 	if (rb.q_words)
 		MMG_LAUNCH(c, k_encode_reads, mmg_blocks(rb.q_words, 256), 256, 0, c->d_ascii.as<uint8_t>(), c->d_seq_off.as<uint64_t>(),
 		           c->d_seq_len.as<int32_t>(), c->d_q_off.as<uint64_t>(), c->d_flip.as<uint8_t>(), n_seq, rb.q_words, c->d_Q.as<uint32_t>());
-	// no synchronisation: every source of the copies above is pinned memory the ctx owns until its next upload
 	return MMG_OK;
+}
+
+extern "C" int mmg_batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg_batch_t *b)
+{
+	mmg_stage_t st;
+	MMG_TRY(mmg_stage(c, 0, b->n_frag, b->n_seq, b->n_bases, b->flip != nullptr, b->ukey != nullptr, &st));
+	memcpy(st.bases, b->bases, b->n_bases);
+	memcpy(st.seq_len, b->seq_len, (size_t)b->n_seq * 4);
+	memcpy(st.seq_off, b->seq_off, (size_t)b->n_seq * 8);
+	memcpy(st.n_seg, b->n_seg, (size_t)b->n_frag * 4);
+	memcpy(st.seg_off, b->seg_off, (size_t)b->n_frag * 4);
+	if (b->flip) memcpy(st.flip, b->flip, (size_t)b->n_seq);
+	if (b->ukey) memcpy(st.ukey, b->ukey, (size_t)b->n_frag * 4);
+	return mmg_upload_stage(c, opt, 0);
 }
 
 struct PassBufs {
@@ -1826,7 +1783,7 @@ extern "C" int mmg_seed_chain_resident(mmg_ctx_t *c, const mmg_idx_t *mi, const 
 	NameTabs nt = {nullptr, nullptr, nullptr};
 	if (opt->flag & (MMG_F_NO_DIAG | MMG_F_NO_DUAL)) { // never filter on keys of another index or batch
 		if (mi->d_tkey == nullptr) { mmg_set_error("the self/dual filters need the target name keys (mmg_idx_set_name_keys)"); return MMG_EINVAL; }
-		if (rb.n_ukey != nf) { mmg_set_error("the self/dual filters need the name keys of this batch (mmg_batch_set_name_keys)"); return MMG_EINVAL; }
+		if (!rb.has_ukey) { mmg_set_error("the self/dual filters need the name keys of this batch (mmg_batch_t.ukey)"); return MMG_EINVAL; }
 		nt.tkey = mi->d_tkey, nt.tlen = mi->d_seq_len, nt.ukey = c->d_ukey.as<uint32_t>();
 	}
 	MMG_CUDA(cudaEventRecord(c->ev[0], c->stream));
@@ -1964,6 +1921,7 @@ extern "C" int mmg_sketch(mmg_ctx_t *c, const char *str, int len, int w, int k, 
 	mmg_mapopt_t opt; memset(&opt, 0, sizeof(opt));
 	int32_t one = 1, zero = 0, l = len; uint64_t o = 0;
 	mmg_batch_t b; b.n_frag = 1, b.n_seq = 1, b.n_seg = &one, b.seg_off = &zero, b.seq_len = &l, b.seq_off = &o, b.bases = str, b.n_bases = (uint64_t)len;
+	b.flip = nullptr, b.ukey = nullptr;
 	MMG_TRY(mmg_batch_upload(c, &opt, &b));
 	std::vector<SketchUnit> units;
 	const int chunk = is_hpc ? len : 96;

@@ -107,10 +107,10 @@ typedef struct {          /* one GPU's share of a mini-batch */
 	char *stage_dst; const uint64_t *stage_off;
 	size_t m_jobs;
 	int rc;
-	int slot, stage_mode; /* staging slot of the ctx; 0: stage and upload, 1: stage only (host), 2: upload what an earlier stage-only call left in the slot */
+	int ci, slot, ops;    /* ctx index in the bucket, its staging slot this shard uses, SH_* */
 	const void *batch;    /* the mini-batch the shard belongs to (identifies what a slot holds) */
 	const uint8_t *flip;  /* --no-pairing: [read] 1 if the read is mapped reverse-complemented, decided by the pair it was read in; 0: by pe_ori and the fragment */
-	uint32_t *ukey;       /* self/dual filters: name key of every unit of the shard, in a pinned staging slot of the ctx */
+	uint32_t *ukey;       /* self/dual filters: name key of every unit of the shard, written into the staging slot */
 	double t_name_keys;
 } shard_t;
 
@@ -310,82 +310,58 @@ static void stage_unit_key(void *data, long i, int tid)
 	sh->ukey[i] = mm_b200_unit_key(sh->mi, sh->seq[sh->seg_off[sh->f0 + i]].name);
 }
 
-/* stage the reads of fragments [f0,f1) on the shard's GPU: the host part fills one of the ctx's two pinned staging slots
- * (concatenated reads and the four tables), the device part is mmg_batch_upload (H2D + 4-bit encode).  mm_b200_map_batches
- * runs the host part of a lane group's next mini-batch while the current one is mapped. */
-static void *shard_upload(void *data)
+/* what map_step_group does with every shard: fill a pinned staging slot of its ctx (host), upload the slot (H2D + 4-bit
+ * encode), map the resident batch */
+enum { SH_STAGE = 1, SH_SEND = 2, SH_MAP = 4 };
+
+/* the host part of an upload: the reads of units [f0,f1), their four tables, the flips and the unit keys into staging slot
+ * sh->slot of the ctx.  mm_b200_map_batches runs it for a lane group's next mini-batch while the current one is mapped. */
+static void shard_stage(shard_t *sh)
 {
-	shard_t *sh = (shard_t*)data;
-	const int nf = sh->f1 - sh->f0, mode = sh->stage_mode;
 	struct mm_idx_bucket_s *B = sh->mi->B;
-	int i, n_seq = 0, ci;
+	const int nf = sh->f1 - sh->f0;
+	const double t0 = realtime();
+	int i, n_seq = 0;
 	uint64_t n_bases = 0, o;
-	char *bases;
-	int32_t *n_seg, *seg_off, *seq_len;
-	uint64_t *seq_off;
-	uint8_t *flip = 0;
-	mmg_batch_t b;
-	double t0;
-	sh->rc = 0;
-	if (nf <= 0) return 0;
-	for (ci = 0; ci < 16 * MM_B200_MAX_LANES && B->ctx[ci] != sh->ctx; ++ci) {}
-	if (mode != 1 && sh->up_token) pthread_mutex_lock(sh->up_token);
-	t0 = realtime();
-	sh->s0 = sh->seg_off[sh->f0];
-	if (mode == 2 && B->staged[ci][sh->slot].batch == sh->batch && B->staged[ci][sh->slot].f0 == sh->f0 && B->staged[ci][sh->slot].f1 == sh->f1) {
-		n_seq = B->staged[ci][sh->slot].n_seq, n_bases = B->staged[ci][sh->slot].n_bases;
-		bases = (char*)mmg_staging_slot(sh->ctx, sh->slot, n_bases + 1);
-		mmg_staging_tables_slot(sh->ctx, sh->slot, n_seq, nf, &seq_len, &seq_off, &n_seg, &seg_off);
-		if ((sh->flip && mmg_staging_flips_slot(sh->ctx, sh->slot, n_seq, &flip) != MMG_OK) ||
-		    (use_name_filters(sh->opt) && mmg_staging_name_keys_slot(sh->ctx, sh->slot, nf, &sh->ukey) != MMG_OK)) {
-			shard_fail(sh, "cannot allocate the staging buffers"); if (sh->up_token) pthread_mutex_unlock(sh->up_token); return 0;
-		}
-	} else {
-		for (i = sh->f0; i < sh->f1; ++i) n_seq += sh->n_seg[i];
-		for (i = 0; i < n_seq; ++i) n_bases += sh->seq[sh->s0 + i].l_seq;
-		bases = (char*)mmg_staging_slot(sh->ctx, sh->slot, n_bases + 1);
-		if (bases == 0 || mmg_staging_tables_slot(sh->ctx, sh->slot, n_seq, nf, &seq_len, &seq_off, &n_seg, &seg_off) != MMG_OK) {
-			shard_fail(sh, "cannot allocate the staging buffers"); if (mode != 1 && sh->up_token) pthread_mutex_unlock(sh->up_token); return 0;
-		}
-		if (sh->flip) { /* the reads are uploaded as read; the device flips them from this table */
-			if (mmg_staging_flips_slot(sh->ctx, sh->slot, n_seq, &flip) != MMG_OK) {
-				shard_fail(sh, "cannot allocate the staging buffers"); if (mode != 1 && sh->up_token) pthread_mutex_unlock(sh->up_token); return 0;
-			}
-			memcpy(flip, sh->flip + sh->s0, (size_t)n_seq);
-		}
-		if (use_name_filters(sh->opt)) {
-			const double tk = realtime();
-			if (mmg_staging_name_keys_slot(sh->ctx, sh->slot, nf, &sh->ukey) != MMG_OK) {
-				shard_fail(sh, "cannot allocate the staging buffers"); if (mode != 1 && sh->up_token) pthread_mutex_unlock(sh->up_token); return 0;
-			}
-			parallel_for(sh->n_threads, stage_unit_key, sh, nf);
-			sh->t_name_keys += realtime() - tk;
-		}
-		for (i = 0, o = 0; i < n_seq; ++i) {
-			seq_len[i] = sh->seq[sh->s0 + i].l_seq, seq_off[i] = o;
-			o += seq_len[i];
-		}
-		sh->stage_dst = bases, sh->stage_off = seq_off;
-		parallel_for(sh->n_threads, stage_copy_read, sh, n_seq);
-		for (i = 0; i < nf; ++i) n_seg[i] = sh->n_seg[sh->f0 + i], seg_off[i] = sh->seg_off[sh->f0 + i] - sh->s0;
-		if (getenv("MM2_B200_TRACE")) fprintf(stderr, "[T::upload] staged %d reads in %.4f s\n", n_seq, realtime() - t0);
-		if (mode == 1) {
-			B->staged[ci][sh->slot].batch = sh->batch, B->staged[ci][sh->slot].f0 = sh->f0, B->staged[ci][sh->slot].f1 = sh->f1;
-			B->staged[ci][sh->slot].n_seq = n_seq, B->staged[ci][sh->slot].n_bases = n_bases;
-			sh->st.t_upload += realtime() - t0;
-			return 0;
-		}
+	mmg_stage_t st;
+	B->staged[sh->ci][sh->slot].batch = 0; /* the slot holds nothing whole until the end */
+	for (i = sh->f0; i < sh->f1; ++i) n_seq += sh->n_seg[i];
+	for (i = 0; i < n_seq; ++i) n_bases += sh->seq[sh->s0 + i].l_seq;
+	if (mmg_stage(sh->ctx, sh->slot, nf, n_seq, n_bases, sh->flip != 0, use_name_filters(sh->opt), &st) != MMG_OK) {
+		shard_fail(sh, "cannot allocate the staging buffers");
+		return;
 	}
-	b.n_frag = nf, b.n_seq = n_seq, b.n_seg = n_seg, b.seg_off = seg_off, b.seq_len = seq_len, b.seq_off = seq_off, b.bases = bases, b.n_bases = n_bases;
-	if ((flip ? mmg_batch_upload_flips(sh->ctx, &sh->dopt, &b, flip) : mmg_batch_upload(sh->ctx, &sh->dopt, &b)) != MMG_OK) shard_fail(sh, "read upload failed");
-	else if (use_name_filters(sh->opt) && mmg_batch_set_name_keys(sh->ctx, nf, sh->ukey) != MMG_OK) shard_fail(sh, "name key upload failed");
-	if (getenv("MM2_B200_TRACE")) fprintf(stderr, "[T::upload] +device upload %.4f s\n", realtime() - t0);
+	if (sh->flip) memcpy(st.flip, sh->flip + sh->s0, (size_t)n_seq); /* the reads are uploaded as read; the device flips them from this table */
+	if (st.ukey) {
+		const double tk = realtime();
+		sh->ukey = st.ukey;
+		parallel_for(sh->n_threads, stage_unit_key, sh, nf);
+		sh->t_name_keys += realtime() - tk;
+	}
+	for (i = 0, o = 0; i < n_seq; ++i) {
+		st.seq_len[i] = sh->seq[sh->s0 + i].l_seq, st.seq_off[i] = o;
+		o += st.seq_len[i];
+	}
+	sh->stage_dst = st.bases, sh->stage_off = st.seq_off;
+	parallel_for(sh->n_threads, stage_copy_read, sh, n_seq);
+	for (i = 0; i < nf; ++i) st.n_seg[i] = sh->n_seg[sh->f0 + i], st.seg_off[i] = sh->seg_off[sh->f0 + i] - sh->s0;
+	B->staged[sh->ci][sh->slot].batch = sh->batch, B->staged[sh->ci][sh->slot].f0 = sh->f0, B->staged[sh->ci][sh->slot].f1 = sh->f1;
+	if (getenv("MM2_B200_TRACE")) fprintf(stderr, "[T::upload] staged %d reads in %.4f s\n", n_seq, realtime() - t0);
 	sh->st.n_frag += nf, sh->st.n_reads += n_seq, sh->st.n_bases += n_bases;
 	sh->st.t_upload += realtime() - t0;
-	if (sh->up_token) pthread_mutex_unlock(sh->up_token);
-	return 0;
 }
 
+/* the device part: upload what the slot holds */
+static void shard_send(shard_t *sh)
+{
+	const double t0 = realtime();
+	if (mmg_upload_stage(sh->ctx, &sh->dopt, sh->slot) != MMG_OK) {
+		shard_fail(sh, "read upload failed");
+		return;
+	}
+	if (getenv("MM2_B200_TRACE")) fprintf(stderr, "[T::upload] device upload %.4f s\n", realtime() - t0);
+	sh->st.t_upload += realtime() - t0;
+}
 
 /* ---- device path (short-read presets): hits, per-mate split, alignment walk and CIGAR post-processing run on the GPU
  * (csrc/mmg_post.cu: designed device stages over flat arrays, mmg_hits.h / mmg_aln.h / mmg_post.h, MAPQ and pairing included); the
@@ -606,19 +582,38 @@ static step_t *step_read(pipeline_t *p)
 	return s;
 }
 
-static void *shard_both(void *data) { shard_upload(data); return map_shard(data); }
+/* whether the shard's staging slot holds this shard, filled by an earlier SH_STAGE call */
+static int slot_holds(const shard_t *sh)
+{
+	const struct mm_idx_bucket_s *B = sh->mi->B;
+	return B->staged[sh->ci][sh->slot].batch == sh->batch && B->staged[sh->ci][sh->slot].f0 == sh->f0 && B->staged[sh->ci][sh->slot].f1 == sh->f1;
+}
 
-/* mode 0: upload + map; 1: upload only; 2: map the batch uploaded by an earlier mode-1 call.
+static void *shard_run(void *data)
+{
+	shard_t *sh = (shard_t*)data;
+	const int send = !!(sh->ops & SH_SEND);
+	if (sh->f1 <= sh->f0) return 0;
+	if (send && sh->up_token) pthread_mutex_lock(sh->up_token);
+	if ((sh->ops & SH_STAGE) || (send && !slot_holds(sh))) shard_stage(sh);
+	if (send && !sh->rc) shard_send(sh);
+	if (send && sh->up_token) pthread_mutex_unlock(sh->up_token);
+	if (sh->ops & SH_MAP) map_shard(sh);
+	return 0;
+}
+
+/* ops (SH_*): what to do with every shard of the step.  SH_SEND without SH_STAGE stages a shard first unless its slot holds it.
+ * slot: the staging slot of every ctx this call uses.
  * group/n_groups: the lanes of every GPU are split into n_groups sets and this call uses set `group`, so that calls on
  * different groups may run at the same time (mm_b200_map_batches) */
-static int map_step_group(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_threads, step_t *s, int mode, int group, int n_groups, int slot, int stage_mode)
+static int map_step_group(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_threads, step_t *s, int ops, int group, int n_groups, int slot)
 {
 	struct mm_idx_bucket_s *B = mi->B;
 	const int lanes = B->lanes / n_groups;  /* shards per GPU of this call, each with its own stream */
 	const int n_dev = B->n_dev * lanes;
 	shard_t *sh = (shard_t*)calloc(n_dev, sizeof(shard_t));
 	pthread_t *tid = (pthread_t*)calloc(n_dev, sizeof(pthread_t));
-	int d, f = 0, rc = 0, pass;
+	int d, f = 0, rc = 0;
 	int64_t tot = 0, acc = 0;
 	const double t_start = realtime();
 	/* the mapping units: the fragments as read, or with --no-pairing every read on its own (worker_for, map.c:475-485); the
@@ -643,7 +638,7 @@ static int map_step_group(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_thre
 		 * can hide) is short and the second, larger upload runs under its kernels */
 		const int64_t goal = (lanes == 2 && use_device_path(mi, opt)) ? (tot * (d / 2) + (d % 2 == 0 ? tot * 3 / 10 : tot)) / B->n_dev : tot * (d + 1) / n_dev;
 		const int gpu = d / lanes;
-		h->mi = mi, h->opt = opt, h->ctx = B->ctx[gpu * B->lanes + group * lanes + d % lanes], h->didx = B->didx[gpu];
+		h->mi = mi, h->opt = opt, h->ci = gpu * B->lanes + group * lanes + d % lanes, h->ctx = B->ctx[h->ci], h->didx = B->didx[gpu];
 		mm_mapopt_to_dev(opt, &h->dopt);
 		mm_arena_init(&h->arena);
 		/* lanes of one GPU alternate between device and host stages, so each may use that GPU's whole share of host threads */
@@ -652,7 +647,7 @@ static int map_step_group(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_thre
 		 * may overlap freely (the latency-bound tails of one shard fill the gaps of the other) */
 		h->gpu_token = B->lanes > 1 && (!use_device_path(mi, opt) || g_serial_shards) ? &B->gpu_token[gpu] : 0;
 		h->up_token = B->lanes > 1 && use_device_path(mi, opt) ? &B->up_token[gpu] : 0;
-		h->slot = slot, h->stage_mode = stage_mode, h->batch = s;
+		h->slot = slot, h->ops = ops, h->batch = s;
 		h->seq = s->seq, h->n_seg = u_seg, h->seg_off = u_off, h->n_reg = s->n_reg, h->rep_len = s->rep_len, h->frag_gap = s->frag_gap, h->reg = s->reg;
 		h->flip = u_flip;
 		h->f0 = f;
@@ -664,15 +659,10 @@ static int map_step_group(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_thre
 		h->f1 = f;
 		if (h->f1 > h->f0) h->s0 = u_off[h->f0];
 	}
-	if (stage_mode == 1) mode = 1; /* host staging only */
-	for (pass = 0; pass < 2; ++pass) {
-		void *(*fn)(void*) = mode == 0 ? shard_both : pass == 0 ? shard_upload : map_shard;
-		if ((pass == 0 && mode == 2) || (pass == 1 && mode == 1) || (pass == 1 && mode == 0)) continue;
-		if (n_dev == 1) fn(&sh[0]);
-		else {
-			for (d = 0; d < n_dev; ++d) pthread_create(&tid[d], 0, fn, &sh[d]);
-			for (d = 0; d < n_dev; ++d) pthread_join(tid[d], 0);
-		}
+	if (n_dev == 1) shard_run(&sh[0]);
+	else {
+		for (d = 0; d < n_dev; ++d) pthread_create(&tid[d], 0, shard_run, &sh[d]);
+		for (d = 0; d < n_dev; ++d) pthread_join(tid[d], 0);
 	}
 	pthread_mutex_lock(&g_stats_mu);
 	for (d = 0; d < n_dev; ++d) {
@@ -701,9 +691,10 @@ static int map_step_group(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_thre
 	return rc;
 }
 
-static int map_step(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_threads, step_t *s, int mode) { return map_step_group(mi, opt, n_threads, s, mode, 0, 1, 0, 0); }
+/* the mode of mm_b200_map_batch(es): 0 stage, upload and map; 1 stage and upload; 2 map what mode 1 left resident */
+static int mode_ops(int mode) { return mode == 1 ? SH_STAGE | SH_SEND : mode == 2 ? SH_MAP : SH_STAGE | SH_SEND | SH_MAP; }
 
-static int step_map(pipeline_t *p, step_t *s) { return map_step(p->mi, p->opt, p->n_threads, s, 0); }
+static int step_map(pipeline_t *p, step_t *s) { return map_step_group(p->mi, p->opt, p->n_threads, s, SH_STAGE | SH_SEND | SH_MAP, 0, 1, 0); }
 
 /* Several mini-batches, two in flight: batch i runs on lane group i % 2 of every GPU, so the upload, the latency-bound tails
  * (the serial replays of a few repeat-family fragments) and the host finish of one batch run under the kernels of the other.
@@ -716,7 +707,7 @@ typedef struct { mb_arg_t *a; int i, slot, n_threads; } mb_stage_t;
 static void *map_batches_stage(void *data)
 { /* host staging of batch i into the pinned slot the lane group does not map from */
 	mb_stage_t *t = (mb_stage_t*)data;
-	map_step_group(t->a->mi, t->a->opt, t->n_threads, t->a->b[t->i], 1, t->a->group, t->a->n_groups, t->slot, 1);
+	map_step_group(t->a->mi, t->a->opt, t->n_threads, t->a->b[t->i], SH_STAGE, t->a->group, t->a->n_groups, t->slot);
 	return 0;
 }
 
@@ -726,7 +717,7 @@ static void *map_batches_main(void *data)
 	int i, slot = 0;
 	if (a->mode != 0) { /* upload only / map resident: nothing to overlap */
 		for (i = a->group; i < a->n; i += a->n_groups)
-			if (map_step_group(a->mi, a->opt, a->n_threads, a->b[i], a->mode, a->group, a->n_groups, 0, 0) != 0) a->rc = -1;
+			if (map_step_group(a->mi, a->opt, a->n_threads, a->b[i], mode_ops(a->mode), a->group, a->n_groups, 0) != 0) a->rc = -1;
 		return 0;
 	}
 	{ mb_stage_t t0 = {a, a->group, 0, a->n_threads}; if (a->group < a->n) map_batches_stage(&t0); }
@@ -735,7 +726,7 @@ static void *map_batches_main(void *data)
 		pthread_t tid;
 		mb_stage_t t = {a, nx, slot ^ 1, a->n_threads > 2 ? a->n_threads / 2 : 1};
 		if (nx < a->n) pthread_create(&tid, 0, map_batches_stage, &t); /* the next batch of this group is staged while this one is mapped */
-		if (map_step_group(a->mi, a->opt, a->n_threads, a->b[i], 0, a->group, a->n_groups, slot, 2) != 0) a->rc = -1;
+		if (map_step_group(a->mi, a->opt, a->n_threads, a->b[i], SH_SEND | SH_MAP, a->group, a->n_groups, slot) != 0) a->rc = -1;
 		if (nx < a->n) pthread_join(tid, 0);
 	}
 	return 0;
@@ -930,7 +921,7 @@ static void *mapper_main(void *a)
 	int i;
 	while ((s = slot_get(m->in)) != 0) {
 		const long idx = s->order;
-		if (!p->failed && map_step_group(p->mi, p->opt, m->n_threads, s, 0, m->group, m->lane_groups, 0, 0) != 0) p->failed = 1;
+		if (!p->failed && map_step_group(p->mi, p->opt, m->n_threads, s, SH_STAGE | SH_SEND | SH_MAP, m->group, m->lane_groups, 0) != 0) p->failed = 1;
 		pthread_mutex_lock(&m->turn->mu);
 		while (m->turn->turn != idx) pthread_cond_wait(&m->turn->cv, &m->turn->mu);
 		pthread_mutex_unlock(&m->turn->mu);
@@ -1076,8 +1067,8 @@ void mm_map_frag(const mm_idx_t *mi, int n_segs, const int *qlens, const char **
 	mm_mapopt_to_dev(&o2, &sh.dopt);
 	sh.n_threads = 1, sh.f0 = 0, sh.f1 = 1;
 	sh.seq = seq, sh.n_seg = &n_seg, sh.seg_off = &one_off, sh.n_reg = n_regs, sh.rep_len = rep, sh.frag_gap = gap, sh.reg = regs;
-	shard_upload(&sh);
-	map_shard(&sh);
+	sh.ops = SH_STAGE | SH_SEND | SH_MAP;
+	shard_run(&sh);
 	if (sh.rc) { fprintf(stderr, "[ERROR] mapping failed; no CPU fallback exists\n"); exit(1); }
 	if (b) b->rep_len = rep[0], b->frag_gap = gap[0];
 	for (j = 0; j < n_segs; ++j) free(seq[j].seq);
@@ -1140,7 +1131,7 @@ void mm_b200_batch_info(const mm_b200_batch_t *b, int *n_seq, int *n_frag, int64
 
 int mm_b200_map_batch(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_threads, mm_b200_batch_t *b, int mode)
 {
-	return map_step(mi, opt, n_threads > 1 ? n_threads : 1, (step_t*)b, mode);
+	return map_step_group(mi, opt, n_threads > 1 ? n_threads : 1, (step_t*)b, mode_ops(mode), 0, 1, 0);
 }
 
 /* drop the hits of a mapped batch so that it can be mapped again */

@@ -57,7 +57,7 @@ struct mm_idx_bucket_s {
 	int dev_id[16];
 	mmg_ctx_t *ctx[16 * MM_B200_MAX_LANES]; /* ctx[d * lanes + lane]: own stream and arenas, same device */
 	mmg_idx_t *didx[16];
-	struct { const void *batch; int f0, f1, n_seq; uint64_t n_bases; } staged[16 * MM_B200_MAX_LANES][2]; /* what the ctx's staging slots hold (mm_b200_map_batches) */
+	struct { const void *batch; int f0, f1; } staged[16 * MM_B200_MAX_LANES][MMG_STAGE_SLOTS]; /* which shard the ctx's staging slots hold */
 	pthread_mutex_t up_token[16];  /* device path: the shards of a GPU stage their reads one after the other */
 	pthread_mutex_t gpu_token[16]; /* with lanes > 1: one shard per GPU runs device stages at a time, the others do their host stages */
 	int32_t max_occ_cache_set; float max_occ_cache_f; int32_t max_occ_cache;

@@ -155,6 +155,11 @@ typedef struct {            /* one mini-batch of fragments: inputs are HOST poin
 	const uint64_t *seq_off;/* [n_seq] offset of each read in `bases` */
 	const char *bases;      /* concatenated ASCII reads, original orientation */
 	uint64_t n_bases;
+	/* [n_seq] 1 = reverse-complement the read before mapping, whatever fragment it is in (--no-pairing, map.c:458-498: the mates
+	 * of a pair are flipped as for a pair but mapped one by one); null: the mates are flipped per pe_ori within each fragment */
+	const uint8_t *flip;
+	/* [n_frag] unit keys (see "name keys"), which the self/dual filters need; null: the batch has none */
+	const uint32_t *ukey;
 } mmg_batch_t;
 
 typedef struct {            /* per-fragment chaining output, HOST arrays owned by the ctx (valid until the next batch call) */
@@ -175,28 +180,27 @@ typedef struct {            /* per-fragment chaining output, HOST arrays owned b
 /* upload + encode reads (mate flip per pe_ori, map.c:467-469), then sketch -> seed -> chain (+ re-chain) */
 int  mmg_seed_chain_batch(mmg_ctx_t *ctx, const mmg_idx_t *idx, const mmg_mapopt_t *opt, const mmg_batch_t *batch,
                           mmg_chains_t *out);
-/* same, split so that a caller can time device-resident work separately */
+/* Uploads go through the ctx's MMG_STAGE_SLOTS pinned staging slots.  A caller fills a slot with mmg_stage and uploads it
+ * with mmg_upload_stage, so that it can fill one slot for its next batch while the batch uploaded from the other is mapped.
+ * mmg_stage first waits until the device has read what the slot's last upload copied, so the host never overwrites data a
+ * copy still reads.  The upload makes its batch the resident one: it replaces the previous batch, flips and unit keys included.
+ * mmg_seed_chain_resident refuses (MMG_EINVAL) options with MM_F_NO_DIAG or MM_F_NO_DUAL when the index has no target keys
+ * or the batch was uploaded without unit keys. */
+#define MMG_STAGE_SLOTS 2
+typedef struct {            /* writable pinned arrays of one staging slot, laid out as the fields of mmg_batch_t */
+	char *bases;            /* [n_bases] */
+	int32_t *seq_len;       /* [n_seq] */
+	uint64_t *seq_off;      /* [n_seq] */
+	int32_t *n_seg, *seg_off; /* [n_frag] */
+	uint8_t *flip;          /* [n_seq] when asked for, else null */
+	uint32_t *ukey;         /* [n_frag] when asked for, else null */
+} mmg_stage_t;
+int  mmg_stage(mmg_ctx_t *ctx, int slot, int n_frag, int n_seq, uint64_t n_bases, int with_flip, int with_ukey, mmg_stage_t *out);
+/* upload what the slot holds and encode the reads (mate flip per the slot's flip table or pe_ori, map.c:467-469) */
+int  mmg_upload_stage(mmg_ctx_t *ctx, const mmg_mapopt_t *opt, int slot);
+/* the upload half of mmg_seed_chain_batch, so that a caller can time device-resident work separately: the batch's host arrays
+ * are copied into slot 0 (mmg_stage), then uploaded from there */
 int  mmg_batch_upload(mmg_ctx_t *ctx, const mmg_mapopt_t *opt, const mmg_batch_t *batch);
-/* pinned staging buffer of the ctx: fill it with the concatenated reads and pass it as batch->bases to skip one host copy */
-void *mmg_staging(mmg_ctx_t *ctx, size_t bytes);
-/* pinned arrays of the ctx for the four tables of mmg_batch_t (seq_len and seq_off with n_seq entries, n_seg and seg_off with n_frag):
- * fill them and pass the same pointers in the batch to skip another host copy */
-int  mmg_staging_tables(mmg_ctx_t *ctx, int n_seq, int n_frag, int32_t **seq_len, uint64_t **seq_off, int32_t **n_seg, int32_t **seg_off);
-/* the same with an explicit slot (0 or 1): a caller can fill slot 1 for its next batch while the batch staged in slot 0 is mapped */
-void *mmg_staging_slot(mmg_ctx_t *ctx, int slot, size_t bytes);
-int  mmg_staging_tables_slot(mmg_ctx_t *ctx, int slot, int n_seq, int n_frag, int32_t **seq_len, uint64_t **seq_off, int32_t **n_seg, int32_t **seg_off);
-/* mmg_batch_upload with the flip of every read given (flip[n_seq]: 1 = reverse-complement the read before mapping) instead of
- * derived from pe_ori and each fragment's segment count.  For batches whose fragments are single reads cut from pairs
- * (--no-pairing, map.c:458-498): the mates are still flipped as for a pair, but mapped one by one. */
-int  mmg_batch_upload_flips(mmg_ctx_t *ctx, const mmg_mapopt_t *opt, const mmg_batch_t *batch, const uint8_t *flip);
-/* pinned array of the ctx for that flip table in slot 0 or 1 (n_seq bytes): fill it and pass it to skip a host copy */
-int  mmg_staging_flips_slot(mmg_ctx_t *ctx, int slot, int n_seq, uint8_t **flip);
-/* unit keys (see "name keys") of the n_frag fragments of the batch just uploaded; an upload discards the keys of the batch before.
- * mmg_seed_chain_resident refuses (MMG_EINVAL) options with MM_F_NO_DIAG or MM_F_NO_DUAL when either key table is missing. */
-int  mmg_batch_set_name_keys(mmg_ctx_t *ctx, int n_frag, const uint32_t *ukey);
-/* pinned array of the ctx for those keys in slot 0 or 1 (n_frag entries): fill it and pass it to skip a host copy */
-int  mmg_staging_name_keys_slot(mmg_ctx_t *ctx, int slot, int n_frag, uint32_t **ukey);
-/* page-locked job / result arrays owned by the ctx (kept across batches) for mmg_ksw_batch; plain malloc'd arrays work too, slower */
 
 int  mmg_seed_chain_resident(mmg_ctx_t *ctx, const mmg_idx_t *idx, const mmg_mapopt_t *opt, mmg_chains_t *out, int download);
 
@@ -219,6 +223,7 @@ int  mmg_ksw_batch(mmg_ctx_t *ctx, const mmg_idx_t *idx, const mmg_mapopt_t *opt
                    mmg_ksw_res_t *res, const uint32_t **cigars, double *kernel_ms, uint64_t *cells);
 /* jobs and true-band cells the last mmg_ksw_batch() ran in the thread-per-job fast form (band never clips) and in the literal 16-lane form */
 void mmg_ksw_last_split(const mmg_ctx_t *ctx, uint64_t *jobs_fast, uint64_t *cells_fast, uint64_t *jobs_literal, uint64_t *cells_literal);
+/* page-locked job / result arrays owned by the ctx (kept across batches) for mmg_ksw_batch; plain malloc'd arrays work too, slower */
 int  mmg_job_buffers(mmg_ctx_t *ctx, size_t n_jobs, mmg_ksw_job_t **jobs, mmg_ksw_res_t **res);
 
 /* ------------------------------------------- post-chaining stages on the device (short-read presets)

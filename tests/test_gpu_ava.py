@@ -100,13 +100,34 @@ def test_batch_chains_equal_oracle(gpu, mode):
             assert int(ch["rechained"].sum()) > 0
 
 
-def test_missing_keys_refused(gpu):
+def test_flips_and_names_in_one_upload(gpu):
+    """a flip table and unit keys in one upload: the queries uploaded reverse-complemented, every flip set, chain exactly as the
+    queries as read, both under their names, and the name filters drop the same hits"""
+    api, ctx, idx, T, queries = gpu
+    opt = api.ont_opt(1000)
+    opt.flag |= A.MM_F_NO_DIAG | A.MM_F_NO_DUAL | A.MM_F_HEAP_SORT
+    names = [n for n, _ in queries]
+    runs = []
+    for frags, flips in (([[q] for _, q in queries], None), ([[L.revcomp(q)] for _, q in queries], np.ones(len(queries), np.uint8))):
+        batch, keep = api.Context.make_batch(frags)
+        ctx.path_counts(reset=True)
+        ctx.batch_upload(opt, batch, flips=flips, names=names, idx=idx)
+        runs.append((api.chains_to_py(ctx.seed_chain_resident(idx, opt, True)), int(ctx.path_counts()[7])))
+    (want, want_named), (got, got_named) = runs
+    for k in ("n_u", "n_a", "rep_len", "n_mini", "rechained", "u_off", "a_off", "mini_off"):
+        assert np.array_equal(got[k], want[k]), k
+    assert got["u"].tobytes() == want["u"].tobytes() and got["a"].tobytes() == want["a"].tobytes()
+    assert np.array_equal(got["mini_pos"], want["mini_pos"])
+    assert got_named == want_named > 0 and int(want["n_u"].sum()) > 0
+
+
+def test_missing_name_keys_refused(gpu):
     api, ctx, idx, T, queries = gpu
     opt = api.ont_opt(1000)
     opt.flag |= A.MM_F_NO_DUAL
     batch, keep = api.Context.make_batch([[q] for _, q in queries])
     ctx.batch_upload(opt, batch)  # no unit keys for this batch
-    with pytest.raises(api.MmgError, match="mmg_batch_set_name_keys"):
+    with pytest.raises(api.MmgError, match=r"mmg_batch_t\.ukey"):
         ctx.seed_chain_resident(idx, opt, True)
     bare = api.Index(ctx, T.seqs, A.W, A.K)  # no target keys
     try:

@@ -52,7 +52,7 @@ def _write_rc(src, dst):
 # ---------------------------------------------------------------------------------------------------- device layer
 
 def test_device_flips_from_table():
-    """mmg_batch_upload_flips: single-read fragments whose flips come from a table chain exactly as the same reads uploaded
+    """mmg_batch_t.flip: single-read fragments whose flips come from a table chain exactly as the same reads uploaded
     already reverse-complemented (K1-K3 and the re-chain pass see one-segment units)."""
     import airlift_b200.api as api
     from test_oracle_vs_ref import _mk_ref, _frags
