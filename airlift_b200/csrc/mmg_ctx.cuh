@@ -158,6 +158,11 @@ struct mmg_ctx_s {
 // use, both slots grow together: page-locking is slow and synchronises the device, so it should happen once, not per slot.
 int mmg_stage_grow(mmg_ctx_t *c, int slot, PinBuf StageSlot::*buf, size_t bytes);
 
+// allow the kernels of mmg_ksw.cu / mmg_stages.cu that launch with more than 48 KB of dynamic shared memory to do so on the
+// current device: kernel attributes belong to a device, so mmg_init sets them for every context
+int mmg_ksw_set_smem_attrs();
+int mmg_stages_set_smem_attrs();
+
 #define MMG_LAUNCH(ctx, kern, grid, block, smem, ...) MMG_LAUNCH_AS(ctx, #kern, kern, grid, block, smem, __VA_ARGS__)
 // the same under a given profile name (the instantiations of one kernel template share their template's name)
 #define MMG_LAUNCH_AS(ctx, label, kern, grid, block, smem, ...) do { \

@@ -31,6 +31,8 @@ extern "C" int mmg_init(int device, mmg_ctx_t **out)
 	if (n <= 0) { mmg_set_error("no CUDA device: this library has no CPU path"); return MMG_ENODEV; }
 	if (device < 0 || device >= n) { mmg_set_error("device %d out of range (%d present)", device, n); return MMG_EINVAL; }
 	MMG_CUDA(cudaSetDevice(device));
+	MMG_TRY(mmg_ksw_set_smem_attrs());
+	MMG_TRY(mmg_stages_set_smem_attrs());
 	mmg_ctx_t *c = new mmg_ctx_s();
 	c->dev = device;
 	MMG_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));

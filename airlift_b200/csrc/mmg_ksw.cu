@@ -1,11 +1,14 @@
 // mmg_ksw.cu -- K4: batched ksw_extd2 (ksw2_extd2_sse.c:19-393) on the device.
 //
-// One DP job is run by a group of 16 lanes -- one lane per int8 lane of the reference's SSE
-// registers -- so that the widened 16-lane band, the stale out-of-band lanes and the block
-// boundary carry-in rule (SURVEY.md H5) are reproduced by construction.  The lane arrays
-// u|v|x|y|x2|y2|s|sf|qr keep the reference's memory order (ksw2_extd2_sse.c:99-102); they live
-// in shared memory when a job is small enough (all short-read jobs) and in a global arena
-// otherwise.  Neighbour lanes are exchanged with width-16 shuffles instead of byte shifts.
+// k_ksw_prep puts every job into one of four forms by its shape; jobs are sorted by form and size and each form is one launch:
+//  - fast (k_ksw_tpj): one thread per job whose band never clips, in size classes whose state fits shared memory;
+//  - wavefront (k_ksw_wave): one warp per job whose band never clips but which is too large for the fast classes;
+//  - literal warp (k_ksw_dpx): every other job, one warp each, running the SSE program itself so that the widened 16-lane
+//    band, the stale out-of-band lanes and the block boundary carry-in rule (SURVEY.md H5) are reproduced by construction.
+//    The lane arrays keep the reference's order (ksw2_extd2_sse.c:99-102) with two cells per lane on 16x2 SIMD
+//    (mmg_kswdpx.h); they live in a shared-memory slot when they fit (all short-read jobs) and in a global arena otherwise;
+//  - literal CTA (k_ksw_dpx_block): the same program for jobs whose state exceeds the warp's slot, one CTA per job with the
+//    state in its shared memory.
 #include <algorithm>
 #include <cub/cub.cuh>
 #include "mmg_ctx.cuh"
@@ -23,24 +26,59 @@ struct KswJobDev {       // a job as the kernel sees it: mmg_ksw_job_t resolved 
 struct KswScore { int32_t m; int8_t mat[25]; int8_t q, e, q2, e2; };
 struct KswResDev { KswEz ez; uint64_t cigar_off; };   // == mmg_ksw_res_t
 
-#define KSW_GROUP 16
-#define KSW_JOBS_PER_BLOCK 8
-#define KSW_SMEM_PER_JOB 4096
+// the device tables every K4 kernel reads and writes, and the scoring.  __restrict__ does not reach the members of a struct: the
+// kernels read the job tables and the sequences through __ldg, the read-only path restrict parameters would give them.
+struct KswTabs {
+	const mmg_ksw_job_t *jobs;
+	const uint32_t *Q, *S;                                // packed reads of the resident batch, packed reference
+	const uint64_t *q_off, *ref_off;                      // base offset of each read in Q, of each contig in S
+	const int32_t *read_len;
+	const uint64_t *mem_off, *p_off, *cig_off;            // per job: its arena slot, traceback and CIGAR (k_ksw_prep sizes, scanned)
+	int8_t *gmem;
+	uint8_t *gp;
+	uint32_t *gcig;
+	KswEz *res;
+	KswScore sc;
+};
+
+__device__ __forceinline__ mmg_ksw_job_t ksw_ldg_job(const mmg_ksw_job_t *p)
+{
+	mmg_ksw_job_t j;
+	static_assert(sizeof(j) % 4 == 0, "a job is 4-byte words");
+#pragma unroll
+	for (int i = 0; i < (int)(sizeof(j) / 4); ++i) reinterpret_cast<int32_t*>(&j)[i] = __ldg(reinterpret_cast<const int32_t*>(p) + i);
+	return j;
+}
+
+// a job as the kernels see it: mmg_ksw_job_t resolved against the resident batch and the index
+__device__ __forceinline__ KswJobDev ksw_job(const KswTabs &t, int ji)
+{
+	const mmg_ksw_job_t hj = ksw_ldg_job(t.jobs + ji);
+	KswJobDev jb;
+	jb.q_base = __ldg(t.q_off + hj.seq_id), jb.q_readlen = __ldg(t.read_len + hj.seq_id), jb.q_rev = hj.q_rev, jb.q_start = hj.q_start, jb.q_len = hj.q_len;
+	jb.t_base = __ldg(t.ref_off + hj.rid) + (uint64_t)hj.t_start, jb.t_len = hj.t_len, jb.reversed = hj.reversed;
+	jb.w = hj.w, jb.zdrop = hj.zdrop, jb.end_bonus = hj.end_bonus, jb.flag = hj.flag;
+	jb.mem_off = __ldg(t.mem_off + ji), jb.p_off = __ldg(t.p_off + ji), jb.cig_off = __ldg(t.cig_off + ji);
+	return jb;
+}
+
 #define KSWDPX_SMEM_PER_JOB 5120    /* pair layout (mmg_kswdpx.h): 14 B per target column + query + 16 */
 #define KSWDPX_JOBS_PER_BLOCK 4     /* one warp per job */
+
+__device__ __forceinline__ int ksw_seq4(const uint32_t *S, uint64_t i) { return __ldg(S + (i >> 3)) >> ((i & 7) << 2) & 0xf; } // mmg_seq4_get
 
 __device__ __forceinline__ uint8_t ksw_qbase(const uint32_t *Q, const KswJobDev &jb, int j)
 { // element j of the query handed to ksw (align.c:691-697,721,761): a slice of qseq0[rev], possibly reversed
 	const int idx = jb.reversed ? jb.q_start + jb.q_len - 1 - j : jb.q_start + j;
-	if (!jb.q_rev) return (uint8_t)mmg_seq4_get(Q, jb.q_base + idx);
-	const int c = mmg_seq4_get(Q, jb.q_base + (jb.q_readlen - 1 - idx)); // align.c:869
+	if (!jb.q_rev) return (uint8_t)ksw_seq4(Q, jb.q_base + idx);
+	const int c = ksw_seq4(Q, jb.q_base + (jb.q_readlen - 1 - idx)); // align.c:869
 	return (uint8_t)(c < 4 ? 3 - c : 4);
 }
 
 __device__ __forceinline__ uint8_t ksw_tbase(const uint32_t *S, const KswJobDev &jb, int i)
 {
 	const int ti = jb.reversed ? jb.t_len - 1 - i : i;
-	return (uint8_t)mmg_seq4_get(S, jb.t_base + ti); // mm_idx_getseq, index.c:152-162
+	return (uint8_t)ksw_seq4(S, jb.t_base + ti); // mm_idx_getseq, index.c:152-162
 }
 
 __device__ __forceinline__ int ksw_ncol(int qlen, int tlen, int w)
@@ -53,18 +91,18 @@ __device__ __forceinline__ int ksw_ncol(int qlen, int tlen, int w)
 // Fast-form size classes: a job whose band never clips runs one-thread-per-job (k_ksw_tpj) in the first class it fits:
 // min(qlen,tlen) <= mc (depth of the circular state window), tlen <= tc, qlen <= qc; nt = threads (jobs) per CTA.
 #define KSW_N_FAST 3
-#define KSW_CLS_LITERAL KSW_N_FAST            /* literal form, 16 lanes per job */
-#define KSW_CLS_LITERAL_WIDE (KSW_N_FAST + 1)  /* literal form, 32 lanes per job: bands wider than two SSE blocks */
-#define KSW_CLS_BLOCK1 (KSW_N_FAST + 2)        /* literal form, one CTA per job: state too large for the warp kernel's shared-memory slot */
-#define KSW_CLS_BLOCK2 (KSW_N_FAST + 3)        /* the same with up to KSWB_SMEM2 bytes of state */
-#define KSW_CLS_WAVE (KSW_N_FAST + 4)          /* wavefront form: one warp per large job whose band never clips */
-#define KSW_N_CLS (KSW_N_FAST + 5)
+#define KSW_CLS_LITERAL KSW_N_FAST            /* literal form, one warp per job */
+#define KSW_CLS_BLOCK1 (KSW_N_FAST + 1)        /* literal form, one CTA per job: state too large for the warp kernel's shared-memory slot */
+#define KSW_CLS_BLOCK2 (KSW_N_FAST + 2)        /* the same with up to KSWB_SMEM2 bytes of state */
+#define KSW_CLS_WAVE (KSW_N_FAST + 3)          /* wavefront form: one warp per large job whose band never clips */
+#define KSW_N_CLS (KSW_N_FAST + 4)
 #define KSWB_WARPS 8                           /* warps of the CTA form */
 #define KSWB_MAXG 2                            /* groups of four SSE blocks per warp and anti-diagonal: bands up to 64 blocks */
 #define KSWB_SMEM1 (48 * 1024)
 #define KSWB_SMEM2 (200 * 1024)
 struct KswFastClass { int32_t mc, tc, qc, nt; };
 struct KswFastTab { KswFastClass c[KSW_N_FAST]; };
+static const KswFastTab ksw_ftab = {{{24, 56, 56, 128}, {48, 104, 104, 128}, {80, 160, 160, 64}}};
 // per thread: the window of pair slots (mmg_kswfast2.h), the target bases, the query bases with a padding element at either end
 // (the target bases are read from the packed reference when a cell enters: keeping them too cost a resident CTA per SM)
 static inline size_t ksw_fast_smem(const KswFastClass &k) { return (size_t)k.nt * ((size_t)((k.mc >> 1) + 3) * 16 + (size_t)k.qc + 2); }
@@ -115,19 +153,12 @@ __global__ void k_ksw_prep(const mmg_ksw_job_t *__restrict__ jobs, int n, KswSco
 					const uint64_t est = (uint64_t)qlen * (uint64_t)tlen;
 					k = (uint32_t)cls << 28 | (63u - (uint32_t)(63 - __clzll((long long)(est | 1))));
 				} else if (cls == KSW_CLS_LITERAL) {
-					// 32 lanes pay off for wide bands whose lane arrays sit in shared memory (measured: +9 % on the short-read jobs, -5 % on
-					// long-read jobs whose arrays live in the HBM arena)
-					{ int bw = qlen < tlen ? qlen : tlen; if (g.w + 1 < bw) bw = g.w + 1;
-					  if (bw > 32 && !g.bail && mmg_ksw_mem_bytes(qlen, tlen) + (size_t)((tlen + 15) / 16) * 64 <= KSW_SMEM_PER_JOB) cls = KSW_CLS_LITERAL_WIDE; }
-					const size_t mem_bytes = mmg_ksw_mem_bytes(qlen, tlen), H_bytes = (size_t)((tlen + 15) / 16) * 64;
-					if (mem_bytes + H_bytes > KSW_SMEM_PER_JOB) m = (mem_bytes + H_bytes + 63) & ~(size_t)63;
-					if (mmg_kswdpx_mem_bytes(qlen, tlen) > KSWDPX_SMEM_PER_JOB) { const size_t md = (mmg_kswdpx_mem_bytes(qlen, tlen) + 63) & ~(size_t)63; if (md > m) m = md; }
+					const size_t md = mmg_kswdpx_mem_bytes(qlen, tlen);
+					if (md > KSWDPX_SMEM_PER_JOB) m = (md + 63) & ~(size_t)63; // state beyond the warp kernel's slot goes to the arena
 					if (!(j.flag & MMG_EZ_SCORE_ONLY)) p = ((uint64_t)(qlen + tlen - 1) * ksw_ncol(qlen, tlen, j.w) + 1) * 16;
-					{ // state beyond the warp kernel's slot: a CTA walks the job with the state in its own shared memory
-						const size_t md = mmg_kswdpx_mem_bytes(qlen, tlen);
-						if (!g.bail && (md > KSWDPX_SMEM_PER_JOB || force_block) && md <= KSWB_SMEM2 && g.n_col_ <= 4 * KSWB_WARPS * KSWB_MAXG)
-							cls = md <= KSWB_SMEM1 ? KSW_CLS_BLOCK1 : KSW_CLS_BLOCK2, m = 0;
-					}
+					// or, when it fits, a CTA walks the job with the state in its own shared memory
+					if (!g.bail && (md > KSWDPX_SMEM_PER_JOB || force_block) && md <= KSWB_SMEM2 && g.n_col_ <= 4 * KSWB_WARPS * KSWB_MAXG)
+						cls = md <= KSWB_SMEM1 ? KSW_CLS_BLOCK1 : KSW_CLS_BLOCK2, m = 0;
 					const uint64_t est = (uint64_t)(qlen + tlen) * (uint64_t)(qlen < tlen ? qlen : tlen);
 					k = (uint32_t)cls << 28 | (63u - (uint32_t)(63 - __clzll((long long)(est | 1)))); // big jobs first
 				} else {
@@ -150,192 +181,11 @@ __global__ void k_ksw_prep(const mmg_ksw_job_t *__restrict__ jobs, int n, KswSco
 	if ((threadIdx.x & 31) == 0 && cells) atomicAdd(cells_total, cells);
 }
 
-// G lanes walk one job: 16 (one SSE register per step, two jobs per warp) or 32 (two neighbouring 16-lane blocks per step,
-// one job per warp: fewer steps per anti-diagonal and no divergence between two jobs for the wide bands of the large jobs)
-template <int kMode, int G>
-__device__ __forceinline__ void ksw_run(const KswGeom &g, const KswJobDev &jb, int8_t *mem, int32_t *H, uint8_t *p, KswEz &ez,
-                                        const int lane, const unsigned gmask)
-{
-	const int l16 = lane & 15, half = lane >> 4; // lane inside its 16-lane block; which block of the pair (always 0 when G == 16)
-	const int tl16 = g.tlen_ * 16;
-	int8_t *u = mem, *v = u + tl16, *x = v + tl16, *y = x + tl16, *x2 = y + tl16, *y2 = x2 + tl16, *s = y2 + tl16;
-	const uint8_t *sf = reinterpret_cast<const uint8_t*>(s + tl16), *qr = sf + tl16;
-	const int qlen = g.qlen, tlen = g.tlen, flag = jb.flag;
-	const bool approx = (flag & MMG_EZ_APPROX_MAX) != 0;
-	int last_st = -1, last_en = -1;
-	int32_t H0 = 0, last_H0_t = 0;
-	for (int r = 0; r < qlen + tlen - 1; ++r) {
-		int st0, en0;
-		if (!mmg_ksw_band(g, r, &st0, &en0)) { ez.zdropped = 1; break; }
-		const int st = st0 / 16 * 16, en = (en0 + 16) / 16 * 16 - 1;
-		int x1, x21, v1;
-		if (st > 0) {
-			if (st - 1 >= last_st && st - 1 <= last_en) x1 = x[st - 1], x21 = x2[st - 1], v1 = v[st - 1];
-			else x1 = -g.q - g.e, x21 = -g.q2 - g.e2, v1 = -g.q - g.e;
-		} else {
-			x1 = -g.q - g.e, x21 = -g.q2 - g.e2;
-			v1 = mmg_ksw_first_col(g, r);
-		}
-		if (en >= r && lane == 0) {
-			y[r] = (int8_t)(-g.q - g.e), y2[r] = (int8_t)(-g.q2 - g.e2);
-			u[r] = (int8_t)mmg_ksw_first_col(g, r);
-		}
-		{ // scores, 16-byte chunks starting at st0 (ksw2_extd2_sse.c:158-172)
-			const uint8_t *qrr = qr + (qlen - 1 - r);
-			for (int t = st0 + half * 16; t <= en0; t += G) s[t + l16] = mmg_ksw_score(g, sf[t + l16], qrr[t + l16]);
-		}
-		__syncwarp(gmask);
-		const int st_ = st / 16, en_ = en / 16;
-		if (G == 16) {
-			for (int blk = st_; blk <= en_; ++blk) {
-				const int i = blk * 16 + lane;
-				const int xo = x[i], vo = v[i], x2o = x2[i];
-				int xt1 = __shfl_up_sync(gmask, xo, 1, 16), vt1 = __shfl_up_sync(gmask, vo, 1, 16), x2t1 = __shfl_up_sync(gmask, x2o, 1, 16);
-				if (lane == 0) xt1 = x1, vt1 = v1, x2t1 = x21;
-				x1 = __shfl_sync(gmask, xo, 15, 16);
-				v1 = __shfl_sync(gmask, vo, 15, 16);
-				x21 = __shfl_sync(gmask, x2o, 15, 16);
-				const KswCell c = mmg_ksw_cell<kMode>(g, s[i], (int8_t)xt1, (int8_t)vt1, u[i], y[i], (int8_t)x2t1, y2[i]);
-				u[i] = c.u, v[i] = c.v, x[i] = c.x, y[i] = c.y, x2[i] = c.x2, y2[i] = c.y2;
-				if (kMode) p[((size_t)r * g.n_col_ + (blk - st_)) * 16 + lane] = c.d;
-			}
-		} else {
-			for (int bp = st_ >> 1; bp <= en_ >> 1; ++bp) { // blocks 2bp and 2bp+1 side by side; a block outside [st_, en_] sits out
-				const int blk = bp * 2 + half, i = bp * 32 + lane;
-				const bool act = blk >= st_ && blk <= en_;
-				int xo = 0, vo = 0, x2o = 0;
-				if (act) xo = x[i], vo = v[i], x2o = x2[i];
-				int xt1 = __shfl_up_sync(gmask, xo, 1, 32), vt1 = __shfl_up_sync(gmask, vo, 1, 32), x2t1 = __shfl_up_sync(gmask, x2o, 1, 32);
-				// lane 0 of the band's first block takes the carry-in; so does the first lane of every pair (old values of the pair before)
-				if (lane == 0 || (lane == 16 && blk == st_)) xt1 = x1, vt1 = v1, x2t1 = x21;
-				x1 = __shfl_sync(gmask, xo, 31, 32);
-				v1 = __shfl_sync(gmask, vo, 31, 32);
-				x21 = __shfl_sync(gmask, x2o, 31, 32);
-				if (act) {
-					const KswCell c = mmg_ksw_cell<kMode>(g, s[i], (int8_t)xt1, (int8_t)vt1, u[i], y[i], (int8_t)x2t1, y2[i]);
-					u[i] = c.u, v[i] = c.v, x[i] = c.x, y[i] = c.y, x2[i] = c.x2, y2[i] = c.y2;
-					if (kMode) p[((size_t)r * g.n_col_ + (blk - st_)) * 16 + l16] = c.d;
-				}
-			}
-		}
-		__syncwarp(gmask);
-		if (!approx) { // exact max over the band with the reference's tie order (ksw2_extd2_sse.c:315-358)
-			int32_t max_H, max_t, H_en0;
-			if (r > 0) {
-				H_en0 = en0 > 0 ? H[en0 - 1] + u[en0] : H[en0] + v[en0];
-				__syncwarp(gmask);
-				int32_t bh = H_en0, bt = en0; uint32_t br = 0;
-				for (int t = st0 + lane; t < en0; t += G) {
-					const int32_t h = H[t] + v[t];
-					H[t] = h;
-					const uint32_t rk = mmg_ksw_max_rank(t, st0, en0);
-					if (h > bh || (h == bh && rk < br)) bh = h, bt = t, br = rk;
-				}
-				if (lane == 0) H[en0] = H_en0;
-#pragma unroll
-				for (int d = G / 2; d >= 1; d >>= 1) {
-					const int32_t oh = __shfl_xor_sync(gmask, bh, d, G), ot = __shfl_xor_sync(gmask, bt, d, G);
-					const uint32_t orank = __shfl_xor_sync(gmask, br, d, G);
-					if (oh > bh || (oh == bh && orank < br)) bh = oh, bt = ot, br = orank;
-				}
-				max_H = bh, max_t = bt;
-			} else {
-				H_en0 = v[0] - g.qe_pre;
-				if (lane == 0) H[0] = H_en0;
-				max_H = H_en0, max_t = 0;
-			}
-			__syncwarp(gmask);
-			if (en0 == tlen - 1 && H_en0 > ez.mte) ez.mte = H_en0, ez.mte_q = r - en;
-			if (r - st0 == qlen - 1) { const int32_t hs = H[st0]; if (hs > ez.mqe) ez.mqe = hs, ez.mqe_t = st0; }
-			if (mmg_ksw_zdrop(&ez, max_H, r, max_t, jb.zdrop, g.e2)) break;
-			if (r == qlen + tlen - 2 && en0 == tlen - 1) ez.score = H[tlen - 1];
-		} else { // ksw2_extd2_sse.c:359-375
-			if (r > 0) {
-				if (last_H0_t >= st0 && last_H0_t <= en0 && last_H0_t + 1 >= st0 && last_H0_t + 1 <= en0) {
-					const int32_t d0 = v[last_H0_t], d1 = u[last_H0_t + 1];
-					if (d0 > d1) H0 += d0;
-					else H0 += d1, ++last_H0_t;
-				} else if (last_H0_t >= st0 && last_H0_t <= en0) {
-					H0 += v[last_H0_t];
-				} else {
-					++last_H0_t, H0 += u[last_H0_t];
-				}
-			} else H0 = v[0] - g.qe_pre, last_H0_t = 0;
-			if ((flag & MMG_EZ_APPROX_DROP) && mmg_ksw_zdrop(&ez, H0, r, last_H0_t, jb.zdrop, g.e2)) break;
-			if (r == qlen + tlen - 2 && en0 == tlen - 1) ez.score = H0;
-		}
-		last_st = st, last_en = en;
-	}
-}
-
-template <int G>
-__global__ void __launch_bounds__(G * KSW_JOBS_PER_BLOCK)
-k_ksw(const mmg_ksw_job_t *__restrict__ jobs, const int32_t *__restrict__ order, int n_jobs, KswScore sc, const uint32_t *__restrict__ Q,
-      const uint32_t *__restrict__ S, const uint64_t *__restrict__ q_off, const int32_t *__restrict__ read_len, const uint64_t *__restrict__ ref_off,
-      const uint64_t *__restrict__ mem_off, const uint64_t *__restrict__ p_off, const uint64_t *__restrict__ cig_off,
-      int8_t *__restrict__ gmem, uint8_t *__restrict__ gp, uint32_t *__restrict__ gcig, KswEz *__restrict__ res)
-{
-	extern __shared__ __align__(16) uint8_t smem[];
-	const int grp = threadIdx.x / G, lane = threadIdx.x % G;
-	const int slot = blockIdx.x * KSW_JOBS_PER_BLOCK + grp;
-	if (slot >= n_jobs) return;
-	const unsigned gmask = G == 32 ? 0xffffffffu : 0xffffu << (threadIdx.x & 16);
-	const int ji = order[slot];
-	const mmg_ksw_job_t hj = jobs[ji];
-	KswJobDev jb;
-	jb.q_base = q_off[hj.seq_id], jb.q_readlen = read_len[hj.seq_id], jb.q_rev = hj.q_rev, jb.q_start = hj.q_start, jb.q_len = hj.q_len;
-	jb.t_base = ref_off[hj.rid] + (uint64_t)hj.t_start, jb.t_len = hj.t_len, jb.reversed = hj.reversed;
-	jb.w = hj.w, jb.zdrop = hj.zdrop, jb.end_bonus = hj.end_bonus, jb.flag = hj.flag;
-	jb.mem_off = mem_off[ji], jb.p_off = p_off[ji], jb.cig_off = cig_off[ji];
-	const KswGeom g = mmg_ksw_geom(jb.q_len, jb.t_len, sc.m, sc.mat, sc.q, sc.e, sc.q2, sc.e2, jb.w);
-	KswEz ez;
-	mmg_ksw_reset(&ez);
-	if (g.bail) { if (lane == 0) res[ji] = ez; return; }
-	const int tl16 = g.tlen_ * 16;
-	const size_t mem_bytes = mmg_ksw_mem_bytes(jb.q_len, jb.t_len), H_bytes = (size_t)tl16 * 4;
-	int8_t *mem; int32_t *H;
-	if (mem_bytes + H_bytes <= KSW_SMEM_PER_JOB) {
-		mem = reinterpret_cast<int8_t*>(smem + (size_t)grp * KSW_SMEM_PER_JOB);
-		H = reinterpret_cast<int32_t*>(mem + mem_bytes);
-	} else {
-		mem = gmem + jb.mem_off; // arena slot = lane arrays followed by H[] (sized in k_ksw_prep)
-		H = reinterpret_cast<int32_t*>(gmem + jb.mem_off + mem_bytes);
-	}
-	// initial lane state (ksw2_extd2_sse.c:99-121)
-	{
-		int8_t *u = mem;
-		const int8_t n1 = (int8_t)(-g.q - g.e), n2 = (int8_t)(-g.q2 - g.e2);
-		for (int i = lane; i < tl16; i += G) {
-			u[i] = n1, u[tl16 + i] = n1, u[2 * tl16 + i] = n1, u[3 * tl16 + i] = n1; // u v x y
-			u[4 * tl16 + i] = n2, u[5 * tl16 + i] = n2;                              // x2 y2
-			u[6 * tl16 + i] = 0;                                                      // s (kcalloc)
-			u[7 * tl16 + i] = i < jb.t_len ? (int8_t)ksw_tbase(S, jb, i) : 0;         // sf
-			H[i] = MMG_KSW_NEG_INF;
-		}
-		int8_t *qr = u + 8 * tl16;
-		const int qn = g.qlen_ * 16 + 16;
-		for (int i = lane; i < qn; i += G) qr[i] = i < jb.q_len ? (int8_t)ksw_qbase(Q, jb, jb.q_len - 1 - i) : 0;
-	}
-	__syncwarp(gmask);
-	uint8_t *p = gp + jb.p_off;
-	const bool with_cigar = !(jb.flag & MMG_EZ_SCORE_ONLY);
-	if (!with_cigar) ksw_run<0, G>(g, jb, mem, H, p, ez, lane, gmask);
-	else if (!(jb.flag & MMG_EZ_RIGHT)) ksw_run<1, G>(g, jb, mem, H, p, ez, lane, gmask);
-	else ksw_run<2, G>(g, jb, mem, H, p, ez, lane, gmask);
-	__syncwarp(gmask);
-	if (lane == 0) {
-		int i0, j0;
-		if (with_cigar && mmg_ksw_trace_start(g, jb.flag, jb.end_bonus, &ez, &i0, &j0))
-			ez.n_cigar = mmg_ksw_backtrack(g, !!(jb.flag & MMG_EZ_REV_CIGAR), p, i0, j0, gcig + jb.cig_off);
-		res[ji] = ez;
-	}
-}
-
 // ---- K4, literal form on 16x2 SIMD: one warp per job, two adjacent cells per lane (mmg_kswdpx.h) ------------------------
-// The same program as ksw_run above -- widened band, stale lanes, block carry-in, score refresh in 16-byte chunks from st0 with
-// its spill into sf[], exact-max tie order -- with four 16-lane SSE blocks side by side in the warp: lane L holds cells 2(L & 7)
-// and 2(L & 7) + 1 of block st_ + 4 i + (L >> 3) in step i.  (Eight lanes per job, four jobs per warp, was no faster than the
-// byte-lane kernel: jobs of different shapes in one warp diverge and issue one after the other.)
+// The program of ksw2_extd2_sse.c:123-378 -- widened band, stale lanes, block carry-in, score refresh in 16-byte chunks from st0
+// with its spill into sf[], exact-max tie order -- with four 16-lane SSE blocks side by side in the warp: lane L holds cells
+// 2(L & 7) and 2(L & 7) + 1 of block st_ + 4 i + (L >> 3) in step i.  (Eight lanes per job, four jobs per warp, was measured no
+// faster than one lane per SSE byte lane: jobs of different shapes in one warp diverge and issue one after the other.)
 template <int kMode>
 __device__ __forceinline__ void ksw_run_dpx(const KswGeom &g, const KswJobDev &jb, uint8_t *mem, int32_t *H, uint8_t *p, KswEz &ez, const int lane)
 {
@@ -459,31 +309,24 @@ __device__ __forceinline__ void ksw_run_dpx(const KswGeom &g, const KswJobDev &j
 	}
 }
 
-__global__ void __launch_bounds__(32 * KSWDPX_JOBS_PER_BLOCK)
-k_ksw_dpx(const mmg_ksw_job_t *__restrict__ jobs, const int32_t *__restrict__ order, int n_jobs, KswScore sc, const uint32_t *__restrict__ Q,
-          const uint32_t *__restrict__ S, const uint64_t *__restrict__ q_off, const int32_t *__restrict__ read_len, const uint64_t *__restrict__ ref_off,
-          const uint64_t *__restrict__ mem_off, const uint64_t *__restrict__ p_off, const uint64_t *__restrict__ cig_off,
-          int8_t *__restrict__ gmem, uint8_t *__restrict__ gp, uint32_t *__restrict__ gcig, KswEz *__restrict__ res)
+__global__ void __launch_bounds__(32 * KSWDPX_JOBS_PER_BLOCK, 7) // 72 registers: seven CTAs per SM
+k_ksw_dpx(KswTabs t, const int32_t *__restrict__ order, int n_jobs)
 {
 	extern __shared__ __align__(16) uint8_t smem[];
 	const int grp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 	const int slot = blockIdx.x * KSWDPX_JOBS_PER_BLOCK + grp;
 	if (slot >= n_jobs) return;
 	const int ji = order[slot];
-	const mmg_ksw_job_t hj = jobs[ji];
-	KswJobDev jb;
-	jb.q_base = q_off[hj.seq_id], jb.q_readlen = read_len[hj.seq_id], jb.q_rev = hj.q_rev, jb.q_start = hj.q_start, jb.q_len = hj.q_len;
-	jb.t_base = ref_off[hj.rid] + (uint64_t)hj.t_start, jb.t_len = hj.t_len, jb.reversed = hj.reversed;
-	jb.w = hj.w, jb.zdrop = hj.zdrop, jb.end_bonus = hj.end_bonus, jb.flag = hj.flag;
-	jb.mem_off = mem_off[ji], jb.p_off = p_off[ji], jb.cig_off = cig_off[ji];
+	const KswJobDev jb = ksw_job(t, ji);
+	const KswScore sc = t.sc;
 	const KswGeom g = mmg_ksw_geom(jb.q_len, jb.t_len, sc.m, sc.mat, sc.q, sc.e, sc.q2, sc.e2, jb.w);
 	KswEz ez;
 	mmg_ksw_reset(&ez);
-	if (g.bail) { if (lane == 0) res[ji] = ez; return; }
+	if (g.bail) { if (lane == 0) t.res[ji] = ez; return; }
 	const int tl16 = g.tlen_ * 16;
 	const size_t lane_bytes = (mmg_kswdpx_lane_bytes(jb.q_len, jb.t_len) + 15) & ~(size_t)15;
 	uint8_t *mem = mmg_kswdpx_mem_bytes(jb.q_len, jb.t_len) <= KSWDPX_SMEM_PER_JOB ? smem + (size_t)grp * KSWDPX_SMEM_PER_JOB
-	                                                                              : reinterpret_cast<uint8_t*>(gmem) + jb.mem_off; // arena slot sized in k_ksw_prep
+	                                                                              : reinterpret_cast<uint8_t*>(t.gmem) + jb.mem_off; // arena slot sized in k_ksw_prep
 	int32_t *H = reinterpret_cast<int32_t*>(mem + lane_bytes);
 	{ // initial lane state (ksw2_extd2_sse.c:99-121) in the pair layout
 		const uint32_t w1 = 0x01010101u * (uint8_t)(int8_t)(-g.q - g.e), w2 = 0x01010101u * (uint8_t)(int8_t)(-g.q2 - g.e2);
@@ -492,15 +335,15 @@ k_ksw_dpx(const mmg_ksw_job_t *__restrict__ jobs, const int32_t *__restrict__ or
 		int8_t *s = reinterpret_cast<int8_t*>(mem) + (size_t)tl16 * 8;
 		for (int i = lane; i < tl16; i += 32) {
 			s[i] = 0;                                                           // s (kcalloc)
-			s[tl16 + i] = i < jb.t_len ? (int8_t)ksw_tbase(S, jb, i) : 0;       // sf
+			s[tl16 + i] = i < jb.t_len ? (int8_t)ksw_tbase(t.S, jb, i) : 0;     // sf
 			H[i] = MMG_KSW_NEG_INF;
 		}
 		int8_t *qr = s + 2 * tl16;
 		const int qn = g.qlen_ * 16 + 16;
-		for (int i = lane; i < qn; i += 32) qr[i] = i < jb.q_len ? (int8_t)ksw_qbase(Q, jb, jb.q_len - 1 - i) : 0;
+		for (int i = lane; i < qn; i += 32) qr[i] = i < jb.q_len ? (int8_t)ksw_qbase(t.Q, jb, jb.q_len - 1 - i) : 0;
 	}
 	__syncwarp();
-	uint8_t *p = gp + jb.p_off;
+	uint8_t *p = t.gp + jb.p_off;
 	const bool with_cigar = !(jb.flag & MMG_EZ_SCORE_ONLY);
 	if (!with_cigar) ksw_run_dpx<0>(g, jb, mem, H, p, ez, lane);
 	else if (!(jb.flag & MMG_EZ_RIGHT)) ksw_run_dpx<1>(g, jb, mem, H, p, ez, lane);
@@ -509,8 +352,8 @@ k_ksw_dpx(const mmg_ksw_job_t *__restrict__ jobs, const int32_t *__restrict__ or
 	if (lane == 0) {
 		int i0, j0;
 		if (with_cigar && mmg_ksw_trace_start(g, jb.flag, jb.end_bonus, &ez, &i0, &j0))
-			ez.n_cigar = mmg_ksw_backtrack(g, !!(jb.flag & MMG_EZ_REV_CIGAR), p, i0, j0, gcig + jb.cig_off);
-		res[ji] = ez;
+			ez.n_cigar = mmg_ksw_backtrack(g, !!(jb.flag & MMG_EZ_REV_CIGAR), p, i0, j0, t.gcig + jb.cig_off);
+		t.res[ji] = ez;
 	}
 }
 
@@ -669,21 +512,14 @@ __device__ __forceinline__ void ksw_run_dpx_block(const KswGeom &g, const KswJob
 }
 
 __global__ void __launch_bounds__(32 * KSWB_WARPS)
-k_ksw_dpx_block(const mmg_ksw_job_t *__restrict__ jobs, const int32_t *__restrict__ order, int n_jobs, KswScore sc, const uint32_t *__restrict__ Q,
-                const uint32_t *__restrict__ S, const uint64_t *__restrict__ q_off, const int32_t *__restrict__ read_len, const uint64_t *__restrict__ ref_off,
-                const uint64_t *__restrict__ p_off, const uint64_t *__restrict__ cig_off, uint8_t *__restrict__ gp, uint32_t *__restrict__ gcig,
-                KswEz *__restrict__ res)
+k_ksw_dpx_block(KswTabs t, const int32_t *__restrict__ order, int n_jobs)
 {
 	extern __shared__ __align__(16) uint8_t smem[];
 	__shared__ int32_t s_red[3 * KSWB_WARPS];
 	const int tid = threadIdx.x, NT = 32 * KSWB_WARPS;
 	const int ji = order[blockIdx.x];
-	const mmg_ksw_job_t hj = jobs[ji];
-	KswJobDev jb;
-	jb.q_base = q_off[hj.seq_id], jb.q_readlen = read_len[hj.seq_id], jb.q_rev = hj.q_rev, jb.q_start = hj.q_start, jb.q_len = hj.q_len;
-	jb.t_base = ref_off[hj.rid] + (uint64_t)hj.t_start, jb.t_len = hj.t_len, jb.reversed = hj.reversed;
-	jb.w = hj.w, jb.zdrop = hj.zdrop, jb.end_bonus = hj.end_bonus, jb.flag = hj.flag;
-	jb.mem_off = 0, jb.p_off = p_off[ji], jb.cig_off = cig_off[ji];
+	const KswJobDev jb = ksw_job(t, ji);
+	const KswScore sc = t.sc;
 	const KswGeom g = mmg_ksw_geom(jb.q_len, jb.t_len, sc.m, sc.mat, sc.q, sc.e, sc.q2, sc.e2, jb.w);
 	KswEz ez;
 	mmg_ksw_reset(&ez);
@@ -698,15 +534,15 @@ k_ksw_dpx_block(const mmg_ksw_job_t *__restrict__ jobs, const int32_t *__restric
 		int8_t *s = reinterpret_cast<int8_t*>(mem) + (size_t)tl16 * 8;
 		for (int i = tid; i < tl16; i += NT) {
 			s[i] = 0;
-			s[tl16 + i] = i < jb.t_len ? (int8_t)ksw_tbase(S, jb, i) : 0;
+			s[tl16 + i] = i < jb.t_len ? (int8_t)ksw_tbase(t.S, jb, i) : 0;
 			H[i] = MMG_KSW_NEG_INF;
 		}
 		int8_t *qr = s + 2 * tl16;
 		const int qn = g.qlen_ * 16 + 16;
-		for (int i = tid; i < qn; i += NT) qr[i] = i < jb.q_len ? (int8_t)ksw_qbase(Q, jb, jb.q_len - 1 - i) : 0;
+		for (int i = tid; i < qn; i += NT) qr[i] = i < jb.q_len ? (int8_t)ksw_qbase(t.Q, jb, jb.q_len - 1 - i) : 0;
 	}
 	__syncthreads();
-	uint8_t *p = gp + jb.p_off;
+	uint8_t *p = t.gp + jb.p_off;
 	const bool with_cigar = !(jb.flag & MMG_EZ_SCORE_ONLY);
 	if (!with_cigar) ksw_run_dpx_block<0>(g, jb, mem, H, p, ez, s_red);
 	else if (!(jb.flag & MMG_EZ_RIGHT)) ksw_run_dpx_block<1>(g, jb, mem, H, p, ez, s_red);
@@ -715,8 +551,8 @@ k_ksw_dpx_block(const mmg_ksw_job_t *__restrict__ jobs, const int32_t *__restric
 	if (tid == 0) {
 		int i0, j0;
 		if (with_cigar && mmg_ksw_trace_start(g, jb.flag, jb.end_bonus, &ez, &i0, &j0))
-			ez.n_cigar = mmg_ksw_backtrack(g, !!(jb.flag & MMG_EZ_REV_CIGAR), p, i0, j0, gcig + jb.cig_off);
-		res[ji] = ez;
+			ez.n_cigar = mmg_ksw_backtrack(g, !!(jb.flag & MMG_EZ_REV_CIGAR), p, i0, j0, t.gcig + jb.cig_off);
+		t.res[ji] = ez;
 	}
 }
 
@@ -724,10 +560,7 @@ k_ksw_dpx_block(const mmg_ksw_job_t *__restrict__ jobs, const int32_t *__restric
 // threads of a CTA interleave their per-job arrays in shared memory ([element][thread]): a warp's accesses fall on consecutive
 // banks (16-byte pair slots: one LDS.128 / STS.128 per two cells).
 __global__ void __launch_bounds__(128)
-k_ksw_tpj(const mmg_ksw_job_t *__restrict__ jobs, const int32_t *__restrict__ order, int n_jobs, KswScore sc, KswFastClass fc,
-          const uint32_t *__restrict__ Q, const uint32_t *__restrict__ S, const uint64_t *__restrict__ q_off, const int32_t *__restrict__ read_len,
-          const uint64_t *__restrict__ ref_off, const uint64_t *__restrict__ p_off, const uint64_t *__restrict__ cig_off,
-          uint8_t *__restrict__ gp, uint32_t *__restrict__ gcig, KswEz *__restrict__ res)
+k_ksw_tpj(KswTabs t, const int32_t *__restrict__ order, int n_jobs, KswFastClass fc)
 {
 	extern __shared__ __align__(16) uint8_t smem[];
 	const int NT = blockDim.x, tid = threadIdx.x;
@@ -736,19 +569,20 @@ k_ksw_tpj(const mmg_ksw_job_t *__restrict__ jobs, const int32_t *__restrict__ or
 	KswSlot *st = reinterpret_cast<KswSlot*>(smem) + tid;
 	uint8_t *qb = smem + (size_t)((fc.mc >> 1) + 3) * NT * 16 + tid + NT; // qb[-1] and qb[qlen] are padding
 	const int ji = order[slot];
-	const mmg_ksw_job_t hj = jobs[ji];
+	const mmg_ksw_job_t hj = ksw_ldg_job(t.jobs + ji);
 	const int qlen = hj.q_len, tlen = hj.t_len;
+	const KswScore sc = t.sc;
 	const KswGeom g = mmg_ksw_geom(qlen, tlen, sc.m, sc.mat, sc.q, sc.e, sc.q2, sc.e2, hj.w);
 	// target slice of S (mm_idx_getseq, index.c:152-162), reversed for left extensions (align.c:694-695): read base by base as cells enter
-	const uint64_t t_a0 = ref_off[hj.rid] + (uint64_t)hj.t_start;
+	const uint64_t t_a0 = __ldg(t.ref_off + hj.rid) + (uint64_t)hj.t_start;
 	const bool t_rev = hj.reversed != 0;
-	auto tbase = [&](int i) -> uint32_t { const uint64_t a = t_a0 + (uint64_t)(t_rev ? tlen - 1 - i : i); return __ldg(S + (a >> 3)) >> ((a & 7) << 2) & 0xf; };
+	auto tbase = [&](int i) -> uint32_t { const uint64_t a = t_a0 + (uint64_t)(t_rev ? tlen - 1 - i : i); return (uint32_t)ksw_seq4(t.S, a); };
 	{ // query slice of qseq0[q_rev] (align.c:865-870)
-		const uint64_t qbase = q_off[hj.seq_id];
-		const int rl = read_len[hj.seq_id];
+		const uint64_t qbase = __ldg(t.q_off + hj.seq_id);
+		const int rl = __ldg(t.read_len + hj.seq_id);
 		const int lo = hj.q_rev ? rl - hj.q_start - qlen : hj.q_start, hi = lo + qlen;
 		for (int wp = lo >> 3; wp <= (hi - 1) >> 3; ++wp) {
-			const uint32_t word = Q[(qbase >> 3) + wp]; // reads start on 8-base boundaries
+			const uint32_t word = __ldg(t.Q + (qbase >> 3) + wp); // reads start on 8-base boundaries
 #pragma unroll
 			for (int k = 0; k < 8; ++k) {
 				const int pos = wp * 8 + k;
@@ -763,8 +597,8 @@ k_ksw_tpj(const mmg_ksw_job_t *__restrict__ jobs, const int32_t *__restrict__ or
 	}
 	qb[-(ptrdiff_t)NT] = 4, qb[(size_t)qlen * NT] = 4;
 	KswEz ez;
-	mmg_ksw_fast2(g, hj.flag, hj.zdrop, hj.end_bonus, st, tbase, qb - NT, NT, reinterpret_cast<uint32_t*>(gp + p_off[ji]), &ez, gcig + cig_off[ji]);
-	res[ji] = ez;
+	mmg_ksw_fast2(g, hj.flag, hj.zdrop, hj.end_bonus, st, tbase, qb - NT, NT, reinterpret_cast<uint32_t*>(t.gp + __ldg(t.p_off + ji)), &ez, t.gcig + __ldg(t.cig_off + ji));
+	t.res[ji] = ez;
 }
 
 
@@ -867,31 +701,25 @@ MMG_HDN inline int ksw_wave_backtrack(const KswGeom &g, int is_rev, const uint8_
 }
 
 __global__ void __launch_bounds__(32 * KW_WARPS)
-k_ksw_wave(const mmg_ksw_job_t *__restrict__ jobs, const int32_t *__restrict__ order, int n_jobs, KswScore sc, const uint32_t *__restrict__ Q,
-           const uint32_t *__restrict__ S, const uint64_t *__restrict__ q_off, const int32_t *__restrict__ read_len, const uint64_t *__restrict__ ref_off,
-           const uint64_t *__restrict__ mem_off, const uint64_t *__restrict__ p_off, const uint64_t *__restrict__ cig_off,
-           int8_t *__restrict__ gmem, uint8_t *__restrict__ gp, uint32_t *__restrict__ gcig, KswEz *__restrict__ res)
+k_ksw_wave(KswTabs t, const int32_t *__restrict__ order, int n_jobs)
 {
 	const int lane = threadIdx.x & 31, slot = blockIdx.x * KW_WARPS + (threadIdx.x >> 5);
 	if (slot >= n_jobs) return;
 	const int ji = order[slot];
-	const mmg_ksw_job_t hj = jobs[ji];
-	KswJobDev jb;
-	jb.q_base = q_off[hj.seq_id], jb.q_readlen = read_len[hj.seq_id], jb.q_rev = hj.q_rev, jb.q_start = hj.q_start, jb.q_len = hj.q_len;
-	jb.t_base = ref_off[hj.rid] + (uint64_t)hj.t_start, jb.t_len = hj.t_len, jb.reversed = hj.reversed;
-	jb.w = hj.w, jb.zdrop = hj.zdrop, jb.end_bonus = hj.end_bonus, jb.flag = hj.flag;
+	const KswJobDev jb = ksw_job(t, ji);
+	const KswScore sc = t.sc;
 	const KswGeom g = mmg_ksw_geom(jb.q_len, jb.t_len, sc.m, sc.mat, sc.q, sc.e, sc.q2, sc.e2, jb.w);
 	const int qlen = g.qlen, tlen = g.tlen, R = qlen + tlen - 1;
-	unsigned long long *diag = reinterpret_cast<unsigned long long*>(gmem + mem_off[ji]);
+	unsigned long long *diag = reinterpret_cast<unsigned long long*>(t.gmem + jb.mem_off);
 	int32_t *hrow = reinterpret_cast<int32_t*>(diag + (qlen + tlen)), *hcol = hrow + tlen;
 	int4 *edge = reinterpret_cast<int4*>((reinterpret_cast<size_t>(hcol + qlen) + 15) & ~(size_t)15);
-	uint8_t *p2 = gp + p_off[ji];
+	uint8_t *p2 = t.gp + jb.p_off;
 	const bool with_cigar = !(jb.flag & MMG_EZ_SCORE_ONLY), exact = !(jb.flag & MMG_EZ_APPROX_MAX);
 	if (exact) for (int r = lane; r < R; r += 32) diag[r] = 0;
 	__syncwarp();
-	if (!with_cigar) ksw_wave_sweep<0>(g, jb, Q, S, p2, diag, hrow, hcol, edge, exact, lane);
-	else if (!(jb.flag & MMG_EZ_RIGHT)) ksw_wave_sweep<1>(g, jb, Q, S, p2, diag, hrow, hcol, edge, exact, lane);
-	else ksw_wave_sweep<2>(g, jb, Q, S, p2, diag, hrow, hcol, edge, exact, lane);
+	if (!with_cigar) ksw_wave_sweep<0>(g, jb, t.Q, t.S, p2, diag, hrow, hcol, edge, exact, lane);
+	else if (!(jb.flag & MMG_EZ_RIGHT)) ksw_wave_sweep<1>(g, jb, t.Q, t.S, p2, diag, hrow, hcol, edge, exact, lane);
+	else ksw_wave_sweep<2>(g, jb, t.Q, t.S, p2, diag, hrow, hcol, edge, exact, lane);
 	__threadfence_block();
 	__syncwarp();
 	if (lane != 0) return;
@@ -913,8 +741,8 @@ k_ksw_wave(const mmg_ksw_job_t *__restrict__ jobs, const int32_t *__restrict__ o
 	}
 	int i0, j0;
 	if (with_cigar && mmg_ksw_trace_start(g, jb.flag, jb.end_bonus, &ez, &i0, &j0))
-		ez.n_cigar = ksw_wave_backtrack(g, !!(jb.flag & MMG_EZ_REV_CIGAR), p2, ksw_wave_tpad(tlen), i0, j0, gcig + cig_off[ji]);
-	res[ji] = ez;
+		ez.n_cigar = ksw_wave_backtrack(g, !!(jb.flag & MMG_EZ_REV_CIGAR), p2, ksw_wave_tpad(tlen), i0, j0, t.gcig + __ldg(t.cig_off + ji)); // read here: not held across the sweep
+	t.res[ji] = ez;
 }
 
 __global__ void k_res_ncig(int n_jobs, const KswEz *__restrict__ res, int32_t *__restrict__ ncig)
@@ -948,6 +776,17 @@ template <class T> static int scan_excl(mmg_ctx_t *c, const T *d_in, int64_t *d_
 	return MMG_OK;
 }
 
+// the dynamic shared memory the K4 kernels launch with, allowed on the current device (mmg_init, once per context)
+int mmg_ksw_set_smem_attrs()
+{
+	size_t mx = 0;
+	for (int q = 0; q < KSW_N_FAST; ++q) mx = std::max(mx, ksw_fast_smem(ksw_ftab.c[q]));
+	MMG_CUDA(cudaFuncSetAttribute(k_ksw_tpj, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mx));
+	MMG_CUDA(cudaFuncSetAttribute(k_ksw_dpx, cudaFuncAttributeMaxDynamicSharedMemorySize, KSWDPX_SMEM_PER_JOB * KSWDPX_JOBS_PER_BLOCK));
+	MMG_CUDA(cudaFuncSetAttribute(k_ksw_dpx_block, cudaFuncAttributeMaxDynamicSharedMemorySize, KSWB_SMEM2));
+	return MMG_OK;
+}
+
 #define KSW_SPLIT 1 // ksw_launch: the jobs' DP state exceeds the budget given; nothing was run
 
 // d_jobs: n jobs already on the device.  q_off/read_len/ref_off: device tables the jobs index into.  budget: device bytes the
@@ -966,10 +805,9 @@ static int ksw_launch(mmg_ctx_t *c, const mmg_ksw_job_t *d_jobs, int n, const ui
 	uint32_t *d_cls = reinterpret_cast<uint32_t*>(d_cells + 2 + KSW_N_CLS); // d_cells: total, then per class; d_cls: KSW_N_CLS job counters
 	uint32_t *key = d_cls + 8, *key2 = key + n1;
 	int32_t *idx = reinterpret_cast<int32_t*>(key2 + n1), *order = idx + n1, *ncig = order + n1;
-	static const KswFastTab ftab = {{{24, 56, 56, 128}, {48, 104, 104, 128}, {80, 160, 160, 64}}};
 	static const bool force_block = getenv("MMG_KSW_FORCE_BLOCK") != nullptr; // test aid: every literal job the CTA form can take goes through it
 	MMG_CUDA(cudaMemsetAsync(d_cells, 0, (2 + KSW_N_CLS) * 8 + 32, c->stream));
-	MMG_LAUNCH(c, k_ksw_prep, mmg_blocks(n1, 128), 128, 0, d_jobs, n, sc, ftab, mem_sz, p_sz, cig_sz, key, idx, d_cells, d_cls, force_block ? 1 : 0);
+	MMG_LAUNCH(c, k_ksw_prep, mmg_blocks(n1, 128), 128, 0, d_jobs, n, sc, ksw_ftab, mem_sz, p_sz, cig_sz, key, idx, d_cells, d_cls, force_block ? 1 : 0);
 	MMG_TRY(scan_excl(c, mem_sz, mem_off, (int)n1));
 	MMG_TRY(scan_excl(c, p_sz, p_off, (int)n1));
 	MMG_TRY(scan_excl(c, cig_sz, cg_off, (int)n1));
@@ -985,8 +823,8 @@ static int ksw_launch(mmg_ctx_t *c, const mmg_ksw_job_t *d_jobs, int n, const ui
 	MMG_CUDA(cudaStreamSynchronize(c->stream));
 	if (budget && n > 1 && (size_t)(tot[0] + tot[1] + tot[2] * 4) > budget) return KSW_SPLIT;
 	if (cells) *cells = h_cells[0];
-	c->k_last_jobs_literal = h_cls[KSW_CLS_LITERAL] + h_cls[KSW_CLS_LITERAL_WIDE] + h_cls[KSW_CLS_BLOCK1] + h_cls[KSW_CLS_BLOCK2]; // the wavefront form counts as a fast form
-	c->k_last_cells_literal = h_cells[1 + KSW_CLS_LITERAL] + h_cells[1 + KSW_CLS_LITERAL_WIDE] + h_cells[1 + KSW_CLS_BLOCK1] + h_cells[1 + KSW_CLS_BLOCK2];
+	c->k_last_jobs_literal = h_cls[KSW_CLS_LITERAL] + h_cls[KSW_CLS_BLOCK1] + h_cls[KSW_CLS_BLOCK2]; // the wavefront form counts as a fast form
+	c->k_last_cells_literal = h_cells[1 + KSW_CLS_LITERAL] + h_cells[1 + KSW_CLS_BLOCK1] + h_cells[1 + KSW_CLS_BLOCK2];
 	c->k_last_jobs_fast = (uint64_t)n - c->k_last_jobs_literal, c->k_last_cells_fast = h_cells[0] - c->k_last_cells_literal;
 	if (getenv("MMG_KSW_DEBUG")) {
 		fprintf(stderr, "[mmg_ksw] %d jobs, %llu cells:", n, h_cells[0]);
@@ -999,67 +837,28 @@ static int ksw_launch(mmg_ctx_t *c, const mmg_ksw_job_t *d_jobs, int n, const ui
 	MMG_TRY(c->k_res.ensure(((n1 * sizeof(KswEz) + 15) & ~(size_t)15) + n1 * sizeof(KswResDev)));
 	KswEz *d_ez = c->k_res.as<KswEz>();
 	KswResDev *d_res = reinterpret_cast<KswResDev*>(c->k_res.as<uint8_t>() + ((n1 * sizeof(KswEz) + 15) & ~(size_t)15));
+	KswTabs t;
+	t.jobs = d_jobs, t.Q = d_Q, t.S = d_S, t.q_off = d_q_off, t.ref_off = d_ref_off, t.read_len = d_read_len;
+	t.mem_off = reinterpret_cast<const uint64_t*>(mem_off), t.p_off = reinterpret_cast<const uint64_t*>(p_off), t.cig_off = reinterpret_cast<const uint64_t*>(cg_off);
+	t.gmem = c->k_mem.as<int8_t>(), t.gp = c->k_p.as<uint8_t>(), t.gcig = c->k_cig.as<uint32_t>(), t.res = d_ez, t.sc = sc;
 	MMG_CUDA(cudaEventRecord(c->ev[0], c->stream));
-	{
-		static bool attr_set[16] = {false};
-		if (c->dev < 16 && !attr_set[c->dev]) {
-			size_t mx = 0;
-			for (int q = 0; q < KSW_N_FAST; ++q) mx = std::max(mx, ksw_fast_smem(ftab.c[q]));
-			MMG_CUDA(cudaFuncSetAttribute(k_ksw_tpj, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mx));
-			attr_set[c->dev] = true;
-		}
-	}
-	uint32_t first = 0;
-	for (int q = 0; q < KSW_N_FAST; ++q) { // fast-form classes, then the literal 16-lane form for everything else
-		const uint32_t nq = h_cls[q];
-		if (nq)
-			MMG_LAUNCH(c, k_ksw_tpj, mmg_blocks(nq, ftab.c[q].nt), ftab.c[q].nt, ksw_fast_smem(ftab.c[q]), d_jobs, order + first, (int)nq, sc, ftab.c[q],
-			           d_Q, d_S, d_q_off, d_read_len, d_ref_off, reinterpret_cast<const uint64_t*>(p_off), reinterpret_cast<const uint64_t*>(cg_off),
-			           c->k_p.as<uint8_t>(), c->k_cig.as<uint32_t>(), d_ez);
-		first += nq;
-	}
-	static const bool legacy_literal = getenv("MMG_KSW_LEGACY") != nullptr; // the one-lane-per-byte-lane kernels, kept for A/B runs
-	if (!legacy_literal) {
-		static bool dpx_attr[16] = {false};
-		if (c->dev < 16 && !dpx_attr[c->dev]) {
-			MMG_CUDA(cudaFuncSetAttribute(k_ksw_dpx, cudaFuncAttributeMaxDynamicSharedMemorySize, KSWDPX_SMEM_PER_JOB * KSWDPX_JOBS_PER_BLOCK));
-			dpx_attr[c->dev] = true;
-		}
-		const uint32_t nl = h_cls[KSW_CLS_LITERAL] + h_cls[KSW_CLS_LITERAL_WIDE]; // consecutive in the scheduling order
-		if (nl)
-			MMG_LAUNCH(c, k_ksw_dpx, mmg_blocks(nl, KSWDPX_JOBS_PER_BLOCK), 32 * KSWDPX_JOBS_PER_BLOCK, KSWDPX_SMEM_PER_JOB * KSWDPX_JOBS_PER_BLOCK,
-			           d_jobs, order + first, (int)nl, sc, d_Q, d_S, d_q_off, d_read_len, d_ref_off, reinterpret_cast<const uint64_t*>(mem_off),
-			           reinterpret_cast<const uint64_t*>(p_off), reinterpret_cast<const uint64_t*>(cg_off), c->k_mem.as<int8_t>(), c->k_p.as<uint8_t>(),
-			           c->k_cig.as<uint32_t>(), d_ez);
-	}
-	if (legacy_literal && h_cls[KSW_CLS_LITERAL])
-		MMG_LAUNCH(c, k_ksw<16>, mmg_blocks(h_cls[KSW_CLS_LITERAL], KSW_JOBS_PER_BLOCK), 16 * KSW_JOBS_PER_BLOCK, KSW_SMEM_PER_JOB * KSW_JOBS_PER_BLOCK,
-		           d_jobs, order + first, (int)h_cls[KSW_CLS_LITERAL], sc, d_Q, d_S, d_q_off, d_read_len, d_ref_off, reinterpret_cast<const uint64_t*>(mem_off),
-		           reinterpret_cast<const uint64_t*>(p_off), reinterpret_cast<const uint64_t*>(cg_off), c->k_mem.as<int8_t>(), c->k_p.as<uint8_t>(),
-		           c->k_cig.as<uint32_t>(), d_ez);
-	first += h_cls[KSW_CLS_LITERAL];
-	if (legacy_literal && h_cls[KSW_CLS_LITERAL_WIDE])
-		MMG_LAUNCH(c, k_ksw<32>, mmg_blocks(h_cls[KSW_CLS_LITERAL_WIDE], KSW_JOBS_PER_BLOCK), 32 * KSW_JOBS_PER_BLOCK, KSW_SMEM_PER_JOB * KSW_JOBS_PER_BLOCK,
-		           d_jobs, order + first, (int)h_cls[KSW_CLS_LITERAL_WIDE], sc, d_Q, d_S, d_q_off, d_read_len, d_ref_off, reinterpret_cast<const uint64_t*>(mem_off),
-		           reinterpret_cast<const uint64_t*>(p_off), reinterpret_cast<const uint64_t*>(cg_off), c->k_mem.as<int8_t>(), c->k_p.as<uint8_t>(),
-		           c->k_cig.as<uint32_t>(), d_ez);
-	first += h_cls[KSW_CLS_LITERAL_WIDE];
-	for (int q = KSW_CLS_BLOCK1; q <= KSW_CLS_BLOCK2; ++q) { // literal jobs with more state than a warp's slot: a CTA each, state in its shared memory
-		static bool blk_attr[16] = {false};
-		if (c->dev < 16 && !blk_attr[c->dev]) {
-			MMG_CUDA(cudaFuncSetAttribute(k_ksw_dpx_block, cudaFuncAttributeMaxDynamicSharedMemorySize, KSWB_SMEM2));
-			blk_attr[c->dev] = true;
-		}
+	uint32_t first = 0; // the classes are consecutive in the scheduling order
+	for (int q = 0; q < KSW_N_FAST; ++q) {
 		if (h_cls[q])
-			MMG_LAUNCH(c, k_ksw_dpx_block, h_cls[q], 32 * KSWB_WARPS, q == KSW_CLS_BLOCK1 ? KSWB_SMEM1 : KSWB_SMEM2, d_jobs, order + first, (int)h_cls[q], sc, d_Q, d_S,
-			           d_q_off, d_read_len, d_ref_off, reinterpret_cast<const uint64_t*>(p_off), reinterpret_cast<const uint64_t*>(cg_off), c->k_p.as<uint8_t>(),
-			           c->k_cig.as<uint32_t>(), d_ez);
+			MMG_LAUNCH(c, k_ksw_tpj, mmg_blocks(h_cls[q], ksw_ftab.c[q].nt), ksw_ftab.c[q].nt, ksw_fast_smem(ksw_ftab.c[q]), t, order + first, (int)h_cls[q], ksw_ftab.c[q]);
+		first += h_cls[q];
+	}
+	if (h_cls[KSW_CLS_LITERAL])
+		MMG_LAUNCH(c, k_ksw_dpx, mmg_blocks(h_cls[KSW_CLS_LITERAL], KSWDPX_JOBS_PER_BLOCK), 32 * KSWDPX_JOBS_PER_BLOCK, KSWDPX_SMEM_PER_JOB * KSWDPX_JOBS_PER_BLOCK,
+		           t, order + first, (int)h_cls[KSW_CLS_LITERAL]);
+	first += h_cls[KSW_CLS_LITERAL];
+	for (int q = KSW_CLS_BLOCK1; q <= KSW_CLS_BLOCK2; ++q) { // literal jobs with more state than a warp's slot: a CTA each, state in its shared memory
+		if (h_cls[q])
+			MMG_LAUNCH(c, k_ksw_dpx_block, h_cls[q], 32 * KSWB_WARPS, q == KSW_CLS_BLOCK1 ? KSWB_SMEM1 : KSWB_SMEM2, t, order + first, (int)h_cls[q]);
 		first += h_cls[q];
 	}
 	if (h_cls[KSW_CLS_WAVE])
-		MMG_LAUNCH(c, k_ksw_wave, mmg_blocks(h_cls[KSW_CLS_WAVE], KW_WARPS), 32 * KW_WARPS, 0, d_jobs, order + first, (int)h_cls[KSW_CLS_WAVE], sc, d_Q, d_S, d_q_off,
-		           d_read_len, d_ref_off, reinterpret_cast<const uint64_t*>(mem_off), reinterpret_cast<const uint64_t*>(p_off), reinterpret_cast<const uint64_t*>(cg_off),
-		           c->k_mem.as<int8_t>(), c->k_p.as<uint8_t>(), c->k_cig.as<uint32_t>(), d_ez);
+		MMG_LAUNCH(c, k_ksw_wave, mmg_blocks(h_cls[KSW_CLS_WAVE], KW_WARPS), 32 * KW_WARPS, 0, t, order + first, (int)h_cls[KSW_CLS_WAVE]);
 	MMG_CUDA(cudaEventRecord(c->ev[1], c->stream));
 	MMG_LAUNCH(c, k_res_ncig, mmg_blocks(n1, 256), 256, 0, n, d_ez, ncig);
 	MMG_TRY(scan_excl(c, ncig, nc_off, (int)n1));
@@ -1114,7 +913,7 @@ int mmg_ksw_device(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, i
 }
 
 extern "C" void mmg_ksw_last_split(const mmg_ctx_t *c, uint64_t *jobs_fast, uint64_t *cells_fast, uint64_t *jobs_literal, uint64_t *cells_literal)
-{ // how the last mmg_ksw_batch() divided its jobs between the thread-per-job fast form and the literal 16-lane form
+{ // how the last mmg_ksw_batch() divided its jobs between the fast forms (thread per job, wavefront) and the literal forms
 	if (jobs_fast) *jobs_fast = c->k_last_jobs_fast;
 	if (cells_fast) *cells_fast = c->k_last_cells_fast;
 	if (jobs_literal) *jobs_literal = c->k_last_jobs_literal;

@@ -1066,7 +1066,6 @@ __device__ __forceinline__ int block_incl_scan(int v, int *s, int *total)
 }
 
 #define TAIL_BLOCK_SMEM (216 * 1024)
-__device__ int g_tail_walk = 0;        /* 1: the chain tail walks every chain (the form before the level-by-level one); MMG_TAIL_WALK=1 */
 #define TAIL_HEAVY_N 2048               /* first-pass fragments with more anchors go to the CTA form */
 #define TAIL_HEAVY_SMEM (64 * 1024)     /* staging area of the CTA form in the first pass: three CTAs of 512 threads per SM */
 __global__ void __launch_bounds__(1024)
@@ -1075,7 +1074,8 @@ k_chain_tail_block(FragTab ft, const int32_t *__restrict__ list, int n_list, con
                    uint64_t *__restrict__ u, mm128 *__restrict__ bb, RsFrame *__restrict__ stack, int32_t *__restrict__ nu_out,
                    int32_t *__restrict__ nv_out, const int32_t *__restrict__ heavy /* slots by descending anchor count */,
                    int32_t *__restrict__ n_heavy /* [0] how many of them this kernel takes, [1] the next one to hand out */, size_t smem_cap,
-                   const int32_t *__restrict__ rep, int rechain_enabled, uint8_t *__restrict__ flag_out /* first pass only */)
+                   const int32_t *__restrict__ rep, int rechain_enabled, uint8_t *__restrict__ flag_out /* first pass only */,
+                   int walk /* 1: walk every chain, the form before the level-by-level one (MMG_TAIL_WALK=1) */)
 {
 	__shared__ int s_scan[1024], s_nu, s_tie, s_it;
 	extern __shared__ __align__(16) unsigned char dyn_tail[];
@@ -1124,7 +1124,7 @@ k_chain_tail_block(FragTab ft, const int32_t *__restrict__ list, int n_list, con
 			// fire-and-forget atomic per anchor -- a chain keeps exactly the anchors it owns (they are consecutive on its path), and an
 			// owned anchor's slot in b[] follows from the two depths.
 			int n_keep = 0;
-			bool par = P.min_cnt >= 2 && !g_tail_walk;
+			bool par = P.min_cnt >= 2 && !walk;
 			int maxd = 0;
 			if (par) {
 				unsigned long long *P2 = reinterpret_cast<unsigned long long*>(W); // (jump << 32 | distance) per anchor
@@ -1583,6 +1583,13 @@ struct PassBufs {
 	DevBuf *na, *aoff, *rep, *nmini, *mini, *a, *work, *u, *b, *stack, *nu, *nv;
 };
 
+// the dynamic shared memory the chain tail's CTA form launches with, allowed on the current device (mmg_init, once per context)
+int mmg_stages_set_smem_attrs()
+{
+	MMG_CUDA(cudaFuncSetAttribute(k_chain_tail_block, cudaFuncAttributeMaxDynamicSharedMemorySize, TAIL_BLOCK_SMEM));
+	return MMG_OK;
+}
+
 // plan -> scan -> fill -> chain for the fragments in `list` (null = all) with cut-off max_occ
 static int run_pass(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, const FragTab &ft, const NameTabs &nt, const int32_t *d_list, int n_list,
                     int64_t n_mv, int max_occ, const PassBufs &pb, bool want_mini, uint8_t *d_flag, int64_t *n_anchors)
@@ -1729,18 +1736,11 @@ static int run_pass(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, 
 		           c->d_seg_long.as<int32_t>(), d_nlong, d_next, c->d_frag_iter.as<unsigned long long>());
 	}
 	{
-		static bool attr_set = false;
-		if (!attr_set) {
-			MMG_CUDA(cudaFuncSetAttribute(k_chain_tail_block, cudaFuncAttributeMaxDynamicSharedMemorySize, TAIL_BLOCK_SMEM));
-			if (getenv("MMG_TAIL_WALK")) { const int one = 1; MMG_CUDA(cudaMemcpyToSymbol(g_tail_walk, &one, sizeof(one))); } // A/B aid
-			attr_set = true;
-		}
-	}
-	{
 		// The fragments with thousands of anchors get a CTA each, with its sorts staged in shared memory: all fragments of the re-chain
 		// pass (one CTA per SM, the whole shared memory), a few per thousand of the first pass (ahead of the warp kernel that takes
 		// everything else).  The CTAs pull fragments from a counter, largest first.
 		static const int heavy_env = getenv("MMG_TAIL_HEAVY_N") ? atoi(getenv("MMG_TAIL_HEAVY_N")) : TAIL_HEAVY_N;
+		static const int walk = getenv("MMG_TAIL_WALK") ? 1 : 0;
 		const bool second = d_flag == nullptr;
 		const int heavy_n = second ? -1 : heavy_env, rechain_enabled = opt->max_occ > opt->mid_occ ? 1 : 0;
 		MMG_TRY(c->d_heavy.ensure(((size_t)n_list * 4 + 16) * 4));
@@ -1758,11 +1758,11 @@ static int run_pass(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, 
 		if (second)
 			MMG_LAUNCH(c, k_chain_tail_block, n_list < 148 ? n_list : 148, 1024, TAIL_BLOCK_SMEM, ft, d_list, n_list, c->d_misc.as<int32_t>(), co, pb.aoff->as<int64_t>(),
 			           pb.na->as<int32_t>(), pb.a->as<mm128>(), pb.work->as<int32_t>(), pb.u->as<uint64_t>(), pb.b->as<mm128>(), pb.stack->as<RsFrame>(),
-			           pb.nu->as<int32_t>(), pb.nv->as<int32_t>(), heavy, n_heavy, (size_t)TAIL_BLOCK_SMEM, nullptr, 0, nullptr);
+			           pb.nu->as<int32_t>(), pb.nv->as<int32_t>(), heavy, n_heavy, (size_t)TAIL_BLOCK_SMEM, nullptr, 0, nullptr, walk);
 		else
 			MMG_LAUNCH(c, k_chain_tail_block, 148 * 3, 512, TAIL_HEAVY_SMEM, ft, d_list, n_list, c->d_misc.as<int32_t>(), co, pb.aoff->as<int64_t>(),
 			           pb.na->as<int32_t>(), pb.a->as<mm128>(), pb.work->as<int32_t>(), pb.u->as<uint64_t>(), pb.b->as<mm128>(), pb.stack->as<RsFrame>(),
-			           pb.nu->as<int32_t>(), pb.nv->as<int32_t>(), heavy, n_heavy, (size_t)TAIL_HEAVY_SMEM, pb.rep->as<int32_t>(), rechain_enabled, d_flag);
+			           pb.nu->as<int32_t>(), pb.nv->as<int32_t>(), heavy, n_heavy, (size_t)TAIL_HEAVY_SMEM, pb.rep->as<int32_t>(), rechain_enabled, d_flag, walk);
 		if (!second)
 		MMG_LAUNCH(c, k_chain_tail_warp, mmg_blocks((size_t)n_list * 32, 128), 128, 0, ft, d_list, n_list, c->d_misc.as<int32_t>(), co, pb.aoff->as<int64_t>(),
 		           pb.na->as<int32_t>(), pb.a->as<mm128>(), pb.work->as<int32_t>(), pb.u->as<uint64_t>(), pb.b->as<mm128>(), pb.stack->as<RsFrame>(),
