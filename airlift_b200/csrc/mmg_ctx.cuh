@@ -114,6 +114,12 @@ struct ResidentBatch {
 
 struct ProfRec { const char *name; cudaEvent_t a, b; };
 
+// the arrays of one seed-and-chain pass over a list of fragments (mmg_stages.cu: PassTab is their device view)
+struct PassArena {
+	DevBuf na, aoff, rep, nmini, mini, a, work, u, b, stack, nu, nv;
+	void release() { for (DevBuf *d : {&na, &aoff, &rep, &nmini, &mini, &a, &work, &u, &b, &stack, &nu, &nv}) d->release(); }
+};
+
 struct mmg_ctx_s {
 	int dev = 0;
 	cudaStream_t stream = nullptr;
@@ -127,11 +133,10 @@ struct mmg_ctx_s {
 	ResidentBatch rb;
 	// device arenas (grown on demand, reused across batches)
 	DevBuf d_ascii, d_Q, d_seq_len, d_seq_off, d_q_off, d_flip, d_units, d_unit_cnt, d_unit_off, d_mv, d_m_n, d_m_val,
-	       d_frag_unit0, d_frag_qlen, d_frag_na, d_frag_aoff, d_frag_rep, d_frag_nmini, d_mini, d_a, d_work, d_u, d_b, d_heap,
-	       d_stack, d_frag_nu, d_frag_nv, d_frag_flag, d_frag_iter, d_cub, d_out_u, d_out_a, d_out_mini, d_uoff, d_voff, d_moff,
-	       d_frag_list, d_misc, d_seg_head, d_seg_start, d_seg_avg, d_replay, d_skey, d_sval, d_sseg, d_tie, d_m_aoff, d_hrank, d_hpop, d_hlist, d_seg_li, d_seg_long, d_unit0, d_fseg_off, d_sk_stage, d_heavy, d_ukey;
-	// second-pass (re-chain with max_occ) arenas
-	DevBuf d2_frag_na, d2_frag_aoff, d2_frag_rep, d2_frag_nmini, d2_mini, d2_a, d2_work, d2_u, d2_b, d2_stack, d2_frag_nu, d2_frag_nv;
+	       d_frag_unit0, d_frag_qlen, d_frag_nseg, d_heap, d_frag_flag, d_frag_iter, d_cub, d_out_u, d_out_a, d_out_mini, d_uoff, d_voff, d_moff,
+	       d_frag_list, d_seg_head, d_seg_start, d_seg_avg, d_replay, d_skey, d_sval, d_sseg, d_tie, d_m_aoff, d_hrank, d_hpop, d_hlist, d_seg_li, d_seg_long, d_unit0, d_fseg_off, d_sk_stage, d_heavy, d_ukey;
+	// pass[0]: every fragment with the mid_occ cut-off; pass[1]: the fragments re-chained with max_occ (map.c:353-375)
+	PassArena pass[2];
 	// ksw arenas
 	DevBuf k_jobs, k_mem, k_H, k_p, k_cig, k_res, k_cig_out, k_cig_off;
 	const void *k_last_res = nullptr; // device {ez, cigar offset} array of the last ksw_launch
@@ -149,7 +154,7 @@ struct mmg_ctx_s {
 	// after z-drop cuts, [5] hits cut at a z-drop, [6] seed hits whose merge order was replayed, [7] seed hits the self/dual filters dropped
 	uint64_t path[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 	StageSlot stage[MMG_STAGE_SLOTS];
-	PinBuf h_path;                     // device counters of the pass in flight land here
+	PinBuf h_path;                     // the device's path counters of the batch in flight land here (PathCounters, mmg_stages.cu)
 	PinBuf h_p_hash, h_p_nreg, h_p_offs, h_p_blob, h_p_rep;
 	PinBuf h_meta, h_out_meta, h_out_u, h_out_a, h_out_mini, h_k_jobs, h_k_res, h_k_cig;
 };

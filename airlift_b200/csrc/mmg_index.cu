@@ -48,18 +48,17 @@ extern "C" void mmg_destroy(mmg_ctx_t *c)
 	cudaSetDevice(c->dev);
 	cudaStreamSynchronize(c->stream);
 	DevBuf *bufs[] = {&c->d_ascii, &c->d_Q, &c->d_seq_len, &c->d_seq_off, &c->d_q_off, &c->d_flip, &c->d_units, &c->d_unit_cnt,
-		&c->d_unit_off, &c->d_mv, &c->d_m_n, &c->d_m_val, &c->d_frag_unit0, &c->d_frag_qlen, &c->d_frag_na, &c->d_frag_aoff,
-		&c->d_frag_rep, &c->d_frag_nmini, &c->d_mini, &c->d_a, &c->d_work, &c->d_u, &c->d_b, &c->d_heap, &c->d_stack, &c->d_frag_nu,
-		&c->d_frag_nv, &c->d_frag_flag, &c->d_frag_iter, &c->d_cub, &c->d_out_u, &c->d_out_a, &c->d_out_mini, &c->d_uoff, &c->d_voff,
-		&c->d_moff, &c->d_frag_list, &c->d_misc, &c->d_seg_head, &c->d_seg_start, &c->d_seg_avg, &c->d_replay, &c->d_skey, &c->d_sval, &c->d_sseg, &c->d_tie, &c->d_m_aoff, &c->d_hrank, &c->d_hpop, &c->d_hlist, &c->d_seg_li, &c->d_seg_long, &c->d_unit0, &c->d_fseg_off, &c->d_sk_stage, &c->d_heavy, &c->d_ukey, &c->d2_frag_na, &c->d2_frag_aoff, &c->d2_frag_rep, &c->d2_frag_nmini, &c->d2_mini,
-		&c->d2_a, &c->d2_work, &c->d2_u, &c->d2_b, &c->d2_stack, &c->d2_frag_nu, &c->d2_frag_nv, &c->k_jobs, &c->k_mem, &c->k_H,
-		&c->k_p, &c->k_cig, &c->k_res, &c->k_cig_out, &c->k_cig_off};
+		&c->d_unit_off, &c->d_mv, &c->d_m_n, &c->d_m_val, &c->d_frag_unit0, &c->d_frag_qlen, &c->d_frag_nseg, &c->d_heap,
+		&c->d_frag_flag, &c->d_frag_iter, &c->d_cub, &c->d_out_u, &c->d_out_a, &c->d_out_mini, &c->d_uoff, &c->d_voff,
+		&c->d_moff, &c->d_frag_list, &c->d_seg_head, &c->d_seg_start, &c->d_seg_avg, &c->d_replay, &c->d_skey, &c->d_sval, &c->d_sseg, &c->d_tie, &c->d_m_aoff, &c->d_hrank, &c->d_hpop, &c->d_hlist, &c->d_seg_li, &c->d_seg_long, &c->d_unit0, &c->d_fseg_off, &c->d_sk_stage, &c->d_heavy, &c->d_ukey,
+		&c->k_jobs, &c->k_mem, &c->k_H, &c->k_p, &c->k_cig, &c->k_res, &c->k_cig_out, &c->k_cig_off};
 	if (getenv("MM2_B200_TRACE"))
 		fprintf(stderr, "[T::buffers] %llu device and %llu pinned (re-)allocations so far, %.3f s and %.3f s inside them\n", g_mmg_grow[0], g_mmg_grow[1],
 		        g_mmg_grow_ns[0] * 1e-9, g_mmg_grow_ns[1] * 1e-9);
 	const unsigned long long t_rel = mmg_now_ns();
 	for (DevBuf *b : bufs) b->release();
 	for (DevBuf &b : c->pb) b.release();
+	for (PassArena &p : c->pass) p.release();
 	PinBuf *pins[] = {&c->h_meta, &c->h_out_meta, &c->h_out_u, &c->h_out_a, &c->h_out_mini, &c->h_k_jobs, &c->h_k_res, &c->h_k_cig,
 	                  &c->h_p_hash, &c->h_p_nreg, &c->h_p_offs, &c->h_p_blob, &c->h_p_rep, &c->h_path};
 	for (PinBuf *b : pins) b->release();

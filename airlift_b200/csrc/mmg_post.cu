@@ -233,10 +233,10 @@ extern "C" int mmg_post_chain(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapop
 	}
 	MMG_CUDA(cudaMemsetAsync(B[X::PB_CTR].p, 0, 64, c->stream));
 	MMG_CUDA(cudaMemsetAsync(B[X::PB_CAP].p, 0, (size_t)(n_seq + 2) * 4, c->stream));
-	hs.n_seg = c->d_misc.as<int32_t>(), hs.seg_off = B[X::PB_SEGOFF].as<int32_t>(), hs.seq_len = c->d_seq_len.as<int32_t>();
+	hs.n_seg = c->d_frag_nseg.as<int32_t>(), hs.seg_off = B[X::PB_SEGOFF].as<int32_t>(), hs.seq_len = c->d_seq_len.as<int32_t>();
 	hs.q_off = c->d_q_off.as<uint64_t>(), hs.flip = c->d_flip.as<uint8_t>(), hs.Q = c->d_Q.as<uint32_t>(), hs.S = mi->d_S;
 	hs.ref_off = mi->d_seq_off, hs.ref_len = mi->d_seq_len;
-	hs.nu = c->d_frag_nu.as<int32_t>(), hs.rep = c->d_frag_rep.as<int32_t>(), hs.uoff = c->d_uoff.as<int64_t>(), hs.voff = c->d_voff.as<int64_t>();
+	hs.nu = c->pass[0].nu.as<int32_t>(), hs.rep = c->pass[0].rep.as<int32_t>(), hs.uoff = c->d_uoff.as<int64_t>(), hs.voff = c->d_voff.as<int64_t>();
 	hs.u = c->d_out_u.as<uint64_t>(), hs.a = c->d_out_a.as<mm128>(), hs.hash = B[X::PB_HASH].as<uint32_t>();
 	// ---- fragment-level hit arrays (one slot per chain)
 	const size_t nu1 = (size_t)tot_u + 1;
@@ -369,7 +369,7 @@ extern "C" int mmg_post_chain(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapop
 	MMG_D2H(c, c->h_p_nreg.p, hs.n_reg, (size_t)n_seq * 4);
 	MMG_D2H(c, c->h_p_offs.p, B[X::PB_OFFS].p, (size_t)(n_seq + 1) * 8);
 	if (blob_bytes) MMG_D2H(c, c->h_p_blob.p, B[X::PB_BLOB].p, (size_t)blob_bytes);
-	MMG_D2H(c, c->h_p_rep.p, c->d_frag_rep.p, (size_t)nf * 4);
+	MMG_D2H(c, c->h_p_rep.p, c->pass[0].rep.p, (size_t)nf * 4);
 	{
 		cudaError_t e = cudaStreamSynchronize(c->stream);
 		if (e != cudaSuccess) { mmg_set_error("post-chaining stages (pack): %s", cudaGetErrorString(e)); return MMG_ECUDA; }

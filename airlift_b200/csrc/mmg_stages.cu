@@ -574,33 +574,28 @@ __device__ int64_t fill_heap_prefetch(const mm128 *mv, const int32_t *m_n, const
 	return n_a;
 }
 
-// K2c: anchors per fragment, in the reference's order (map.c:149-247)
+// K2c, literal form: anchors in the reference's order (map.c:149-211) for the fragments the rank replay cannot take (replay[] == 2)
 template <bool kNamed>
 __global__ void k_fill(FragTab ft, const int32_t *__restrict__ list, int n_list, const mm128 *__restrict__ mv, const int32_t *__restrict__ m_n,
                        const uint64_t *__restrict__ m_val, const uint64_t *__restrict__ pos, int max_occ, int64_t flag,
-                       const int64_t *__restrict__ aoff, int32_t *__restrict__ na, mm128 *__restrict__ a, mm128 *__restrict__ heap, RsFrame *__restrict__ stack,
-                       const uint8_t *__restrict__ replay /* null: every fragment */, int want /* value of replay[] that selects a fragment */, int per_warp,
-                       NameTabs nt, unsigned long long *__restrict__ n_named)
+                       const int64_t *__restrict__ aoff, int32_t *__restrict__ na, mm128 *__restrict__ a, mm128 *__restrict__ heap,
+                       const uint8_t *__restrict__ replay, int per_warp, NameTabs nt, unsigned long long *__restrict__ n_named)
 {
 	// per_warp: one fragment per warp (lane 0 works).  The re-chain pass lists a few hundred fragments of ~10^5 anchors each; as
 	// neighbouring threads of one warp their serial replays diverged and ran one after the other (36 ms for 192 fragments)
 	const int gt = blockIdx.x * blockDim.x + threadIdx.x, li = per_warp ? gt >> 5 : gt;
 	if (li >= n_list || (per_warp && (gt & 31))) return;
-	if (replay && replay[li] != want) return;
+	if (replay[li] != 2) return;
 	const int f = list ? list[li] : li;
 	const int64_t b = ft.unit_off[ft.unit0[f]], e = ft.unit_off[ft.unit0[f + 1]];
 	const int64_t ao = aoff[li];
 	const NameFilt nf = name_filt(nt, f);
 	int64_t n, nn;
-	if (flag & MMG_F_HEAP_SORT) {
-		__shared__ mm128 s_heap[2][128];
-		__shared__ uint64_t s_nxt[2][128];
-		if (per_warp && e - b <= 128)
-			n = fill_heap_prefetch<kNamed>(mv + b, m_n + b, m_val + b, (int)(e - b), max_occ, pos, flag, nf, ft.qlen[f], na[li], s_heap[threadIdx.x >> 5], s_nxt[threadIdx.x >> 5], a + ao, &nn);
-		else n = mmg_fill_heap<kNamed>(mv + b, m_n + b, m_val + b, (int)(e - b), max_occ, pos, flag, nf, ft.qlen[f], na[li], heap + b, a + ao, &nn);
-	}
-	else
-		n = mmg_fill_flat<kNamed>(mv + b, m_n + b, m_val + b, (int)(e - b), max_occ, pos, flag, nf, ft.qlen[f], a + ao, stack + ao / 65 + 2 * (int64_t)li, &nn);
+	__shared__ mm128 s_heap[2][128];
+	__shared__ uint64_t s_nxt[2][128];
+	if (per_warp && e - b <= 128)
+		n = fill_heap_prefetch<kNamed>(mv + b, m_n + b, m_val + b, (int)(e - b), max_occ, pos, flag, nf, ft.qlen[f], na[li], s_heap[threadIdx.x >> 5], s_nxt[threadIdx.x >> 5], a + ao, &nn);
+	else n = mmg_fill_heap<kNamed>(mv + b, m_n + b, m_val + b, (int)(e - b), max_occ, pos, flag, nf, ft.qlen[f], na[li], heap + b, a + ao, &nn);
 	na[li] = (int32_t)n;
 	if (kNamed && nn) atomicAdd(n_named, (unsigned long long)nn);
 }
@@ -1533,11 +1528,11 @@ extern "C" int mmg_upload_stage(mmg_ctx_t *c, const mmg_mapopt_t *opt, int slot)
 	MMG_TRY(c->d_units.ensure((size_t)(rb.n_units + 1) * sizeof(SketchUnit)));
 	MMG_TRY(c->d_frag_unit0.ensure((size_t)(n_frag + 2) * 4));
 	MMG_TRY(c->d_frag_qlen.ensure((size_t)(n_frag + 2) * 4));
-	MMG_TRY(c->d_misc.ensure((size_t)(n_frag + 2) * 4));     // n_seg
+	MMG_TRY(c->d_frag_nseg.ensure((size_t)(n_frag + 2) * 4));
 	MMG_TRY(c->d_fseg_off.ensure((size_t)(n_frag + 2) * 4));
 	MMG_H2D(c, c->d_seq_len.p, t_len, (size_t)(n_seq + 1) * 4);
 	MMG_H2D(c, c->d_seq_off.p, t_off, (size_t)(n_seq + 1) * 8);
-	MMG_H2D(c, c->d_misc.p, t_nseg, (size_t)n_frag * 4);
+	MMG_H2D(c, c->d_frag_nseg.p, t_nseg, (size_t)n_frag * 4);
 	MMG_H2D(c, c->d_fseg_off.p, t_segoff, (size_t)n_frag * 4);
 	if (s.has_flip && n_seq > 0) MMG_H2D(c, c->d_flip.p, s.flip.p, (size_t)n_seq);
 	if (s.has_ukey) {
@@ -1556,7 +1551,7 @@ extern "C" int mmg_upload_stage(mmg_ctx_t *c, const mmg_mapopt_t *opt, int slot)
 		MMG_CUDA(cub::DeviceScan::ExclusiveSum(c->d_cub.p, t2, it_u, c->d_unit0.as<int64_t>(), n_seq + 1, c->stream));
 		c->launches += 2;
 	}
-	MMG_LAUNCH(c, k_batch_tables, mmg_blocks((size_t)n_frag + 1, 256), 256, 0, n_frag, n_seq, c->d_misc.as<int32_t>(), c->d_fseg_off.as<int32_t>(),
+	MMG_LAUNCH(c, k_batch_tables, mmg_blocks((size_t)n_frag + 1, 256), 256, 0, n_frag, n_seq, c->d_frag_nseg.as<int32_t>(), c->d_fseg_off.as<int32_t>(),
 	           c->d_seq_len.as<int32_t>(), c->d_q_off.as<uint64_t>(), c->d_unit0.as<int64_t>(), opt->pe_ori, s.has_flip ? 1 : 0, c->d_units.as<SketchUnit>(),
 	           c->d_flip.as<uint8_t>(), c->d_frag_unit0.as<int32_t>(), c->d_frag_qlen.as<int32_t>());
 	if (rb.q_words)
@@ -1579,10 +1574,6 @@ extern "C" int mmg_batch_upload(mmg_ctx_t *c, const mmg_mapopt_t *opt, const mmg
 	return mmg_upload_stage(c, opt, 0);
 }
 
-struct PassBufs {
-	DevBuf *na, *aoff, *rep, *nmini, *mini, *a, *work, *u, *b, *stack, *nu, *nv;
-};
-
 // the dynamic shared memory the chain tail's CTA form launches with, allowed on the current device (mmg_init, once per context)
 int mmg_stages_set_smem_attrs()
 {
@@ -1590,49 +1581,82 @@ int mmg_stages_set_smem_attrs()
 	return MMG_OK;
 }
 
-// plan -> scan -> fill -> chain for the fragments in `list` (null = all) with cut-off max_occ
-static int run_pass(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, const FragTab &ft, const NameTabs &nt, const int32_t *d_list, int n_list,
-                    int64_t n_mv, int max_occ, const PassBufs &pb, bool want_mini, uint8_t *d_flag, int64_t *n_anchors)
+// the device counters of a batch that feed c->path[] (mmg_path_counts), read back into the pinned c->h_path
+struct PathCounters {
+	int32_t heap[2][4];        // per pass (k_heap_list): [0] fragments replayed on ranks, [1] k_heap_replay's cursor, [2] fragments left to k_fill
+	unsigned long long pops;   // seed hits whose merge order was replayed (k_heap_emit)
+	unsigned long long named;  // seed hits the self/dual filters dropped; one copy from d_frag_iter fills this and pops
+};
+
+// one pass: the fragments it takes and the typed pointers of its arena
+struct PassTab {
+	const int32_t *list;       // fragment of every slot; null: slot li is fragment li
+	int n_list;
+	int64_t *aoff;             // [n_list+1] first anchor slot of every fragment
+	int32_t *na, *rep, *nmini, *nu, *nv;
+	uint64_t *mini;            // null when nothing reads the minimizer positions
+	mm128 *a, *b;
+	int32_t *work;             // per anchor f|p|t|v, then the chain-order array
+	uint64_t *u;
+	RsFrame *stack;
+};
+
+// the view of pass `pass`'s arena; taken again whenever the arena has grown
+static PassTab pass_tab(mmg_ctx_t *c, int pass, const int32_t *d_list, int n_list, bool want_mini)
 {
+	const PassArena &A = c->pass[pass];
+	PassTab t;
+	t.list = d_list, t.n_list = n_list;
+	t.aoff = A.aoff.as<int64_t>(), t.na = A.na.as<int32_t>(), t.rep = A.rep.as<int32_t>(), t.nmini = A.nmini.as<int32_t>();
+	t.mini = want_mini ? A.mini.as<uint64_t>() : nullptr;
+	t.a = A.a.as<mm128>(), t.work = A.work.as<int32_t>(), t.u = A.u.as<uint64_t>(), t.b = A.b.as<mm128>(), t.stack = A.stack.as<RsFrame>();
+	t.nu = A.nu.as<int32_t>(), t.nv = A.nv.as<int32_t>();
+	return t;
+}
+
+// K2 of pass `pass` (0: every fragment with mid_occ; 1: the fragments in d_list, re-chained with max_occ): plan -> scan -> sort ->
+// heap replay on ranks and literal heap merge, or the radix-order replay of the non-heap presets.  The anchors stay in the pass's
+// arena; *pt is its view.
+static int seed_pass(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, const FragTab &ft, const NameTabs &nt, int pass, const int32_t *d_list, int n_list,
+                     int max_occ, int64_t n_mv, bool want_mini, PassTab *pt, int64_t *n_anchors)
+{
+	PassArena &A = c->pass[pass];
 	unsigned long long *n_named = c->d_frag_iter.as<unsigned long long>() + 2;
 	const bool named = nt.ukey != nullptr;
-	*n_anchors = 0;
-	if (n_list == 0) return MMG_OK;
-	MMG_TRY(pb.na->ensure((size_t)(n_list + 1) * 4));
-	MMG_TRY(pb.aoff->ensure((size_t)(n_list + 1) * 8));
-	MMG_TRY(pb.rep->ensure((size_t)(n_list + 1) * 4));
-	MMG_TRY(pb.nmini->ensure((size_t)(n_list + 1) * 4));
-	MMG_TRY(pb.nu->ensure((size_t)(n_list + 1) * 4));
-	MMG_TRY(pb.nv->ensure((size_t)(n_list + 1) * 4));
-	if (want_mini) MMG_TRY(pb.mini->ensure((size_t)(n_mv + 1) * 8));
+	MMG_TRY(A.na.ensure((size_t)(n_list + 1) * 4));
+	MMG_TRY(A.aoff.ensure((size_t)(n_list + 1) * 8));
+	MMG_TRY(A.rep.ensure((size_t)(n_list + 1) * 4));
+	MMG_TRY(A.nmini.ensure((size_t)(n_list + 1) * 4));
+	MMG_TRY(A.nu.ensure((size_t)(n_list + 1) * 4));
+	MMG_TRY(A.nv.ensure((size_t)(n_list + 1) * 4));
+	if (want_mini) MMG_TRY(A.mini.ensure((size_t)(n_mv + 1) * 8));
 	const bool heap_path = (opt->flag & MMG_F_HEAP_SORT) != 0;
 	MMG_TRY(c->d_replay.ensure((size_t)n_list + 16));
-	MMG_CUDA(cudaMemsetAsync(pb.na->p, 0, (size_t)(n_list + 1) * 4, c->stream));
-	MMG_CUDA(cudaMemsetAsync(pb.nu->p, 0, (size_t)(n_list + 1) * 4, c->stream)); // slot n_list must read 0 for the scans
-	MMG_CUDA(cudaMemsetAsync(pb.nv->p, 0, (size_t)(n_list + 1) * 4, c->stream));
-	MMG_CUDA(cudaMemsetAsync(pb.nmini->p, 0, (size_t)(n_list + 1) * 4, c->stream));
-	MMG_LAUNCH(c, k_plan, mmg_blocks(n_list, 128), 128, 0, ft, d_list, n_list, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(), max_occ,
-	           pb.na->as<int32_t>(), pb.rep->as<int32_t>(), pb.nmini->as<int32_t>(), want_mini ? pb.mini->as<uint64_t>() : nullptr,
+	MMG_CUDA(cudaMemsetAsync(A.na.p, 0, (size_t)(n_list + 1) * 4, c->stream));
+	MMG_CUDA(cudaMemsetAsync(A.nu.p, 0, (size_t)(n_list + 1) * 4, c->stream)); // slot n_list must read 0 for the scans
+	MMG_CUDA(cudaMemsetAsync(A.nv.p, 0, (size_t)(n_list + 1) * 4, c->stream));
+	MMG_CUDA(cudaMemsetAsync(A.nmini.p, 0, (size_t)(n_list + 1) * 4, c->stream));
+	PassTab t = pass_tab(c, pass, d_list, n_list, want_mini);
+	MMG_LAUNCH(c, k_plan, mmg_blocks(n_list, 128), 128, 0, ft, d_list, n_list, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(), max_occ, t.na, t.rep, t.nmini, t.mini,
 	           heap_path ? c->d_replay.as<uint8_t>() : nullptr, c->d_m_aoff.as<int32_t>());
-	MMG_TRY(scan_i32_to_i64(c, pb.na->as<int32_t>(), pb.aoff->as<int64_t>(), n_list + 1));
-	int32_t *hp_counters = nullptr, *rlist = nullptr, *hp = nullptr;
+	MMG_TRY(scan_i32_to_i64(c, t.na, t.aoff, n_list + 1));
+	int32_t *hp_counters = nullptr, *rlist = nullptr, *hp = c->h_path.as<PathCounters>()->heap[pass];
 	if (heap_path) { // the fragments whose heap order has to be replayed: their number rides on the synchronisation below
 		MMG_TRY(c->d_hlist.ensure(((size_t)n_list + 8) * 4));
-		MMG_TRY(c->h_path.ensure(64));
-		hp_counters = c->d_hlist.as<int32_t>(), rlist = hp_counters + 4, hp = c->h_path.as<int32_t>() + (d_flag ? 0 : 4);
+		hp_counters = c->d_hlist.as<int32_t>(), rlist = hp_counters + 4;
 		MMG_CUDA(cudaMemsetAsync(hp_counters, 0, 16, c->stream));
 		MMG_LAUNCH(c, k_heap_list, mmg_blocks(n_list, 256), 256, 0, n_list, c->d_replay.as<uint8_t>(), rlist, hp_counters);
 		MMG_D2H(c, hp, hp_counters, 16);
 	}
 	int64_t tot = 0;
-	MMG_D2H(c, &tot, pb.aoff->as<int64_t>() + n_list, 8);
+	MMG_D2H(c, &tot, t.aoff + n_list, 8);
 	MMG_CUDA(cudaStreamSynchronize(c->stream));
-	*n_anchors = tot;
-	MMG_TRY(pb.a->ensure((size_t)(tot + 1) * 16));
-	MMG_TRY(pb.work->ensure((size_t)(tot + 1) * 32)); // f|p|t|v then the chain-order array
-	MMG_TRY(pb.u->ensure((size_t)(tot + 1) * 16));
-	MMG_TRY(pb.b->ensure((size_t)(tot + 1) * 16));
-	MMG_TRY(pb.stack->ensure((size_t)(tot / 65 + 2 * (size_t)n_list + 4) * sizeof(RsFrame)));
+	MMG_TRY(A.a.ensure((size_t)(tot + 1) * 16));
+	MMG_TRY(A.work.ensure((size_t)(tot + 1) * 32)); // f|p|t|v then the chain-order array
+	MMG_TRY(A.u.ensure((size_t)(tot + 1) * 16));
+	MMG_TRY(A.b.ensure((size_t)(tot + 1) * 16));
+	MMG_TRY(A.stack.ensure((size_t)(tot / 65 + 2 * (size_t)n_list + 4) * sizeof(RsFrame)));
+	t = pass_tab(c, pass, d_list, n_list, want_mini);
 	MMG_TRY(c->d_heap.ensure((size_t)(n_mv + 1) * 16));
 	uint8_t *d_tie = nullptr;
 	if (!heap_path) { // radix-sort form: sort everything, replay only the fragments where two anchors share x
@@ -1649,49 +1673,46 @@ static int run_pass(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, 
 		int64_t *seg_b = c->d_sseg.as<int64_t>(), *seg_e = seg_b + n_list + 1;
 		int32_t *n_skipped = reinterpret_cast<int32_t*>(seg_e + n_list + 1);
 		MMG_CUDA(cudaMemsetAsync(n_skipped, 0, (size_t)n_list * 4, c->stream));
-		MMG_LAUNCH_AS(c, "k_expand", (named ? k_expand<true> : k_expand<false>), mmg_blocks(tot, 256), 256, 0, ft, d_list, n_list, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(), c->d_m_val.as<uint64_t>(),
-		           mi->d_pos, max_occ, opt->flag, pb.aoff->as<int64_t>(), c->d_replay.as<uint8_t>(), tot, k0, v0, n_skipped, c->d_m_aoff.as<int32_t>(),
-			           nt, n_named);
-		MMG_LAUNCH(c, k_sort_segments, mmg_blocks(n_list, 256), 256, 0, n_list, pb.aoff->as<int64_t>(), c->d_replay.as<uint8_t>(), seg_b, seg_e);
+		MMG_LAUNCH_AS(c, "k_expand", (named ? k_expand<true> : k_expand<false>), mmg_blocks(tot, 256), 256, 0, ft, d_list, n_list, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(),
+		              c->d_m_val.as<uint64_t>(), mi->d_pos, max_occ, opt->flag, t.aoff, c->d_replay.as<uint8_t>(), tot, k0, v0, n_skipped, c->d_m_aoff.as<int32_t>(), nt, n_named);
+		MMG_LAUNCH(c, k_sort_segments, mmg_blocks(n_list, 256), 256, 0, n_list, t.aoff, c->d_replay.as<uint8_t>(), seg_b, seg_e);
 		{
 			size_t tmp = 0;
 			cub::DeviceSegmentedSort::SortPairs(nullptr, tmp, k0, k1, v0, v1, tot, n_list, seg_b, seg_e, c->stream);
 			MMG_TRY(c->d_cub.ensure(tmp));
 			MMG_TIMED(c, "cub_segmented_sort(seed hits)", cub::DeviceSegmentedSort::SortPairs(c->d_cub.p, tmp, k0, k1, v0, v1, tot, n_list, seg_b, seg_e, c->stream));
 		}
-		MMG_LAUNCH(c, k_emit_sorted, mmg_blocks(tot, 256), 256, 0, n_list, pb.aoff->as<int64_t>(), c->d_replay.as<uint8_t>(), tot, k1, v1, n_skipped,
-		           pb.na->as<int32_t>(), pb.a->as<mm128>(), d_tie);
+		MMG_LAUNCH(c, k_emit_sorted, mmg_blocks(tot, 256), 256, 0, n_list, t.aoff, c->d_replay.as<uint8_t>(), tot, k1, v1, n_skipped, t.na, t.a, d_tie);
 	}
 	if (heap_path && tot > 0) { // fragments where equal positions meet in the heap: replay it on the ranks the sort just produced
 		MMG_TRY(c->d_hrank.ensure(((size_t)tot + 1) * 4));
 		MMG_TRY(c->d_hpop.ensure(((size_t)tot + 1) * 4));
-		int32_t *counters = hp_counters;
 		const uint64_t *k1 = c->d_skey.as<uint64_t>() + tot + 1, *v1 = c->d_sval.as<uint64_t>() + tot + 1;
 		if (hp[0] > 0) {
-			MMG_LAUNCH(c, k_heap_rank, mmg_blocks(tot, 256), 256, 0, n_list, pb.aoff->as<int64_t>(), c->d_replay.as<uint8_t>(), tot, k1, v1, c->d_hrank.as<uint32_t>());
-			MMG_LAUNCH(c, k_heap_replay, hp[0] < 148 * 8 ? hp[0] : 148 * 8, 32, 0, ft, d_list, rlist, counters, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(), c->d_m_val.as<uint64_t>(),
-			           c->d_m_aoff.as<int32_t>(), mi->d_pos, max_occ, opt->flag, pb.aoff->as<int64_t>(), c->d_hrank.as<uint32_t>(), c->d_hpop.as<uint32_t>());
-			MMG_LAUNCH_AS(c, "k_heap_emit", (named ? k_heap_emit<true> : k_heap_emit<false>), hp[0], HEAP_EMIT_THREADS, 0, ft, d_list, rlist, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(), c->d_m_val.as<uint64_t>(),
-			           c->d_m_aoff.as<int32_t>(), mi->d_pos, max_occ, opt->flag, pb.aoff->as<int64_t>(), c->d_hpop.as<uint32_t>(), pb.na->as<int32_t>(), pb.a->as<mm128>(),
-			           c->d_frag_iter.as<unsigned long long>() + 1, nt, n_named);
+			MMG_LAUNCH(c, k_heap_rank, mmg_blocks(tot, 256), 256, 0, n_list, t.aoff, c->d_replay.as<uint8_t>(), tot, k1, v1, c->d_hrank.as<uint32_t>());
+			MMG_LAUNCH(c, k_heap_replay, hp[0] < 148 * 8 ? hp[0] : 148 * 8, 32, 0, ft, d_list, rlist, hp_counters, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(),
+			           c->d_m_val.as<uint64_t>(), c->d_m_aoff.as<int32_t>(), mi->d_pos, max_occ, opt->flag, t.aoff, c->d_hrank.as<uint32_t>(), c->d_hpop.as<uint32_t>());
+			MMG_LAUNCH_AS(c, "k_heap_emit", (named ? k_heap_emit<true> : k_heap_emit<false>), hp[0], HEAP_EMIT_THREADS, 0, ft, d_list, rlist, c->d_mv.as<mm128>(),
+			              c->d_m_n.as<int32_t>(), c->d_m_val.as<uint64_t>(), c->d_m_aoff.as<int32_t>(), mi->d_pos, max_occ, opt->flag, t.aoff, c->d_hpop.as<uint32_t>(),
+			              t.na, t.a, c->d_frag_iter.as<unsigned long long>() + 1, nt, n_named);
 		}
 	}
-	// literal replay: the heap merge for the few fragments the rank replay does not take; fill + klib radix sort for the non-heap presets
+	// literal replay: the heap merge for the few fragments the rank replay does not take; klib's radix sort for the non-heap presets
 	if (!heap_path) {
 		if (tot > 0)
-			MMG_LAUNCH(c, k_fill_flat_warp, mmg_blocks((size_t)n_list * 32, 128), 128, 0, n_list, pb.aoff->as<int64_t>(), d_tie, c->d_skey.as<uint64_t>(),
-			           c->d_sval.as<uint64_t>(), pb.na->as<int32_t>(), pb.a->as<mm128>(), pb.work->as<int32_t>(), pb.stack->as<RsFrame>());
+			MMG_LAUNCH(c, k_fill_flat_warp, mmg_blocks((size_t)n_list * 32, 128), 128, 0, n_list, t.aoff, d_tie, c->d_skey.as<uint64_t>(),
+			           c->d_sval.as<uint64_t>(), t.na, t.a, t.work, t.stack);
 	} else {
-		const int per_warp = d_flag == nullptr || n_list <= 4096 ? 1 : 0; // the re-chain pass (and any small list): spread over warps
-		MMG_LAUNCH_AS(c, "k_fill", (named ? k_fill<true> : k_fill<false>), mmg_blocks(per_warp ? (size_t)n_list * 32 : (size_t)n_list, 64), 64, 0, ft, d_list, n_list, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(),
-		           c->d_m_val.as<uint64_t>(), mi->d_pos, max_occ, opt->flag, pb.aoff->as<int64_t>(), pb.na->as<int32_t>(), pb.a->as<mm128>(), c->d_heap.as<mm128>(),
-		           pb.stack->as<RsFrame>(), heap_path ? c->d_replay.as<uint8_t>() : d_tie, heap_path ? 2 : 1, per_warp, nt, n_named);
+		const int per_warp = pass == 1 || n_list <= 4096 ? 1 : 0; // the re-chain pass (and any small list): spread over warps
+		MMG_LAUNCH_AS(c, "k_fill", (named ? k_fill<true> : k_fill<false>), mmg_blocks(per_warp ? (size_t)n_list * 32 : (size_t)n_list, 64), 64, 0,
+		              ft, d_list, n_list, c->d_mv.as<mm128>(), c->d_m_n.as<int32_t>(), c->d_m_val.as<uint64_t>(), mi->d_pos, max_occ, opt->flag, t.aoff, t.na, t.a,
+		              c->d_heap.as<mm128>(), c->d_replay.as<uint8_t>(), per_warp, nt, n_named);
 	}
 	if (getenv("MMG_TRACE")) { // distribution of the literal-replay work of this pass (debug aid; synchronises)
 		std::vector<uint8_t> hr((size_t)n_list); std::vector<int32_t> hn((size_t)n_list);
 		cudaStreamSynchronize(c->stream);
 		cudaMemcpy(hr.data(), heap_path ? c->d_replay.p : (void*)d_tie, (size_t)n_list, cudaMemcpyDeviceToHost);
-		cudaMemcpy(hn.data(), pb.na->p, (size_t)n_list * 4, cudaMemcpyDeviceToHost);
+		cudaMemcpy(hn.data(), t.na, (size_t)n_list * 4, cudaMemcpyDeviceToHost);
 		int64_t nr = 0, ar = 0, amax = 0, big = 0, abig = 0, big_all = 0, abig_all = 0;
 		for (int i = 0; i < n_list; ++i) {
 			if (hn[i] > 4096) ++big_all, abig_all += hn[i];
@@ -1701,24 +1722,29 @@ static int run_pass(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, 
 		fprintf(stderr, "[mmg::pass] max_occ %d: %d fragments, %lld anchors; > 4096 anchors: %lld fragments with %lld anchors; literal replay: %lld fragments, %lld anchors, largest %lld, "
 		        "of which > 4096 anchors: %lld fragments with %lld anchors\n", max_occ, n_list, (long long)tot, (long long)big_all, (long long)abig_all, (long long)nr, (long long)ar, (long long)amax, (long long)big, (long long)abig);
 	}
-	ChainOptDev co;
-	co.bw = opt->bw, co.max_gap = opt->max_gap, co.max_gap_ref = opt->max_gap_ref, co.max_frag_len = opt->max_frag_len;
-	co.max_skip = opt->max_chain_skip, co.max_iter = opt->max_chain_iter, co.min_cnt = opt->min_cnt, co.min_sc = opt->min_chain_score;
-	co.is_cdna = !!(opt->flag & MMG_F_SPLICE), co.is_sr = !!(opt->flag & MMG_F_SR);
+	*pt = t, *n_anchors = tot;
+	return MMG_OK;
+}
+
+// K3 of pass `pass` on the tot anchors seed_pass left in pt: segments -> fill -> tails.  The first pass flags the fragments the
+// re-chain pass takes in c->d_frag_flag.
+static int chain_pass(mmg_ctx_t *c, const mmg_mapopt_t *opt, const FragTab &ft, const ChainOptDev &co, int pass, const PassTab &pt, int64_t tot)
+{
+	const int n_list = pt.n_list;
+	const int32_t *n_seg = c->d_frag_nseg.as<int32_t>();
 	if (tot > 0) {
 		// segments: head flags -> compacted start indices
 		MMG_TRY(c->d_seg_head.ensure((size_t)tot + 16));
 		MMG_TRY(c->d_seg_start.ensure(((size_t)tot + 2) * 8 + 64));
 		MMG_TRY(c->d_seg_avg.ensure((size_t)(n_list + 1) * 4));
+		MMG_TRY(c->d_seg_li.ensure(((size_t)tot + 1) * 4));   // fragment slot of every segment head (sparse)
+		MMG_TRY(c->d_seg_long.ensure(((size_t)tot / CHAIN_SMALL_SEG + 2) * 4)); // segments left to the warp form
 		int64_t *seg_start = c->d_seg_start.as<int64_t>();
 		int32_t *d_nseg = reinterpret_cast<int32_t*>(seg_start + tot + 1), *d_next = d_nseg + 1, *d_nlong = d_nseg + 2;
 		MMG_CUDA(cudaMemsetAsync(d_nseg, 0, 16, c->stream));
-		MMG_TRY(c->d_seg_li.ensure(((size_t)tot + 1) * 4));   // fragment slot of every segment head (sparse)
-		MMG_TRY(c->d_seg_long.ensure(((size_t)tot / CHAIN_SMALL_SEG + 2) * 4)); // segments left to the warp form
-		MMG_LAUNCH(c, k_chain_heads, mmg_blocks(tot, 256), 256, 0, ft, d_list, n_list, c->d_misc.as<int32_t>(), co, pb.aoff->as<int64_t>(),
-		           pb.na->as<int32_t>(), pb.a->as<mm128>(), tot, c->d_seg_head.as<uint8_t>(), pb.work->as<int32_t>(), c->d_seg_li.as<int32_t>());
-		MMG_LAUNCH(c, k_chain_avgspan, mmg_blocks((size_t)n_list * 32, 128), 128, 0, n_list, pb.aoff->as<int64_t>(), pb.na->as<int32_t>(),
-		           pb.a->as<mm128>(), c->d_seg_avg.as<float>());
+		MMG_LAUNCH(c, k_chain_heads, mmg_blocks(tot, 256), 256, 0, ft, pt.list, n_list, n_seg, co, pt.aoff, pt.na, pt.a, tot, c->d_seg_head.as<uint8_t>(), pt.work,
+		           c->d_seg_li.as<int32_t>());
+		MMG_LAUNCH(c, k_chain_avgspan, mmg_blocks((size_t)n_list * 32, 128), 128, 0, n_list, pt.aoff, pt.na, pt.a, c->d_seg_avg.as<float>());
 		{
 			size_t tmp = 0;
 			cub::CountingInputIterator<int64_t> it(0);
@@ -1728,45 +1754,38 @@ static int run_pass(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, 
 			++c->launches;
 		}
 		// short segments: a thread each; the others: persistent warps pull them from the list the first kernel leaves
-		MMG_LAUNCH(c, k_chain_fill_small, 148 * 16, 128, 0, ft, d_list, c->d_misc.as<int32_t>(), co, pb.aoff->as<int64_t>(), pb.na->as<int32_t>(),
-		           pb.a->as<mm128>(), pb.work->as<int32_t>(), c->d_seg_avg.as<float>(), seg_start, c->d_seg_li.as<int32_t>(), d_nseg,
-		           c->d_seg_long.as<int32_t>(), d_nlong, c->d_frag_iter.as<unsigned long long>());
-		MMG_LAUNCH(c, k_chain_fill, 148 * 8, 128, 0, ft, d_list, n_list, c->d_misc.as<int32_t>(), co, pb.aoff->as<int64_t>(), pb.na->as<int32_t>(),
-		           pb.a->as<mm128>(), pb.work->as<int32_t>(), c->d_seg_avg.as<float>(), seg_start, c->d_seg_li.as<int32_t>(), d_nseg,
-		           c->d_seg_long.as<int32_t>(), d_nlong, d_next, c->d_frag_iter.as<unsigned long long>());
+		MMG_LAUNCH(c, k_chain_fill_small, 148 * 16, 128, 0, ft, pt.list, n_seg, co, pt.aoff, pt.na, pt.a, pt.work, c->d_seg_avg.as<float>(), seg_start,
+		           c->d_seg_li.as<int32_t>(), d_nseg, c->d_seg_long.as<int32_t>(), d_nlong, c->d_frag_iter.as<unsigned long long>());
+		MMG_LAUNCH(c, k_chain_fill, 148 * 8, 128, 0, ft, pt.list, n_list, n_seg, co, pt.aoff, pt.na, pt.a, pt.work, c->d_seg_avg.as<float>(), seg_start,
+		           c->d_seg_li.as<int32_t>(), d_nseg, c->d_seg_long.as<int32_t>(), d_nlong, d_next, c->d_frag_iter.as<unsigned long long>());
 	}
+	// The fragments with thousands of anchors get a CTA each, with its sorts staged in shared memory: all fragments of the re-chain
+	// pass (one CTA per SM, the whole shared memory), a few per thousand of the first pass (ahead of the warp kernel that takes
+	// everything else).  The CTAs pull fragments from a counter, largest first.
+	static const int heavy_env = getenv("MMG_TAIL_HEAVY_N") ? atoi(getenv("MMG_TAIL_HEAVY_N")) : TAIL_HEAVY_N;
+	static const int walk = getenv("MMG_TAIL_WALK") ? 1 : 0;
+	const int heavy_n = pass == 1 ? -1 : heavy_env, rechain_enabled = opt->max_occ > opt->mid_occ ? 1 : 0;
+	MMG_TRY(c->d_heavy.ensure(((size_t)n_list * 4 + 16) * 4));
+	int32_t *n_heavy = c->d_heavy.as<int32_t>(), *val0 = n_heavy + 4, *heavy = val0 + n_list;
+	uint32_t *key0 = reinterpret_cast<uint32_t*>(heavy + n_list), *key1 = key0 + n_list;
+	MMG_CUDA(cudaMemsetAsync(n_heavy, 0, 16, c->stream));
+	MMG_LAUNCH(c, k_tail_heavy_list, mmg_blocks(n_list, 256), 256, 0, n_list, pt.na, heavy_n, key0, val0, n_heavy);
 	{
-		// The fragments with thousands of anchors get a CTA each, with its sorts staged in shared memory: all fragments of the re-chain
-		// pass (one CTA per SM, the whole shared memory), a few per thousand of the first pass (ahead of the warp kernel that takes
-		// everything else).  The CTAs pull fragments from a counter, largest first.
-		static const int heavy_env = getenv("MMG_TAIL_HEAVY_N") ? atoi(getenv("MMG_TAIL_HEAVY_N")) : TAIL_HEAVY_N;
-		static const int walk = getenv("MMG_TAIL_WALK") ? 1 : 0;
-		const bool second = d_flag == nullptr;
-		const int heavy_n = second ? -1 : heavy_env, rechain_enabled = opt->max_occ > opt->mid_occ ? 1 : 0;
-		MMG_TRY(c->d_heavy.ensure(((size_t)n_list * 4 + 16) * 4));
-		int32_t *n_heavy = c->d_heavy.as<int32_t>(), *val0 = n_heavy + 4, *heavy = val0 + n_list;
-		uint32_t *key0 = reinterpret_cast<uint32_t*>(heavy + n_list), *key1 = key0 + n_list;
-		MMG_CUDA(cudaMemsetAsync(n_heavy, 0, 16, c->stream));
-		MMG_LAUNCH(c, k_tail_heavy_list, mmg_blocks(n_list, 256), 256, 0, n_list, pb.na->as<int32_t>(), heavy_n, key0, val0, n_heavy);
-		{
-			size_t tmp = 0;
-			cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp, key0, key1, val0, heavy, n_list, 0, 32, c->stream);
-			MMG_TRY(c->d_cub.ensure(tmp));
-			MMG_CUDA(cub::DeviceRadixSort::SortPairsDescending(c->d_cub.p, tmp, key0, key1, val0, heavy, n_list, 0, 32, c->stream));
-			++c->launches;
-		}
-		if (second)
-			MMG_LAUNCH(c, k_chain_tail_block, n_list < 148 ? n_list : 148, 1024, TAIL_BLOCK_SMEM, ft, d_list, n_list, c->d_misc.as<int32_t>(), co, pb.aoff->as<int64_t>(),
-			           pb.na->as<int32_t>(), pb.a->as<mm128>(), pb.work->as<int32_t>(), pb.u->as<uint64_t>(), pb.b->as<mm128>(), pb.stack->as<RsFrame>(),
-			           pb.nu->as<int32_t>(), pb.nv->as<int32_t>(), heavy, n_heavy, (size_t)TAIL_BLOCK_SMEM, nullptr, 0, nullptr, walk);
-		else
-			MMG_LAUNCH(c, k_chain_tail_block, 148 * 3, 512, TAIL_HEAVY_SMEM, ft, d_list, n_list, c->d_misc.as<int32_t>(), co, pb.aoff->as<int64_t>(),
-			           pb.na->as<int32_t>(), pb.a->as<mm128>(), pb.work->as<int32_t>(), pb.u->as<uint64_t>(), pb.b->as<mm128>(), pb.stack->as<RsFrame>(),
-			           pb.nu->as<int32_t>(), pb.nv->as<int32_t>(), heavy, n_heavy, (size_t)TAIL_HEAVY_SMEM, pb.rep->as<int32_t>(), rechain_enabled, d_flag, walk);
-		if (!second)
-		MMG_LAUNCH(c, k_chain_tail_warp, mmg_blocks((size_t)n_list * 32, 128), 128, 0, ft, d_list, n_list, c->d_misc.as<int32_t>(), co, pb.aoff->as<int64_t>(),
-		           pb.na->as<int32_t>(), pb.a->as<mm128>(), pb.work->as<int32_t>(), pb.u->as<uint64_t>(), pb.b->as<mm128>(), pb.stack->as<RsFrame>(),
-		           pb.nu->as<int32_t>(), pb.nv->as<int32_t>(), pb.rep->as<int32_t>(), rechain_enabled, d_flag, heavy_n);
+		size_t tmp = 0;
+		cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp, key0, key1, val0, heavy, n_list, 0, 32, c->stream);
+		MMG_TRY(c->d_cub.ensure(tmp));
+		MMG_CUDA(cub::DeviceRadixSort::SortPairsDescending(c->d_cub.p, tmp, key0, key1, val0, heavy, n_list, 0, 32, c->stream));
+		++c->launches;
+	}
+	if (pass == 1)
+		MMG_LAUNCH(c, k_chain_tail_block, n_list < 148 ? n_list : 148, 1024, TAIL_BLOCK_SMEM, ft, pt.list, n_list, n_seg, co, pt.aoff, pt.na, pt.a, pt.work,
+		           pt.u, pt.b, pt.stack, pt.nu, pt.nv, heavy, n_heavy, (size_t)TAIL_BLOCK_SMEM, nullptr, 0, nullptr, walk);
+	else {
+		uint8_t *flag = c->d_frag_flag.as<uint8_t>();
+		MMG_LAUNCH(c, k_chain_tail_block, 148 * 3, 512, TAIL_HEAVY_SMEM, ft, pt.list, n_list, n_seg, co, pt.aoff, pt.na, pt.a, pt.work, pt.u, pt.b, pt.stack,
+		           pt.nu, pt.nv, heavy, n_heavy, (size_t)TAIL_HEAVY_SMEM, pt.rep, rechain_enabled, flag, walk);
+		MMG_LAUNCH(c, k_chain_tail_warp, mmg_blocks((size_t)n_list * 32, 128), 128, 0, ft, pt.list, n_list, n_seg, co, pt.aoff, pt.na, pt.a, pt.work, pt.u,
+		           pt.b, pt.stack, pt.nu, pt.nv, pt.rep, rechain_enabled, flag, heavy_n);
 	}
 	return MMG_OK;
 }
@@ -1798,17 +1817,22 @@ extern "C" int mmg_seed_chain_resident(mmg_ctx_t *c, const mmg_idx_t *mi, const 
 	if (n_mv) MMG_LAUNCH(c, k_lookup, mmg_blocks(n_mv, 256), 256, 0, mi->view(), c->d_mv.as<mm128>(), n_mv, c->d_m_n.as<int32_t>(), c->d_m_val.as<uint64_t>());
 	FragTab ft;
 	ft.unit0 = c->d_frag_unit0.as<int32_t>(), ft.unit_off = c->d_unit_off.as<int64_t>(), ft.qlen = c->d_frag_qlen.as<int32_t>();
+	ChainOptDev co;
+	co.bw = opt->bw, co.max_gap = opt->max_gap, co.max_gap_ref = opt->max_gap_ref, co.max_frag_len = opt->max_frag_len;
+	co.max_skip = opt->max_chain_skip, co.max_iter = opt->max_chain_iter, co.min_cnt = opt->min_cnt, co.min_sc = opt->min_chain_score;
+	co.is_cdna = !!(opt->flag & MMG_F_SPLICE), co.is_sr = !!(opt->flag & MMG_F_SR);
 	const bool want_mini = !(opt->flag & MMG_F_SR); // only mm_est_err reads mini_pos (map.c:388)
 	MMG_TRY(c->d_frag_flag.ensure((size_t)nf + 16));
 	MMG_TRY(c->d_frag_iter.ensure(32)); // chain iterations | replayed merge pops | hits the self/dual filters dropped
 	MMG_CUDA(cudaMemsetAsync(c->d_frag_flag.p, 0, (size_t)nf + 16, c->stream));
 	MMG_CUDA(cudaMemsetAsync(c->d_frag_iter.p, 0, 32, c->stream));
-	MMG_TRY(c->h_path.ensure(64));
-	memset(c->h_path.p, 0, 64);
-	PassBufs p1 = {&c->d_frag_na, &c->d_frag_aoff, &c->d_frag_rep, &c->d_frag_nmini, &c->d_mini, &c->d_a, &c->d_work, &c->d_u, &c->d_b,
-	               &c->d_stack, &c->d_frag_nu, &c->d_frag_nv};
+	MMG_TRY(c->h_path.ensure(sizeof(PathCounters)));
+	PathCounters *pc = c->h_path.as<PathCounters>();
+	memset(pc, 0, sizeof(*pc));
+	PassTab p1, p2;
 	int64_t n_anch1 = 0, n_anch2 = 0;
-	MMG_TRY(run_pass(c, mi, opt, ft, nt, nullptr, nf, n_mv, opt->mid_occ, p1, want_mini, c->d_frag_flag.as<uint8_t>(), &n_anch1));
+	MMG_TRY(seed_pass(c, mi, opt, ft, nt, 0, nullptr, nf, opt->mid_occ, n_mv, want_mini, &p1, &n_anch1));
+	MMG_TRY(chain_pass(c, opt, ft, co, 0, p1, n_anch1));
 	// second pass: fragments whose best chain misses a segment, with the higher cut-off (map.c:353-375)
 	std::vector<int32_t> list;
 	std::vector<uint8_t> hflag(nf);
@@ -1820,23 +1844,20 @@ extern "C" int mmg_seed_chain_resident(mmg_ctx_t *c, const mmg_idx_t *mi, const 
 		MMG_CUDA(cudaStreamSynchronize(c->stream));
 		for (int f = 0; f < nf; ++f) if (hflag[f]) list.push_back(f);
 	}
-	PassBufs p2 = {&c->d2_frag_na, &c->d2_frag_aoff, &c->d2_frag_rep, &c->d2_frag_nmini, &c->d2_mini, &c->d2_a, &c->d2_work, &c->d2_u, &c->d2_b,
-	               &c->d2_stack, &c->d2_frag_nu, &c->d2_frag_nv};
 	const int n2 = (int)list.size();
 	if (n2) {
 		MMG_H2D(c, d_list, list.data(), (size_t)n2 * 4);
-		MMG_TRY(run_pass(c, mi, opt, ft, nt, d_list, n2, n_mv, opt->max_occ, p2, want_mini, nullptr, &n_anch2));
-		MMG_LAUNCH(c, k_merge_pass2, mmg_blocks(n2, 128), 128, 0, n2, d_list, c->d2_frag_nu.as<int32_t>(), c->d2_frag_nv.as<int32_t>(),
-		           c->d2_frag_rep.as<int32_t>(), c->d2_frag_nmini.as<int32_t>(), c->d_frag_nu.as<int32_t>(), c->d_frag_nv.as<int32_t>(),
-		           c->d_frag_rep.as<int32_t>(), c->d_frag_nmini.as<int32_t>(), d_src);
-	}
+		MMG_TRY(seed_pass(c, mi, opt, ft, nt, 1, d_list, n2, opt->max_occ, n_mv, want_mini, &p2, &n_anch2));
+		MMG_TRY(chain_pass(c, opt, ft, co, 1, p2, n_anch2));
+		MMG_LAUNCH(c, k_merge_pass2, mmg_blocks(n2, 128), 128, 0, n2, d_list, p2.nu, p2.nv, p2.rep, p2.nmini, p1.nu, p1.nv, p1.rep, p1.nmini, d_src);
+	} else p2 = pass_tab(c, 1, d_list, 0, want_mini); // unread: no fragment has a second-pass slot
 	// dense outputs
 	MMG_TRY(c->d_uoff.ensure((size_t)(nf + 1) * 8));
 	MMG_TRY(c->d_voff.ensure((size_t)(nf + 1) * 8));
 	MMG_TRY(c->d_moff.ensure((size_t)(nf + 1) * 8));
-	MMG_TRY(scan_i32_to_i64(c, c->d_frag_nu.as<int32_t>(), c->d_uoff.as<int64_t>(), nf + 1));
-	MMG_TRY(scan_i32_to_i64(c, c->d_frag_nv.as<int32_t>(), c->d_voff.as<int64_t>(), nf + 1));
-	if (want_mini) MMG_TRY(scan_i32_to_i64(c, c->d_frag_nmini.as<int32_t>(), c->d_moff.as<int64_t>(), nf + 1));
+	MMG_TRY(scan_i32_to_i64(c, p1.nu, c->d_uoff.as<int64_t>(), nf + 1));
+	MMG_TRY(scan_i32_to_i64(c, p1.nv, c->d_voff.as<int64_t>(), nf + 1));
+	if (want_mini) MMG_TRY(scan_i32_to_i64(c, p1.nmini, c->d_moff.as<int64_t>(), nf + 1));
 	int64_t tot[3] = {0, 0, 0};
 	MMG_D2H(c, &tot[0], c->d_uoff.as<int64_t>() + nf, 8);
 	MMG_D2H(c, &tot[1], c->d_voff.as<int64_t>() + nf, 8);
@@ -1846,16 +1867,14 @@ extern "C" int mmg_seed_chain_resident(mmg_ctx_t *c, const mmg_idx_t *mi, const 
 	MMG_TRY(c->d_out_u.ensure((size_t)(tot[0] + 1) * 8));
 	MMG_TRY(c->d_out_a.ensure((size_t)(tot[1] + 1) * 16));
 	MMG_TRY(c->d_out_mini.ensure((size_t)(tot[2] + 1) * 8));
-	MMG_LAUNCH(c, k_gather, nf, 64, 0, nf, d_src, c->d_frag_aoff.as<int64_t>(), c->d_u.as<uint64_t>(), c->d_a.as<mm128>(),
-	           c->d2_frag_aoff.as<int64_t>(), c->d2_u.as<uint64_t>(), c->d2_a.as<mm128>(), c->d_frag_nu.as<int32_t>(), c->d_frag_nv.as<int32_t>(),
-	           c->d_uoff.as<int64_t>(), c->d_voff.as<int64_t>(), c->d_out_u.as<uint64_t>(), c->d_out_a.as<mm128>());
+	MMG_LAUNCH(c, k_gather, nf, 64, 0, nf, d_src, p1.aoff, p1.u, p1.a, p2.aoff, p2.u, p2.a, p1.nu, p1.nv, c->d_uoff.as<int64_t>(), c->d_voff.as<int64_t>(),
+	           c->d_out_u.as<uint64_t>(), c->d_out_a.as<mm128>());
 	if (want_mini)
-		MMG_LAUNCH(c, k_gather_mini, nf, 64, 0, nf, ft, d_src, c->d_mini.as<uint64_t>(), c->d2_mini.as<uint64_t>(), c->d_frag_nmini.as<int32_t>(),
-		           c->d_moff.as<int64_t>(), c->d_out_mini.as<uint64_t>());
+		MMG_LAUNCH(c, k_gather_mini, nf, 64, 0, nf, ft, d_src, p1.mini, p2.mini, p1.nmini, c->d_moff.as<int64_t>(), c->d_out_mini.as<uint64_t>());
 	MMG_CUDA(cudaEventRecord(c->ev[1], c->stream));
 	unsigned long long iters = 0;
 	MMG_D2H(c, &iters, c->d_frag_iter.p, 8);
-	MMG_D2H(c, c->h_path.as<unsigned long long>() + 5, c->d_frag_iter.as<unsigned long long>() + 1, 16); // hits whose merge order was replayed, hits dropped by name
+	MMG_D2H(c, &pc->pops, c->d_frag_iter.as<unsigned long long>() + 1, 16);
 	out->n_minimizers = (uint64_t)n_mv, out->n_anchors = (uint64_t)(n_anch1 + n_anch2);
 	if (download) {
 		// meta: n_u | n_a | rep_len | n_mini | rechained (int32 each) then u_off | a_off | mini_off (uint64 each, nf+1)
@@ -1866,10 +1885,10 @@ extern "C" int mmg_seed_chain_resident(mmg_ctx_t *c, const mmg_idx_t *mi, const 
 		MMG_TRY(c->h_out_mini.ensure((size_t)(tot[2] + 1) * 8));
 		int32_t *hi = c->h_out_meta.as<int32_t>();
 		uint64_t *ho = reinterpret_cast<uint64_t*>(c->h_out_meta.as<uint8_t>() + ((meta_i + 15) & ~(size_t)15));
-		MMG_D2H(c, hi, c->d_frag_nu.p, (size_t)nf * 4);
-		MMG_D2H(c, hi + nf, c->d_frag_nv.p, (size_t)nf * 4);
-		MMG_D2H(c, hi + 2 * nf, c->d_frag_rep.p, (size_t)nf * 4);
-		MMG_D2H(c, hi + 3 * nf, c->d_frag_nmini.p, (size_t)nf * 4);
+		MMG_D2H(c, hi, p1.nu, (size_t)nf * 4);
+		MMG_D2H(c, hi + nf, p1.nv, (size_t)nf * 4);
+		MMG_D2H(c, hi + 2 * nf, p1.rep, (size_t)nf * 4);
+		MMG_D2H(c, hi + 3 * nf, p1.nmini, (size_t)nf * 4);
 		MMG_D2H(c, hi + 4 * nf, d_src, (size_t)nf * 4);
 		MMG_D2H(c, ho, c->d_uoff.p, (size_t)(nf + 1) * 8);
 		MMG_D2H(c, ho + (nf + 1), c->d_voff.p, (size_t)(nf + 1) * 8);
@@ -1887,11 +1906,9 @@ extern "C" int mmg_seed_chain_resident(mmg_ctx_t *c, const mmg_idx_t *mi, const 
 		float ms = 0;
 		cudaEventElapsedTime(&ms, c->ev[1], c->ev[2]); out->t_d2h_ms = ms;
 	} else MMG_CUDA(cudaStreamSynchronize(c->stream));
-	{ // path counters of this batch (the stream is idle here)
-		const int32_t *hp = c->h_path.as<int32_t>();
-		c->path[0] += (uint64_t)n2, c->path[1] += (uint64_t)(hp[0] + hp[4]), c->path[2] += (uint64_t)(hp[2] + hp[6]);
-		c->path[6] += c->h_path.as<unsigned long long>()[5], c->path[7] += c->h_path.as<unsigned long long>()[6];
-	}
+	// path counters of this batch (the stream is idle here)
+	c->path[0] += (uint64_t)n2, c->path[1] += (uint64_t)(pc->heap[0][0] + pc->heap[1][0]), c->path[2] += (uint64_t)(pc->heap[0][2] + pc->heap[1][2]);
+	c->path[6] += pc->pops, c->path[7] += pc->named;
 	float ms = 0;
 	cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]); out->t_kernels_ms = ms;
 	out->n_chain_iter = iters;
