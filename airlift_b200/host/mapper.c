@@ -543,14 +543,6 @@ static void *map_shard(void *data)
 /* ------------------------------------------------------------------ the three-step pipeline */
 
 typedef struct {
-	int n_seq, n_frag;
-	mm_bseq1_t *seq;
-	int *n_reg, *seg_off, *n_seg, *rep_len, *frag_gap;
-	mm_reg1_t **reg;
-	long order; /* position in the input (file driver: batches of two mappers leave in this order) */
-} step_t;
-
-typedef struct {
 	int mini_batch_size, n_processed, n_threads, n_fp;
 	const mm_mapopt_t *opt;
 	mm_bseq_file_t **fp;
@@ -1017,7 +1009,7 @@ int mm_map_file(const mm_idx_t *idx, const char *fn, const mm_mapopt_t *opt, int
 	return mm_map_file_frag(idx, 1, &fn, opt, n_threads);
 }
 
-/* ------------------------------------------------------------------ per-fragment API (a batch of one) */
+/* ------------------------------------------------------------------ per-fragment API (shared mini-batches, apiq.c) */
 
 struct mm_tbuf_s { int rep_len, frag_gap; };
 int mm_b200_check_opt(const mm_mapopt_t *opt)
@@ -1036,44 +1028,23 @@ int mm_b200_check_opt(const mm_mapopt_t *opt)
 mm_tbuf_t *mm_tbuf_init(void) { return (mm_tbuf_t*)calloc(1, sizeof(mm_tbuf_t)); }
 void mm_tbuf_destroy(mm_tbuf_t *b) { free(b); }
 
+/* what the request queue maps a round with: the batch path on every GPU of the index */
+static int apiq_map_batches(void *round, step_t **b, int n)
+{
+	const mm_apiq_round_t *r = (const mm_apiq_round_t*)round;
+	return mm_b200_map_batches(r->mi, r->opt, r->n_threads, (mm_b200_batch_t**)b, n, 0);
+}
+
 void mm_map_frag(const mm_idx_t *mi, int n_segs, const int *qlens, const char **seqs, int *n_regs, mm_reg1_t **regs, mm_tbuf_t *b,
                  const mm_mapopt_t *opt, const char *qname)
-{ /* map.c:272-424 */
-	shard_t sh;
-	mm_bseq1_t *seq;
-	int j, one_off = 0, n_seg = n_segs, rep[MM_MAX_SEG], gap[MM_MAX_SEG];
-	mm_mapopt_t o2;
+{ /* map.c:272-424, for the fragments of all concurrent callers at once */
+	int j, rep_len = 0, frag_gap = 0;
 	for (j = 0; j < n_segs; ++j) n_regs[j] = 0, regs[j] = 0;
 	if (n_segs <= 0 || n_segs > MM_MAX_SEG) return;
 	if (mi == 0 || mi->B == 0 || mi->B->n_dev < 1) { fprintf(stderr, "[ERROR] the index is not resident on a GPU\n"); exit(1); }
 	if (mm_b200_check_opt(opt) < 0 || (use_name_filters(opt) && mm_b200_name_keys_ready(mi) < 0)) exit(1);
-	/* the resident batch, staging buffers and pools belong to ctx[0], not to the caller's mm_tbuf_t: one call at a time */
-	pthread_mutex_lock(&mi->B->api_mu);
-	seq = (mm_bseq1_t*)calloc(n_segs, sizeof(mm_bseq1_t));
-	for (j = 0; j < n_segs; ++j) {
-		seq[j].l_seq = qlens[j], seq[j].name = (char*)qname, seq[j].seq = (char*)malloc((size_t)qlens[j] + 1);
-		memcpy(seq[j].seq, seqs[j], qlens[j]); seq[j].seq[qlens[j]] = 0;
-	}
-	memset(&sh, 0, sizeof(sh));
-	mm_arena_init(&sh.arena);
-	/* MM_F_INDEPEND_SEG is read by the file and batch drivers only (worker_for, map.c:475-485): the reference's mm_map_frag maps
-	 * the segments it is given jointly whatever the flag, and so does this one (shard_t::flip stays 0).
-	 * worker_for flips the mates of a pair around this call (map.c:467-469,486-497); callers of the library API
-	 * pass sequences already in mapping orientation, so neither the host nor the device flips here.
-	 * pe_ori = 0 keeps `pe_ori >= 0` (pairing on, map.c:404) while naming no mate to flip. */
-	o2 = *opt;
-	if (o2.pe_ori > 0) o2.pe_ori = 0;
-	sh.mi = mi, sh.opt = &o2, sh.ctx = mi->B->ctx[0], sh.didx = mi->B->didx[0];
-	mm_mapopt_to_dev(&o2, &sh.dopt);
-	sh.n_threads = 1, sh.f0 = 0, sh.f1 = 1;
-	sh.seq = seq, sh.n_seg = &n_seg, sh.seg_off = &one_off, sh.n_reg = n_regs, sh.rep_len = rep, sh.frag_gap = gap, sh.reg = regs;
-	sh.ops = SH_STAGE | SH_SEND | SH_MAP;
-	shard_run(&sh);
-	if (sh.rc) { fprintf(stderr, "[ERROR] mapping failed; no CPU fallback exists\n"); exit(1); }
-	if (b) b->rep_len = rep[0], b->frag_gap = gap[0];
-	for (j = 0; j < n_segs; ++j) free(seq[j].seq);
-	free(seq);
-	pthread_mutex_unlock(&mi->B->api_mu);
+	mm_apiq_map_frag(mi, apiq_map_batches, mm_b200_batches_in_flight, opt, n_segs, qlens, seqs, qname, n_regs, regs, &rep_len, &frag_gap);
+	if (b) b->rep_len = rep_len, b->frag_gap = frag_gap;
 }
 
 mm_reg1_t *mm_map(const mm_idx_t *mi, int qlen, const char *seq, int *n_regs, mm_tbuf_t *b, const mm_mapopt_t *opt, const char *qname)

@@ -61,7 +61,8 @@ struct mm_idx_bucket_s {
 	pthread_mutex_t up_token[16];  /* device path: the shards of a GPU stage their reads one after the other */
 	pthread_mutex_t gpu_token[16]; /* with lanes > 1: one shard per GPU runs device stages at a time, the others do their host stages */
 	int32_t max_occ_cache_set; float max_occ_cache_f; int32_t max_occ_cache;
-	pthread_mutex_t api_mu; /* mm_map_frag()/mm_map() share ctx[0]: concurrent callers take turns */
+	pthread_mutex_t apiq_mu;  /* guards the lazy start of apiq */
+	struct mm_apiq_s *apiq;   /* mm_map_frag()/mm_map(): request queue and its dispatcher thread (apiq.c); 0 until the first call */
 	pthread_mutex_t key_mu; /* guards the lazy set-up of the name keys */
 	const char **sorted_names; /* the target names in strcmp order, once the name keys were made (namekey.c) */
 };
@@ -230,5 +231,24 @@ uint32_t mm_b200_unit_key(const mm_idx_t *mi, const char *qname); /* after mm_b2
 /* mapper.c */
 mmg_ctx_t *mm_b200_ctx(const mm_idx_t *mi, int dev_slot);
 void mm_mapopt_to_dev(const mm_mapopt_t *opt, mmg_mapopt_t *d);
+
+/* a mini-batch of fragments (the reference's step_t, map.c:449-456, minus the per-thread buffers); mm_b200_batch_t is one */
+typedef struct {
+	int n_seq, n_frag;
+	mm_bseq1_t *seq;
+	int *n_reg, *seg_off, *n_seg, *rep_len, *frag_gap;
+	mm_reg1_t **reg;
+	long order; /* position in the input (file driver: batches of two mappers leave in this order) */
+} step_t;
+
+/* apiq.c: mm_map_frag() callers of any number of threads enqueue requests; one dispatcher thread per index maps what is
+ * queued when it comes round, as up to two mini-batches through `map`, and hands every caller its own hits */
+typedef struct { const mm_idx_t *mi; const mm_mapopt_t *opt; int n_threads; } mm_apiq_round_t; /* what `map` receives as its first argument */
+typedef int (*mm_apiq_map_f)(void *round, step_t **b, int n);               /* 0, or -1 when mapping failed */
+typedef int (*mm_apiq_in_flight_f)(const mm_idx_t *mi, const mm_mapopt_t *opt); /* batches `map` overlaps for these options */
+/* maps one fragment; the first call on an index starts its dispatcher with `map` and `in_flight` */
+void mm_apiq_map_frag(const mm_idx_t *mi, mm_apiq_map_f map, mm_apiq_in_flight_f in_flight, const mm_mapopt_t *opt, int n_segs,
+                      const int *qlens, const char **seqs, const char *qname, int *n_regs, mm_reg1_t **regs, int *rep_len, int *frag_gap);
+void mm_apiq_stop(struct mm_idx_bucket_s *B); /* maps what is queued, then stops and joins the dispatcher */
 
 #endif

@@ -48,7 +48,7 @@ static mm_idx_t *idx_from_seqs(int w, int k, int b, int flag, int n, char **seq,
 	}
 	B->n_dev = g_n_dev;
 	B->lanes = g_lanes;
-	pthread_mutex_init(&B->api_mu, 0);
+	pthread_mutex_init(&B->apiq_mu, 0);
 	pthread_mutex_init(&B->key_mu, 0);
 	for (d = 0; d < g_n_dev; ++d) {
 		int l;
@@ -73,6 +73,7 @@ void mm_idx_destroy(mm_idx_t *mi)
 	int d;
 	if (mi == 0) return;
 	if (mi->B) {
+		mm_apiq_stop(mi->B); /* no thread outlives the index */
 		for (d = 0; d < mi->B->n_dev; ++d) mmg_idx_free(mi->B->didx[d]);
 		for (d = 0; d < mi->B->n_dev * mi->B->lanes; ++d) mmg_destroy(mi->B->ctx[d]);
 		free(mi->B->sorted_names);
@@ -442,7 +443,7 @@ mm_idx_t *mm_b200_idx_alloc_named(const mm_idxopt_t *opt, int n_seq, const char 
 		sum += lens[i];
 	}
 	B->n_dev = 1, B->lanes = g_lanes, B->dev_id[0] = g_dev[0];
-	pthread_mutex_init(&B->api_mu, 0);
+	pthread_mutex_init(&B->apiq_mu, 0);
 	pthread_mutex_init(&B->key_mu, 0);
 	pthread_mutex_init(&B->gpu_token[0], 0);
 	pthread_mutex_init(&B->up_token[0], 0);

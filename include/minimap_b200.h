@@ -5,7 +5,8 @@
  * recompiles against this header unchanged.  Differences, all behind the API:
  *   - mm_idx_t::B no longer points at per-bucket khash tables; it holds the handle of the HBM-resident index;
  *   - mapping is batched: mm_map_file_frag() drives the GPU stages once per mini-batch instead of once
- *     per fragment, and mm_map_frag()/mm_map() are a batch of one;
+ *     per fragment, and the mm_map_frag()/mm_map() calls that are waiting at the same time, from any number of threads,
+ *     are mapped together as one mini-batch;
  *   - a CUDA device is required: every entry point fails with an [ERROR] on stderr otherwise.
  */
 #ifndef MINIMAP_B200_H
@@ -196,8 +197,10 @@ int mm_b200_idx_finalize(mm_idx_t *mi);
 /* options this build does not implement (splice, -D/-X/--dual=no, -T, --split-prefix) are refused, never ignored: 0 if
  * opt can be mapped with, else -1 after an [ERROR] line.  MM_F_INDEPEND_SEG (--no-pairing) maps the two reads of a pair
  * one by one in mm_map_file_frag() and mm_b200_map_batch(es); mm_map_frag() maps the segments it is given jointly, as the
- * reference does.  mm_map_frag()/mm_map() take turns on a lock (one resident batch per GPU context), so concurrent
- * callers are safe but serialised. */
+ * reference does.  mm_map_frag()/mm_map() may be called from any number of threads at once, each with its own mm_tbuf_t:
+ * one dispatcher thread per index (started by the first call, joined by mm_idx_destroy) maps the calls that are waiting
+ * with equal options as shared mini-batches on every GPU of the index, and a lone caller is never held back to fill one.
+ * Calling them while mm_b200_map_batch(es) or mm_map_file(_frag) maps on the same index is not supported. */
 int mm_b200_check_opt(const mm_mapopt_t *opt);
 /* name keys of the self/dual-hit filters (see "name keys" in mmg.h): sorted[] receives the n names in strcmp order (a NULL name
  * counts as ""), tkey[] the target key of each; mm_b200_name_ukey gives the unit key of qname against those sorted names
