@@ -97,10 +97,10 @@ void mm_write_sam_hdr(const mm_idx_t *idx, const char *rg, const char *ver, int 
 
 /* ---- cs / MD (format.c:137-250) */
 
-static void write_cs(mm_str_t *s, const uint8_t *tseq, const uint8_t *qseq, const mm_reg1_t *r, char *tmp, int no_iden)
+static void write_cs(mm_str_t *s, const uint8_t *tseq, const uint8_t *qseq, const mm_reg1_t *r, char *tmp, int no_iden, int write_tag)
 {
 	int i, q_off = 0, t_off = 0;
-	sb_str(s, "\tcs:Z:");
+	if (write_tag) sb_str(s, "\tcs:Z:");
 	for (i = 0; i < (int)r->p->n_cigar; ++i) {
 		const int op = r->p->cigar[i] & 0xf, len = r->p->cigar[i] >> 4;
 		int j;
@@ -138,10 +138,10 @@ static void write_cs(mm_str_t *s, const uint8_t *tseq, const uint8_t *qseq, cons
 	assert(t_off == r->re - r->rs && q_off == r->qe - r->qs);
 }
 
-static void write_md(mm_str_t *s, const uint8_t *tseq, const uint8_t *qseq, const mm_reg1_t *r, char *tmp)
+static void write_md(mm_str_t *s, const uint8_t *tseq, const uint8_t *qseq, const mm_reg1_t *r, char *tmp, int write_tag)
 {
 	int i, q_off = 0, t_off = 0, l_MD = 0;
-	sb_str(s, "\tMD:Z:");
+	if (write_tag) sb_str(s, "\tMD:Z:");
 	for (i = 0; i < (int)r->p->n_cigar; ++i) {
 		const int op = r->p->cigar[i] & 0xf, len = r->p->cigar[i] >> 4;
 		int j;
@@ -162,7 +162,9 @@ static void write_md(mm_str_t *s, const uint8_t *tseq, const uint8_t *qseq, cons
 	assert(t_off == r->re - r->rs && q_off == r->qe - r->qs);
 }
 
-static void write_cs_or_md(mm_str_t *s, const mm_idx_t *mi, const mm_bseq1_t *t, const mm_reg1_t *r, int no_iden, int is_md)
+/* the cs (is_md: MD) string of r appended to s, after its "\tcs:Z:" / "\tMD:Z:" tag when write_tag; seq is the query as it was
+ * mapped (format.c:137-250).  The PAF/SAM writers and mm_gen_cs / mm_gen_MD share it. */
+static void write_cs_or_md(mm_str_t *s, const mm_idx_t *mi, const char *seq, const mm_reg1_t *r, int no_iden, int is_md, int write_tag)
 {
 	int i;
 	const int ql = r->qe - r->qs, tl = r->re - r->rs;
@@ -173,11 +175,33 @@ static void write_cs_or_md(mm_str_t *s, const mm_idx_t *mi, const mm_bseq1_t *t,
 	tseq = (uint8_t*)malloc(tl > 0 ? tl : 1);
 	tmp = (char*)malloc((tl > ql ? tl : ql) + 1);
 	mm_idx_getseq(mi, r->rid, r->rs, r->re, tseq);
-	if (!r->rev) for (i = r->qs; i < r->qe; ++i) qseq[i - r->qs] = seq_nt4_table[(uint8_t)t->seq[i]];
-	else for (i = r->qs; i < r->qe; ++i) { const uint8_t c = seq_nt4_table[(uint8_t)t->seq[i]]; qseq[r->qe - i - 1] = c >= 4 ? 4 : 3 - c; }
-	if (is_md) write_md(s, tseq, qseq, r, tmp);
-	else write_cs(s, tseq, qseq, r, tmp, no_iden);
+	if (!r->rev) for (i = r->qs; i < r->qe; ++i) qseq[i - r->qs] = seq_nt4_table[(uint8_t)seq[i]];
+	else for (i = r->qs; i < r->qe; ++i) { const uint8_t c = seq_nt4_table[(uint8_t)seq[i]]; qseq[r->qe - i - 1] = c >= 4 ? 4 : 3 - c; }
+	if (is_md) write_md(s, tseq, qseq, r, tmp, write_tag);
+	else write_cs(s, tseq, qseq, r, tmp, no_iden, write_tag);
 	free(qseq); free(tseq); free(tmp);
+}
+
+static int gen_cs_or_md(char **buf, int *max_len, const mm_idx_t *mi, const mm_reg1_t *r, const char *seq, int no_iden, int is_md)
+{ /* mm_gen_cs_or_MD (format.c): the string alone, in a buffer the caller keeps across calls */
+	mm_str_t s;
+	s.s = *buf, s.l = 0, s.m = *max_len > 0 ? (unsigned)*max_len : 0;
+	write_cs_or_md(&s, mi, seq, r, no_iden, is_md, 0);
+	if (s.s && s.m > 0) s.s[s.l] = 0;
+	*buf = s.s, *max_len = (int)s.m;
+	return (int)s.l;
+}
+
+int mm_gen_cs(void *km, char **buf, int *max_len, const mm_idx_t *mi, const mm_reg1_t *r, const char *seq, int no_iden)
+{
+	(void)km;
+	return gen_cs_or_md(buf, max_len, mi, r, seq, no_iden, 0);
+}
+
+int mm_gen_MD(void *km, char **buf, int *max_len, const mm_idx_t *mi, const mm_reg1_t *r, const char *seq)
+{
+	(void)km;
+	return gen_cs_or_md(buf, max_len, mi, r, seq, 0, 1);
 }
 
 static double event_identity(const mm_reg1_t *r)
@@ -241,7 +265,7 @@ void mm_write_paf3(mm_str_t *s, const mm_idx_t *mi, const mm_bseq1_t *t, const m
 		for (k = 0; k < r->p->n_cigar; ++k) { sb_int(s, r->p->cigar[k] >> 4); sb_chr(s, "MIDNSHP=XB"[r->p->cigar[k] & 0xf]); }
 	}
 	if (r->p && (opt_flag & (MM_F_OUT_CS|MM_F_OUT_MD)))
-		write_cs_or_md(s, mi, t, r, !(opt_flag & MM_F_OUT_CS_LONG), opt_flag & MM_F_OUT_MD);
+		write_cs_or_md(s, mi, t->seq, r, !(opt_flag & MM_F_OUT_CS_LONG), opt_flag & MM_F_OUT_MD, 1);
 	if ((opt_flag & MM_F_COPY_COMMENT) && t->comment) { sb_chr(s, '\t'); sb_str(s, t->comment); }
 }
 
@@ -422,7 +446,7 @@ void mm_write_sam3(mm_str_t *s, const mm_idx_t *mi, const mm_bseq1_t *t, int seg
 			}
 		}
 		if (r->p && (opt_flag & (MM_F_OUT_CS|MM_F_OUT_MD)))
-			write_cs_or_md(s, mi, t, r, !(opt_flag & MM_F_OUT_CS_LONG), opt_flag & MM_F_OUT_MD);
+			write_cs_or_md(s, mi, t->seq, r, !(opt_flag & MM_F_OUT_CS_LONG), opt_flag & MM_F_OUT_MD, 1);
 		if (cigar_in_tag) sam_cigar(s, flag, 1, t->l_seq, r, opt_flag);
 	}
 	if (rep_len >= 0) sb_tag_i(s, "\trl:i:", rep_len);

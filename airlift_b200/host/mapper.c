@@ -1012,16 +1012,24 @@ int mm_map_file(const mm_idx_t *idx, const char *fn, const mm_mapopt_t *opt, int
 /* ------------------------------------------------------------------ per-fragment API (shared mini-batches, apiq.c) */
 
 struct mm_tbuf_s { int rep_len, frag_gap; };
-int mm_b200_check_opt(const mm_mapopt_t *opt)
+const char *mm_b200_opt_error(const mm_mapopt_t *opt)
 { /* what the device stages do not implement is refused with a message; nothing is silently dropped */
-	const char *what = 0;
-	if (opt->flag & MM_F_SPLICE) what = "spliced alignment (--splice, ksw_exts2)";
+#define NOT_SUPPORTED " is not supported by this build"
+	if (opt->flag & MM_F_SPLICE) return "spliced alignment (--splice, ksw_exts2)" NOT_SUPPORTED;
 	/* the short-read presets' device post stages (aln_plan_sr, mmg_aln.h) do not bound the extension of a self-chain (MM_SEED_SELF) */
-	else if ((opt->flag & (MM_F_NO_DIAG | MM_F_NO_DUAL)) && (opt->flag & MM_F_SR)) what = "the self/dual-hit filters of the all-vs-all modes (-D, -X, --dual=no, ava-ont, ava-pb; map.c:128-137)";
-	else if (opt->sdust_thres > 0) what = "SDUST masking of query minimizers (-T, map.c:41-62)";
-	else if (opt->split_prefix) what = "--split-prefix (the index is a single part in HBM)";
-	if (what == 0) return 0;
-	fprintf(stderr, "[ERROR] %s is not supported by this build\n", what);
+	if ((opt->flag & (MM_F_NO_DIAG | MM_F_NO_DUAL)) && (opt->flag & MM_F_SR))
+		return "the self/dual-hit filters of the all-vs-all modes (-D, -X, --dual=no, ava-ont, ava-pb; map.c:128-137)" NOT_SUPPORTED;
+	if (opt->sdust_thres > 0) return "SDUST masking of query minimizers (-T, map.c:41-62)" NOT_SUPPORTED;
+	if (opt->split_prefix) return "--split-prefix (the index is a single part in HBM)" NOT_SUPPORTED;
+	return 0;
+#undef NOT_SUPPORTED
+}
+
+int mm_b200_check_opt(const mm_mapopt_t *opt)
+{
+	const char *msg = mm_b200_opt_error(opt);
+	if (msg == 0) return 0;
+	fprintf(stderr, "[ERROR] %s\n", msg);
 	return -1;
 }
 

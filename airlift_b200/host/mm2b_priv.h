@@ -162,6 +162,7 @@ void mm_bseq_free1(mm_bseq1_t *s, int packed);
 int mm_qname_len(const char *s);
 int mm_qname_same(const char *s1, const char *s2);
 void mm_revcomp_bseq(mm_bseq1_t *s);
+int mm_bseq_pack1(mm_bseq1_t *s, const char *name, const char *seq, int l_seq);
 
 /* hits.c */
 #ifndef MM_DEVICE_BUILD

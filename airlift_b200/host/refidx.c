@@ -109,6 +109,15 @@ int mm_idx_getseq(const mm_idx_t *mi, uint32_t rid, uint32_t st, uint32_t en, ui
 	return (int)(en - st);
 }
 
+int mm_idx_name2id(const mm_idx_t *mi, const char *name)
+{ /* a linear scan: bindings look a name up once per call, and the index keeps no name table */
+	uint32_t i;
+	if (name == 0) return -1;
+	for (i = 0; i < mi->n_seq; ++i)
+		if (mi->seq[i].name && strcmp(mi->seq[i].name, name) == 0) return (int)i;
+	return -1;
+}
+
 int32_t mm_idx_cal_max_occ(const mm_idx_t *mi, float f)
 {
 	int32_t t = 0;

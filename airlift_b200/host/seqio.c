@@ -415,3 +415,61 @@ mm_bseq1_t *mm_bseq_read_frag2(int n_fp, mm_bseq_file_t **fp, int chunk_size, in
 	*n_ = a.n;
 	return a.a;
 }
+
+int mm_bseq_pack1(mm_bseq1_t *s, const char *name, const char *seq, int l_seq)
+{ /* a packed record (see slab_t) on a slab of its own, for batches built from memory; 0, or -1 when out of memory */
+	const size_t l_name = name ? strlen(name) : 0, off = (sizeof(slab_t) + 7) & ~(size_t)7;
+	char *p = (char*)malloc(off + sizeof(slab_t*) + l_name + 1 + (size_t)l_seq + 1), *b;
+	if (p == 0) return -1;
+	((slab_t*)p)->live = 1;
+	*(slab_t**)(p + off) = (slab_t*)p;
+	b = p + off + sizeof(slab_t*);
+	memset(s, 0, sizeof(*s));
+	s->name = b, memcpy(b, name ? name : "", l_name + 1);
+	s->seq = b + l_name + 1, memcpy(s->seq, seq, l_seq), s->seq[l_seq] = 0;
+	s->l_seq = l_seq;
+	return 0;
+}
+
+/* ---- record-at-a-time reader for bindings (mappy.fastx_read): the records mm_bseq_read3 gives, one per call */
+
+struct mm_fastx_s { mm_bseq_file_t *fp; mm_bseq1_t *a; int n, i, with_comment; };
+
+mm_fastx_t *mm_fastx_open(const char *fn, int with_comment)
+{
+	mm_fastx_t *r;
+	mm_bseq_file_t *fp = mm_bseq_open(fn);
+	if (fp == 0) return 0;
+	r = (mm_fastx_t*)calloc(1, sizeof(*r));
+	r->fp = fp, r->with_comment = with_comment;
+	return r;
+}
+
+static void fastx_drop(mm_fastx_t *r)
+{
+	int i;
+	for (i = 0; i < r->n; ++i) mm_bseq_free1(&r->a[i], 0);
+	free(r->a);
+	r->a = 0, r->n = r->i = 0;
+}
+
+int mm_fastx_read(mm_fastx_t *r, const char **name, const char **seq, const char **qual, const char **comment)
+{
+	const mm_bseq1_t *t;
+	if (r->i == r->n) {
+		fastx_drop(r);
+		r->a = mm_bseq_read3(r->fp, 1, 1, r->with_comment, 0, &r->n); /* chunk of one base: one record (more after empty ones) */
+		if (r->n == 0) return -1;
+	}
+	t = &r->a[r->i++];
+	*name = t->name, *seq = t->seq, *qual = t->qual, *comment = t->comment;
+	return t->l_seq;
+}
+
+void mm_fastx_close(mm_fastx_t *r)
+{
+	if (r == 0) return;
+	fastx_drop(r);
+	mm_bseq_close(r->fp);
+	free(r);
+}

@@ -174,6 +174,7 @@ void mm_idx_destroy(mm_idx_t *mi);
 #endif
 MM_FN int mm_idx_getseq(const mm_idx_t *mi, uint32_t rid, uint32_t st, uint32_t en, uint8_t *seq);
 int32_t mm_idx_cal_max_occ(const mm_idx_t *mi, float f);
+int mm_idx_name2id(const mm_idx_t *mi, const char *name); /* -1 when no target has that name */
 
 /* mapping (map.c) */
 mm_tbuf_t *mm_tbuf_init(void);
@@ -183,6 +184,18 @@ void mm_map_frag(const mm_idx_t *mi, int n_segs, const int *qlens, const char **
                  const mm_mapopt_t *opt, const char *qname);
 int mm_map_file(const mm_idx_t *idx, const char *fn, const mm_mapopt_t *opt, int n_threads);
 int mm_map_file_frag(const mm_idx_t *idx, int n_segs, const char **fn, const mm_mapopt_t *opt, int n_threads);
+
+/* cs / MD of a hit (format.c, mm_gen_cs / mm_gen_MD), the string alone: *buf is realloc'd to *max_len bytes and the length
+ * is returned; seq is the query as mapped; km is not used.  The PAF/SAM writers print the same strings. */
+int mm_gen_cs(void *km, char **buf, int *max_len, const mm_idx_t *mi, const mm_reg1_t *r, const char *seq, int no_iden);
+int mm_gen_MD(void *km, char **buf, int *max_len, const mm_idx_t *mi, const mm_reg1_t *r, const char *seq);
+
+/* FASTA/FASTQ (gzip'd or not) one record at a time, as the mapper reads it (bseq.c): mm_fastx_read returns the sequence
+ * length, or -1 at the end; the strings (qual and comment may be 0) stay valid until the next call */
+typedef struct mm_fastx_s mm_fastx_t;
+mm_fastx_t *mm_fastx_open(const char *fn, int with_comment);
+int mm_fastx_read(mm_fastx_t *r, const char **name, const char **seq, const char **qual, const char **comment);
+void mm_fastx_close(mm_fastx_t *r);
 
 /* B200 additions */
 int mm_b200_set_devices(int n_gpus, const int *dev_ids); /* before building the index; default: device 0 */
@@ -202,6 +215,7 @@ int mm_b200_idx_finalize(mm_idx_t *mi);
  * with equal options as shared mini-batches on every GPU of the index, and a lone caller is never held back to fill one.
  * Calling them while mm_b200_map_batch(es) or mm_map_file(_frag) maps on the same index is not supported. */
 int mm_b200_check_opt(const mm_mapopt_t *opt);
+const char *mm_b200_opt_error(const mm_mapopt_t *opt); /* the message mm_b200_check_opt prints (no "[ERROR] "), or 0: nothing printed */
 /* name keys of the self/dual-hit filters (see "name keys" in mmg.h): sorted[] receives the n names in strcmp order (a NULL name
  * counts as ""), tkey[] the target key of each; mm_b200_name_ukey gives the unit key of qname against those sorted names
  * (MMG_NAME_NONE for a NULL qname) */
@@ -237,6 +251,25 @@ int  mm_b200_set_in_flight(int n); /* mini-batches mm_b200_map_batches keeps in 
 int  mm_b200_batches_in_flight(const mm_idx_t *mi, const mm_mapopt_t *opt); /* what mm_b200_map_batches overlaps for these options */
 int  mm_b200_map_batches(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_threads, mm_b200_batch_t **b, int n, int mode);
 int  mm_b200_n_devices(const mm_idx_t *mi);
+
+/* Hits for bindings that do not mirror mm_reg1_t (airlift_b200/mappy.py): one malloc'd block, released with mm_b200_hits_free,
+ * holding n_hits rows of MM_B200_HITS_COLS integers, the CIGAR words of every hit in row order, and the cs (short form) / MD
+ * strings asked for, each NUL-terminated.  Columns: frag, seg_id, rid, rs, re, qs, qe, rev, mapq, primary (id == parent), mlen,
+ * blen, n_ambi, trans_strand, dp_score, dp_max, n_cigar, cigar_off, cs_off, cs_len, md_off, md_len (string offsets: -1 when
+ * not made). */
+#define MM_B200_HITS_COLS 22
+#define MM_B200_HITS_CS   0x1
+#define MM_B200_HITS_MD   0x2
+typedef struct { int64_t n_hits, n_cigar, n_str; const int64_t *rows; const uint32_t *cigar; const char *str; } mm_b200_hits_t;
+/* one fragment of one or two reads through mm_map_frag (any thread): the second read is given as sequenced, mapped as its reverse
+ * complement, and its hits are reported in its own orientation, as the PAF writer prints a pair */
+mm_b200_hits_t *mm_b200_map_hits(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_segs, const int *qlens, const char **seqs,
+                                 const char *qname, int flags);
+mm_b200_hits_t *mm_b200_batch_hits_flat(const mm_idx_t *mi, const mm_b200_batch_t *b, int flags); /* of a mapped batch */
+void mm_b200_hits_free(mm_b200_hits_t *h);
+/* a batch of n_frag fragments from memory, for mm_b200_map_batch(es): fragment f has n_segs[f] reads, the next ones of
+ * qlens / seqs, named names[f] (names may be 0) */
+mm_b200_batch_t *mm_b200_make_batch(int n_frag, const int *n_segs, const int *qlens, const char *const *seqs, const char *const *names);
 void mm_b200_path_counts(const mm_idx_t *mi, uint64_t out[8], int reset); /* see mmg_path_counts (mmg.h) */
 
 typedef struct { /* accumulated over mm_b200_map_batch / mm_map_file_frag calls; seconds and counts */
