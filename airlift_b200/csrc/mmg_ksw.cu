@@ -9,6 +9,10 @@
 //    (mmg_kswdpx.h); they live in a shared-memory slot when they fit (all short-read jobs) and in a global arena otherwise;
 //  - literal CTA (k_ksw_dpx_block): the same program for jobs whose state exceeds the warp's slot, one CTA per job with the
 //    state in its shared memory.
+//
+// Two environment variables, read once per process, are test aids: MMG_KSW_FORCE_BLOCK=1 sends every literal job the CTA form can
+// take through it; MMG_KSW_BUDGET=<bytes> replaces the device memory mmg_ksw_batch lets one round of DP state take (a third of
+// what is free), so that the split into parts (ksw_batch_parts) runs without filling the device.
 #include <algorithm>
 #include <cub/cub.cuh>
 #include "mmg_ctx.cuh"
@@ -964,7 +968,8 @@ extern "C" int mmg_ksw_batch(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt
 	// the DP state may take a third of what the device has free (the ctx's own DP buffers count as free: they are reused)
 	size_t fr = 0, total = 0;
 	MMG_CUDA(cudaMemGetInfo(&fr, &total));
-	const size_t budget = (fr + c->k_mem.cap + c->k_p.cap + c->k_cig.cap) / 3;
+	static const size_t budget_env = getenv("MMG_KSW_BUDGET") ? strtoull(getenv("MMG_KSW_BUDGET"), nullptr, 10) : 0; // test aid, see the header
+	const size_t budget = budget_env ? budget_env : (fr + c->k_mem.cap + c->k_p.cap + c->k_cig.cap) / 3;
 	const int rc = ksw_launch(c, c->k_jobs.as<mmg_ksw_job_t>(), n_jobs, c->d_Q.as<uint32_t>(), mi->d_S, c->d_q_off.as<uint64_t>(), c->d_seq_len.as<int32_t>(),
 	                          mi->d_seq_off, make_score(opt), res, cigars, kernel_ms, cells, true, budget);
 	if (rc != KSW_SPLIT) return rc;

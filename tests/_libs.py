@@ -249,6 +249,50 @@ def simple_mat(a, b, sc_ambi):
     return m
 
 
+class KswScoring:
+    """One scoring of the DP kernels with the job parameters the tests use with it.  b and sc_ambi may be given with either sign:
+    simple_mat, like make_score on the device and ksw_gen_simple_mat in the reference, takes their magnitude."""
+
+    def __init__(self, name, a, b, sc_ambi, q, e, q2, e2, zdrop, end_bonus, band):
+        self.name, self.a, self.b, self.sc_ambi = name, a, b, sc_ambi
+        self.q, self.e, self.q2, self.e2 = q, e, q2, e2
+        self.zdrop, self.end_bonus, self.band = zdrop, end_bonus, band
+
+    @property
+    def mat(self):
+        return simple_mat(self.a, self.b, self.sc_ambi)
+
+    @property
+    def pen(self):
+        return (self.q, self.e, self.q2, self.e2)
+
+    def set_opt(self, opt):
+        """the scoring fields of an api.MapOpt, as the CLI or mappy would set them"""
+        opt.a, opt.b, opt.q, opt.e, opt.q2, opt.e2, opt.sc_ambi = self.a, self.b, self.q, self.e, self.q2, self.e2, self.sc_ambi
+        return opt
+
+    def __repr__(self):
+        return self.name
+
+
+# Every scoring the DP kernels are held to the oracle under.  sr and ont are the presets' own; the asm presets (host/opts.c) come
+# close to the int8 limit of the reference's lanes, (q+e)+(q2+e2) <= 127, and edge127 sits on it; eq is the single-affine case
+# (q == q2, e == e2); N0 gives N a zero score, which ksw2 replaces by -e2; bigA has large scores and a large N penalty; under
+# bail the worst score exceeds 2(q+e), where ksw2 returns before any DP.  asm20 gives b negative, bigA sc_ambi negative.
+KSW_SCORINGS = {s.name: s for s in [
+    KswScoring("sr", 2, 8, 1, 12, 2, 24, 1, 100, 10, 151),
+    KswScoring("ont", 2, 4, 1, 4, 2, 24, 1, 400, -1, 751),          # map-ont
+    KswScoring("asm5", 1, 19, 1, 39, 3, 81, 1, 200, -1, 500),
+    KswScoring("asm10", 1, 9, 1, 16, 2, 41, 1, 200, 5, 500),
+    KswScoring("asm20", 1, -4, 1, 6, 2, 26, 1, 200, 10, 500),
+    KswScoring("edge127", 1, 20, 1, 40, 3, 83, 1, 400, 10, 500),
+    KswScoring("eq", 1, 4, 1, 6, 1, 6, 1, 200, 5, 200),
+    KswScoring("N0", 2, 4, 0, 4, 2, 24, 1, 400, -1, 751),
+    KswScoring("bigA", 10, 20, -5, 20, 4, 60, 2, 300, 20, 300),
+    KswScoring("bail", 2, 20, 1, 4, 2, 24, 1, 100, 10, 151),
+]}
+
+
 def orc_ksw(q, t, mat, gq, ge, gq2, ge2, w, zdrop, end_bonus, flag):
     ez = Extz()
     q = np.ascontiguousarray(q, dtype=np.uint8)

@@ -155,6 +155,11 @@ def test_seed_and_chain(emu, mode):
         L.oracle().orc_idx_destroy(oi)
 
 
+def _n_cases(preset, n):
+    """the K4 tests below run every scoring of L.KSW_SCORINGS; the three they began with keep their full case count"""
+    return n if preset in ("sr", "ont", "eq") else n // 3
+
+
 def emu_ksw(E, q, t, mat, pen, w, zd, eb, fl):
     ez = Ez()
     cig = np.zeros(len(q) + len(t) + 4, dtype=np.uint32)
@@ -164,16 +169,14 @@ def emu_ksw(E, q, t, mat, pen, w, zd, eb, fl):
                 mte_q=ez.mte_q, score=ez.score, reach_end=ez.reach_end, cigar=cig[:ez.n_cigar].tolist())
 
 
-@pytest.mark.parametrize("preset", ["sr", "ont"])
+@pytest.mark.parametrize("preset", list(L.KSW_SCORINGS))
 def test_ksw_pieces(emu, preset):
     from test_oracle_vs_ref import _ksw_cases
     rng = np.random.default_rng(5150)
-    if preset == "sr":
-        mat, pen, bw, zd, eb = L.simple_mat(2, 8, 1), (12, 2, 24, 1), 151, 100, 10
-    else:
-        mat, pen, bw, zd, eb = L.simple_mat(2, 4, 1), (4, 2, 24, 1), 751, 400, -1
+    sc = L.KSW_SCORINGS[preset]
+    mat, pen, bw, zd, eb = sc.mat, sc.pen, sc.band, sc.zdrop, sc.end_bonus
     n = 0
-    for q, t in _ksw_cases(rng, 180):
+    for q, t in _ksw_cases(rng, _n_cases(preset, 180)):
         for fl in [0xC2, 0x40, 0x08, 0x00, 0x01, 0x02]:
             for w in ([bw, 20, -1] if n % 5 == 0 else [bw]):
                 a = L.orc_ksw(q, t, mat, *pen, w, zd, eb if fl & 0x40 else -1, fl)
@@ -207,20 +210,16 @@ def emu_ksw_fast2(E, q, t, mat, pen, w, zd, eb, fl, stride):
                 mte_q=ez.mte_q, score=ez.score, reach_end=ez.reach_end, cigar=cig[:ez.n_cigar].tolist())
 
 
-@pytest.mark.parametrize("preset", ["sr", "ont", "eq"])
+@pytest.mark.parametrize("preset", list(L.KSW_SCORINGS))
 def test_ksw_fast_form_in_pairs(emu, preset):
     """The thread-per-job form on 16x2 pairs (mmg_kswfast2.h: two cells per instruction, pairs aligned on the target coordinate, the
     out-of-matrix half of the first / last pair computed and ignored) equals ksw_extd2 bit for bit: all flags, w = -1, odd and
     even lengths, 1 x n and n x 1 jobs, N bases."""
     from test_oracle_vs_ref import _ksw_cases
     rng = np.random.default_rng(4242)
-    if preset == "sr":
-        mat, pen, bw, zd, eb = L.simple_mat(2, 8, 1), (12, 2, 24, 1), 151, 100, 10
-    elif preset == "ont":
-        mat, pen, bw, zd, eb = L.simple_mat(2, 4, 1), (4, 2, 24, 1), 751, 400, -1
-    else:
-        mat, pen, bw, zd, eb = L.simple_mat(1, 4, 1), (6, 1, 6, 1), 200, 200, 5
-    cases = list(_ksw_cases(rng, 240))
+    sc = L.KSW_SCORINGS[preset]
+    mat, pen, bw, zd, eb = sc.mat, sc.pen, sc.band, sc.zdrop, sc.end_bonus
+    cases = list(_ksw_cases(rng, _n_cases(preset, 240)))
     for ql, tl in [(1, 1), (1, 2), (2, 1), (1, 7), (7, 1), (2, 2), (3, 2), (2, 3), (5, 4), (4, 5), (16, 17), (17, 16), (33, 31)]:
         cases.append((rng.integers(0, 5, ql, dtype=np.uint8), rng.integers(0, 5, tl, dtype=np.uint8)))
     n_fast = 0
@@ -235,20 +234,18 @@ def test_ksw_fast_form_in_pairs(emu, preset):
                     a["cigar"] = []
                 assert a == b, (len(q), len(t), fl, w)
                 n_fast += 1
-    assert n_fast > 1500
+    assert n_fast > 1500 * _n_cases(preset, 240) // 240
 
 
-@pytest.mark.parametrize("preset", ["sr", "ont"])
+@pytest.mark.parametrize("preset", list(L.KSW_SCORINGS))
 def test_ksw_fast_form(emu, preset):
     """The thread-per-job form used when the band never clips equals ksw_extd2 bit for bit (all flags, incl. w=-1)."""
     from test_oracle_vs_ref import _ksw_cases
     rng = np.random.default_rng(777)
-    if preset == "sr":
-        mat, pen, bw, zd, eb = L.simple_mat(2, 8, 1), (12, 2, 24, 1), 151, 100, 10
-    else:
-        mat, pen, bw, zd, eb = L.simple_mat(2, 4, 1), (4, 2, 24, 1), 751, 400, -1
+    sc = L.KSW_SCORINGS[preset]
+    mat, pen, bw, zd, eb = sc.mat, sc.pen, sc.band, sc.zdrop, sc.end_bonus
     n_fast = n_skip = 0
-    for q, t in _ksw_cases(rng, 240):
+    for q, t in _ksw_cases(rng, _n_cases(preset, 240)):
         for fl in [0xC2, 0x40, 0x08, 0x18, 0x00, 0x01, 0x02, 0x80]:
             for w in [bw, -1]:
                 b = emu_ksw_fast(emu, q, t, mat, pen, w, zd, eb if fl & 0x40 else -1, fl, 1 + (n_fast % 3))
@@ -260,7 +257,7 @@ def test_ksw_fast_form(emu, preset):
                     a["cigar"] = []
                 assert a == b, (len(q), len(t), fl, w)
                 n_fast += 1
-    assert n_fast > 1500 and (preset != "sr" or n_skip > 0)
+    assert n_fast > 1500 * _n_cases(preset, 240) // 240 and (preset != "sr" or n_skip > 0)
 
 
 def _heap_case(rng, n_lists, max_cnt, dup_frac):
@@ -316,18 +313,16 @@ def emu_ksw_dpx(E, q, t, mat, pen, w, zd, eb, fl):
                 mte_q=ez.mte_q, score=ez.score, reach_end=ez.reach_end, cigar=cig[:ez.n_cigar].tolist())
 
 
-@pytest.mark.parametrize("preset", ["sr", "ont"])
+@pytest.mark.parametrize("preset", list(L.KSW_SCORINGS))
 def test_ksw_literal_form_on_16x2_simd(emu, preset):
     """The literal form in the pair layout (two cells per lane, 16x2 arithmetic, direction from one max over value*8+preference)
     equals ksw_extd2 bit for bit: all flags, bands that clip (stale lanes are read), w=-1, N bases."""
     from test_oracle_vs_ref import _ksw_cases
     rng = np.random.default_rng(4242)
-    if preset == "sr":
-        mat, pen, bw, zd, eb = L.simple_mat(2, 8, 1), (12, 2, 24, 1), 151, 100, 10
-    else:
-        mat, pen, bw, zd, eb = L.simple_mat(2, 4, 1), (4, 2, 24, 1), 751, 400, -1
+    sc = L.KSW_SCORINGS[preset]
+    mat, pen, bw, zd, eb = sc.mat, sc.pen, sc.band, sc.zdrop, sc.end_bonus
     n = 0
-    for q, t in _ksw_cases(rng, 200):
+    for q, t in _ksw_cases(rng, _n_cases(preset, 200)):
         for fl in [0xC2, 0x40, 0x08, 0x18, 0x00, 0x01, 0x02, 0x80]:
             for w in ([bw, 20, 7, -1] if n % 3 == 0 else [bw, 20]):
                 a = L.orc_ksw(q, t, mat, *pen, w, zd, eb if fl & 0x40 else -1, fl)
@@ -336,6 +331,45 @@ def test_ksw_literal_form_on_16x2_simd(emu, preset):
                     a["cigar"] = []
                 assert a == b, (len(q), len(t), fl, w)
         n += 1
+
+
+@pytest.mark.parametrize("preset", list(L.KSW_SCORINGS))
+def test_ksw_forms_equal_exact_dp(emu, preset):
+    """The oracle and every emulated form against the plain int64 DP of tests/_kswref.py on jobs whose band never clips, z-drop
+    off: score, max, mqe, mte, H at the max cell, the cells the CIGAR spans and its score.  Under bail every form returns the
+    reset result without a CIGAR."""
+    from test_oracle_vs_ref import _ksw_cases
+    from _kswref import KswRef, check_job
+    sc = L.KSW_SCORINGS[preset]
+    mat, pen = sc.mat, sc.pen
+    rng = np.random.default_rng(6006)
+    cases = list(_ksw_cases(rng, 48))
+    for ql, tl in [(1, 1), (1, 9), (9, 1), (1, 300), (300, 1), (17, 16), (64, 700)]:
+        cases.append((rng.integers(0, 5, ql, dtype=np.uint8), rng.integers(0, 5, tl, dtype=np.uint8)))
+    reset = dict(max=0, zdropped=0, max_q=-1, max_t=-1, mqe=-0x40000000, mqe_t=-1, mte=-0x40000000, mte_q=-1, score=-0x40000000,
+                 reach_end=0, cigar=[])
+    n_fast = 0
+    for q, t in cases:
+        ref = KswRef(q, t, mat, *pen) if preset != "bail" else None
+        for fl in [0x00, 0x40, 0x08, 0x02, 0xC2, 0x4A, 0x80, 0x01]:
+            eb = sc.end_bonus if fl & 0x40 else -1
+            a = L.orc_ksw(q, t, mat, *pen, -1, -1, eb, fl)
+            forms = {"scalar": emu_ksw(emu, q, t, mat, pen, -1, -1, eb, fl), "literal 16x2": emu_ksw_dpx(emu, q, t, mat, pen, -1, -1, eb, fl),
+                     "fast": emu_ksw_fast(emu, q, t, mat, pen, -1, -1, eb, fl, 2), "fast pairs": emu_ksw_fast2(emu, q, t, mat, pen, -1, -1, eb, fl, 3)}
+            if fl & 0x01:
+                a["cigar"] = []
+            if preset == "bail":
+                assert a == reset, a
+            else:
+                check_job(a, q, t, mat, pen, fl, eb, ref)
+            for name, b in forms.items():
+                if b is None:  # outside the fast forms' limits
+                    continue
+                n_fast += name.startswith("fast")
+                if preset != "bail":
+                    check_job(b, q, t, mat, pen, fl, eb, ref)
+                assert a == b, (name, len(q), len(t), fl)
+    assert n_fast == 2 * 8 * len(cases)  # no clipping band and small jobs: the fast forms take every one
 
 
 @pytest.mark.parametrize("w,k", [(11, 21), (10, 15), (5, 19), (19, 19), (3, 5), (1, 15), (4, 7), (32, 27)])

@@ -103,23 +103,25 @@ def test_seeds_and_chain_single(ctx, api, refseqs, mode):
         L.oracle().orc_idx_destroy(oi)
 
 
-@pytest.mark.parametrize("preset", ["sr", "ont"])
+@pytest.mark.parametrize("preset", list(L.KSW_SCORINGS))
 def test_ksw_single(ctx, preset):
+    """every scoring of L.KSW_SCORINGS; sr and ont with the full case count.  The last cases give the gap pieces in the other
+    order (q2, e2, q, e): the CLI refuses that, the kernels swap them as ksw2 does (after taking q+e of the order given)."""
     from test_oracle_vs_ref import _ksw_cases
     rng = np.random.default_rng(808)
-    if preset == "sr":
-        mat, pen, bw, zd, eb = L.simple_mat(2, 8, 1), (12, 2, 24, 1), 151, 100, 10
-    else:
-        mat, pen, bw, zd, eb = L.simple_mat(2, 4, 1), (4, 2, 24, 1), 751, 400, -1
+    sc = L.KSW_SCORINGS[preset]
+    mat, pen, bw, zd, eb = sc.mat, sc.pen, sc.band, sc.zdrop, sc.end_bonus
+    n_cases = 90 if preset in ("sr", "ont") else 30
     n = 0
-    for q, t in _ksw_cases(rng, 90):
+    for q, t in _ksw_cases(rng, n_cases + 6):
+        p = pen if n < n_cases else (pen[2], pen[3], pen[0], pen[1])
         for fl in [0xC2, 0x40, 0x08, 0x00, 0x01, 0x02]:
             for w in ([bw, 20, -1] if n % 5 == 0 else [bw]):
-                a = L.orc_ksw(q, t, mat, *pen, w, zd, eb if fl & 0x40 else -1, fl)
-                b = ctx.ksw_extd2(q, t, mat, *pen, w, zd, eb if fl & 0x40 else -1, fl)
+                a = L.orc_ksw(q, t, mat, *p, w, zd, eb if fl & 0x40 else -1, fl)
+                b = ctx.ksw_extd2(q, t, mat, *p, w, zd, eb if fl & 0x40 else -1, fl)
                 if fl & 0x01:
                     a["cigar"] = []
-                assert a == b, (len(q), len(t), fl, w)
+                assert a == b, (len(q), len(t), fl, w, p)
         n += 1
 
 
@@ -202,6 +204,17 @@ def test_seed_chain_batch(ctx, api, refseqs, mode):
 
 def test_ksw_batch(ctx, api, refseqs):
     """DP jobs described against the resident reads and the index (align.c:690-771 call shapes)."""
+    _ksw_batch(ctx, api, refseqs, L.KSW_SCORINGS["sr"], 400)
+
+
+@pytest.mark.parametrize("preset", [p for p in L.KSW_SCORINGS if p != "sr"])
+def test_ksw_batch_scoring(ctx, api, refseqs, preset):
+    """test_ksw_batch under the other scorings of L.KSW_SCORINGS: the scoring reaches the kernels through the mapping options
+    (make_score), as from the CLI or mappy."""
+    _ksw_batch(ctx, api, refseqs, L.KSW_SCORINGS[preset], 150)
+
+
+def _ksw_batch(ctx, api, refseqs, sc, n_jobs):
     from test_oracle_vs_ref import _frags
     w, k = 11, 21
     idx = api.Index(ctx, refseqs, w, k)
@@ -209,15 +222,15 @@ def test_ksw_batch(ctx, api, refseqs):
     try:
         frags_mapped = _frags(rng, refseqs, 60, True)
         frags = [[f[0], L.revcomp(f[1])] for f in frags_mapped]
-        opt = api.sr_opt()
+        opt = sc.set_opt(api.sr_opt())
         batch, keep = api.Context.make_batch(frags)
         ctx.batch_upload(opt, batch)
         reads = [s for f in frags_mapped for s in f]  # mapping orientation, as resident on the device
         codes = [L.nt4(r) for r in reads]
         refcodes = [L.nt4(s) for s in refseqs]
-        jobs = np.zeros(400, dtype=api.ksw_job_dtype)
+        jobs = np.zeros(n_jobs, dtype=api.ksw_job_dtype)
         want = []
-        mat = L.simple_mat(2, 8, 1)
+        mat = sc.mat
         for j in range(len(jobs)):
             sid = int(rng.integers(0, len(reads)))
             ql_read = len(reads[sid])
@@ -227,13 +240,14 @@ def test_ksw_batch(ctx, api, refseqs):
             ts = int(rng.integers(0, len(refseqs[rid]) - 400)); tl = int(rng.integers(1, 300))
             rev = int(rng.integers(0, 2))
             fl = [0xC2, 0x40, 0x08, 0x00][j % 4]
-            wj = [151, 40][j % 2]
-            jobs[j] = (sid, q_rev, qs, ql, rid, ts, tl, rev, wj, 100, 10 if fl & 0x40 else -1, fl)
+            wj = [sc.band, 40][j % 2]
+            eb = sc.end_bonus if fl & 0x40 else -1
+            jobs[j] = (sid, q_rev, qs, ql, rid, ts, tl, rev, wj, sc.zdrop, eb, fl)
             strand = codes[sid] if not q_rev else np.where(codes[sid][::-1] < 4, 3 - codes[sid][::-1], 4).astype(np.uint8)
             q = strand[qs:qs + ql]; t = refcodes[rid][ts:ts + tl]
             if rev:
                 q, t = q[::-1], t[::-1]
-            want.append(L.orc_ksw(q, t, mat, 12, 2, 24, 1, wj, 100, 10 if fl & 0x40 else -1, fl))
+            want.append(L.orc_ksw(q, t, mat, *sc.pen, wj, sc.zdrop, eb, fl))
         got, ms, cells = ctx.ksw_batch(idx, opt, jobs)
         for j in range(len(jobs)):
             assert got[j] == want[j], (j, jobs[j])
