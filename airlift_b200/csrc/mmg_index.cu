@@ -286,14 +286,49 @@ extern "C" int mmg_idx_set_name_keys(mmg_idx_t *mi, const uint32_t *tkey)
 	return MMG_OK;
 }
 
-static int idx_alloc(mmg_idx_t *mi)
+static int idx_alloc(mmg_idx_t *mi, bool with_S)
 {
-	MMG_CUDA(cudaMalloc(&mi->d_S, ((mi->total_len + 7) / 8 + 4) * 4));
+	if (with_S) MMG_CUDA(cudaMalloc(&mi->d_S, ((mi->total_len + 7) / 8 + 4) * 4));
 	MMG_CUDA(cudaMalloc(&mi->d_seq_off, (size_t)(mi->n_seq + 1) * 8));
 	MMG_CUDA(cudaMalloc(&mi->d_seq_len, (size_t)(mi->n_seq + 1) * 4));
 	MMG_CUDA(cudaMalloc(&mi->d_slots, mi->n_slots * sizeof(IdxSlot)));
 	MMG_CUDA(cudaMalloc(&mi->d_pos, (mi->n_pos + 1) * 8));
 	return MMG_OK;
+}
+
+// one slot per distinct minimizer (power-of-two slots at load <= 0.5), filled from the key-sorted (ukey, counts, ustart) and pos[]
+static int idx_table(mmg_ctx_t *c, mmg_idx_t *mi, const uint64_t *d_ukey, const int64_t *d_ustart)
+{
+	uint64_t n_slots = 1024; int bits = 10;
+	while (n_slots < (uint64_t)mi->n_keys * 2) n_slots <<= 1, ++bits;
+	mi->n_slots = n_slots, mi->slot_shift = 64 - bits;
+	MMG_CUDA(cudaMalloc(&mi->d_slots, n_slots * sizeof(IdxSlot)));
+	MMG_LAUNCH(c, k_fill_u64, mmg_blocks(n_slots * 2, 256), 256, 0, reinterpret_cast<uint64_t*>(mi->d_slots), n_slots * 2, MMG_SLOT_EMPTY);
+	if (mi->n_keys)
+		MMG_LAUNCH(c, k_idx_insert, mmg_blocks(mi->n_keys, 256), 256, 0, d_ukey, mi->d_counts, d_ustart, mi->n_keys, mi->d_pos, mi->d_slots, n_slots - 1, mi->slot_shift);
+	return MMG_OK;
+}
+
+static int idx_seq_table(mmg_ctx_t *c, mmg_idx_t *mi)
+{
+	MMG_CUDA(cudaMalloc(&mi->d_seq_off, (size_t)(mi->n_seq + 1) * 8));
+	MMG_CUDA(cudaMalloc(&mi->d_seq_len, (size_t)(mi->n_seq + 1) * 4));
+	MMG_CUDA(cudaMemcpyAsync(mi->d_seq_off, mi->h_seq_off.data(), (size_t)(mi->n_seq + 1) * 8, cudaMemcpyHostToDevice, c->stream));
+	MMG_CUDA(cudaMemcpyAsync(mi->d_seq_len, mi->h_seq_len.data(), (size_t)(mi->n_seq + 1) * 4, cudaMemcpyHostToDevice, c->stream));
+	MMG_CUDA(cudaStreamSynchronize(c->stream));
+	return MMG_OK;
+}
+
+static mmg_idx_t *idx_new(mmg_ctx_t *c, int w, int k, int is_hpc, int n_seq, const uint32_t *lens)
+{
+	mmg_idx_t *mi = new mmg_idx_s();
+	mi->dev = c->dev, mi->w = w, mi->k = k, mi->is_hpc = is_hpc, mi->n_seq = n_seq;
+	mi->h_seq_off.resize(n_seq + 1); mi->h_seq_len.resize(n_seq + 1);
+	uint64_t tot = 0;
+	for (int i = 0; i < n_seq; ++i) { mi->h_seq_off[i] = tot; mi->h_seq_len[i] = lens[i]; tot += lens[i]; }
+	mi->h_seq_off[n_seq] = tot; mi->h_seq_len[n_seq] = 0;
+	mi->total_len = tot;
+	return mi;
 }
 
 extern "C" int mmg_idx_build(mmg_ctx_t *c, int w, int k, int is_hpc, int n_seq, const char *const *seqs, const uint32_t *lens, mmg_idx_t **out)
@@ -304,13 +339,8 @@ extern "C" int mmg_idx_build(mmg_ctx_t *c, int w, int k, int is_hpc, int n_seq, 
 		return (w > MMG_MAX_W) ? MMG_ELIMIT : MMG_EINVAL;
 	}
 	MMG_CUDA(cudaSetDevice(c->dev));
-	mmg_idx_t *mi = new mmg_idx_s();
-	mi->dev = c->dev, mi->w = w, mi->k = k, mi->is_hpc = is_hpc, mi->n_seq = n_seq;
-	mi->h_seq_off.resize(n_seq + 1); mi->h_seq_len.resize(n_seq + 1);
-	uint64_t tot = 0;
-	for (int i = 0; i < n_seq; ++i) { mi->h_seq_off[i] = tot; mi->h_seq_len[i] = lens[i]; tot += lens[i]; }
-	mi->h_seq_off[n_seq] = tot; mi->h_seq_len[n_seq] = 0;
-	mi->total_len = tot;
+	mmg_idx_t *mi = idx_new(c, w, k, is_hpc, n_seq, lens);
+	const uint64_t tot = mi->total_len;
 	int rc = MMG_OK;
 	uint8_t *d_ascii = nullptr;
 	SketchUnit *d_units = nullptr;
@@ -423,26 +453,12 @@ extern "C" int mmg_idx_build(mmg_ctx_t *c, int w, int k, int is_hpc, int n_seq, 
 		IDX_CUDA(cub::DeviceScan::ExclusiveSum(c->d_cub.p, tmp, mi->d_counts, d_ustart, n_keys, c->stream));
 		++c->launches;
 	}
-	// 6. table: power-of-two slots at load <= 0.5
-	uint64_t n_slots = 1024; int bits = 10;
-	while (n_slots < (uint64_t)n_keys * 2) n_slots <<= 1, ++bits;
-	mi->n_slots = n_slots, mi->slot_shift = 64 - bits;
-	IDX_CUDA(cudaMalloc(&mi->d_slots, n_slots * sizeof(IdxSlot)));
-	k_fill_u64<<<mmg_blocks(n_slots * 2, 256), 256, 0, c->stream>>>(reinterpret_cast<uint64_t*>(mi->d_slots), n_slots * 2, MMG_SLOT_EMPTY); ++c->launches;
-	IDX_CUDA(cudaGetLastError());
 	// positions: keep the sorted value array as pos[]
 	mi->d_pos = vb.Current();
 	if (vb.Current() == d_val[0]) d_val[0] = nullptr; else d_val[1] = nullptr;
-	if (n_keys) {
-		k_idx_insert<<<mmg_blocks(n_keys, 256), 256, 0, c->stream>>>(d_ukey, mi->d_counts, d_ustart, n_keys, mi->d_pos, mi->d_slots, n_slots - 1, mi->slot_shift); ++c->launches;
-		IDX_CUDA(cudaGetLastError());
-	}
-	// 7. sequence table
-	IDX_CUDA(cudaMalloc(&mi->d_seq_off, (size_t)(n_seq + 1) * 8));
-	IDX_CUDA(cudaMalloc(&mi->d_seq_len, (size_t)(n_seq + 1) * 4));
-	IDX_CUDA(cudaMemcpyAsync(mi->d_seq_off, mi->h_seq_off.data(), (size_t)(n_seq + 1) * 8, cudaMemcpyHostToDevice, c->stream));
-	IDX_CUDA(cudaMemcpyAsync(mi->d_seq_len, mi->h_seq_len.data(), (size_t)(n_seq + 1) * 4, cudaMemcpyHostToDevice, c->stream));
-	IDX_CUDA(cudaStreamSynchronize(c->stream));
+	// 6. table, 7. sequence table
+	IDX_TRY(idx_table(c, mi, d_ukey, d_ustart));
+	IDX_TRY(idx_seq_table(c, mi));
 	cleanup();
 	c->d_cub.release();
 	*out = mi;
@@ -451,16 +467,190 @@ extern "C" int mmg_idx_build(mmg_ctx_t *c, int w, int k, int is_hpc, int n_seq, 
 #undef IDX_TRY
 }
 
+// ------------------------------------------------------------------ build from an index file's minimizer lists
+
+#define LISTS_SINGLE (1ULL << 63)
+#define LISTS_SHORT 32 // runs up to this long are copied by one thread, longer ones by a warp
+
+__global__ void k_lists_keys(const uint64_t *__restrict__ key, int64_t n, uint64_t *__restrict__ skey, uint32_t *__restrict__ sidx)
+{
+	const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+	if (i >= n) return;
+	skey[i] = key[i] & ~LISTS_SINGLE, sidx[i] = (uint32_t)i;
+}
+
+// file order -> minimizer order; bad[0] is set when a minimizer is listed twice
+__global__ void k_lists_gather(const uint64_t *__restrict__ skey, const uint32_t *__restrict__ sidx, int64_t n, const uint64_t *__restrict__ key,
+                               const uint32_t *__restrict__ cnt, const uint64_t *__restrict__ src, uint32_t *__restrict__ ucnt,
+                               uint64_t *__restrict__ usrc, unsigned int *bad)
+{
+	const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+	if (j >= n) return;
+	const uint32_t i = sidx[j];
+	const bool single = (key[i] & LISTS_SINGLE) != 0;
+	ucnt[j] = single ? 1u : cnt[i];
+	usrc[j] = src[i] | (single ? LISTS_SINGLE : 0);
+	if (j > 0 && skey[j] == skey[j - 1]) atomicOr(bad, 1u);
+}
+
+// a thread per short run; the long ones are queued for k_lists_scatter_long.  A singleton's one position is its own value.
+__global__ void k_lists_scatter(const uint32_t *__restrict__ ucnt, const uint64_t *__restrict__ usrc, const int64_t *__restrict__ ustart, int64_t n,
+                                const uint64_t *__restrict__ p, uint64_t *__restrict__ pos, int64_t *__restrict__ long_runs, unsigned long long *n_long)
+{
+	const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+	if (j >= n) return;
+	const uint32_t m = ucnt[j];
+	const uint64_t s = usrc[j];
+	uint64_t *dst = pos + ustart[j];
+	if (s & LISTS_SINGLE) { dst[0] = s & ~LISTS_SINGLE; return; }
+	if (m > LISTS_SHORT) { long_runs[atomicAdd(n_long, 1ULL)] = j; return; }
+	for (uint32_t t = 0; t < m; ++t) dst[t] = p[s + t];
+}
+
+__global__ void k_lists_scatter_long(const uint32_t *__restrict__ ucnt, const uint64_t *__restrict__ usrc, const int64_t *__restrict__ ustart,
+                                     const int64_t *__restrict__ long_runs, const unsigned long long *n_long, const uint64_t *__restrict__ p,
+                                     uint64_t *__restrict__ pos)
+{
+	const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+	const int lane = threadIdx.x & 31;
+	for (int64_t r = warp; r < (int64_t)*n_long; r += n_warps) {
+		const int64_t j = long_runs[r];
+		const uint32_t m = ucnt[j];
+		const uint64_t *s = p + usrc[j];
+		uint64_t *dst = pos + ustart[j];
+		for (uint32_t t = lane; t < m; t += 32) dst[t] = s[t];
+	}
+}
+
+// host -> device through the pinned bases buffer of staging slot 0, in chunks: a human-size p[] is several GB
+static int upload_chunked(mmg_ctx_t *c, void *dst, const void *src, size_t bytes)
+{
+	const size_t stage = 64u << 20;
+	if (bytes == 0) return MMG_OK;
+	MMG_TRY(mmg_stage_grow(c, 0, &StageSlot::bases, stage));
+	uint8_t *h = c->stage[0].bases.as<uint8_t>();
+	for (size_t o = 0; o < bytes; o += stage) {
+		const size_t l = bytes - o < stage ? bytes - o : stage;
+		memcpy(h, static_cast<const uint8_t*>(src) + o, l);
+		MMG_CUDA(cudaMemcpyAsync(static_cast<uint8_t*>(dst) + o, h, l, cudaMemcpyHostToDevice, c->stream));
+		MMG_CUDA(cudaStreamSynchronize(c->stream));
+	}
+	return MMG_OK;
+}
+
+extern "C" int mmg_idx_build_lists(mmg_ctx_t *c, int w, int k, int is_hpc, int n_seq, const uint32_t *lens, int64_t n_keys, const uint64_t *key,
+                                   const uint32_t *cnt, const uint64_t *src, uint64_t n_p, const uint64_t *p, mmg_idx_t **out)
+{
+	*out = nullptr;
+	if (w < 1 || w > MMG_MAX_W || k < 1 || k > 28 || n_seq <= 0 || n_keys < 0 || n_keys >= (1LL << 32)) {
+		mmg_set_error("mmg_idx_build_lists: need 1<=w<=%d, 1<=k<=28, n_seq>0, 0<=n_keys<2^32", MMG_MAX_W);
+		return (w > MMG_MAX_W) ? MMG_ELIMIT : MMG_EINVAL;
+	}
+	for (int64_t i = 0; i < n_keys; ++i) { // nothing out of range reaches the device
+		if ((key[i] & ~LISTS_SINGLE) >> (2 * k)) { mmg_set_error("mmg_idx_build_lists: minimizer %lld has more than %d bits", (long long)i, 2 * k); return MMG_EINVAL; }
+		if (!(key[i] & LISTS_SINGLE) && (cnt[i] == 0 || src[i] > n_p || cnt[i] > n_p - src[i])) {
+			mmg_set_error("mmg_idx_build_lists: the positions of minimizer %lld lie outside p[] (%llu entries)", (long long)i, (unsigned long long)n_p);
+			return MMG_EINVAL;
+		}
+	}
+	MMG_CUDA(cudaSetDevice(c->dev));
+	mmg_idx_t *mi = idx_new(c, w, k, is_hpc, n_seq, lens);
+	mi->n_keys = n_keys;
+	int rc = MMG_OK;
+	const size_t nk = (size_t)n_keys + 1;
+	uint64_t *d_key = nullptr, *d_src = nullptr, *d_p = nullptr, *d_sk[2] = {nullptr, nullptr}, *d_usrc = nullptr;
+	uint32_t *d_cnt = nullptr, *d_si[2] = {nullptr, nullptr};
+	int64_t *d_ustart = nullptr, *d_long = nullptr;
+	unsigned long long *d_ctr = nullptr; // [0] long runs, [1] a minimizer listed twice
+	auto cleanup = [&]() {
+		cudaFree(d_key); cudaFree(d_src); cudaFree(d_p); cudaFree(d_sk[0]); cudaFree(d_sk[1]); cudaFree(d_usrc);
+		cudaFree(d_cnt); cudaFree(d_si[0]); cudaFree(d_si[1]); cudaFree(d_ustart); cudaFree(d_long); cudaFree(d_ctr);
+	};
+#define IDX_CUDA(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { mmg_set_error("%s:%d: %s: %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); cleanup(); mmg_idx_free(mi); return MMG_ECUDA; } } while (0)
+#define IDX_TRY(call) do { rc = (call); if (rc != MMG_OK) { cleanup(); mmg_idx_free(mi); return rc; } } while (0)
+#define LAUNCH_IDX(kern, grid, block, ...) do { kern<<<(grid), (block), 0, c->stream>>>(__VA_ARGS__); ++c->launches; IDX_CUDA(cudaGetLastError()); } while (0)
+
+	// 1. upload the lists as the file gives them
+	IDX_CUDA(cudaMalloc(&d_key, nk * 8));
+	IDX_CUDA(cudaMalloc(&d_cnt, nk * 4));
+	IDX_CUDA(cudaMalloc(&d_src, nk * 8));
+	IDX_CUDA(cudaMalloc(&d_p, ((size_t)n_p + 1) * 8));
+	IDX_TRY(upload_chunked(c, d_key, key, (size_t)n_keys * 8));
+	IDX_TRY(upload_chunked(c, d_cnt, cnt, (size_t)n_keys * 4));
+	IDX_TRY(upload_chunked(c, d_src, src, (size_t)n_keys * 8));
+	IDX_TRY(upload_chunked(c, d_p, p, (size_t)n_p * 8));
+
+	// 2. order by minimizer
+	for (int i = 0; i < 2; ++i) { IDX_CUDA(cudaMalloc(&d_sk[i], nk * 8)); IDX_CUDA(cudaMalloc(&d_si[i], nk * 4)); }
+	cub::DoubleBuffer<uint64_t> kb(d_sk[0], d_sk[1]);
+	cub::DoubleBuffer<uint32_t> ib(d_si[0], d_si[1]);
+	if (n_keys) {
+		LAUNCH_IDX(k_lists_keys, mmg_blocks(n_keys, 256), 256, d_key, n_keys, d_sk[0], d_si[0]);
+		size_t tmp = 0;
+		cub::DeviceRadixSort::SortPairs(nullptr, tmp, kb, ib, n_keys, 0, 2 * k, c->stream);
+		IDX_TRY(c->d_cub.ensure(tmp));
+		IDX_CUDA(cub::DeviceRadixSort::SortPairs(c->d_cub.p, tmp, kb, ib, n_keys, 0, 2 * k, c->stream));
+		++c->launches;
+	}
+	// 3. counts in minimizer order and each run's start in pos[]
+	IDX_CUDA(cudaMalloc(&mi->d_counts, nk * 4));
+	IDX_CUDA(cudaMalloc(&d_usrc, nk * 8));
+	IDX_CUDA(cudaMalloc(&d_ustart, (nk + 1) * 8));
+	IDX_CUDA(cudaMalloc(&d_ctr, 16));
+	IDX_CUDA(cudaMemsetAsync(d_ctr, 0, 16, c->stream));
+	IDX_CUDA(cudaMemsetAsync(mi->d_counts, 0, nk * 4, c->stream)); // counts[n_keys] = 0: the scan leaves the total in ustart[n_keys]
+	if (n_keys)
+		LAUNCH_IDX(k_lists_gather, mmg_blocks(n_keys, 256), 256, kb.Current(), ib.Current(), n_keys, d_key, d_cnt, d_src, mi->d_counts, d_usrc,
+		               reinterpret_cast<unsigned int*>(d_ctr + 1));
+	{
+		size_t tmp = 0;
+		cub::DeviceScan::ExclusiveSum(nullptr, tmp, mi->d_counts, d_ustart, (int64_t)nk, c->stream);
+		IDX_TRY(c->d_cub.ensure(tmp));
+		IDX_CUDA(cub::DeviceScan::ExclusiveSum(c->d_cub.p, tmp, mi->d_counts, d_ustart, (int64_t)nk, c->stream));
+		++c->launches;
+	}
+	int64_t n_pos = 0;
+	unsigned long long dup = 0;
+	IDX_CUDA(cudaMemcpyAsync(&n_pos, d_ustart + n_keys, 8, cudaMemcpyDeviceToHost, c->stream));
+	IDX_CUDA(cudaMemcpyAsync(&dup, d_ctr + 1, 8, cudaMemcpyDeviceToHost, c->stream));
+	IDX_CUDA(cudaStreamSynchronize(c->stream));
+	if (dup) { mmg_set_error("mmg_idx_build_lists: a minimizer is listed more than once"); cleanup(); mmg_idx_free(mi); return MMG_EINVAL; }
+	mi->n_pos = (uint64_t)n_pos;
+	// only the sorted minimizers, the runs and p[] are read from here on
+	cudaFree(d_key); d_key = nullptr; cudaFree(d_cnt); d_cnt = nullptr; cudaFree(d_src); d_src = nullptr;
+	cudaFree(d_si[0]); cudaFree(d_si[1]); d_si[0] = d_si[1] = nullptr;
+	if (kb.Current() == d_sk[0]) { cudaFree(d_sk[1]); d_sk[1] = nullptr; } else { cudaFree(d_sk[0]); d_sk[0] = nullptr; }
+	// 4. scatter every run into pos[], its positions in the order the file lists them
+	IDX_CUDA(cudaMalloc(&mi->d_pos, (mi->n_pos + 1) * 8));
+	IDX_CUDA(cudaMalloc(&d_long, nk * 8));
+	if (n_keys) {
+		LAUNCH_IDX(k_lists_scatter, mmg_blocks(n_keys, 256), 256, mi->d_counts, d_usrc, d_ustart, n_keys, d_p, mi->d_pos, d_long, d_ctr);
+		LAUNCH_IDX(k_lists_scatter_long, 148 * 16, 256, mi->d_counts, d_usrc, d_ustart, d_long, d_ctr, d_p, mi->d_pos);
+	}
+	// 5. the table, as mmg_idx_build fills it from the same (minimizer, count, start); no sequence is kept
+	IDX_TRY(idx_table(c, mi, kb.Current(), d_ustart));
+	IDX_TRY(idx_seq_table(c, mi));
+	cleanup();
+	c->d_cub.release();
+	*out = mi;
+	return MMG_OK;
+#undef IDX_CUDA
+#undef IDX_TRY
+#undef LAUNCH_IDX
+}
+
 extern "C" int64_t mmg_idx_n_minimizers(const mmg_idx_t *mi) { return (int64_t)mi->n_pos; }
 extern "C" int64_t mmg_idx_n_keys(const mmg_idx_t *mi) { return mi->n_keys; }
 extern "C" uint64_t mmg_idx_total_len(const mmg_idx_t *mi) { return mi->total_len; }
 extern "C" size_t mmg_idx_bytes(const mmg_idx_t *mi)
 {
-	return ((mi->total_len + 7) / 8) * 4 + mi->n_slots * sizeof(IdxSlot) + mi->n_pos * 8 + (size_t)mi->n_seq * 12;
+	return (mi->d_S ? ((mi->total_len + 7) / 8) * 4 : 0) + mi->n_slots * sizeof(IdxSlot) + mi->n_pos * 8 + (size_t)mi->n_seq * 12;
 }
+extern "C" int mmg_idx_has_seq(const mmg_idx_t *mi) { return mi->d_S != nullptr; }
 
 extern "C" int mmg_idx_copy_S(const mmg_idx_t *mi, uint32_t *S_host)
 {
+	if (mi->d_S == nullptr) { mmg_set_error("mmg_idx_copy_S: the index holds no sequence (built from a .mmi written with --idx-no-seq)"); return MMG_EINVAL; }
 	MMG_CUDA(cudaSetDevice(mi->dev));
 	MMG_CUDA(cudaMemcpy(S_host, mi->d_S, ((mi->total_len + 7) / 8) * 4, cudaMemcpyDeviceToHost));
 	return MMG_OK;
@@ -508,7 +698,7 @@ extern "C" int mmg_idx_export(const mmg_idx_t *mi, mmg_idx_image_t *img)
 {
 	img->w = mi->w, img->k = mi->k, img->is_hpc = mi->is_hpc, img->n_seq = mi->n_seq;
 	img->total_len = mi->total_len, img->n_slots = mi->n_slots, img->n_pos = mi->n_pos, img->n_keys = mi->n_keys;
-	img->d_S = mi->d_S, img->bytes_S = ((mi->total_len + 7) / 8) * 4;
+	img->d_S = mi->d_S, img->bytes_S = mi->d_S ? ((mi->total_len + 7) / 8) * 4 : 0;
 	img->d_seq_off = mi->d_seq_off, img->bytes_seq_off = (size_t)(mi->n_seq + 1) * 8;
 	img->d_seq_len = mi->d_seq_len, img->bytes_seq_len = (size_t)(mi->n_seq + 1) * 4;
 	img->d_slots = mi->d_slots, img->bytes_slots = mi->n_slots * sizeof(IdxSlot);
@@ -525,7 +715,7 @@ extern "C" int mmg_idx_alloc_like(mmg_ctx_t *c, mmg_idx_image_t *img, mmg_idx_t 
 	mi->total_len = img->total_len, mi->n_slots = img->n_slots, mi->n_pos = img->n_pos, mi->n_keys = img->n_keys;
 	int bits = 0; while ((1ULL << bits) < mi->n_slots) ++bits;
 	mi->slot_shift = 64 - bits;
-	int rc = idx_alloc(mi);
+	int rc = idx_alloc(mi, img->bytes_S > 0 || img->total_len == 0); // an index without sequence has total_len > 0 and no S bytes
 	if (rc != MMG_OK) { mmg_idx_free(mi); return rc; }
 	img->d_S = mi->d_S, img->d_seq_off = mi->d_seq_off, img->d_seq_len = mi->d_seq_len, img->d_slots = mi->d_slots, img->d_pos = mi->d_pos;
 	*out = mi;
@@ -553,7 +743,7 @@ extern "C" int mmg_idx_clone_to(mmg_ctx_t *c, const mmg_idx_t *src, mmg_idx_t **
 		cudaDeviceCanAccessPeer(&can, c->dev, src->dev);
 		if (can) { cudaError_t e = cudaDeviceEnablePeerAccess(src->dev, 0); if (e != cudaSuccess) cudaGetLastError(); }
 	}
-	MMG_CUDA(cudaMemcpyPeerAsync(d.d_S, c->dev, s.d_S, src->dev, s.bytes_S, c->stream));
+	if (s.bytes_S) MMG_CUDA(cudaMemcpyPeerAsync(d.d_S, c->dev, s.d_S, src->dev, s.bytes_S, c->stream));
 	MMG_CUDA(cudaMemcpyPeerAsync(d.d_seq_off, c->dev, s.d_seq_off, src->dev, s.bytes_seq_off, c->stream));
 	MMG_CUDA(cudaMemcpyPeerAsync(d.d_seq_len, c->dev, s.d_seq_len, src->dev, s.bytes_seq_len, c->stream));
 	MMG_CUDA(cudaMemcpyPeerAsync(d.d_slots, c->dev, s.d_slots, src->dev, s.bytes_slots, c->stream));

@@ -909,6 +909,7 @@ int mmg_ksw_device(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt_t *opt, i
 	*d_res = nullptr, *d_cigars = nullptr;
 	if (kernel_ms) *kernel_ms = 0;
 	if (cells) *cells = 0;
+	if (mi->d_S == nullptr) { mmg_set_error("DP alignment needs the reference sequence, and the index holds none (--idx-no-seq)"); return MMG_EINVAL; }
 	if (n_jobs <= 0) return MMG_OK;
 	MMG_TRY(ksw_launch(c, d_jobs, n_jobs, c->d_Q.as<uint32_t>(), mi->d_S, c->d_q_off.as<uint64_t>(), c->d_seq_len.as<int32_t>(), mi->d_seq_off, make_score(opt),
 	                   nullptr, d_cigars, kernel_ms, cells, false));
@@ -956,6 +957,7 @@ extern "C" int mmg_ksw_batch(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapopt
 	*cigars = nullptr;
 	if (kernel_ms) *kernel_ms = 0;
 	if (cells) *cells = 0;
+	if (mi->d_S == nullptr) { mmg_set_error("mmg_ksw_batch: DP alignment needs the reference sequence, and the index holds none (--idx-no-seq)"); return MMG_EINVAL; }
 	if (n_jobs <= 0) return MMG_OK;
 	MMG_CUDA(cudaSetDevice(c->dev));
 	const ResidentBatch &rb = c->rb;

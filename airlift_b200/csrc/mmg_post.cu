@@ -193,6 +193,11 @@ extern "C" int mmg_post_chain(mmg_ctx_t *c, const mmg_idx_t *mi, const mmg_mapop
 	memset(out, 0, sizeof(*out));
 	if (opt_bytes != sizeof(FullOpt)) { mmg_set_error("mmg_post_chain: mm_mapopt_t size mismatch"); return MMG_EINVAL; }
 	(void)idx_flag;
+	// only the CIGAR stages (post_plan, post_build) read the reference; without MM_F_CIGAR an index without sequence maps as any other
+	if ((static_cast<const FullOpt*>(opt_full)->flag & HIT_F_CIGAR) && mi->d_S == nullptr) {
+		mmg_set_error("mmg_post_chain: CIGAR output needs the reference sequence, and the index holds none (--idx-no-seq)");
+		return MMG_EINVAL;
+	}
 	MMG_CUDA(cudaSetDevice(c->dev));
 	const ResidentBatch &rb = c->rb;
 	const int nf = rb.n_frag, n_seq = rb.n_seq;

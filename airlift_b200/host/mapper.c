@@ -134,6 +134,7 @@ static int chain_gap_ref(const mm_mapopt_t *opt, int qlen_sum)
 }
 
 static int use_device_path(const mm_idx_t *mi, const mm_mapopt_t *opt);
+static int check_seq(const mm_idx_t *mi, const mm_mapopt_t *opt);
 static void stage_align(void *data, long i, int tid);
 static void stage_finish(void *data, long i, int tid);
 
@@ -613,7 +614,7 @@ static int map_step_group(const mm_idx_t *mi, const mm_mapopt_t *opt, int n_thre
 	int n_unit = s->n_frag, *u_seg = s->n_seg, *u_off = s->seg_off, *u_tab = 0;
 	uint8_t *u_flip = 0;
 	mm_b200_tune_malloc();
-	if (mm_b200_check_opt(opt) < 0 || (use_name_filters(opt) && mm_b200_name_keys_ready(mi) < 0)) { free(sh); free(tid); return -1; }
+	if (mm_b200_check_opt(opt) < 0 || check_seq(mi, opt) < 0 || (use_name_filters(opt) && mm_b200_name_keys_ready(mi) < 0)) { free(sh); free(tid); return -1; }
 	if (opt->flag & MM_F_INDEPEND_SEG) {
 		int k, j;
 		u_tab = (int*)malloc(2 * (size_t)s->n_seq * sizeof(int) + 1);
@@ -939,7 +940,7 @@ int mm_map_file_frag(const mm_idx_t *idx, int n_segs, const char **fn, const mm_
 	int i;
 	if (n_segs < 1) return -1;
 	if (idx == 0 || idx->B == 0 || idx->B->n_dev < 1) { fprintf(stderr, "[ERROR] the index is not resident on a GPU\n"); return -1; }
-	if (mm_b200_check_opt(opt) < 0) return -1;
+	if (mm_b200_check_opt(opt) < 0 || check_seq(idx, opt) < 0) return -1;
 	memset(&pl, 0, sizeof(pl));
 	pl.n_fp = n_segs;
 	pl.fp = (mm_bseq_file_t**)calloc(n_segs, sizeof(mm_bseq_file_t*));
@@ -1025,6 +1026,19 @@ const char *mm_b200_opt_error(const mm_mapopt_t *opt)
 #undef NOT_SUPPORTED
 }
 
+const char *mm_b200_seq_error(const mm_idx_t *mi, const mm_mapopt_t *opt)
+{ /* main.c:361-366 of the reference refuses the same for the command line */
+	return (opt->flag & MM_F_CIGAR) && mi->S == 0 ? "the prebuilt index doesn't contain sequences." : 0;
+}
+
+static int check_seq(const mm_idx_t *mi, const mm_mapopt_t *opt)
+{
+	const char *msg = mm_b200_seq_error(mi, opt);
+	if (msg == 0) return 0;
+	fprintf(stderr, "[ERROR] %s\n", msg);
+	return -1;
+}
+
 int mm_b200_check_opt(const mm_mapopt_t *opt)
 {
 	const char *msg = mm_b200_opt_error(opt);
@@ -1050,7 +1064,7 @@ void mm_map_frag(const mm_idx_t *mi, int n_segs, const int *qlens, const char **
 	for (j = 0; j < n_segs; ++j) n_regs[j] = 0, regs[j] = 0;
 	if (n_segs <= 0 || n_segs > MM_MAX_SEG) return;
 	if (mi == 0 || mi->B == 0 || mi->B->n_dev < 1) { fprintf(stderr, "[ERROR] the index is not resident on a GPU\n"); exit(1); }
-	if (mm_b200_check_opt(opt) < 0 || (use_name_filters(opt) && mm_b200_name_keys_ready(mi) < 0)) exit(1);
+	if (mm_b200_check_opt(opt) < 0 || check_seq(mi, opt) < 0 || (use_name_filters(opt) && mm_b200_name_keys_ready(mi) < 0)) exit(1);
 	mm_apiq_map_frag(mi, apiq_map_batches, mm_b200_batches_in_flight, opt, n_segs, qlens, seqs, qname, n_regs, regs, &rep_len, &frag_gap);
 	if (b) b->rep_len = rep_len, b->frag_gap = frag_gap;
 }
@@ -1188,6 +1202,7 @@ void mm_b200_free_batch(mm_b200_batch_t *b)
 }
 
 mmg_ctx_t *mm_b200_ctx(const mm_idx_t *mi, int dev_slot) { return mi->B->ctx[dev_slot]; }
+mmg_idx_t *mm_b200_didx(const mm_idx_t *mi, int dev) { return mi->B->didx[dev]; }
 int mm_b200_n_devices(const mm_idx_t *mi) { return mi->B->n_dev; }
 
 void mm_b200_profile(const mm_idx_t *mi, int enable)

@@ -231,6 +231,7 @@ uint32_t mm_b200_unit_key(const mm_idx_t *mi, const char *qname); /* after mm_b2
 
 /* mapper.c */
 mmg_ctx_t *mm_b200_ctx(const mm_idx_t *mi, int dev_slot);
+mmg_idx_t *mm_b200_didx(const mm_idx_t *mi, int dev); /* the device index on GPU dev of the index */
 void mm_mapopt_to_dev(const mm_mapopt_t *opt, mmg_mapopt_t *d);
 
 /* a mini-batch of fragments (the reference's step_t, map.c:449-456, minus the per-thread buffers); mm_b200_batch_t is one */

@@ -30,8 +30,8 @@ static void die_gpu(const char *what)
 	exit(1);
 }
 
-/* build the device index from in-memory sequences and wrap it in an mm_idx_t */
-static mm_idx_t *idx_from_seqs(int w, int k, int b, int flag, int n, char **seq, const uint32_t *len, char **name)
+/* an mm_idx_t with names, lengths and the GPU contexts, without its device index yet */
+static mm_idx_t *idx_shell(int w, int k, int b, int flag, int n, const uint32_t *len, char **name)
 {
 	mm_idx_t *mi = (mm_idx_t*)calloc(1, sizeof(mm_idx_t));
 	struct mm_idx_bucket_s *B = (struct mm_idx_bucket_s*)calloc(1, sizeof(*B));
@@ -58,12 +58,28 @@ static mm_idx_t *idx_from_seqs(int w, int k, int b, int flag, int n, char **seq,
 		for (l = 0; l < B->lanes; ++l)
 			if (mmg_init(g_dev[d], &B->ctx[d * B->lanes + l]) != MMG_OK) die_gpu("cannot initialise the GPU");
 	}
-	if (mmg_idx_build(B->ctx[0], w, k, !!(flag & MM_I_HPC), n, (const char *const*)seq, len, &B->didx[0]) != MMG_OK) die_gpu("index construction failed");
-	for (d = 1; d < g_n_dev; ++d) /* replicate over NVLink; nothing else ever crosses GPUs */
-		if (mmg_idx_clone_to(B->ctx[d * B->lanes], B->didx[0], &B->didx[d]) != MMG_OK) die_gpu("index replication failed");
+	return mi;
+}
+
+static void idx_replicate(mm_idx_t *mi)
+{
+	int d;
+	for (d = 1; d < mi->B->n_dev; ++d) /* replicate over NVLink; nothing else ever crosses GPUs */
+		if (mmg_idx_clone_to(mi->B->ctx[d * mi->B->lanes], mi->B->didx[0], &mi->B->didx[d]) != MMG_OK) die_gpu("index replication failed");
+}
+
+/* build the device index from in-memory sequences and wrap it in an mm_idx_t */
+static mm_idx_t *idx_from_seqs(int w, int k, int b, int flag, int n, char **seq, const uint32_t *len, char **name)
+{
+	mm_idx_t *mi = idx_shell(w, k, b, flag, n, len, name);
+	uint64_t sum = 0;
+	int i;
+	for (i = 0; i < n; ++i) sum += len[i];
+	if (mmg_idx_build(mi->B->ctx[0], mi->w, k, !!(flag & MM_I_HPC), n, (const char *const*)seq, len, &mi->B->didx[0]) != MMG_OK) die_gpu("index construction failed");
+	idx_replicate(mi);
 	/* the host keeps the packed sequence: CIGAR post-processing and cs/MD read it (index.c:152-162) */
 	mi->S = (uint32_t*)calloc((sum + 7) / 8 + 1, 4);
-	if (mmg_idx_copy_S(B->didx[0], mi->S) != MMG_OK) die_gpu("cannot fetch the packed reference");
+	if (mmg_idx_copy_S(mi->B->didx[0], mi->S) != MMG_OK) die_gpu("cannot fetch the packed reference");
 	return mi;
 }
 
@@ -102,7 +118,7 @@ mm_idx_t *mm_idx_str(int w, int k, int is_hpc, int bucket_bits, int n, const cha
 int mm_idx_getseq(const mm_idx_t *mi, uint32_t rid, uint32_t st, uint32_t en, uint8_t *seq)
 { /* index.c:152-162 */
 	uint64_t i, st1, en1;
-	if (rid >= mi->n_seq || st >= mi->seq[rid].len) return -1;
+	if (mi->S == 0 || rid >= mi->n_seq || st >= mi->seq[rid].len) return -1; /* S: null for an index loaded without sequences */
 	if (en > mi->seq[rid].len) en = mi->seq[rid].len;
 	st1 = mi->seq[rid].offset + st, en1 = mi->seq[rid].offset + en;
 	for (i = st1; i < en1; ++i) seq[i - st1] = mm_seq4_get(mi->S, i);
@@ -142,7 +158,8 @@ void mm_idx_stat(const mm_idx_t *mi)
  * klib hash table in slot order.  The device table has another shape, so mm_idx_dump() asks the device for the keys in
  * bucket order and replays khash's placement (khash.h:232-330) on slot numbers alone: the file comes out byte for byte
  * as the reference writes it.  mm_idx_load() takes the parameters, names and the 4-bit sequence from the file and
- * re-derives the tables on the GPU -- they are a function of exactly those -- then checks the counts the file states. */
+ * re-derives the tables on the GPU -- they are a function of exactly those -- then checks the counts the file states.  A file
+ * written without sequences (MM_I_NO_SEQ) has nothing to re-derive from: its minimizer lists go to mmg_idx_build_lists. */
 
 typedef struct { int32_t *slot; uint8_t *live, *taken; uint32_t cap; } kh_replay_t;
 
@@ -262,6 +279,81 @@ void mm_idx_dump(FILE *fp, const mm_idx_t *mi)
 	free(keys); free(vals); free(pos); free(p); free(h); free(o.slot); free(o.live); free(o.taken);
 }
 
+/* The minimizer lists of one index part written without sequences, as mmg_idx_build_lists takes them.  Per bucket i the file
+ * holds p[] and the {key, val} pairs of its hash table (index.c:438-477): key = minimizer >> b << 1 | singleton, val = the
+ * position of a singleton, else start << 32 | n with start indexing the bucket's p[].  Here: key = minimizer (| KEY_ONCE for a
+ * singleton), in the file's order; src = the singleton's position, or the run's first entry in p[], all buckets' p[] in one array. */
+typedef struct { int64_t n_keys; uint64_t n_p, m_keys, m_p; uint64_t *key, *src, *p; uint32_t *cnt; } mmi_lists_t;
+
+static void mmi_lists_free(mmi_lists_t *l) { free(l->key); free(l->src); free(l->p); free(l->cnt); }
+
+/* 0; -1 when the file ends early; -2 when a run lies outside its bucket's p[] */
+static int mmi_read_lists(FILE *fp, int b, mmi_lists_t *l)
+{
+	uint64_t *kv = 0, m_kv = 0;
+	uint32_t i, j;
+	int rc = 0;
+	memset(l, 0, sizeof(*l));
+	for (i = 0; i < 1U << b && rc == 0; ++i) {
+		int32_t n;
+		uint32_t size;
+		const uint64_t p0 = l->n_p;
+		if (fread(&n, 4, 1, fp) != 1 || n < 0) { rc = -1; break; }
+		if (l->n_p + n > l->m_p) { l->m_p = l->n_p + n + ((l->n_p + n) >> 1); l->p = (uint64_t*)realloc(l->p, l->m_p * 8); }
+		if (fread(l->p + l->n_p, 8, n, fp) != (size_t)n) { rc = -1; break; }
+		l->n_p += n;
+		if (fread(&size, 4, 1, fp) != 1) { rc = -1; break; }
+		if ((uint64_t)l->n_keys + size > l->m_keys) {
+			l->m_keys = l->n_keys + size + ((l->n_keys + size) >> 1);
+			l->key = (uint64_t*)realloc(l->key, l->m_keys * 8), l->src = (uint64_t*)realloc(l->src, l->m_keys * 8);
+			l->cnt = (uint32_t*)realloc(l->cnt, l->m_keys * 4);
+		}
+		if (2 * (uint64_t)size > m_kv) { m_kv = 2 * (uint64_t)size; kv = (uint64_t*)realloc(kv, m_kv * 8); }
+		if (fread(kv, 16, size, fp) != size) { rc = -1; break; }
+		for (j = 0; j < size; ++j) {
+			const uint64_t y0 = kv[2 * j], y1 = kv[2 * j + 1], m = y0 >> 1 << b | i;
+			const int64_t e = l->n_keys++;
+			if (y0 & 1) l->key[e] = m | KEY_ONCE, l->cnt[e] = 1, l->src[e] = y1;
+			else {
+				l->key[e] = m, l->cnt[e] = (uint32_t)y1, l->src[e] = p0 + (y1 >> 32);
+				if ((y1 >> 32) + (uint32_t)y1 > (uint64_t)n) { rc = -2; break; }
+			}
+		}
+	}
+	free(kv);
+	if (rc) mmi_lists_free(l), memset(l, 0, sizeof(*l));
+	return rc;
+}
+
+/* test hook: the lists of the first part of a no-sequence index file, exactly as mm_idx_load hands them to mmg_idx_build_lists.
+ * Returns the number of distinct minimizers, or -1 with the loader's message; free the arrays with mm_b200_mmi_lists_free */
+int64_t mm_b200_mmi_lists(const char *fn, uint64_t **key, uint32_t **cnt, uint64_t **src, uint64_t *n_p, uint64_t **p)
+{
+	FILE *fp = fopen(fn, "rb");
+	char magic[4];
+	uint32_t x[5], i, len;
+	mmi_lists_t l;
+	int rc = -1;
+	if (fp == 0) return -1;
+	if (fread(magic, 1, 4, fp) != 4 || strncmp(magic, MM_IDX_MAGIC, 4) != 0 || fread(x, 4, 5, fp) != 5 || !(x[4] & MM_I_NO_SEQ)) {
+		fprintf(stderr, "[ERROR] not an index file written without sequences\n");
+		fclose(fp);
+		return -1;
+	}
+	for (i = 0; i < x[3]; ++i) {
+		uint8_t nl;
+		if (fread(&nl, 1, 1, fp) != 1 || fseeko(fp, nl, SEEK_CUR) != 0 || fread(&len, 4, 1, fp) != 1) break;
+	}
+	if (i == x[3]) rc = mmi_read_lists(fp, (int)x[2], &l);
+	fclose(fp);
+	if (rc == -1) { fprintf(stderr, "[ERROR] the index file is truncated\n"); return -1; }
+	if (rc < 0) { fprintf(stderr, "[ERROR] the index file lists positions outside their bucket\n"); return -1; }
+	*key = l.key, *cnt = l.cnt, *src = l.src, *n_p = l.n_p, *p = l.p;
+	return l.n_keys;
+}
+
+void mm_b200_mmi_lists_free(uint64_t *key, uint32_t *cnt, uint64_t *src, uint64_t *p) { free(key); free(cnt); free(src); free(p); }
+
 mm_idx_t *mm_idx_load(FILE *fp)
 {
 	char magic[4], **seq, **name;
@@ -271,10 +363,6 @@ mm_idx_t *mm_idx_load(FILE *fp)
 	if (fread(magic, 1, 4, fp) != 4) return 0;
 	if (strncmp(magic, MM_IDX_MAGIC, 4) != 0) return 0;
 	if (fread(x, 4, 5, fp) != 5) return 0;
-	if (x[4] & MM_I_NO_SEQ) {
-		fprintf(stderr, "[ERROR] the prebuilt index doesn't contain sequences; this build needs them on the GPU\n");
-		exit(1);
-	}
 	seq = (char**)calloc(x[3], sizeof(char*)), name = (char**)calloc(x[3], sizeof(char*)), len = (uint32_t*)calloc(x[3], 4);
 	for (i = 0; i < x[3]; ++i) {
 		uint8_t l;
@@ -285,6 +373,21 @@ mm_idx_t *mm_idx_load(FILE *fp)
 		}
 		if (fread(&len[i], 4, 1, fp) != 1) goto truncated;
 		sum_len += len[i];
+	}
+	if (x[4] & MM_I_NO_SEQ) { /* no sequence to re-derive the tables from: the device builds them from the file's lists */
+		mmi_lists_t l;
+		const int rc = mmi_read_lists(fp, (int)x[2], &l);
+		if (rc == -1) goto truncated;
+		if (rc < 0) { fprintf(stderr, "[ERROR] the index file lists positions outside their bucket\n"); exit(1); }
+		mi = idx_shell((int)x[0], (int)x[1], (int)x[2], (int)x[4], (int)x[3], len, name);
+		if (mmg_idx_build_lists(mi->B->ctx[0], mi->w, mi->k, !!(mi->flag & MM_I_HPC), mi->n_seq, len, l.n_keys, l.key, l.cnt, l.src, l.n_p, l.p,
+		                        &mi->B->didx[0]) != MMG_OK)
+			die_gpu("index construction failed");
+		idx_replicate(mi); /* mi->S stays null: nothing on the host may read the sequence */
+		mmi_lists_free(&l);
+		for (i = 0; i < x[3]; ++i) free(name[i]);
+		free(seq); free(name); free(len);
+		return mi;
 	}
 	for (i = 0; i < 1U << x[2]; ++i) { /* the tables are rebuilt from the sequence; only their sizes are taken from the file */
 		int32_t n;
@@ -500,6 +603,7 @@ int mm_b200_idx_finalize(mm_idx_t *mi)
 	uint32_t i;
 	for (i = 0; i < mi->n_seq; ++i) sum += mi->seq[i].len;
 	if (mmg_idx_finalize(mi->B->didx[0]) != MMG_OK) die_gpu("index replica");
+	if (!mmg_idx_has_seq(mi->B->didx[0])) return 0;
 	mi->S = (uint32_t*)calloc((sum + 7) / 8 + 1, 4);
 	if (mmg_idx_copy_S(mi->B->didx[0], mi->S) != MMG_OK) die_gpu("cannot fetch the packed reference");
 	return 0;

@@ -21,6 +21,7 @@ What differs from the reference's mappy:
 """
 import ctypes as C
 import os
+import struct
 import threading
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -30,6 +31,7 @@ MM_F_CIGAR = 0x004
 MM_F_SPLICE = 0x080
 MM_F_INDEPEND_SEG = 0x20000
 MM_I_HPC = 0x1
+MM_I_NO_SEQ = 0x2
 MM_B200_HITS_COLS = 22
 MM_B200_HITS_CS, MM_B200_HITS_MD = 0x1, 0x2
 (_FRAG, _SEG, _RID, _RS, _RE, _QS, _QE, _REV, _MAPQ, _PRI, _MLEN, _BLEN, _N_AMBI, _TS, _DP_SCORE, _DP_MAX, _N_CIGAR, _CIGAR_OFF,
@@ -204,6 +206,17 @@ class _SharedLock:
             self._cv.notify_all()
 
 
+def _mmi_without_seq(fn):
+    """True for an index file written with --idx-no-seq (header flag MM_I_NO_SEQ).  Aligner always asks for CIGARs, as the
+    reference's mappy does, and they need the target sequence."""
+    try:
+        with open(fn, "rb") as f:
+            head = f.read(24)
+    except OSError:
+        return False
+    return len(head) == 24 and head[:4] == b"MMI\x02" and (struct.unpack("<5I", head[4:])[4] & MM_I_NO_SEQ) != 0
+
+
 def _enc(s):
     return s if isinstance(s, bytes) else s.encode()
 
@@ -256,7 +269,8 @@ class Aligner:
     [a,b,q,e], [a,b,q,e,q2,e2] or the same plus sc_ambi), then mm_mapopt_update.  The index is read from fn_idx_in (FASTA/FASTQ, gzip'd or not, or a .mmi; fn_idx_out writes
     the .mmi) or built from the one sequence seq.  bool(aligner) is False when no index could be read.
 
-    Raises ValueError for options this build refuses, with the library's message, and RuntimeError without a CUDA device.
+    Raises ValueError for options this build refuses, with the library's message, and for a .mmi written with --idx-no-seq
+    (CIGARs need the sequence), and RuntimeError without a CUDA device.
 
     map() may be called from any number of threads at once.  map_batch() maps on the index alone: mm_map_frag and the batch
     path must not map on one index at the same time, so map_batch waits for running map() calls and holds new ones back while
@@ -269,6 +283,8 @@ class Aligner:
         L = _L()
         io, mo = set_options(preset, k, w, min_cnt, min_chain_score, min_dp_score, bw, best_n, max_frag_len, extra_flags, scoring)
         self._idx_opt, self._map_opt = io, mo
+        if seq is None and fn_idx_in is not None and _mmi_without_seq(fn_idx_in):
+            raise ValueError("the prebuilt index doesn't contain sequences.")
         if L.mmg_device_count() < 1:
             raise RuntimeError("no CUDA device: this mapper has no CPU path")
         if seq is None:

@@ -216,6 +216,14 @@ int mm_b200_idx_finalize(mm_idx_t *mi);
  * Calling them while mm_b200_map_batch(es) or mm_map_file(_frag) maps on the same index is not supported. */
 int mm_b200_check_opt(const mm_mapopt_t *opt);
 const char *mm_b200_opt_error(const mm_mapopt_t *opt); /* the message mm_b200_check_opt prints (no "[ERROR] "), or 0: nothing printed */
+/* An index loaded from a .mmi written with --idx-no-seq keeps no sequence (mi->S is null): it maps, but CIGARs (-a, -c, --cs,
+ * --MD: MM_F_CIGAR) cannot be computed against it.  mm_b200_seq_error returns the message for that case, or 0; the mapping calls
+ * refuse it as they refuse mm_b200_check_opt's options (the batch calls return -1, mm_map_frag exits) */
+const char *mm_b200_seq_error(const mm_idx_t *mi, const mm_mapopt_t *opt);
+/* the minimizer lists of the first part of a no-sequence .mmi, as its loader hands them to mmg_idx_build_lists (see mmg.h);
+ * returns the number of distinct minimizers, or -1 with the loader's message printed */
+int64_t mm_b200_mmi_lists(const char *fn, uint64_t **key, uint32_t **cnt, uint64_t **src, uint64_t *n_p, uint64_t **p);
+void mm_b200_mmi_lists_free(uint64_t *key, uint32_t *cnt, uint64_t *src, uint64_t *p);
 /* name keys of the self/dual-hit filters (see "name keys" in mmg.h): sorted[] receives the n names in strcmp order (a NULL name
  * counts as ""), tkey[] the target key of each; mm_b200_name_ukey gives the unit key of qname against those sorted names
  * (MMG_NAME_NONE for a NULL qname) */

@@ -62,12 +62,21 @@ void mmg_growth_counts(uint64_t out[2], int reset);
  * Positions returned per minimizer are identical, in value and order, to mm_idx_get's. */
 int  mmg_idx_build(mmg_ctx_t *ctx, int w, int k, int is_hpc, int n_seq, const char *const *seqs, const uint32_t *lens,
                    mmg_idx_t **idx);
+/* Build the same index from the minimizer lists of an index file written without sequences (--idx-no-seq; mm_idx_load,
+ * index.c:479-531).  n_keys distinct minimizers, in any order: key[i] = the minimizer, bit 63 set when it occurs once;
+ * src[i] = that one position, or else the index in p[] of the first of its cnt[i] positions, which pos[] keeps in the order
+ * p[] lists them.  p[] (n_p entries) holds the lists of every bucket one after another.  The index holds no sequence:
+ * mmg_idx_copy_S, mmg_ksw_batch and mmg_post_chain with MM_F_CIGAR refuse it with MMG_EINVAL before any launch. */
+int  mmg_idx_build_lists(mmg_ctx_t *ctx, int w, int k, int is_hpc, int n_seq, const uint32_t *lens, int64_t n_keys, const uint64_t *key,
+                         const uint32_t *cnt, const uint64_t *src, uint64_t n_p, const uint64_t *p, mmg_idx_t **idx);
+int  mmg_idx_has_seq(const mmg_idx_t *idx);           /* 0 for an index built by mmg_idx_build_lists */
 void mmg_idx_free(mmg_idx_t *idx);
 int64_t mmg_idx_n_minimizers(const mmg_idx_t *idx);   /* occurrences */
 int64_t mmg_idx_n_keys(const mmg_idx_t *idx);         /* distinct minimizers */
 uint64_t mmg_idx_total_len(const mmg_idx_t *idx);
 size_t mmg_idx_bytes(const mmg_idx_t *idx);           /* HBM footprint */
-/* copy the 4-bit packed reference (mm_idx_t::S layout, mmpriv.h:28-29) to the host: (total_len+7)/8 words */
+/* copy the 4-bit packed reference (mm_idx_t::S layout, mmpriv.h:28-29) to the host: (total_len+7)/8 words.  MMG_EINVAL for
+ * an index without sequence, whose image (mmg_idx_export) has bytes_S = 0 and d_S = NULL */
 int  mmg_idx_copy_S(const mmg_idx_t *idx, uint32_t *S_host);
 int  mmg_idx_cal_max_occ(mmg_idx_t *idx, float f, int32_t *thres);
 /* batched mm_idx_get: for each minier[i] write n[i] and up to max_pos positions at pos + i*max_pos */
